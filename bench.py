@@ -8,6 +8,7 @@ one launch of the fused kernel for the sizes that have a specialised one.  Episo
 region: every N = J*M steps the batch is reset (two more launches), as the reference's loop does.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload A|B|C] [--repeats R]
+                    [--dump-outputs DIR]
 
 The K-step timed region (barrier + synchronize on both sides, CUDA events, max over ranks) is repeated R >= 15 times
 and the MEDIAN is reported, so that short runs (--steps 20 is a 1.8 ms region) are stable to < 2 %.  At N = 1 the same
@@ -164,9 +165,9 @@ def cpu_port_rate(wl, nthreads, target_seconds):
 def real_reference_rate(seconds=12.0):
     """SURVEY.md 8(d) i-ii: the UNMODIFIED Python reference (trainer/parallel_env.Parallel_env over networkx, batch 16,
     J6M6E2 instances of the shipped generator's seed-0 stream, random valid actions under the ESA mask) timed on this
-    box's host cores: one process = one core (how the reference runs), then one process per core.  Needs the reference
-    tree under baseline/_ref (git-ignored copy made by __graft_entry__.build() where /root/reference exists)."""
-    ref_root = os.path.join(ROOT, "baseline", "_ref")
+    box's host cores: one process = one core (how the reference runs), then one process per core.  Needs a checkout of the
+    reference project named by $MTFJSP_REFERENCE_ROOT; the leg is left out without one."""
+    ref_root = os.environ.get("MTFJSP_REFERENCE_ROOT", "")
     if not os.path.isdir(os.path.join(ref_root, "graph-jsp-env", "src", "graph_jsp_env")):
         return None
     script = os.path.join(ROOT, "oracle", "time_reference.py")
@@ -261,9 +262,35 @@ def run_reference(args, wl):
     print(json.dumps(line), flush=True)
 
 
-def measure_env(wl, B, K, W, repeats, rank, world, dev, barrier, sh, envm, torch, want_e2e):
+DUMP_MAX_ENVS = 4096
+DUMP_MAX_BYTES = 48 << 20
+
+
+def snapshot_outputs(env, torch):
+    """What `random_step` hands its caller (action, candidate-machine features, rewards, flags, observation, job mask and
+    candidates) for a fixed, seeded sample of the batch's envs, as host float32 / float64 arrays.  Integer outputs are
+    widened to float64, which holds them exactly."""
+    import numpy as np
+
+    outs = {"op": env.op, "mach": env.mach, "mfea1": env.mfea1_buf, "mach_mask": env.mach_mask, "reward5": env.reward5,
+            "scaled4": env.scaled4, "done": env.done, "invalid": env.invalid, "task_fea": env.task_fea,
+            "mach_fea": env.mach_fea, "adj_w": env.adj_w, "adj_src": env.adj_src, "job_mask": env.job_mask,
+            "candidate": env.candidate}
+    per_env = sum(x[0].numel() * 8 for x in outs.values())
+    n = max(1, min(env.B, DUMP_MAX_ENVS, DUMP_MAX_BYTES // per_env))
+    idx = np.sort(np.random.default_rng(0).choice(env.B, size=n, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    dump = {"env_index": idx.astype(np.float64)}
+    for name, x in outs.items():
+        y = x.index_select(0, sel).cpu()
+        dump[name] = y.numpy() if y.dtype in (torch.float32, torch.float64) else y.to(torch.float64).numpy()
+    return dump
+
+
+def measure_env(wl, B, K, W, repeats, rank, world, dev, barrier, sh, envm, torch, want_e2e, want_dump=False):
     """Everything measured on one workload: whole-job throughput of the timed region, the kernels alone (one CUDA-event
-    pair per launch on the launching stream), changed observation rows, and (want_e2e) the host-buffer C-ABI call."""
+    pair per launch on the launching stream), changed observation rows, and (want_e2e) the host-buffer C-ABI call.
+    want_dump: also keep a sample of what the last timed step computed (snapshot_outputs)."""
     J, M, E = wl["J"], wl["M"], wl["E"]
     N = J * M
     first, count, d, w = sh.make_shard(B * world, rank, world, J, M, E, wl["seed"])
@@ -300,6 +327,8 @@ def measure_env(wl, B, K, W, repeats, rank, world, dev, barrier, sh, envm, torch
     ms = median(times)
     out = {"env": env, "first": first, "w": w, "d": d, "ms": ms, "times": times, "launches": launches,
            "value": B * world * K / (ms * 1e-3)}
+    if want_dump:
+        out["dump"] = snapshot_outputs(env, torch)
 
     # ---- record one episode of actions; count the observation rows a step changes (diff of consecutive observations) ----
     env.reset(w); env.scaler_reset()
@@ -483,7 +512,8 @@ def run_ours(args, wl):
     if sampler:
         sampler.start()
     # weak scaling: B envs per GPU, env i of the B*world job lives on rank i // B (contiguous slices)
-    mm = measure_env(wl, B, K, W, R, rank, world, dev, barrier, sh, envm, torch, want_e2e=True)
+    mm = measure_env(wl, B, K, W, R, rank, world, dev, barrier, sh, envm, torch, want_e2e=True,
+                     want_dump=bool(args.dump_outputs) and rank == 0)
     env, first, w, d = mm["env"], mm["first"], mm["w"], mm["d"]
     rec_op, rec_mc = mm["rec_op"], mm["rec_mc"]
     ms, value, launches, peak, peak_src, kern = mm["ms"], mm["value"], mm["launches"], mm["peak"], mm["peak_src"], mm["kern"]
@@ -681,6 +711,10 @@ def run_ours(args, wl):
             line["cpu_baseline"] = cpu
         if cpu_ref:
             line["cpu_baseline_reference"] = cpu_ref
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in mm["dump"].items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         if stdout_fd is not None:
             sys.stdout.flush()
             os.dup2(stdout_fd, 1)
@@ -707,8 +741,12 @@ def main():
     ap.add_argument("--no-dropin", action="store_true", help="skip the Parallel_env (reference-typed) call measurement")
     ap.add_argument("--no-train", action="store_true", help="skip the rollout + PPO update measurement")
     ap.add_argument("--no-workloads", action="store_true", help="skip the J10M10E3 / J30M20E5 lines")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (a fixed, seeded sample of rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args, wl)
     else:

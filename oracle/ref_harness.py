@@ -2,10 +2,9 @@
 
 TEST INFRASTRUCTURE ONLY.  This module exists to (a) validate the C restatement in
 ``oracle/mtfjsp_oracle.c`` against the reference implementation, (b) generate the golden
-vectors committed under ``tests/golden/`` (see ``tests/golden/gen_golden.py``) and (c) time / drive the
-unmodified reference next to the CUDA path (bench.py's cpu_baseline_reference leg, tests/test_single_env.py).
-It reads ``/root/reference`` in the build container and the git-ignored copy ``baseline/_ref`` on the
-GPU box; the product package never imports it.
+vectors committed under ``tests/golden/`` (see ``tests/golden/gen_golden.py``) and (c) time the unmodified
+reference (bench.py's cpu_baseline_reference leg).  It reads the reference checkout named by
+``$MTFJSP_REFERENCE_ROOT``; the product package never imports it.
 
 Recipe (SURVEY.md Appendix D): three stub packages (gym, matplotlib.pyplot, plotly.figure_factory)
 under ``oracle/ref_shims``, a pre-seeded ``graph_jsp_env.wzl_ima_banner`` module, and the reference
@@ -21,10 +20,7 @@ import types
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# the read-only mount in the build container, else the git-ignored copy that travels to the GPU box (made by
-# __graft_entry__.build(); it carries the unmodified tree so the reference can be TIMED and driven there)
-_COPY = os.path.join(os.path.dirname(_HERE), "baseline", "_ref")
-REF_ROOT = os.environ.get("MTFJSP_REFERENCE_ROOT") or ("/root/reference" if os.path.isdir("/root/reference") else _COPY)
+REF_ROOT = os.environ.get("MTFJSP_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:

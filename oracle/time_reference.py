@@ -3,7 +3,7 @@ networkx, batch 16, J6M6E2 instances of the reference generator's seed-0 stream,
 job mask, each step = cal_cur_task_machine_feature + DGFJSPEnv_paral_step + job-mask update, one process = one core.
 
 TEST / BASELINE INFRASTRUCTURE ONLY (bench.py's cpu_baseline_reference leg runs it in a subprocess).  The reference tree
-is read from $MTFJSP_REFERENCE_ROOT (baseline/_ref on the GPU box: a git-ignored copy made by __graft_entry__.build()).
+is read from $MTFJSP_REFERENCE_ROOT.
 
     python oracle/time_reference.py --seconds 12 --seed 0   ->  {"env_steps_per_s": ..., ...}
 """

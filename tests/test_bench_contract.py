@@ -1,10 +1,14 @@
-"""bench.py contract checks that need no GPU: the reference arm (`--impl reference`, the C restatement of the reference
+"""bench.py contract checks.  Without a GPU: the reference arm (`--impl reference`, the C restatement of the reference
 env timed on the host cores) prints exactly one JSON line with the keys the driver reads, and names the same metric,
-unit and workload as the device arm."""
+unit and workload as the device arm.  On the GPU: `--dump-outputs` writes the last timed step's outputs, the same ones
+on every run with the same arguments."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -53,3 +57,27 @@ def test_needed_bytes_accounting():
     full = 8 + 2 * 1113 + (48 * 36 + 18 * 36 + 32 * 6 + 5 * 6 + 41)
     assert full == 4873 and nb["total"] < full                     # never credits bytes the kernel does not write
     assert bench.median([3, 1, 2]) == 2 and bench.median([4, 1, 2, 3]) == 2.5
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_exactly_and_follow_steps(tmp_path):
+    def run(name, steps):
+        d = tmp_path / name
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "2",
+                              "--repeats", "2", "--batch", "512", "--no-cpu-baseline", "--no-policy", "--no-dropin",
+                              "--no-train", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert len([l for l in out.stdout.splitlines() if l.strip()]) == 1
+        return {f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))}
+
+    a, b, c = run("a", 5), run("b", 5), run("c", 6)
+    assert set(a) == {"env_index", "op", "mach", "mfea1", "mach_mask", "reward5", "scaled4", "done", "invalid", "task_fea",
+                      "mach_fea", "adj_w", "adj_src", "job_mask", "candidate"}
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    n = len(a["env_index"])
+    assert n == 512 and (np.diff(a["env_index"]) > 0).all()
+    for k, x in a.items():
+        assert x.dtype in (np.float32, np.float64) and len(x) == n, k
+        np.testing.assert_array_equal(x, b[k], err_msg=k)
+    assert not (a["invalid"] != 0).any()
+    assert any(not np.array_equal(a[k], c[k]) for k in ("op", "reward5", "task_fea"))   # two more timed steps

@@ -1,20 +1,19 @@
 """The single-env class (reference: graph-jsp-env/.../disjunctive_graph_jsp_env_singlestep.py:97-130 ctor,
 1183-1245 reset -> 9-tuple, 716-974 step -> 14-tuple) against the UNMODIFIED reference, on the GPU box.
 
-The reference tree is read from baseline/_ref (a git-ignored copy staged by __graft_entry__.build(); see
-oracle/ref_harness.py), so these tests skip where it is absent.  Three layers:
+What the reference class returned is stored in tests/golden/single_env_golden.npz (tests/golden/gen_single_env_golden.py;
+digests of canonical forms, oracle/single_env_trace.py), so these tests need nothing outside the repository.  Three layers:
   1. every element of the reset 9-tuple and step 14-tuple, the node attributes, machine routes, final-cost attributes
      and the valid-action mask, step by step against the reference class on the same actions (both left-shift modes);
-  2. the unmodified dispatching-rule rollout tester/pdrs.py:611-839 driving OUR class: the shipped result CSV rows 0 / 1
-     (FIFO+SPT, FIFO+SEC) bit for bit;
-  3. the unmodified validation loop trainer/validate.py:60-297 with the reference's own networks and the shipped
-     checkpoint driving OUR class: same final costs and objective as with the reference class, bit for bit.
+  2. the calls the unmodified dispatching-rule rollout tester/pdrs.py:611-839 makes, replayed on OUR class: every return
+     as the reference class gave it, and the shipped result CSV rows 0 / 1 / 4 / 11 bit for bit;
+  3. the calls the unmodified validation loop trainer/validate.py:60-297 makes with the reference's own networks and the
+     shipped checkpoint, replayed on OUR class: every return, node attribute, final cost and the objective as with the
+     reference class, bit for bit.
 """
-import contextlib
 import importlib
-import io
 import os
-import types
+import random
 
 import numpy as np
 import pytest
@@ -23,6 +22,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 from oracle import ref_harness as rh  # noqa: E402
+from oracle import single_env_trace as tr  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 ins = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.instances")
@@ -33,137 +33,82 @@ def _mine():
     return importlib.import_module("e2e-mappo-for-mt-fjsp_b200.single_env").DisjunctiveGraphJspEnv_singleStep
 
 
-def _need_reference():
-    if not rh.reference_available():
-        pytest.skip("reference tree not staged under baseline/_ref")
+def _golden():
+    return np.load(os.path.join(GOLD, "single_env_golden.npz"))
 
 
-def _make(cls, t, p, tt, args, left_shift):
-    with contextlib.redirect_stdout(io.StringIO()):
-        return cls(jps_instance=np.array([t, p]), reward_function_parameters=args["reward_scaling"],
-                   default_visualisations=["gantt_console", "graph_console"], reward_function="wrk", ability_tr_mm=tt,
-                   perform_left_shift_if_possible=left_shift, configs=args)
+def _same(got, want, what):
+    """Digests of what our class returned against the reference class's."""
+    got, want = np.atleast_1d(np.asarray(got, dtype=np.uint64)), np.atleast_1d(want)
+    bad = np.nonzero(got != want)[0]
+    assert bad.size == 0, "%s: element(s) %s differ from the reference" % (what, bad.tolist())
 
 
-def _same(a, b, what):
-    if isinstance(a, dict):
-        assert set(a) == set(b), (what, set(a) ^ set(b))
-        for k in a:
-            if k == "gantt_df":
-                assert a[k].reset_index(drop=True).equals(b[k].reset_index(drop=True)), what
-            else:
-                _same(a[k], b[k], "%s[%s]" % (what, k))
-    elif isinstance(a, (np.ndarray, list, tuple)):
-        eq(np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64), err_msg=what)
-        if isinstance(a, np.ndarray) and isinstance(b, np.ndarray) and what.startswith(("step[0]", "reset[0]")):
-            assert a.dtype == b.dtype, (what, a.dtype, b.dtype)
-    elif isinstance(a, (bool, np.bool_, str)) or a is None:
-        assert a == b and type(b) in (type(a), bool, np.bool_), (what, a, b)
-    else:   # numbers: the reference mixes python ints, floats and numpy scalars (e.g. a start time of exactly 0 is int 0)
-        assert float(a) == float(b), (what, a, b)
-
-
-@pytest.mark.parametrize("cfg", [(6, 6, 2, True, 3), (6, 6, 2, False, 4), (3, 4, 2, True, 5), (10, 10, 3, True, 6)])
+@pytest.mark.parametrize("cfg", tr.STEP_CFGS)
 def test_tuples_and_attributes_match_the_reference_class_step_by_step(cfg):
-    _need_reference()
     J, M, E, ls, seed = cfg
     N = J * M
-    ref = rh.load_reference()
+    g, key = _golden(), "step/%s/" % tr.cfg_key(cfg)
+    acts, resets, steps, state, final = (g[key + k] for k in ("actions", "reset", "step", "state", "final"))
     d = ins.reference_stream_instances(4, J, M, E, seed=3) if (J, M) == (6, 6) else ins.synthetic_instances(0, 4, J, M, E, seed)
     args = rh.make_args(J, M, E, 1)
-    rng = np.random.default_rng(seed)
     for i in range(2):
         t, p, tt = d["t"][i], d["p"][i], d["transT"][i]
-        a_env, b_env = _make(ref.Env, t, p, tt, args, ls), _make(_mine(), t, p, tt, args, ls)
-        for kind in ("eval", "01"):
-            import random
-
+        env = tr.make_env(_mine(), t, p, tt, args, ls)
+        for k, kind in enumerate(("eval", "01")):
             random.seed(11 + i)
-            ra = a_env.reset(Random_weight_type=kind)
-            random.seed(11 + i)
-            rb = b_env.reset(Random_weight_type=kind)
-            assert len(ra) == len(rb) == 9
-            for k in range(9):
-                _same(ra[k], rb[k], "reset[%d]" % k)
-            eq(a_env.reward_random_weight, b_env.reward_random_weight)
-            nxt = np.zeros(J, dtype=int)
+            rb = env.reset(Random_weight_type=kind)
+            assert len(rb) == 9
+            _same(tr.tuple_digests(rb), resets[i, k], "reset")
+            eq(env.reward_random_weight, g[key + "weights"][i, k])
             for s in range(N):
-                assert a_env.valid_action_mask() == b_env.valid_action_mask()
-                j = rng.choice(np.nonzero(nxt < M)[0])
-                op = j * M + nxt[j]
-                nxt[j] += 1
-                feas = np.nonzero(t[op] >= 0)[0]
-                m = feas[0] if rng.random() < 0.4 else rng.choice(feas)   # lowest index: same-machine chains
-                with contextlib.redirect_stdout(io.StringIO()):
-                    sa = a_env.step([int(op), int(m)])
-                sb = b_env.step([int(op), int(m)])
-                assert len(sa) == len(sb) == 14
-                for k in range(14):
-                    _same(sa[k], sb[k], "step[%d] s=%d" % (k, s))
-                for task_id in range(1, N + 1):
-                    na, nb = a_env.G.nodes[task_id], b_env.G.nodes[task_id]
-                    for key in ("machine", "scheduled", "finish_time", "job", "duration"):
-                        assert na[key] == nb[key], (s, task_id, key, na[key], nb[key])
-                    if na["scheduled"]:
-                        assert na["start_time"] == nb["start_time"]
-                for mm in range(M):
-                    eq(np.asarray(a_env.machine_routes[mm], dtype=np.int64), np.asarray(b_env.machine_routes[mm], dtype=np.int64))
-            for name in ("makespan_previous_step", "total_e1_previous_step", "trans_t_previous_step", "idle_t_previous_step"):
-                assert getattr(a_env, name) == getattr(b_env, name), name
-            assert sa[2] is True or sa[2] == True  # noqa: E712  done
-        assert "M0" in b_env.render(mode="text")
-        b_env.close()
+                _same(tr.digest(env.valid_action_mask()), state[i, k, s, 0], "valid_action_mask s=%d" % s)
+                sb = tr.step_quiet(env, acts[i, k, s])
+                assert len(sb) == 14
+                _same(tr.tuple_digests(sb), steps[i, k, s], "step s=%d" % s)
+                _same(tr.nodes_digest(env, N), state[i, k, s, 1], "node attributes s=%d" % s)
+                _same(tr.routes_digest(env, M), state[i, k, s, 2], "machine routes s=%d" % s)
+            got = [env.makespan_previous_step, env.total_e1_previous_step, env.trans_t_previous_step, env.idle_t_previous_step]
+            eq(np.array(got), final[i, k])
+            assert sb[2] is True
+        assert "M0" in env.render(mode="text")
+        env.close()
 
 
-def _load_pdrs():
-    rh.load_reference()
-    import sys
-
-    if "trainer.fig_kpi" not in sys.modules:
-        fk = types.ModuleType("trainer.fig_kpi")
-        fk.result_box_plot = lambda *a, **k: None
-        fk.get_GPU_usage = lambda *a, **k: None
-        sys.modules["trainer.fig_kpi"] = fk
-    with contextlib.redirect_stdout(io.StringIO()):
-        from tester import pdrs
-    return pdrs
-
-
-def test_unmodified_pdr_rollout_reproduces_shipped_csv_rows_on_our_class(monkeypatch):
-    _need_reference()
-    pdrs = _load_pdrs()
-    g = np.load(os.path.join(GOLD, "pdr_golden.npz"))
-    monkeypatch.setattr(pdrs, "DisjunctiveGraphJspEnv_singleStep", _mine())   # the only change: which class the name binds
-    ds = types.SimpleNamespace(t=g["t"], p=g["p"], transT=g["transT"], edge=g["edge"])
+def test_unmodified_pdr_rollout_reproduces_shipped_csv_rows_on_our_class():
+    g, pdr = _golden(), np.load(os.path.join(GOLD, "pdr_golden.npz"))
     args = rh.make_args(6, 6, 2, 1)
-    rules = {(0, 0): 0, (0, 1): 1, (2, 0): 2, (5, 1): 9}   # (o_rule, m_rule) -> row of pdr_golden (CSV rows 0, 1, 4, 11)
-    for (o_rule, m_rule), row in rules.items():
-        for i in range(12):
-            with contextlib.redirect_stdout(io.StringIO()):
-                _, _, real4 = pdrs.run_Rules_jointActions_withMinus_1217(args, o_rule, m_rule, ds, i, None, None)
-            eq(np.array(real4), g["gold"][row, i], err_msg="rule %s instance %d" % ((o_rule, m_rule), i))
+    for r, ((o_rule, m_rule), row) in enumerate(tr.PDR_ROWS.items()):
+        for i in range(tr.PDR_INSTANCES):
+            what = "rule %s instance %d" % ((o_rule, m_rule), i)
+            env = tr.make_env(_mine(), pdr["t"][i], pdr["p"][i], pdr["transT"][i], args, False)
+            _same(tr.combined_digest(env.reset(Random_weight_type="eval")), g["pdr/reset"][r, i], what + " reset")
+            for s in range(36):
+                out = tr.step_quiet(env, (pdr["ops"][row, i, s], pdr["mch"][row, i, s]))
+                _same(tr.combined_digest(out), g["pdr/step"][r, i, s], what + " step %d" % s)
+            assert out[2]
+            eq(np.array(tr.final_costs(env, 36)), pdr["gold"][row, i], err_msg=what)
+            env.reset()
+            env.close()
 
 
-def test_unmodified_validation_loop_with_shipped_checkpoint_on_our_class(monkeypatch):
-    _need_reference()
-    import random
-
-    ppo, args = rh.make_reference_ppo(6, 6, "cuda:0")
-    with contextlib.redirect_stdout(io.StringIO()):
-        from trainer import validate
-    g = np.load(os.path.join(GOLD, "pdr_golden.npz"))   # the 100 shipped test instances
-    ds = types.SimpleNamespace(t=g["t"], p=g["p"], transT=g["transT"], edge=g["edge"])
-    ref_cls = validate.DisjunctiveGraphJspEnv_singleStep
-    out = {}
-    for name, cls in (("reference", ref_cls), ("ours", _mine())):
-        monkeypatch.setattr(validate, "DisjunctiveGraphJspEnv_singleStep", cls)
-        res = []
-        for i in range(10):
-            random.seed(i)   # the trailing env.reset() of the loop draws reward weights from python's `random`
-            torch.manual_seed(0)
-            with contextlib.redirect_stdout(io.StringIO()):
-                _, final4, obj = validate.validate_cost_gcn_jointActor_GAT(ppo, False, ds, i, "random", greedy=True, args=args)
-            res.append(list(final4) + [obj])
-        out[name] = np.array(res)
-    eq(out["ours"], out["reference"])
-    assert np.isfinite(out["ours"]).all() and (out["ours"][:, 0] > 0).all()
+def test_unmodified_validation_loop_with_shipped_checkpoint_on_our_class():
+    g, pdr = _golden(), np.load(os.path.join(GOLD, "pdr_golden.npz"))   # the 100 shipped test instances
+    args = rh.default_model_args(6, 6)
+    res = []
+    for i in range(tr.VALIDATE_INSTANCES):
+        env = tr.make_env(_mine(), pdr["t"][i], pdr["p"][i], pdr["transT"][i], args, True)
+        _same(tr.combined_digest(env.reset(Random_weight_type="eval")), g["validate/reset"][i], "instance %d reset" % i)
+        for s in range(36):
+            out = tr.step_quiet(env, g["validate/actions"][i, s])
+            _same(tr.combined_digest(out), g["validate/step"][i, s], "instance %d step %d" % (i, s))
+            _same(tr.nodes_digest(env, 36), g["validate/nodes"][i, s], "instance %d node attributes after step %d" % (i, s))
+        assert out[2]
+        mk, pt, transT, idleT = tr.final_costs(env, 36)
+        res.append([mk, pt, transT, idleT, args["weight_mk"] * mk + args["weight_ec"] * (pt + idleT) + args["weight_tt"] * transT])
+        random.seed(i)
+        env.reset()
+        env.close()
+    res = np.array(res)
+    eq(res, g["validate/final"])
+    assert np.isfinite(res).all() and (res[:, 0] > 0).all()
