@@ -31,6 +31,7 @@
 //                            ord[off_m, off_m + cnt[m]) with off_m = cnt[0] + ... + cnt[m-1]; rpred = route predecessor)
 //   xs  [B][xs_stride] f64   static doubles:  mind[N] minpt[N] tt[M][M]
 //   t,p [B][N][M]      f64   instance tables, touched only at (op, machine) and in the mfea1 kernel
+#include <assert.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -74,7 +75,13 @@ struct Params {
     const double* xs;
     const double* t;
     const double* p;
-    const double* weights;  // reset only
+    const double* weights;  // reset, and MODE_FROM_RESET
+    // MODE_FROM_RESET: the step also performs a recorded episode reset (mtfjsp_env::pend_reset): the records are staged
+    // from the snapshot sd0 / si0, the weights from `weights`, the reward scaler's running returns cleared if clear_ret,
+    // and the records written back whole
+    const double* sd0;
+    const int16_t* si0;
+    int clear_ret;
     double cfgw[3], divisor, gamma;
     // step io
     const int32_t* op;
@@ -116,7 +123,8 @@ struct Params {
 };
 
 enum { MODE_STEP = 1, MODE_OBS = 2, MODE_RESET = 4, MODE_POLICY = 8,
-       MODE_HOST = 16 };  // size-specialised kernels: step info / packed records leave as whole-warp runs (host-step calls)
+       MODE_HOST = 16,        // size-specialised kernels: step info / packed records leave as whole-warp runs (host-step calls)
+       MODE_FROM_RESET = 32 };  // size-specialised step kernels: the step also performs a recorded reset (Params::sd0)
 
 // step info (r, done, mk_s, idle_s, pt_s, tt_s) goes to the contiguous [B,6] array and / or the packed host record
 #define INFO6_PUT(b_, k_, v_)                                                                               \
@@ -886,6 +894,14 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     double* g_sd = P.sd + (size_t)bc * S::SD;
     int16_t* g_si = P.si + (size_t)bc * S::SI;
     const double* g_xs = P.xs + (size_t)bc * S::XS;
+    // fused episode reset: an instantiation of its own, so that the kernel of every other step carries none of it
+    constexpr bool fr = (MODE & MODE_FROM_RESET) != 0;
+    static_assert(!fr || (!S::COLD && (MODE & MODE_STEP)), "COLD reads dur / psel from the state record, not the snapshot");
+#ifdef MTFJSP_DEBUG_BOUNDS  // debug builds: the snapshot records read here lie inside the batch
+    if (fr) assert(bc < P.L.B && P.L.sd_stride == S::SD && P.L.si_stride == S::SI);
+#endif
+    const double* src_sd = fr ? P.sd0 + (size_t)bc * S::SD : g_sd;
+    const int16_t* src_si = fr ? P.si0 + (size_t)bc * S::SI : g_si;
 
     // the action is the head of a dependent chain (op -> t[op][m], mind row of its job): issue it first
     int a = 0, m = 0;
@@ -896,11 +912,13 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     if constexpr ((MODE & MODE_POLICY) != 0) {
         const uint8_t* jsrc = (P.mask_mode == MTFJSP_MASK_ESA ? P.jm_esa : P.jm_fin) + (size_t)bc * J;
         if (gl < J) {
-            sel = jsrc[gl] == 0;
-            cj = P.cand_int[(size_t)bc * J + gl];
+            // the reset image (what reset_copy_kernel writes): no job masked, every job's candidate is its first op,
+            // nothing scheduled
+            sel = fr ? true : jsrc[gl] == 0;
+            cj = fr ? gl * M : P.cand_int[(size_t)bc * J + gl];
         }
         if (gl < M && P.mfea1 != nullptr) eid = __ldg(P.edge_id + (size_t)bc * M + gl);
-        nsel_step = g_si[S::O_MISC + 2];
+        nsel_step = fr ? 0 : g_si[S::O_MISC + 2];
     } else if (MODE & MODE_STEP) {
         if (P.act2) { const int2 am = __ldg(P.act2 + bc); a = am.x; m = am.y; }
         else { a = __ldg(P.op + bc); m = __ldg(P.mach + bc); }
@@ -918,7 +936,7 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar),
-                     "r"((uint32_t)(EPW * (S::SM_SD * 8 + S::B_TT + S::SI * 2)))
+                     "r"((uint32_t)(EPW * (S::SM_SD * 8 + S::B_TT + S::SI * 2 + (fr ? (S::SD - (S::O_SC & ~1)) * 8 : 0))))
                      : "memory");
     }
     __syncwarp();
@@ -927,10 +945,20 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
             bulk_g2s(s_sd, g_sd, S::HOT * 8, bar);
             bulk_g2s(s_sd + S::HOT, g_sd + 4 * N, S::TAILBLK * 8, bar);
         } else {
-            bulk_g2s(s_sd, g_sd, S::SD * 8, bar);
+            bulk_g2s(s_sd, src_sd, S::SD * 8, bar);
         }
         if constexpr (S::B_TT > 0) bulk_g2s(base + S::B_SD, g_xs + S::O_TT, S::TT * 8, bar);
-        bulk_g2s(s_si, g_si, S::SI * 2, bar);
+        bulk_g2s(s_si, src_si, S::SI * 2, bar);
+    }
+    // fused reset: the reward-scaler block is the state's (the scaler runs across episodes), staged into the idle-term
+    // scratch from the 16-byte word it starts in; the three weights are the caller's.  Both go over the staged snapshot
+    // once it has landed.
+    constexpr int SC0 = S::O_SC & ~1;
+    static_assert(S::NPT >= S::SD - SC0, "the scaler block is staged in the idle-term scratch");
+    double wv = 0.0;
+    if constexpr (fr) {
+        if (gl == 0) bulk_g2s(s_pt, g_sd + SC0, (S::SD - SC0) * 8, bar);
+        if (gl < 3) wv = P.weights[(size_t)bc * 3 + gl];
     }
     if constexpr (S::TTG) {  // the transport table (M * M doubles) into L1: the step reads a few entries of it
         if (gl < 4) {
@@ -1015,6 +1043,11 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
                 : "r"(bar)
                 : "memory");
         } while (!ok);
+    }
+    if constexpr (fr) {  // R[0..3] are the running returns a folded-in scaler reset clears
+        const double* s_sc0 = s_pt + (S::O_SC - SC0);
+        for (int i = gl; i < 13; i += G) s_sd[S::SM_SC + i] = (i < 4 && P.clear_ret) ? 0.0 : s_sc0[i];
+        if (gl < 3) s_sd[S::SM_W + gl] = wv;
     }
     __syncwarp();
 
@@ -1452,7 +1485,7 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
             }
         }
         __syncwarp();
-        if (valid) {  // selective write-back: 4 scalars, macc[m][3], 13 scaler words
+        if (valid && !fr) {  // selective write-back: 4 scalars, macc[m][3], 13 scaler words
 #pragma unroll
             for (int i = gl; i < 20; i += G) {
                 if (i < 4) g_sd[S::O_SCAL + i] = s_scal[i];
@@ -1626,6 +1659,19 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
             }
             if (P.mfea && gl < M && active) emit_mach(gl, c > 0 ? (int)s_ord[incs - 1] : 0);
         }
+    }
+
+    if (fr && active) {
+        // The records were staged from the snapshot, not from the state: write them back whole, 16 bytes per lane (the
+        // observation part above only reads them)
+        const double2* s2 = reinterpret_cast<const double2*>(s_sd);
+        double2* g2 = reinterpret_cast<double2*>(g_sd);
+#pragma unroll 1
+        for (int i = gl; i < S::SD / 2; i += G) g2[i] = s2[i];
+        const int4* s4 = reinterpret_cast<const int4*>(s_si);
+        int4* g4 = reinterpret_cast<int4*>(g_si);
+#pragma unroll 1
+        for (int i = gl; i < S::SI / 8; i += G) g4[i] = s4[i];
     }
 }
 
@@ -2043,24 +2089,24 @@ __global__ void export_scaler_kernel(Layout L, const double* __restrict__ sd, do
 // Episode reset from the snapshot of the first one: the reset image of an env (initial estimates, counters, links,
 // initial makespan / energy estimates) depends on the instance only, so later resets are one coalesced copy of the env
 // part of `sd` (everything in front of the reward-scaler block; the three reward weights come from the caller), the
-// whole `si` record and the initial job masks / candidates -- instead of re-deriving them per env.
+// whole `si` record and the initial job masks / candidates -- instead of re-deriving them per env.  One block per env,
+// 16 bytes per thread (records are 16-byte aligned).
 __global__ void reset_copy_kernel(Layout L, const double* __restrict__ sd0, const int16_t* __restrict__ si0,
                                   const double* __restrict__ weights, double* __restrict__ sd, int16_t* __restrict__ si,
                                   uint8_t* __restrict__ jm_fin, uint8_t* __restrict__ jm_esa, int32_t* __restrict__ cand) {
-    const int wsi = L.si_stride / 4;  // si record in 8-byte words
-    const int per = L.o_sc + wsi + L.J;
-    const size_t gid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= (size_t)L.B * per) return;
-    const size_t b = gid / per;
-    const int i = (int)(gid - b * per);
-    if (i < L.o_sc) {
-        const size_t k = b * L.sd_stride + i;
-        sd[k] = (i >= L.o_w && i < L.o_w + 3) ? weights[b * 3 + (i - L.o_w)] : sd0[k];
-    } else if (i < L.o_sc + wsi) {
-        const size_t k = b * wsi + (i - L.o_sc);
-        reinterpret_cast<uint2*>(si)[k] = reinterpret_cast<const uint2*>(si0)[k];
-    } else {
-        const int j = i - L.o_sc - wsi;
+    const size_t b = blockIdx.x;
+    const double2* src = reinterpret_cast<const double2*>(sd0 + b * L.sd_stride);
+    double2* dst = reinterpret_cast<double2*>(sd + b * L.sd_stride);
+    auto word = [&](const int i, const double v) { return (i >= L.o_w && i < L.o_w + 3) ? weights[b * 3 + (i - L.o_w)] : v; };
+    for (int k = threadIdx.x; 2 * k < L.o_sc; k += blockDim.x) {  // the part in front of the reward-scaler block
+        const double2 v = src[k];
+        if (2 * k + 1 < L.o_sc) dst[k] = make_double2(word(2 * k, v.x), word(2 * k + 1, v.y));
+        else sd[b * L.sd_stride + 2 * k] = word(2 * k, v.x);
+    }
+    const int4* si_src = reinterpret_cast<const int4*>(si0 + b * L.si_stride);
+    int4* si_dst = reinterpret_cast<int4*>(si + b * L.si_stride);
+    for (int k = threadIdx.x; k < L.si_stride / 8; k += blockDim.x) si_dst[k] = si_src[k];
+    for (int j = threadIdx.x; j < L.J; j += blockDim.x) {
         jm_fin[b * L.J + j] = 0;
         jm_esa[b * L.J + j] = 0;
         cand[b * L.J + j] = j * L.M;
@@ -2103,6 +2149,13 @@ struct mtfjsp_env {
     double* sd0;   // reset snapshot of sd / si (taken after the first reset since the last load)
     int16_t* si0;
     bool reset_snap;
+    // MTFJSP_FUSED_RESET (default on): once the snapshot exists, mtfjsp_reset (and an mtfjsp_scaler_reset behind it) only
+    // record the reset here.  The next step launch of a specialised kernel performs it -- it stages the snapshot instead
+    // of the state and writes its records back whole -- instead of a separate pass over the batch's state.  Every other
+    // entry point first runs the recorded reset as reset_copy_kernel + scaler_kernel (flush_reset).
+    int fused_reset;
+    bool pend_reset, pend_scaler;
+    const double* pend_w;  // the caller's [B,3] weights: valid until the next call on the handle (include/mtfjsp.h)
     int16_t* si;
     int8_t* edge_id;
     uint8_t *jm_fin, *jm_esa;
@@ -2172,9 +2225,37 @@ static Params make_params(mtfjsp_env* h) {
     return P;
 }
 
+// Runs the reset that mtfjsp_reset / mtfjsp_scaler_reset recorded (mtfjsp_env::pend_reset), if any.
+static int flush_reset(mtfjsp_env* h, cudaStream_t s) {
+    const Layout& L = h->L;
+    if (h->pend_reset) {
+        reset_copy_kernel<<<L.B, 128, 0, s>>>(L, h->sd0, h->si0, h->pend_w, h->sd, h->si, h->jm_fin, h->jm_esa, h->cand);
+        h->launches++;
+        h->pend_reset = false;
+        CK(cudaGetLastError(), "reset_copy_kernel");
+    }
+    if (h->pend_scaler) {
+        const size_t n = (size_t)L.B * 4;
+        scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(L, h->sd, 0);
+        h->launches++;
+        h->pend_scaler = false;
+        CK(cudaGetLastError(), "scaler_kernel");
+    }
+    return MTFJSP_OK;
+}
+
+// Head of every entry point that touches env state: selects the device and runs a recorded reset -- unless the call
+// is a step that may perform the reset itself (launch_spec decides; every other launch path flushes).
+static int enter(mtfjsp_env* h, cudaStream_t s, bool step = false) {
+    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    return step ? MTFJSP_OK : flush_reset(h, s);
+}
+
 template <int MODE, typename OutT>
 static int launch_env(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     const Layout& L = h->L;
+    int rc = flush_reset(h, s);
+    if (rc != MTFJSP_OK) return rc;
     size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
     static thread_local int configured_dev = -1;
     static thread_local size_t configured_smem = 0;
@@ -2197,6 +2278,18 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     if (L.sd_stride != S::SD || L.si_stride != S::SI || L.xs_stride != S::XS || L.o_sc != S::O_SC || L.o_misc != S::O_MISC ||
         L.o_eacc != S::O_EACC || L.o_eleaf != S::O_ELEAF || L.o_ipre != S::O_IPRE || L.nich != S::NICH || h->pw.nleaves != S::NLEAF)
         return fail(MTFJSP_E_STATE, "specialised kernel layout mismatch");
+    if constexpr (!S::COLD && (MODE & MODE_STEP) && !(MODE & (MODE_HOST | MODE_FROM_RESET))) {
+        if (h->pend_reset) {  // this step performs the recorded reset
+            Params Q = P;
+            Q.sd0 = h->sd0; Q.si0 = h->si0; Q.weights = h->pend_w; Q.clear_ret = h->pend_scaler ? 1 : 0;
+            h->pend_reset = h->pend_scaler = false;
+            return launch_spec<S, MODE | MODE_FROM_RESET, OutT>(h, Q, s);
+        }
+    }
+    if constexpr (!(MODE & MODE_FROM_RESET)) {
+        const int rc = flush_reset(h, s);
+        if (rc != MTFJSP_OK) return rc;
+    }
     static const size_t extra = getenv("MTFJSP_EXTRA_SMEM") ? (size_t)atoi(getenv("MTFJSP_EXTRA_SMEM")) : 0;  // occupancy experiments
     const size_t smem = (size_t)S::WARPS * S::EPW * S::ENV_BYTES + (S::BAR_IN_PAD ? 0 : 16 * ((S::WARPS * 8 + 15) / 16)) + extra;
     static thread_local int configured_dev = -1;
@@ -2418,6 +2511,7 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
         h->fuse_policy = getenv("MTFJSP_FUSE_POLICY") ? atoi(getenv("MTFJSP_FUSE_POLICY")) : 1;
         h->alternate_order = getenv("MTFJSP_ALTERNATE_ORDER") ? atoi(getenv("MTFJSP_ALTERNATE_ORDER")) : 1;
         h->obs_inc_allowed = !(getenv("MTFJSP_OBS_INCREMENTAL") && atoi(getenv("MTFJSP_OBS_INCREMENTAL")) == 0);  // test hook
+        h->fused_reset = getenv("MTFJSP_FUSED_RESET") ? atoi(getenv("MTFJSP_FUSED_RESET")) : 1;
     }
     h->cfgw[0] = 0.4; h->cfgw[1] = 0.4; h->cfgw[2] = 0.2; h->divisor = 1.0; h->gamma = 0.99;
     size_t Bs = (size_t)B;
@@ -2515,7 +2609,8 @@ int mtfjsp_load(mtfjsp_env* h, const double* t, const double* p, const double* t
                 void* stream) {
     if (!h || !t || !p || !tt || !edge || W < 1) return fail(MTFJSP_E_ARG, "mtfjsp_load: bad argument");
     cudaStream_t s = (cudaStream_t)stream;
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, s);
+    if (rc) return rc;
     const Layout& L = h->L;
     size_t n = (size_t)L.B * L.N * L.M * 8;
     CK(cudaMemcpyAsync(h->t, t, n, cudaMemcpyDeviceToDevice, s), "copy t");
@@ -2533,7 +2628,8 @@ int mtfjsp_load(mtfjsp_env* h, const double* t, const double* p, const double* t
 
 int mtfjsp_scaler_init(mtfjsp_env* h, void* stream) {
     if (!h) return fail(MTFJSP_E_ARG, "null handle");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     size_t n = (size_t)h->L.B * 13;
     scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, 1);
     h->launches++;
@@ -2543,7 +2639,12 @@ int mtfjsp_scaler_init(mtfjsp_env* h, void* stream) {
 
 int mtfjsp_scaler_reset(mtfjsp_env* h, void* stream) {
     if (!h) return fail(MTFJSP_E_ARG, "null handle");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    if (h->pend_reset) {  // performed together with the recorded reset
+        h->pend_scaler = true;
+        return MTFJSP_OK;
+    }
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     size_t n = (size_t)h->L.B * 4;
     scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, 0);
     h->launches++;
@@ -2554,18 +2655,15 @@ int mtfjsp_scaler_reset(mtfjsp_env* h, void* stream) {
 int mtfjsp_reset(mtfjsp_env* h, const double* weights, void* stream) {
     if (!h || !weights) return fail(MTFJSP_E_ARG, "mtfjsp_reset: bad argument");
     if (!h->loaded) return fail(MTFJSP_E_STATE, "mtfjsp_reset before mtfjsp_load");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
     const Layout& L = h->L;
     h->obs_synced = false;
-    if (h->reset_snap) {
-        const size_t total = (size_t)L.B * (L.o_sc + L.si_stride / 4 + L.J);
-        reset_copy_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(L, h->sd0, h->si0, weights, h->sd, h->si, h->jm_fin,
-                                                                      h->jm_esa, h->cand);
-        h->launches++;
-        CK(cudaGetLastError(), "reset_copy_kernel");
-        return MTFJSP_OK;
+    if (h->reset_snap) {  // recorded; a later reset replaces the weights, a pending scaler reset stays
+        h->pend_reset = true;
+        h->pend_w = weights;
+        return h->fused_reset ? MTFJSP_OK : enter(h, s);
     }
+    CK(cudaSetDevice(h->device), "cudaSetDevice");
     Params P = make_params(h);
     P.weights = weights;
     int rc = launch_env<MODE_RESET, double>(h, P, s);
@@ -2584,7 +2682,8 @@ int mtfjsp_step(mtfjsp_env* h, const int32_t* op, const int32_t* mach, double* r
                 uint8_t* done, uint8_t* invalid, void* stream) {
     if (!h || !op || !mach) return fail(MTFJSP_E_ARG, "mtfjsp_step: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_step before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream, true);
+    if (rc) return rc;
     Params P = make_params(h);
     P.op = op; P.mach = mach; P.reward5 = reward5; P.scaled4 = scaled4; P.done = done; P.invalid = invalid;
     h->obs_synced = false;  // the state moves on without any observation buffer following it
@@ -2595,9 +2694,10 @@ int mtfjsp_obs(mtfjsp_env* h, void* task_fea, void* mach_fea, float* adj_w, int1
                int32_t* candidate, int mask_mode, int dtype, void* stream) {
     if (!h) return fail(MTFJSP_E_ARG, "null handle");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_obs before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     Params P = make_params(h);
-    int rc = fill_obs(h, P, task_fea, mach_fea, adj_w, adj_src, job_mask, candidate, mask_mode, dtype);
+    rc = fill_obs(h, P, task_fea, mach_fea, adj_w, adj_src, job_mask, candidate, mask_mode, dtype);
     if (rc) return rc;
     rc = dtype == MTFJSP_F64 ? launch_env_auto<MODE_OBS, double>(h, P, (cudaStream_t)stream)
                              : launch_env_auto<MODE_OBS, float>(h, P, (cudaStream_t)stream);
@@ -2612,9 +2712,10 @@ int mtfjsp_step_obs(mtfjsp_env* h, const int32_t* op, const int32_t* mach, doubl
                     uint8_t* job_mask, int32_t* candidate, int mask_mode, int dtype, void* stream) {
     if (!h || !op || !mach) return fail(MTFJSP_E_ARG, "mtfjsp_step_obs: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_step_obs before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream, true);
+    if (rc) return rc;
     const int inc = obs_inc_now(h, task_fea, mach_fea, adj_w, adj_src, dtype);
-    int rc = step_obs_range(h, op, mach, reward5, scaled4, done, invalid, nullptr, task_fea, mach_fea, adj_w, adj_src,
+    rc = step_obs_range(h, op, mach, reward5, scaled4, done, invalid, nullptr, task_fea, mach_fea, adj_w, adj_src,
                             job_mask, candidate, mask_mode, dtype, 0, h->L.B, (cudaStream_t)stream, nullptr, nullptr, inc);
     if (rc == MTFJSP_OK) obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
     return rc;
@@ -2623,9 +2724,12 @@ int mtfjsp_step_obs(mtfjsp_env* h, const int32_t* op, const int32_t* mach, doubl
 int mtfjsp_mfea1(mtfjsp_env* h, const int32_t* op, void* mfea1, uint8_t* mach_mask, int dtype, void* stream) {
     if (!h || !op || !mfea1) return fail(MTFJSP_E_ARG, "mtfjsp_mfea1: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_mfea1 before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
     const Layout& L = h->L;
     cudaStream_t s = (cudaStream_t)stream;
+    {
+        int rc = enter(h, s);
+        if (rc) return rc;
+    }
     if (dtype != MTFJSP_F32 && dtype != MTFJSP_F64) return fail(MTFJSP_E_ARG, "dtype must be MTFJSP_F32 or MTFJSP_F64");
     {
         int rc = launch_prestep<false>(h, 0, 0, nullptr, const_cast<int32_t*>(op), nullptr, mfea1, mach_mask, dtype, s);
@@ -2647,7 +2751,9 @@ int mtfjsp_dense_adj(mtfjsp_env* h, void* adj, int dtype, void* stream) {
     if (!h || !adj) return fail(MTFJSP_E_ARG, "mtfjsp_dense_adj: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_dense_adj before mtfjsp_reset");
     cudaStream_t s = (cudaStream_t)stream;
-    int rc = mtfjsp_obs(h, nullptr, nullptr, h->tmp_adj_w, h->tmp_adj_src, nullptr, nullptr, MTFJSP_MASK_ESA, MTFJSP_F32, stream);
+    int rc = enter(h, s);
+    if (rc) return rc;
+    rc = mtfjsp_obs(h, nullptr, nullptr, h->tmp_adj_w, h->tmp_adj_src, nullptr, nullptr, MTFJSP_MASK_ESA, MTFJSP_F32, stream);
     if (rc) return rc;
     if (dtype == MTFJSP_F64) dense_adj_kernel<double><<<h->L.B, 256, 0, s>>>(h->L, h->tmp_adj_w, h->tmp_adj_src, (double*)adj);
     else if (dtype == MTFJSP_F32) dense_adj_kernel<float><<<h->L.B, 256, 0, s>>>(h->L, h->tmp_adj_w, h->tmp_adj_src, (float*)adj);
@@ -2660,8 +2766,9 @@ int mtfjsp_dense_adj(mtfjsp_env* h, void* adj, int dtype, void* stream) {
 int mtfjsp_raw_adj(mtfjsp_env* h, int32_t* adj, void* stream) {
     if (!h || !adj) return fail(MTFJSP_E_ARG, "mtfjsp_raw_adj: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_raw_adj before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
+    int rc = enter(h, s);
+    if (rc) return rc;
     const Layout& L = h->L;
     CK(cudaMemsetAsync(adj, 0, (size_t)L.B * L.N * L.N * sizeof(int32_t), s), "cudaMemsetAsync");
     const size_t n = (size_t)L.B * L.N;
@@ -2687,7 +2794,8 @@ int mtfjsp_generate_instances(int B, int J, int M, int E, uint64_t seed, uint64_
 
 int mtfjsp_costs(mtfjsp_env* h, double* cost4, double* total_e1, void* stream) {
     if (!h || (!cost4 && !total_e1)) return fail(MTFJSP_E_ARG, "mtfjsp_costs: bad argument");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     costs_kernel<<<(h->L.B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, cost4, total_e1);
     h->launches++;
     CK(cudaGetLastError(), "costs_kernel");
@@ -2696,8 +2804,9 @@ int mtfjsp_costs(mtfjsp_env* h, double* cost4, double* total_e1, void* stream) {
 
 int mtfjsp_export_state(mtfjsp_env* h, int32_t* mach, double* st, double* ft, int32_t* routes, void* stream) {
     if (!h) return fail(MTFJSP_E_ARG, "null handle");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
+    int rc = enter(h, s);
+    if (rc) return rc;
     const Layout& L = h->L;
     if (routes) {
         size_t n = (size_t)L.B * L.M * L.N;
@@ -2713,7 +2822,8 @@ int mtfjsp_export_state(mtfjsp_env* h, int32_t* mach, double* st, double* ft, in
 
 int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int64_t* n, void* stream) {
     if (!h || !R || !mean || !S || !n) return fail(MTFJSP_E_ARG, "mtfjsp_export_scaler: bad argument");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     export_scaler_kernel<<<(h->L.B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, R, mean, S, n);
     h->launches++;
     CK(cudaGetLastError(), "export_scaler_kernel");
@@ -2724,7 +2834,8 @@ int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int 
                          int32_t* mach, void* stream) {
     if (!h || !op || !mach) return fail(MTFJSP_E_ARG, "mtfjsp_policy_random: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_policy_random before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     const uint8_t* jm = mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin;
     policy_kernel<<<(h->L.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->L, h->t, h->si, jm, h->cand, seed, env_offset, op, mach);
     h->launches++;
@@ -2741,7 +2852,8 @@ int mtfjsp_random_step(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int32_
     int32_t* mc = mach ? mach : h->a_mach;
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_random_step before mtfjsp_reset");
     if (dtype != MTFJSP_F32 && dtype != MTFJSP_F64) return fail(MTFJSP_E_ARG, "dtype must be MTFJSP_F32 or MTFJSP_F64");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream, true);
+    if (rc) return rc;
     {
         Params P = make_params(h);
         P.reward5 = reward5; P.scaled4 = scaled4; P.done = done; P.invalid = invalid;
@@ -2755,7 +2867,9 @@ int mtfjsp_random_step(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int32_
         if (rf > 0) obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
         if (rf != 0) return rf < 0 ? rf : MTFJSP_OK;
     }
-    int rc = launch_prestep<true>(h, seed, env_offset, mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin, o, mc, mfea1,
+    rc = flush_reset(h, (cudaStream_t)stream);  // the separate kernels below read the state
+    if (rc) return rc;
+    rc = launch_prestep<true>(h, seed, env_offset, mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin, o, mc, mfea1,
                                   mach_mask, dtype, (cudaStream_t)stream);
     if (rc < 0) return rc;
     if (rc == 0) {
@@ -2996,7 +3110,8 @@ int mtfjsp_step_host(mtfjsp_env* h, const int32_t* op_host, const int32_t* mach_
                      int16_t* adj_src, int mask_mode, int dtype, void* stream) {
     if (!h || !op_host || !mach_host) return fail(MTFJSP_E_ARG, "mtfjsp_step_host: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_step_host before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     HostIO io = {op_host, mach_host, nullptr, info6_host, job_mask_host, candidate_host, nullptr};
     return host_step_impl(h, io, task_fea, mach_fea, adj_w, adj_src, mask_mode, dtype, (cudaStream_t)stream);
 }
@@ -3005,7 +3120,8 @@ int mtfjsp_step_host_packed(mtfjsp_env* h, const int32_t* actions_host, void* re
                             float* adj_w, int16_t* adj_src, int mask_mode, int dtype, void* stream) {
     if (!h || !actions_host || !records_host) return fail(MTFJSP_E_ARG, "mtfjsp_step_host_packed: bad argument");
     if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_step_host_packed before mtfjsp_reset");
-    CK(cudaSetDevice(h->device), "cudaSetDevice");
+    int rc = enter(h, (cudaStream_t)stream);
+    if (rc) return rc;
     HostIO io = {nullptr, nullptr, actions_host, nullptr, nullptr, nullptr, (unsigned char*)records_host};
     return host_step_impl(h, io, task_fea, mach_fea, adj_w, adj_src, mask_mode, dtype, (cudaStream_t)stream);
 }

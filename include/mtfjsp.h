@@ -67,7 +67,11 @@ int mtfjsp_scaler_reset(mtfjsp_env* h, void* stream);
 
 /* replaces: Parallel_env.init_DGFJSPEnv_state0 / env.reset (trainer/parallel_env.py:87-142, SS:1183-1245).
  * weights: [B,3] f64 per-env reward weights (mk, ec, tt) -- the reference draws them from python's
- * global `random` (SS:1253-1270); here they are data. */
+ * global `random` (SS:1253-1270); here they are data.
+ * Every reset after the first one since a load may be deferred: it is recorded, with mtfjsp_scaler_reset if that
+ * follows, and performed by the next call on the handle, on that call's stream -- inside the step launch where it can,
+ * otherwise before that call's own work.  So `weights` must stay valid and unchanged until the next call on the
+ * handle returns.  MTFJSP_FUSED_RESET=0 in the environment at mtfjsp_create performs every reset at the call. */
 int mtfjsp_reset(mtfjsp_env* h, const double* weights, void* stream);
 
 /* replaces: the transition + reward + reward-scaling half of Parallel_env.DGFJSPEnv_paral_step
