@@ -120,6 +120,12 @@ struct Params {
     uint8_t* jm_fin;
     uint8_t* jm_esa;
     int32_t* cand_int;
+    // launch overlap (size-specialised whole-batch step launches, see ovl_wait): ep != 0 makes each warp release
+    // done_ep[its env range] = ep once its envs are written; wait_ep != 0 makes each warp first wait until that entry
+    // reaches wait_ep (the previous such launch may still be running); ovl_err: mapped host word set on a timeout
+    unsigned long long* done_ep;
+    unsigned long long ep, wait_ep;
+    unsigned* ovl_err;
 };
 
 enum { MODE_STEP = 1, MODE_OBS = 2, MODE_RESET = 4, MODE_POLICY = 8,
@@ -780,6 +786,10 @@ struct Spec {
     static constexpr int ITER = (N + G - 1) / G;
     static constexpr unsigned GMASK = (G_ == 32) ? 0xffffffffu : ((1u << G_) - 1u);
     static constexpr int MINB = minb(NPT, B_TT);
+    // launch overlap (ovl_wait) where it was measured to pay: 4-warp blocks of 16 short envs (J6M6 random step at 65,536
+    // envs, 4.6 waves: 62.5 -> 59.2 us).  The one-warp blocks of the other sizes lost with it (J10M10 at 16,384 envs
+    // 34.7 -> 35.5 us, J30M20 at 4,096 envs 32.2 -> 36.6 us; profiles/README.md, round 5)
+    static constexpr bool OVL = WARPS_ > 1;
 };
 
 // bulk async copy global -> shared (TMA, 1-D), completion counted in bytes on an mbarrier; 16-byte aligned, size % 16 == 0
@@ -850,6 +860,43 @@ __device__ __forceinline__ double np_sum_small(const double* a, int n) {
 // position of the k-th (0-based) set bit of `bits`, -1 if there are not that many (fns.b32: n-th set bit from bit 0 up)
 __device__ __forceinline__ int kth_set_bit(unsigned bits, int k, int /*maxk*/) { return (int)__fns(bits, 0u, k + 1); }
 
+// Launch overlap (Params::done_ep).  Back-to-back whole-batch random steps of one handle are issued with programmatic
+// stream serialization (launch_spec says when) and every block of a whole-batch step launch triggers its dependents when
+// it starts, so launch k+1 becomes resident in the slots that the tail of launch k leaves empty instead of after the
+// whole grid.  A warp of launch k+1 depends only on its own envs
+// in launch k, so it waits for one completion entry per warp-sized env range -- indexed by the env range, not by
+// blockIdx, so both walk directions map to the same entry -- instead of for the whole grid (griddepcontrol.wait).
+// (Per warp rather than per block: the warps of a block share nothing, and no block barrier has to count warps that
+// returned early.)
+// No deadlock: a grid becomes resident only once every CTA of its predecessor has started, so every CTA a warp waits on
+// is resident or finished; by induction over the launches, nothing waits on a CTA that cannot be scheduled.
+// The wait is bounded (1 s of %globaltimer): on expiry the mapped host word is set -- the next call on the handle
+// returns an error -- and the warp proceeds rather than hanging or trapping the device.
+__device__ __forceinline__ void ovl_wait(const unsigned long long* flag, unsigned long long want, unsigned* err) {
+    unsigned long long v;
+    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(flag) : "memory");
+    if (v >= want) return;
+    uint64_t t0, t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
+    unsigned ns = 32;
+    do {
+        __nanosleep(ns);
+        if (ns < 1024) ns <<= 1;
+        asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(flag) : "memory");
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+        if (v < want && t - t0 > 1000000000ull) {
+            *(volatile unsigned*)err = 1u;
+            __threadfence_system();
+            return;
+        }
+    } while (v < want);
+}
+// after every global write of the warp's envs (behind a __syncwarp): publish them.  max: an entry never decreases, so
+// a wait for an epoch that has passed is always satisfied
+__device__ __forceinline__ void ovl_release(unsigned long long* flag, unsigned long long ep) {
+    asm volatile("red.release.gpu.global.max.u64 [%0], %1;" ::"l"(flag), "l"(ep) : "memory");
+}
+
 template <class S, int MODE, typename OutT>
 __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __grid_constant__ Params P) {
     constexpr int J = S::J, M = S::M, N = S::N, G = S::G, EPW = S::EPW, ITER = S::ITER;
@@ -860,6 +907,12 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     const int B = P.b1;
     const int blk = P.rev ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x;
     const int wb0 = P.b0 + (blk * S::WARPS + warp) * EPW;
+    // launch overlap (ovl_wait): the next launch may become resident as soon as every block of this one has started
+    constexpr bool OVL = S::OVL && (MODE & MODE_STEP) && !(MODE & MODE_HOST);
+    if (OVL && P.ep) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    // only the random step without a recorded reset may start early (launch_spec): everything it reads is the handle's
+    // own state, written by the handle's previous step launch
+    constexpr bool WAITS = OVL && (MODE & MODE_POLICY) && !(MODE & MODE_FROM_RESET);
     if (wb0 >= B) return;
     const int b = wb0 + ge;
     const bool active = b < B;
@@ -903,26 +956,32 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     const double* src_sd = fr ? P.sd0 + (size_t)bc * S::SD : g_sd;
     const int16_t* src_si = fr ? P.si0 + (size_t)bc * S::SI : g_si;
 
-    // the action is the head of a dependent chain (op -> t[op][m], mind row of its job): issue it first
     int a = 0, m = 0;
     bool sel = false;  // MODE_POLICY, lane j: job j selectable
     int cj = 0;        //              lane j: candidate op of job j
     int nsel_step = 0; //              ops scheduled so far = the step counter of the random stream
     int eid = 0;       //              lane k: edge group of machine k (candidate-machine feature 5), independent of the action
     if constexpr ((MODE & MODE_POLICY) != 0) {
-        const uint8_t* jsrc = (P.mask_mode == MTFJSP_MASK_ESA ? P.jm_esa : P.jm_fin) + (size_t)bc * J;
-        if (gl < J) {
-            // the reset image (what reset_copy_kernel writes): no job masked, every job's candidate is its first op,
-            // nothing scheduled
-            sel = fr ? true : jsrc[gl] == 0;
-            cj = fr ? gl * M : P.cand_int[(size_t)bc * J + gl];
-        }
         if (gl < M && P.mfea1 != nullptr) eid = __ldg(P.edge_id + (size_t)bc * M + gl);
-        nsel_step = fr ? 0 : g_si[S::O_MISC + 2];
-    } else if (MODE & MODE_STEP) {
-        if (P.act2) { const int2 am = __ldg(P.act2 + bc); a = am.x; m = am.y; }
-        else { a = __ldg(P.op + bc); m = __ldg(P.mach + bc); }
     }
+    // the action is the head of a dependent chain (op -> t[op][m], mind row of its job): issue it first -- with launch
+    // overlap, right behind the wait
+    auto load_action = [&]() {
+        if constexpr ((MODE & MODE_POLICY) != 0) {
+            const uint8_t* jsrc = (P.mask_mode == MTFJSP_MASK_ESA ? P.jm_esa : P.jm_fin) + (size_t)bc * J;
+            if (gl < J) {
+                // the reset image (what reset_copy_kernel writes): no job masked, every job's candidate is its first op,
+                // nothing scheduled
+                sel = fr ? true : jsrc[gl] == 0;
+                cj = fr ? gl * M : P.cand_int[(size_t)bc * J + gl];
+            }
+            nsel_step = fr ? 0 : g_si[S::O_MISC + 2];
+        } else if (MODE & MODE_STEP) {
+            if (P.act2) { const int2 am = __ldg(P.act2 + bc); a = am.x; m = am.y; }
+            else { a = __ldg(P.op + bc); m = __ldg(P.mach + bc); }
+        }
+    };
+    if constexpr (!WAITS) load_action();
     // ---- stage the records: one cp.async.bulk (TMA, 1-D) per record, three per env, issued by the group's first lane and
     // completing on the warp's mbarrier.  (16-byte cp.async copies spread over the G lanes -- 17 LDGSTS per lane at J6M6 --
     // were 5 % slower: 74.4 -> 70.5 us.)
@@ -940,6 +999,19 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
                      : "memory");
     }
     __syncwarp();
+    if constexpr (WAITS && S::B_TT > 0) {  // static: needs nothing from the previous step
+        if (gl == 0) bulk_g2s(base + S::B_SD, g_xs + S::O_TT, S::TT * 8, bar);
+    }
+    // launch overlap: everything below reads or writes what the previous step launch wrote for these envs.  The bulk
+    // copies read it through the async proxy, the previous launch wrote it through the generic one: proxy fence.
+    if constexpr (WAITS) {
+        if (P.wait_ep) {
+            if (lane == 0) ovl_wait(P.done_ep + wb0 / EPW, P.wait_ep, P.ovl_err);
+            __syncwarp();
+            if (gl == 0) asm volatile("fence.proxy.async.global;" ::: "memory");
+        }
+        load_action();
+    }
     if (gl == 0) {
         if constexpr (S::COLD) {
             bulk_g2s(s_sd, g_sd, S::HOT * 8, bar);
@@ -947,7 +1019,7 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
         } else {
             bulk_g2s(s_sd, src_sd, S::SD * 8, bar);
         }
-        if constexpr (S::B_TT > 0) bulk_g2s(base + S::B_SD, g_xs + S::O_TT, S::TT * 8, bar);
+        if constexpr (!WAITS && S::B_TT > 0) bulk_g2s(base + S::B_SD, g_xs + S::O_TT, S::TT * 8, bar);
         bulk_g2s(s_si, src_si, S::SI * 2, bar);
     }
     // fused reset: the reward-scaler block is the state's (the scaler runs across episodes), staged into the idle-term
@@ -1673,6 +1745,13 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
 #pragma unroll 1
         for (int i = gl; i < S::SI / 8; i += G) g4[i] = s4[i];
     }
+    if (OVL && P.ep) {  // the entry index is recomputed rather than kept live through the step (whole batch: b0 = 0)
+        __syncwarp();
+        if ((threadIdx.x & 31) == 0) {
+            const unsigned bk = P.rev ? gridDim.x - 1 - blockIdx.x : blockIdx.x;
+            ovl_release(P.done_ep + bk * S::WARPS + (threadIdx.x >> 5), P.ep);
+        }
+    }
 }
 
 // ---- static tables: min feasible duration / energy per op, edge id per machine ----
@@ -2185,6 +2264,16 @@ struct mtfjsp_env {
     size_t slab_bytes, window_bytes;
     int l2_persist;
     int64_t launches;
+    // MTFJSP_LAUNCH_OVERLAP (default on): whole-batch step launches of the size-specialised kernel may start while the
+    // previous one finishes (programmatic dependent launch; see ovl_wait).  done_ep: one completion epoch per warp-sized
+    // env range, released by every such launch whatever the setting; ep: the epoch of the last one issued.  ovl_err:
+    // mapped host word a launch sets when its wait timed out (ovl_err_d: its device address)
+    // ovl_chain: the handle's last operation was a step launch that released its epoch
+    int launch_overlap;
+    bool ovl_chain;
+    unsigned long long* done_ep;
+    unsigned long long ep;
+    unsigned *ovl_err, *ovl_err_d;
     struct HostPipe* pipe;  // host-step pipeline (streams, events, instantiated graphs), created on first use
 };
 
@@ -2228,6 +2317,7 @@ static Params make_params(mtfjsp_env* h) {
 // Runs the reset that mtfjsp_reset / mtfjsp_scaler_reset recorded (mtfjsp_env::pend_reset), if any.
 static int flush_reset(mtfjsp_env* h, cudaStream_t s) {
     const Layout& L = h->L;
+    if (h->pend_reset || h->pend_scaler) h->ovl_chain = false;
     if (h->pend_reset) {
         reset_copy_kernel<<<L.B, 128, 0, s>>>(L, h->sd0, h->si0, h->pend_w, h->sd, h->si, h->jm_fin, h->jm_esa, h->cand);
         h->launches++;
@@ -2247,7 +2337,10 @@ static int flush_reset(mtfjsp_env* h, cudaStream_t s) {
 // Head of every entry point that touches env state: selects the device and runs a recorded reset -- unless the call
 // is a step that may perform the reset itself (launch_spec decides; every other launch path flushes).
 static int enter(mtfjsp_env* h, cudaStream_t s, bool step = false) {
+    if (*(volatile unsigned*)h->ovl_err)
+        return fail(MTFJSP_E_CUDA, "a step launch waited more than 1 s for the previous one (launch overlap)");
     CK(cudaSetDevice(h->device), "cudaSetDevice");
+    if (!step) h->ovl_chain = false;  // this call may write what a step reads: the next step waits for it in full
     return step ? MTFJSP_OK : flush_reset(h, s);
 }
 
@@ -2268,6 +2361,7 @@ static int launch_env(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     int blocks = (P.b1 - P.b0 + L.warps_per_block - 1) / L.warps_per_block;
     env_kernel<MODE, OutT><<<blocks, L.warps_per_block * 32, smem, s>>>(P);
     h->launches++;
+    h->ovl_chain = false;
     CK(cudaGetLastError(), "env_kernel launch");
     return MTFJSP_OK;
 }
@@ -2305,27 +2399,58 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
         Q.rev = h->flip;
         h->flip ^= 1;
     }
-    if (h->window_bytes && (MODE & MODE_STEP)) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(blocks);
-        cfg.blockDim = dim3(S::WARPS * 32);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = s;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeAccessPolicyWindow;
-        at[0].val.accessPolicyWindow.base_ptr = h->slab;
-        at[0].val.accessPolicyWindow.num_bytes = h->window_bytes;
-        at[0].val.accessPolicyWindow.hitRatio = 1.0f;
-        at[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        at[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
-        CK(cudaLaunchKernelEx(&cfg, env_kernel_s<S, MODE, OutT>, Q), "env_kernel_s launch");
-    } else {
-        env_kernel_s<S, MODE, OutT><<<blocks, S::WARPS * 32, smem, s>>>(Q);
+    // Launch overlap (ovl_wait).  Whole-batch step launches release epochs (Q.ep).  Only a random step without a recorded
+    // reset carries the programmatic attribute, and only when the handle's previous operation was a step launch that released
+    // its epoch (ovl_chain): a predecessor that does not trigger lets the launch start once its blocks have exited, before its
+    // writes need be visible, and the epochs cover only what step launches wrote.  Everything that step reads is the
+    // handle's own state; other work on the stream between two steps may read their outputs but writes nothing it
+    // reads.  Steps fed actions from outside (step, step_obs), fused resets (caller's weights) and every step after
+    // another call on the handle wait for their predecessor in full.  A launch being captured into a graph takes no
+    // part: its epoch would be released only when the graph runs.
+    bool pdl = false;
+    if (S::OVL && (MODE & MODE_STEP) && !(MODE & MODE_HOST) && P.b0 == 0 && P.b1 == L.B && h->launch_overlap) {
+        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(s, &cs) != cudaSuccess) {
+            cudaGetLastError();
+            cs = cudaStreamCaptureStatusActive;
+        }
+        if (cs == cudaStreamCaptureStatusNone) {
+            pdl = (MODE & MODE_POLICY) && !(MODE & MODE_FROM_RESET) && h->ovl_chain;
+            Q.done_ep = h->done_ep;
+            Q.ovl_err = h->ovl_err_d;
+            Q.wait_ep = pdl ? h->ep : 0;
+            Q.ep = h->ep + 1;
+        }
     }
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(blocks);
+    cfg.blockDim = dim3(S::WARPS * 32);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cudaLaunchAttribute at[2];
+    cfg.attrs = at;
+    if (h->window_bytes && (MODE & MODE_STEP)) {
+        cudaLaunchAttribute& a = at[cfg.numAttrs++];
+        a.id = cudaLaunchAttributeAccessPolicyWindow;
+        a.val.accessPolicyWindow.base_ptr = h->slab;
+        a.val.accessPolicyWindow.num_bytes = h->window_bytes;
+        a.val.accessPolicyWindow.hitRatio = 1.0f;
+        a.val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
+        a.val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
+    }
+    if (pdl) {
+        cudaLaunchAttribute& a = at[cfg.numAttrs++];
+        a.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        a.val.programmaticStreamSerializationAllowed = 1;
+    }
+    h->ovl_chain = false;
+    CK(cudaLaunchKernelEx(&cfg, env_kernel_s<S, MODE, OutT>, Q), "env_kernel_s launch");
     h->launches++;
     CK(cudaGetLastError(), "env_kernel_s launch");
+    if (Q.ep) {  // only a launch that was issued releases its epoch
+        h->ep = Q.ep;
+        h->ovl_chain = true;
+    }
     return MTFJSP_OK;
 }
 
@@ -2512,6 +2637,7 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
         h->alternate_order = getenv("MTFJSP_ALTERNATE_ORDER") ? atoi(getenv("MTFJSP_ALTERNATE_ORDER")) : 1;
         h->obs_inc_allowed = !(getenv("MTFJSP_OBS_INCREMENTAL") && atoi(getenv("MTFJSP_OBS_INCREMENTAL")) == 0);  // test hook
         h->fused_reset = getenv("MTFJSP_FUSED_RESET") ? atoi(getenv("MTFJSP_FUSED_RESET")) : 1;
+        h->launch_overlap = getenv("MTFJSP_LAUNCH_OVERLAP") ? atoi(getenv("MTFJSP_LAUNCH_OVERLAP")) : 1;
     }
     h->cfgw[0] = 0.4; h->cfgw[1] = 0.4; h->cfgw[2] = 0.2; h->divisor = 1.0; h->gamma = 0.99;
     size_t Bs = (size_t)B;
@@ -2565,7 +2691,13 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
     ALLOC(h->tmp_adj_src, Bs * N * 2);
     ALLOC(h->sd0, Bs * L.sd_stride * 8);
     ALLOC(h->si0, Bs * L.si_stride * 2);
+    ALLOC(h->done_ep, Bs * sizeof(unsigned long long));  // at most one entry per env
 #undef ALLOC
+    {
+        cudaError_t e_ = cudaHostAlloc((void**)&h->ovl_err, sizeof(unsigned), cudaHostAllocMapped);
+        if (e_ == cudaSuccess) { *h->ovl_err = 0; e_ = cudaHostGetDevicePointer((void**)&h->ovl_err_d, h->ovl_err, 0); }
+        if (e_ != cudaSuccess) { mtfjsp_destroy(h); return fail(MTFJSP_E_CUDA, "cudaHostAlloc", e_); }
+    }
     *out = h;
     return MTFJSP_OK;
 }
@@ -2574,9 +2706,10 @@ int mtfjsp_destroy(mtfjsp_env* h) {
     if (!h) return MTFJSP_OK;
     cudaSetDevice(h->device);
     void* ptrs[] = {h->sd, h->slab, h->t, h->p, h->edge_id, h->a_op, h->a_mach,
-                    h->r5, h->s4, h->info6, h->dn, h->inv, h->tmp_adj_w, h->tmp_adj_src, h->act2, h->rec, h->sd0, h->si0};
+                    h->r5, h->s4, h->info6, h->dn, h->inv, h->tmp_adj_w, h->tmp_adj_src, h->act2, h->rec, h->sd0, h->si0, h->done_ep};
     for (void* q : ptrs)
         if (q) cudaFree(q);
+    if (h->ovl_err) cudaFreeHost(h->ovl_err);
     if (h->pipe) {
         for (auto& e : h->pipe->cache) cudaGraphExecDestroy(e.exec);
         cudaStreamDestroy(h->pipe->ms);
@@ -3127,6 +3260,8 @@ int mtfjsp_step_host_packed(mtfjsp_env* h, const int32_t* actions_host, void* re
 }
 
 int mtfjsp_host_record_bytes(const mtfjsp_env* h) { return h ? h->rec_stride : 0; }
+
+int mtfjsp_launch_overlap_error(const mtfjsp_env* h) { return h ? (int)*(volatile unsigned*)h->ovl_err : 0; }
 
 int64_t mtfjsp_launch_count(const mtfjsp_env* h) { return h ? h->launches : 0; }
 

@@ -264,6 +264,18 @@ class BatchedMTFJSPEnv:
     def launch_count(self):
         return int(self._lib.mtfjsp_launch_count(self._h))
 
+    @property
+    def launch_overlap_error(self):
+        """Nonzero if an overlapped step launch timed out waiting for its predecessor (every later call raises)."""
+        return int(self._lib.mtfjsp_launch_overlap_error(self._h))
+
+    def check_launch_overlap(self):
+        """Raises if a step launch timed out waiting for its predecessor and went on with what it found.  Call it after
+        synchronising with the device: the word is final for every launch that has finished."""
+        if self.launch_overlap_error:
+            raise _lib.MTFJSPError("a step launch waited more than 1 s for the previous one (launch overlap): "
+                                   "its results are not trustworthy")
+
     def bytes_per_step(self):
         return int(self._lib.mtfjsp_bytes_per_step(self._h, self._dt))
 

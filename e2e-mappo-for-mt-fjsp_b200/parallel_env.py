@@ -228,6 +228,7 @@ class Parallel_env(object):
         if self.compat == "ell":
             e = self._env
             info = torch.cat((e.reward5[:, :1], e.done.to(torch.float64).unsqueeze(1), e.scaled4), dim=1).cpu().numpy()
+            e.check_launch_overlap()
             self.oenv_info = info
             if bool(e.invalid.any()):
                 print("============= 'DGFJSPEnv_paral_step': invalid (task, machine) for envs",
@@ -238,6 +239,7 @@ class Parallel_env(object):
         s4 = self._env.scaled4.cpu().numpy()
         done = self._env.done.cpu().numpy()
         inv = self._env.invalid.cpu().numpy()
+        self._env.check_launch_overlap()
         if inv.any():  # the reference prints and corrupts its state; here the step is refused for those envs
             print("============= 'DGFJSPEnv_paral_step': invalid (task, machine) for envs", np.nonzero(inv)[0].tolist())
         rows = np.concatenate([r5[:, :1], done[:, None].astype(np.float64), s4], axis=1).tolist()

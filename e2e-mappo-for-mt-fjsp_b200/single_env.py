@@ -136,6 +136,7 @@ class DisjunctiveGraphJspEnv_singleStep:
         r5 = self._env.reward5.cpu().numpy()[0]
         invalid = bool(self._env.invalid.cpu().numpy()[0])
         done = bool(self._env.done.cpu().numpy()[0])
+        self._env.check_launch_overlap()
         info = {"action": a}
         if invalid:
             info.update({"valid_action": False, "node_id": a + 1})

@@ -295,6 +295,10 @@ int mtfjsp_gae4(const float* r, const float* v, const float* v_next, const float
 /* adv <- (adv - mean) / (std + 1e-5) per stream over `count` values (unbiased std), ppo_algorithm.py:485, 532. */
 int mtfjsp_adv_normalize(float* adv, const double* stats, double count, int T, int64_t B, void* stream);
 
+/* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
+ * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
+ * word: it reflects the launches the device has finished so far (read it after synchronising). */
+int mtfjsp_launch_overlap_error(const mtfjsp_env* h);
 /* Number of kernel launches issued through this handle so far (bench.py reports it). */
 int64_t mtfjsp_launch_count(const mtfjsp_env* h);
 /* Algorithmic bytes per env-step of the fused step+obs kernel for this handle's sizes (SURVEY.md 8d). */
