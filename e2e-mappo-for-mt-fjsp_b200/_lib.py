@@ -96,6 +96,10 @@ SIGNATURES = {
     "mtfjsp_enc_head_tf32": ([_VP, _VP, C.c_int64, _I, _I, _VP, _VP, _I, _VP, _VP, C.c_int64, _VP, _VP, _VP, _VP, _VP, _VP], _I),
     "mtfjsp_enc_wgrad_tf32": ([_VP, _VP, C.c_int64, _I, _VP, _VP, _VP, _VP], _I),
     "mtfjsp_enc_wgrad_workspace_floats": ([_I], C.c_int64),
+    "mtfjsp_enc_esa_mach_stats": ([_VP, _VP, C.c_int64, _I, _VP, _VP, _VP, _VP], _I),
+    "mtfjsp_enc_esa_mach_stats_workspace_doubles": ([], C.c_int64),
+    "mtfjsp_enc_esa_mach_fold": ([_VP, C.c_int64, _VP, _VP, _VP, _VP, C.c_float] + [_VP] * 7, _I),
+    "mtfjsp_enc_esa_mach_head_tf32": ([_VP, _VP, C.c_int64, _I] + [_VP] * 8, _I),
     "mtfjsp_enc_bn_finalize": ([_VP, C.c_int64, _VP, _VP, C.c_float, _VP, _VP, _I, _VP], _I),
     "mtfjsp_gae4": ([_VP, _VP, _VP, _VP, _VP, _VP, _I, C.c_int64, C.c_float, C.c_float, _VP], _I),
     "mtfjsp_adv_normalize": ([_VP, _VP, C.c_double, _I, C.c_int64, _VP], _I),

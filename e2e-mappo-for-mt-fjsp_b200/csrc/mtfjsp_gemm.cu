@@ -1429,6 +1429,263 @@ __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256));
 }
 
+
+// =====================================================================================================================
+// ESA machine actor (model/actor_critic.py:1207-1404 esa_Machine_Actor) in two launches.  Its per-row network is
+//     h1 = BN(f1 W1^T), h2 = BN(f2 W2^T)  (one BatchNorm module, statistics of each call over its own R rows)
+//     s  = 10 ( tanh( tanh( W0 cat(h1, h2, pooled, h_pooled_o) + b0 ) W1m^T + b1 ) . w2 + b2 )
+// BatchNorm is a per-column affine and both projections are linear, so the per-row part of the first layer is ONE K = 14
+// product on the raw features: W0a diag(sc1) W1 f1 + W0b diag(sc2) W2 f2, the shifts join the per-env bias.  The column
+// statistics follow from the feature moments: mean_c = w_c . mu_f, var_c = w_c^T Sigma_f w_c.
+//
+// esa_stats_kernel: feature sums and second moments (the 6 x 6 and 8 x 8 blocks) in FP64, plus the per-env feature means.
+// A CTA stages whole envs (<= 256 rows) of both feature sets in shared memory; thread (m, half) owns moment m over every
+// other row; the CTA's partial goes to workspace[blockIdx] and esa_stats_reduce_kernel adds the partials in block order,
+// so the moments do not depend on scheduling.
+constexpr int ESA_MOMENTS = 14 + 36 + 64, ESA_STATS_THREADS = 256, ESA_STATS_ROWS = 256, ESA_STATS_BLOCKS = 592;
+
+__global__ void __launch_bounds__(ESA_STATS_THREADS) esa_stats_kernel(const float* __restrict__ f1, const float* __restrict__ f2,
+                                                                       long long B, int M, int epc, double* __restrict__ parts,
+                                                                       float* __restrict__ env_mean) {
+    __shared__ float s_f[ESA_STATS_ROWS * 14];
+    __shared__ double s_acc[128];
+    const int tid = threadIdx.x, mom = tid & 127, half = tid >> 7;
+    // moment `mom`: < 14 column sum, < 50 f1 block (i, j), < 114 f2 block (i, j); columns 0..5 = f1, 6..13 = f2
+    int ca = 0, cb = -1;
+    if (mom < 14) ca = mom;
+    else if (mom < 50) { ca = (mom - 14) / 6; cb = (mom - 14) % 6; }
+    else if (mom < ESA_MOMENTS) { ca = 6 + (mom - 50) / 8; cb = 6 + (mom - 50) % 8; }
+    double acc = 0.0;
+    const long long chunks = (B + epc - 1) / epc;
+    for (long long ch = blockIdx.x; ch < chunks; ch += gridDim.x) {
+        const long long e0 = ch * epc;
+        const int ne = (int)(B - e0 < epc ? B - e0 : epc), nr = ne * M;
+        const long long r0 = e0 * M;
+        __syncthreads();  // the previous chunk's readers are done
+        for (int i = tid; i < nr * 6; i += ESA_STATS_THREADS) s_f[(i / 6) * 14 + i % 6] = __ldg(f1 + r0 * 6 + i);
+        for (int i = tid; i < nr * 8; i += ESA_STATS_THREADS) s_f[(i / 8) * 14 + 6 + i % 8] = __ldg(f2 + r0 * 8 + i);
+        __syncthreads();
+        if (mom < ESA_MOMENTS) {
+            if (cb < 0) {
+                for (int r = half; r < nr; r += 2) acc += (double)s_f[r * 14 + ca];
+            } else {
+                for (int r = half; r < nr; r += 2) acc = fma((double)s_f[r * 14 + ca], (double)s_f[r * 14 + cb], acc);
+            }
+        }
+        for (int i = tid; i < ne * 16; i += ESA_STATS_THREADS) {  // per-env means, [B,16] with two zero columns
+            const int e = i >> 4, c = i & 15;
+            double s = 0.0;
+            if (c < 14)
+                for (int m = 0; m < M; m++) s += (double)s_f[(e * M + m) * 14 + c];
+            env_mean[(e0 + e) * 16 + c] = (float)(s / M);
+        }
+    }
+    if (half == 1) s_acc[mom] = acc;
+    __syncthreads();
+    if (half == 0) parts[(size_t)blockIdx.x * 128 + mom] = acc + s_acc[mom];
+}
+
+__global__ void esa_stats_reduce_kernel(const double* __restrict__ parts, int nparts, double* __restrict__ moments) {
+    const int m = threadIdx.x;
+    if (m >= ESA_MOMENTS) return;
+    double t = 0.0;
+    for (int c = 0; c < nparts; c++) t += parts[(size_t)c * 128 + m];
+    moments[m] = t;
+}
+
+// esa_fold_kernel: moments -> BatchNorm affine of both calls -> folded first-layer weights, one thread per hidden column
+// c, FP64 throughout:  sc = gamma / sqrt(w_c^T Sigma w_c + eps), sh = beta - (w_c . mu) sc,  A = diag(sc) W  (so
+// BN(f W^T) = f A^T + sh);  Wf = [W0a A1 | W0b A2 | 0 0],  b0f = b0 + W0a sh1 + W0b sh2,  Wp = [A1 | A2 | 0 0] / 2,
+// bp = (sh1 + sh2) / 2  (the mean over machines commutes with the affine: pooled = env_mean Wp^T + bp).
+__global__ void __launch_bounds__(128) esa_fold_kernel(const double* __restrict__ moments, double inv_rows, const float* __restrict__ W1,
+                                                       const float* __restrict__ W2, const float* __restrict__ gamma,
+                                                       const float* __restrict__ beta, float eps, const float* __restrict__ W0,
+                                                       const float* __restrict__ b0, float* __restrict__ Wf, float* __restrict__ Wp,
+                                                       float* __restrict__ bp, float* __restrict__ b0f) {
+    __shared__ double s_m[ESA_MOMENTS];
+    __shared__ double s_A[128][15];
+    __shared__ double s_sh[2][128];
+    const int c = threadIdx.x;
+    if (c < ESA_MOMENTS) s_m[c] = moments[c] * inv_rows;
+    __syncthreads();
+    double sh[2];
+#pragma unroll
+    for (int set = 0; set < 2; set++) {
+        const int K = set ? 8 : 6, off = set ? 6 : 0;
+        const double* S = s_m + (set ? 50 : 14);
+        const float* W = (set ? W2 : W1) + c * K;
+        double mean = 0.0, var = 0.0;
+        for (int i = 0; i < K; i++) {
+            const double wi = W[i];
+            mean += wi * s_m[off + i];
+            for (int j = 0; j < K; j++) var += wi * (double)W[j] * (S[i * K + j] - s_m[off + i] * s_m[off + j]);
+        }
+        const double sc = (double)gamma[c] / sqrt(fmax(var, 0.0) + (double)eps);
+        sh[set] = (double)beta[c] - mean * sc;
+        for (int i = 0; i < K; i++) s_A[c][off + i] = sc * (double)W[i];
+        s_sh[set][c] = sh[set];
+    }
+    for (int k = 0; k < 16; k++) Wp[c * 16 + k] = k < 14 ? (float)(0.5 * s_A[c][k]) : 0.f;
+    bp[c] = (float)(0.5 * (sh[0] + sh[1]));
+    __syncthreads();
+    double acc[14], accb = (double)b0[c];
+#pragma unroll
+    for (int k = 0; k < 14; k++) acc[k] = 0.0;
+    const float* w0 = W0 + (size_t)c * 512;
+    for (int j = 0; j < 128; j++) {
+        const double a = w0[j], b = w0[128 + j];
+#pragma unroll
+        for (int k = 0; k < 6; k++) acc[k] = fma(a, s_A[j][k], acc[k]);
+#pragma unroll
+        for (int k = 6; k < 14; k++) acc[k] = fma(b, s_A[j][k], acc[k]);
+        accb = fma(a, s_sh[0][j], fma(b, s_sh[1][j], accb));
+    }
+    for (int k = 0; k < 16; k++) Wf[c * 16 + k] = k < 14 ? (float)acc[k] : 0.f;
+    b0f[c] = (float)accb;
+}
+
+// esa_head_tf32_kernel: the machine policy head per 128-row tile, both products on tcgen05.mma kind::tf32:
+//   D1 = [f1 | f2 | 0 0] W0f^T (K = 16, W0f = the folded first-layer weights [128,16]) -> TMEM columns 0..127;
+//   epilogue 1: + bias_env[r / M], tanh, into the A buffer of the second product;  D2 = A2 W1^T -> TMEM 128..255;
+//   epilogue 2: + b1, tanh, . w2, + b2, x 10 -> one float per row.
+// The structure of head_tf32_kernel with its first product replaced: the rows are 56 bytes of raw features instead of
+// a gathered 512-byte embedding, so no [R,128] tensor is read or written.
+constexpr int ESA_HEAD_WARPS = 16;
+
+__global__ void __launch_bounds__(ESA_HEAD_WARPS * 32, 1) esa_head_tf32_kernel(
+    const float* __restrict__ f1, const float* __restrict__ f2, long long rows, int M, const float* __restrict__ W0f,
+    const float* __restrict__ bias_env, const float* __restrict__ W1, const float* __restrict__ b1,
+    const float* __restrict__ w2, const float* __restrict__ b2, float* __restrict__ out, long long num_tiles) {
+    extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr size_t WBYTES = (size_t)TILE_N * 128 * 4, SBYTES = (size_t)TILE_M * 16 * 4;
+    float* sW1 = reinterpret_cast<float*>(smem);
+    float* sA2 = reinterpret_cast<float*>(smem + WBYTES);
+    float* sW0 = reinterpret_cast<float*>(smem + 2 * WBYTES);
+    float* sA1 = reinterpret_cast<float*>(smem + 2 * WBYTES + SBYTES);
+    float* s_part = reinterpret_cast<float*>(smem + 2 * WBYTES + 2 * SBYTES);  // [4][128] partial dots of epilogue 2
+    float* s_b1 = s_part + 4 * 128;
+    float* s_w2 = s_b1 + 128;
+    uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_w2 + 128);
+    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(s_bar + 2);
+
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (tid < 128) {
+        s_b1[tid] = b1 ? b1[tid] : 0.f;
+        s_w2[tid] = w2[tid];
+    }
+    if (tid == 0) {
+        mbar_init(smem_u32(s_bar + 0), 1);
+        mbar_init(smem_u32(s_bar + 1), 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(s_tmem)), "r"(256));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    stage_block<false, ESA_HEAD_WARPS>(sW1, W1, 0, TILE_N, 128, 128, 128, nullptr, nullptr, false, warp, lane);
+    stage_block<false, ESA_HEAD_WARPS>(sW0, W0f, 0, TILE_N, 16, 16, 16, nullptr, nullptr, false, warp, lane);
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    const uint32_t tmem_base = *s_tmem;
+    const uint32_t bar0 = smem_u32(s_bar), bar1 = smem_u32(s_bar + 1);
+    const float b2v = b2 ? __ldg(b2) : 0.f;
+
+    // A1 staging: thread -> (tile row tid / 4, 16-byte piece tid % 4 = features 4p .. 4p+3), UMMA K-major layout with
+    // SBO = 512 (8 rows x 4 pieces); features 0..5 from f1, 6..13 from f2, 14..15 zero
+    const int arow = tid >> 2, apiece = tid & 3;
+    char* const a1dst = reinterpret_cast<char*>(sA1) + (arow >> 3) * 512 + apiece * 128 + (arow & 7) * 16;
+    float v[4];
+    auto fetch = [&](long long tile) {
+        const long long r = tile * TILE_M + arow;
+        const bool ok = tile < num_tiles && r < rows;
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const int k = apiece * 4 + j;
+            v[j] = !ok ? 0.f : k < 6 ? __ldg(f1 + r * 6 + k) : k < 14 ? __ldg(f2 + r * 8 + (k - 6)) : 0.f;
+        }
+    };
+    auto mma = [&](const float* sA, const float* sW, int ksteps, uint32_t sbo, uint32_t dcol) {  // one elected thread
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        const uint32_t aA = smem_u32(sA), aW = smem_u32(sW);
+        for (int k = 0; k < ksteps; k++)
+            umma_tf32(tmem_base + dcol, make_desc(aA + k * 256, 128, sbo), make_desc(aW + k * 256, 128, sbo), k > 0 ? 1u : 0u);
+    };
+
+    const int quad = warp & 3, cg = warp >> 2;  // this warp's TMEM lanes 32 quad .., columns 32 cg ..
+    const int trow = quad * 32 + lane;          // its thread's tile row
+    fetch(blockIdx.x);
+    long long i = 0;
+    for (long long tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, i++) {
+        const uint32_t par = (uint32_t)(i & 1);
+        *reinterpret_cast<float4*>(a1dst) = make_float4(to_tf32(v[0]), to_tf32(v[1]), to_tf32(v[2]), to_tf32(v[3]));
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();
+        if (tid == 0) {
+            mma(sA1, sW0, 2, 512, 0);
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar0) : "memory");
+        }
+        fetch(tile + gridDim.x);  // the next tile's features travel while this tile is multiplied
+        mbar_wait(bar0, par);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        const long long grow = tile * TILE_M + trow;
+        const bool rok = grow < rows;
+        {   // first epilogue: + per-env bias, tanh, into A2 as the second product's operand
+            uint32_t r[32];
+            TMEM_LD32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(cg * 32), r);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            const long long brow = rok ? grow / M : 0;
+            const float4* bp = reinterpret_cast<const float4*>(bias_env + brow * 128 + cg * 32);
+            char* dst = reinterpret_cast<char*>(sA2) + (trow >> 3) * 4096 + (cg * 8) * 128 + (trow & 7) * 16;
+#pragma unroll
+            for (int j = 0; j < 8; j++) {
+                const float4 bb = __ldg(bp + j);
+                float4 x;
+                x.x = to_tf32(tanh_fast(__uint_as_float(r[4 * j]) + bb.x)); x.y = to_tf32(tanh_fast(__uint_as_float(r[4 * j + 1]) + bb.y));
+                x.z = to_tf32(tanh_fast(__uint_as_float(r[4 * j + 2]) + bb.z)); x.w = to_tf32(tanh_fast(__uint_as_float(r[4 * j + 3]) + bb.w));
+                if (!rok) x = make_float4(0.f, 0.f, 0.f, 0.f);
+                *reinterpret_cast<float4*>(dst + j * 128) = x;
+            }
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();
+        if (tid == 0) {
+            mma(sA2, sW1, 16, 4096, TILE_N);
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar1) : "memory");
+        }
+        mbar_wait(bar1, par);
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        {   // second epilogue: + b1, tanh, dot with w2 over this warp's 32 columns
+            uint32_t r[32];
+            TMEM_LD32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(TILE_N + cg * 32), r);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            float acc = 0.f;
+#pragma unroll
+            for (int j = 0; j < 8; j++) {
+                const float4 bb = *reinterpret_cast<const float4*>(s_b1 + cg * 32 + 4 * j);
+                const float4 ww = *reinterpret_cast<const float4*>(s_w2 + cg * 32 + 4 * j);
+                acc = fmaf(tanh_fast(__uint_as_float(r[4 * j]) + bb.x), ww.x, acc);
+                acc = fmaf(tanh_fast(__uint_as_float(r[4 * j + 1]) + bb.y), ww.y, acc);
+                acc = fmaf(tanh_fast(__uint_as_float(r[4 * j + 2]) + bb.z), ww.z, acc);
+                acc = fmaf(tanh_fast(__uint_as_float(r[4 * j + 3]) + bb.w), ww.w, acc);
+            }
+            s_part[cg * 128 + trow] = acc;
+        }
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();
+        if (tid < 128) {
+            const long long orow = tile * TILE_M + tid;
+            if (orow < rows) out[orow] = 10.f * (((s_part[tid] + s_part[128 + tid]) + (s_part[256 + tid] + s_part[384 + tid])) + b2v);
+        }
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256));
+}
+
 }  // namespace
 
 template <int KP>
@@ -1636,6 +1893,49 @@ int mtfjsp_enc_bn_finalize(const double* stats, int64_t rows, const float* gamma
     if (!stats || !gamma || !beta || !scale || !shift || rows < 1 || C < 1) return MTFJSP_E_ARG;
     bn_finalize_kernel<<<(C + 127) / 128, 128, 0, (cudaStream_t)stream>>>(stats, 1.0 / (double)rows, gamma, beta, eps, scale,
                                                                         shift, C);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int64_t mtfjsp_enc_esa_mach_stats_workspace_doubles(void) { return (int64_t)ESA_STATS_BLOCKS * 128; }
+
+int mtfjsp_enc_esa_mach_stats(const float* fea1, const float* fea2, int64_t B, int M, double* moments, float* env_mean,
+                              double* workspace, void* stream) {
+    if (!fea1 || !fea2 || !moments || !env_mean || !workspace || B < 1 || M < 1 || M > ESA_STATS_ROWS) return MTFJSP_E_ARG;
+    const int epc = ESA_STATS_ROWS / M;
+    const long long chunks = (B + epc - 1) / epc;
+    const int grid = (int)(chunks < ESA_STATS_BLOCKS ? chunks : ESA_STATS_BLOCKS);
+    esa_stats_kernel<<<grid, ESA_STATS_THREADS, 0, (cudaStream_t)stream>>>(fea1, fea2, B, M, epc, workspace, env_mean);
+    if (cudaGetLastError() != cudaSuccess) return MTFJSP_E_CUDA;
+    esa_stats_reduce_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(workspace, grid, moments);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_esa_mach_fold(const double* moments, int64_t rows, const float* W1, const float* W2, const float* gamma,
+                             const float* beta, float eps, const float* W0, const float* b0, float* Wf, float* Wp, float* bp,
+                             float* b0f, void* stream) {
+    if (!moments || !W1 || !W2 || !gamma || !beta || !W0 || !b0 || !Wf || !Wp || !bp || !b0f || rows < 1) return MTFJSP_E_ARG;
+    esa_fold_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(moments, 1.0 / (double)rows, W1, W2, gamma, beta, eps, W0, b0, Wf, Wp, bp, b0f);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_esa_mach_head_tf32(const float* fea1, const float* fea2, int64_t B, int M, const float* W0f, const float* bias_env,
+                                  const float* W1, const float* b1, const float* w2, const float* b2, float* out, void* stream) {
+    if (!fea1 || !fea2 || !W0f || !bias_env || !W1 || !w2 || !out || B < 1 || M < 1) return MTFJSP_E_ARG;
+    const long long rows = (long long)B * M;
+    const size_t smem = 2 * (size_t)TILE_N * 128 * 4 + 2 * (size_t)TILE_M * 16 * 4 + (4 * 128 + 2 * 128) * 4 + 2 * 8 + 16;
+    static thread_local bool configured = false;
+    if (!configured) {
+        if (cudaFuncSetAttribute(esa_head_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return MTFJSP_E_CUDA;
+        configured = true;
+    }
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long tiles = (rows + TILE_M - 1) / TILE_M;
+    const int grid = (int)(tiles < sms ? tiles : sms);
+    esa_head_tf32_kernel<<<grid, ESA_HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, rows, M, W0f, bias_env, W1, b1, w2, b2,
+                                                                                  out, tiles);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 

@@ -7,6 +7,8 @@ Forward-only mirrors of the reference networks that consume the environment's na
                      (GIN-style encoder model/gcn_mlp.py:109-197, 204-249; MLPActor / MLPCritic :322-434)
     MachineActor  <- model/actor_critic.py:299-498  Machine_Actor_JointAction_selfGAT_selfCritic
                      (GAT layer model/gat.py:68-159 over the fixed 2-node graph [[1,1],[0,1]])
+    EsaJobActor, EsaMachineActor <- model/actor_critic.py:945-1404  esa_Operation_Actor_Critic, esa_Machine_Actor
+                     (the ESA-PPO baseline the reference's test table compares against; inference only)
 
 What runs where (round 1): the neighbour aggregation (reference: dense adj -> COO -> FP64 cuSPARSE SpMM -> second
 SpMM for the degree) is the hand-written `mtfjsp_enc_aggregate` kernel over ELL; graph pooling is
@@ -34,6 +36,7 @@ from ._lib import check
 _FUSED_HEAD = os.environ.get("MTFJSP_FUSED_HEAD", "1") != "0"
 _FUSED_TRUNK = os.environ.get("MTFJSP_FUSED_TRUNK", "1") != "0"  # likewise for the machine-node trunk
 _FUSED_AGG = os.environ.get("MTFJSP_FUSED_AGG", "1") != "0"      # likewise aggregation + first layer of a GIN MLP
+_FUSED_ESA = os.environ.get("MTFJSP_FUSED_ESA", "1") != "0"      # likewise the ESA machine actor (EsaMachineActor)
 
 
 def _ptr(t):
@@ -355,6 +358,24 @@ def machine_actor_keys(hidden=128):
     return k
 
 
+def esa_job_actor_keys(hidden=128, in_dim=12):
+    """state_dict layout of esa_Operation_Actor_Critic (model/actor_critic.py:945-1205): the job actor with a 4-wide
+    critic (read off the shipped tester/ESWA_MPPO/esa_PPO_operation_actor_*.pth)."""
+    H = hidden
+    k = job_actor_keys(hidden, in_dim)
+    k["job_critic.linears.2.weight"] = (4, H); k["job_critic.linears.2.bias"] = (4,)
+    return k
+
+
+def esa_machine_actor_keys(hidden=128):
+    """state_dict layout of esa_Machine_Actor (model/actor_critic.py:1207-1404).  `gat_layer.*` and `fcl_pooling.weight`
+    are in its state_dict but its forward never reads them."""
+    H = hidden
+    k = machine_actor_keys(hidden)
+    k["m_policy.linears.0.weight"] = (H, 4 * H)
+    return k
+
+
 def seeded_state_dict(keys: dict, seed: int):
     """Deterministic weights for parity fixtures: the same call feeds the reference module (in the build container)
     and this module (on the GPU box), so no checkpoint has to be shipped with the tests."""
@@ -659,12 +680,15 @@ def _check_precision(precision, hidden):
 class JobActor(_GraphEncoder, _Twin):
     """Forward of Operation_Actor_JointAction_selfCritic (model/actor_critic.py:104-296) on native observations."""
 
+    n_values = 2  # width of job_v
+    _keys = staticmethod(job_actor_keys)
+
     def __init__(self, state_dict, n_job, n_machine, hidden=128, in_dim=12, device=None, precision="fp32", trainable=False):
         """precision "fp32": library FP32 GEMMs, bit-for-bit the reference's arithmetic types;
         "tf32": the fused tcgen05 layer kernel (hidden must be 128) -- BatchNorm folded into prologue/epilogue."""
         self.J, self.M, self.N, self.H = n_job, n_machine, n_job * n_machine, hidden
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        self.w = _Params(job_actor_keys(hidden, in_dim), state_dict, self.device, trainable)
+        self.w = _Params(self._keys(hidden, in_dim), state_dict, self.device, trainable)
         _check_precision(precision, hidden)
         self.precision = precision
         self._pending = None
@@ -811,6 +835,8 @@ class _MachineTrunk:
 class MachineActor(_MachineTrunk, _Twin):
     """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498)."""
 
+    n_values = 2  # width of machine_v
+
     def __init__(self, state_dict, n_machine, hidden=128, device=None, precision="fp32", trainable=False):
         self.M, self.H = n_machine, hidden
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -841,6 +867,121 @@ class MachineActor(_MachineTrunk, _Twin):
         nodes, pooled = self.trunk(machine_fea_1, machine_fea_2, groups)
         prob, machine_v = self.heads(nodes, pooled, h_pooled_o, machine_mask, return_logits)
         return prob, pooled, machine_v
+
+
+class EsaJobActor(JobActor):
+    """Forward of esa_Operation_Actor_Critic (model/actor_critic.py:945-1205), the ESA-PPO baseline's job actor: the
+    JobActor network with a 4-wide job critic.  Inference only (the reference has no ESA training)."""
+
+    n_values = 4
+    _keys = staticmethod(esa_job_actor_keys)
+
+    def __init__(self, state_dict, n_job, n_machine, hidden=128, in_dim=12, device=None, precision="fp32"):
+        super().__init__(state_dict, n_job, n_machine, hidden, in_dim, device, precision)
+
+
+_ESA_WS = {}
+
+
+class EsaMachineActor(_Twin):
+    """Forward of esa_Machine_Actor (model/actor_critic.py:1207-1404), the ESA-PPO baseline's machine actor.  No GAT:
+        h1 = BN(fea1 W1^T), h2 = BN(fea2 W2^T)    (one BatchNorm module, batch statistics of each call)
+        pooled = (mean_m h1 + mean_m h2) / 2,   scores = 10 m_policy(cat(h1, h2, pooled, h_pooled_o)),
+        machine_v = machine_critic(pooled)
+    precision "fp32": that chain literally on library FP32 GEMMs (per-instance BatchNorm groups work);
+    "tf32": BatchNorm and both projections folded into the first m_policy layer (K = 14 on the raw features), the
+    statistics from the feature moments -- mtfjsp_enc_esa_mach_stats + mtfjsp_enc_esa_mach_fold + mtfjsp_enc_esa_mach_head_tf32,
+    no [B*M,128] intermediate; one BatchNorm group.  MTFJSP_FUSED_ESA=0 runs the tf32 path layer by layer instead."""
+
+    n_values = 2
+
+    def __init__(self, state_dict, n_machine, hidden=128, device=None, precision="fp32"):
+        self.M, self.H = n_machine, hidden
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.w = _Params(esa_machine_actor_keys(hidden), state_dict, self.device)
+        _check_precision(precision, hidden)
+        self.precision = precision
+
+    def forward(self, machine_fea_1, machine_fea_2, h_pooled_o, machine_mask, groups=1, return_logits=False):
+        """machine_fea_1 [B,M,6], machine_fea_2 [B,M,8], h_pooled_o [B,H], machine_mask [B,M] (1 = infeasible)
+        -> mch_prob [B,M] (the x10 scores with return_logits), h_pooled [B,H], machine_v [B,2]."""
+        w = self.w
+        B = machine_fea_1.shape[0]
+        f1 = machine_fea_1.to(torch.float32).reshape(B * self.M, 6).contiguous()
+        f2 = machine_fea_2.to(torch.float32).reshape(B * self.M, 8).contiguous()
+        if self.precision == "tf32":
+            if groups != 1:
+                raise ValueError("the tf32 ESA machine actor is the rollout path: one BatchNorm group")
+            s, pooled = (self._scores_fused if _FUSED_ESA else self._scores_layers)(f1, f2, h_pooled_o.contiguous(), B)
+            machine_v = _mlp3_tanh_tf32(w, "machine_critic.", pooled)
+        else:
+            s, pooled = self._scores_fp32(f1, f2, h_pooled_o, B, groups)
+            machine_v = _mlp3_tanh(w, "machine_critic.", pooled)
+        if return_logits:
+            return s, pooled, machine_v
+        s = s.masked_fill(machine_mask.reshape(B, self.M).bool(), float("-inf"))     # actor_critic.py:1383-1388
+        return F.softmax(s, dim=-1), pooled, machine_v
+
+    def _scores_fp32(self, f1, f2, h_pooled_o, B, groups):
+        w, M, H = self.w, self.M, self.H
+        h1 = _bn_train(F.linear(f1, w["m_fea_1_fcl.weight"]), w["bn.weight"], w["bn.bias"], groups=groups).reshape(B, M, H)
+        h2 = _bn_train(F.linear(f2, w["m_fea_2_fcl.weight"]), w["bn.weight"], w["bn.bias"], groups=groups).reshape(B, M, H)
+        pooled = (h1.mean(dim=1) + h2.mean(dim=1)) / 2                                  # actor_critic.py:1354-1356
+        x = torch.cat((h1, h2, pooled.unsqueeze(1).expand_as(h1), h_pooled_o.unsqueeze(1).expand_as(h1)), dim=-1)
+        return _mlp3_tanh(w, "m_policy.", x).squeeze(-1) * 10, pooled
+
+    def _env_bias(self, pooled, h_pooled_o, b0):
+        """b0 + W0c pooled + W0d h_pooled_o [B,128]: the per-env column blocks of the first m_policy layer."""
+        w, H = self.w, self.H
+        W0 = w["m_policy.linears.0.weight"]
+        Wc = self._derived("esa_W0c", lambda: W0[:, 2 * H:3 * H])
+        Wd = self._derived("esa_W0d", lambda: W0[:, 3 * H:])
+        return linear_tf32(pooled, Wc, b0) + linear_tf32(h_pooled_o, Wd, None)
+
+    def _scores_fused(self, f1, f2, h_pooled_o, B):
+        w, M = self.w, self.M
+        lib = _lib.lib()
+        dev = f1.device
+        if dev.index not in _ESA_WS:
+            _ESA_WS[dev.index] = torch.empty(int(lib.mtfjsp_enc_esa_mach_stats_workspace_doubles()), dtype=torch.float64, device=dev)
+        moments = torch.empty(114, dtype=torch.float64, device=dev)
+        env_mean = torch.empty((B, 16), dtype=torch.float32, device=dev)
+        check(lib.mtfjsp_enc_esa_mach_stats(_ptr(f1), _ptr(f2), B, M, _ptr(moments), _ptr(env_mean), _ptr(_ESA_WS[dev.index]),
+                                            _stream()), "mtfjsp_enc_esa_mach_stats")
+        Wf = torch.empty((128, 16), dtype=torch.float32, device=dev)
+        Wp = torch.empty_like(Wf)
+        bp = torch.empty(128, dtype=torch.float32, device=dev)
+        b0f = torch.empty_like(bp)
+        check(lib.mtfjsp_enc_esa_mach_fold(_ptr(moments), B * M, _ptr(w["m_fea_1_fcl.weight"]), _ptr(w["m_fea_2_fcl.weight"]),
+                                           _ptr(w["bn.weight"]), _ptr(w["bn.bias"]), 1e-5, _ptr(w["m_policy.linears.0.weight"]),
+                                           _ptr(w["m_policy.linears.0.bias"]), _ptr(Wf), _ptr(Wp), _ptr(bp), _ptr(b0f), _stream()),
+              "mtfjsp_enc_esa_mach_fold")
+        pooled = linear_tf32(env_mean, Wp, bp)
+        bias = self._env_bias(pooled, h_pooled_o, b0f)
+        w2 = self._derived("esa_w2", lambda: w["m_policy.linears.2.weight"].reshape(-1))
+        s = torch.empty((B, M), dtype=torch.float32, device=dev)
+        check(lib.mtfjsp_enc_esa_mach_head_tf32(_ptr(f1), _ptr(f2), B, M, _ptr(Wf), _ptr(bias), _ptr(w["m_policy.linears.1.weight"]),
+                                                _ptr(w["m_policy.linears.1.bias"]), _ptr(w2), _ptr(w["m_policy.linears.2.bias"]),
+                                                _ptr(s), _stream()), "mtfjsp_enc_esa_mach_head_tf32")
+        return s, pooled
+
+    def _scores_layers(self, f1, f2, h_pooled_o, B):
+        """The tf32 path one layer per launch (A/B reference for the fused form): both projections and BatchNorms
+        materialised, the first m_policy layer's per-row block split in two products."""
+        w, M, H = self.w, self.M, self.H
+        W1p = self._derived("esa_W1p", lambda: F.pad(w["m_fea_1_fcl.weight"], (0, 2)))  # K = 8: the kernel takes K % 4 == 0
+        h1 = _bn_train(linear_tf32(F.pad(f1, (0, 2)), W1p, None), w["bn.weight"], w["bn.bias"])
+        h2 = _bn_train(linear_tf32(f2, w["m_fea_2_fcl.weight"], None), w["bn.weight"], w["bn.bias"])
+        pooled = (_graph_mean_raw(h1.view(B, M, H)) + _graph_mean_raw(h2.view(B, M, H))) / 2
+        W0 = w["m_policy.linears.0.weight"]
+        Wa = self._derived("esa_W0a", lambda: W0[:, :H])
+        Wb = self._derived("esa_W0b", lambda: W0[:, H:2 * H])
+        bias = self._env_bias(pooled, h_pooled_o, w["m_policy.linears.0.bias"])
+        z = linear_tf32(h1, Wa, None) + linear_tf32(h2, Wb, None)
+        bias_tanh_(z, bias, M)
+        z = linear_tf32(z, w["m_policy.linears.1.weight"], w["m_policy.linears.1.bias"])
+        w2 = self._derived("esa_w2", lambda: w["m_policy.linears.2.weight"].reshape(-1))
+        return tanh_dot(z, w2, w["m_policy.linears.2.bias"]).view(B, M) * 10, pooled
 
 
 def global_critic_keys(hidden=128, in_dim=12):

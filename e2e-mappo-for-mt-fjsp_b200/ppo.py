@@ -369,6 +369,9 @@ def collect(rollout, weights_per_episode):
     env = rollout.env
     N = env.N
     job, mch = rollout.job, rollout.mch
+    if isinstance(job, _enc.EsaJobActor) or isinstance(mch, _enc.EsaMachineActor):
+        raise TypeError("the ESA-PPO actors are an evaluation baseline (the reference never trains them): roll them out "
+                        "with rollout.Rollout / validate.greedy_validate, not into a PPO buffer")
     buf = RolloutBuffer(len(weights_per_episode), env)
     for w in weights_per_episode:
         rollout.begin_episode(w)

@@ -40,8 +40,8 @@ class Rollout:
         # per-step outputs kept for the PPO buffers
         self.log_a = torch.zeros(B, device=dev)
         self.m_log_a = torch.zeros(B, device=dev)
-        self.job_v = torch.zeros((B, 2), device=dev)
-        self.mch_v = torch.zeros((B, 2), device=dev)
+        self.job_v = torch.zeros((B, getattr(job_actor, "n_values", 2)), device=dev)   # 4 for the ESA job actor
+        self.mch_v = torch.zeros((B, getattr(machine_actor, "n_values", 2)), device=dev)
         self.use_graph = use_cuda_graph
         self._graph = None
         self._warm = 0

@@ -283,6 +283,31 @@ int mtfjsp_enc_aggregate_linear_tf32(const float* X, int64_t B, int N, const flo
 int mtfjsp_enc_wgrad_tf32(const float* dY, const float* X, int64_t rows, int K, float* dW, float* db, float* workspace,
                           void* stream);
 int64_t mtfjsp_enc_wgrad_workspace_floats(int K);
+/* ESA machine actor (model/actor_critic.py:1207-1404 esa_Machine_Actor), hidden = 128, in two launches with no [R,128]
+ * intermediate; fea1 [B*M,6], fea2 [B*M,8] f32, M rows per env.
+ * mtfjsp_enc_esa_mach_stats: the moments the two BatchNorm calls of the actor need, from the raw features:
+ *   moments [114] f64 = column sums of [fea1 | fea2] (14), sum of fea1 fea1^T (6x6 row-major), sum of fea2 fea2^T (8x8);
+ *   env_mean [B,16] f32 = per-env mean of [fea1 | fea2] rows, columns 14, 15 zero.
+ * Per-CTA FP64 partials in `workspace` (mtfjsp_enc_esa_mach_stats_workspace_doubles() doubles) added in CTA order:
+ * run-to-run deterministic.  M <= 256.  Replaces the two [R,128] projections and the BatchNorm statistics passes.
+ * mtfjsp_enc_esa_mach_fold: one thread per hidden column, FP64: the BatchNorm affine of both calls (biased variance
+ * w_c^T Sigma w_c clamped at 0, eps) from moments over `rows` rows, W1 [128,6] / W2 [128,8] the input projections,
+ * W0 [128,512] / b0 the first m_policy layer ->  Wf [128,16] = [W0a diag(sc1) W1 | W0b diag(sc2) W2 | 0 0],
+ * b0f [128] = b0 + W0a sh1 + W0b sh2,  Wp [128,16] = [diag(sc1) W1 | diag(sc2) W2 | 0 0] / 2,  bp = (sh1 + sh2) / 2,
+ * so that pooled = env_mean Wp^T + bp (the mean over machines of (h1 + h2) / 2).
+ * mtfjsp_enc_esa_mach_head_tf32: the machine policy head, one launch, both products on tcgen05.mma kind::tf32:
+ *   out[r] = 10 ( tanh( tanh( [fea1 | fea2 | 0 0][r] W0f^T + bias_env[r / M] ) W1^T + b1 ) . w2 + b2 )
+ * W0f [128,16] = the first layer's h1 / h2 column blocks with the BatchNorm scales and both projections folded in,
+ * bias_env [B,128] = its bias, the BatchNorm shifts and the pooled / h_pooled_o blocks applied per env; b1 / b2 may be
+ * NULL.  Replaces 2 x linear + 2 x BatchNorm + concat + linear + tanh + linear + tanh + linear of the reference. */
+int mtfjsp_enc_esa_mach_stats(const float* fea1, const float* fea2, int64_t B, int M, double* moments, float* env_mean,
+                              double* workspace, void* stream);
+int64_t mtfjsp_enc_esa_mach_stats_workspace_doubles(void);
+int mtfjsp_enc_esa_mach_fold(const double* moments, int64_t rows, const float* W1, const float* W2, const float* gamma,
+                             const float* beta, float eps, const float* W0, const float* b0, float* Wf, float* Wp, float* bp,
+                             float* b0f, void* stream);
+int mtfjsp_enc_esa_mach_head_tf32(const float* fea1, const float* fea2, int64_t B, int M, const float* W0f, const float* bias_env,
+                                  const float* W1, const float* b1, const float* w2, const float* b2, float* out, void* stream);
 /* BatchNorm1d with batch statistics as a per-column affine: scale = gamma/sqrt(var+eps), shift = beta - mean*scale. */
 int mtfjsp_enc_bn_finalize(const double* stats, int64_t rows, const float* gamma, const float* beta, float eps,
                            float* scale, float* shift, int C, void* stream);
