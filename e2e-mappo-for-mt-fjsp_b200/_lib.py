@@ -101,6 +101,12 @@ SIGNATURES = {
     "mtfjsp_enc_esa_mach_fold": ([_VP, C.c_int64, _VP, _VP, _VP, _VP, C.c_float] + [_VP] * 7, _I),
     "mtfjsp_enc_esa_mach_head_tf32": ([_VP, _VP, C.c_int64, _I] + [_VP] * 8, _I),
     "mtfjsp_enc_bn_finalize": ([_VP, C.c_int64, _VP, _VP, C.c_float, _VP, _VP, _I, _VP], _I),
+    "mtfjsp_enc_linear_tf32_grouped": ([_VP, C.c_int64, _I, _I, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP, _VP], _I),
+    "mtfjsp_enc_aggregate_linear_tf32_grouped": ([_VP, C.c_int64, _I] + [_VP] * 6 + [_I, _I, _VP, _VP, _VP], _I),
+    "mtfjsp_enc_aggregate_grouped": ([_VP, _VP, _VP, _VP, C.c_int64, _I, _I, _VP, _VP, _I, _I, _VP], _I),
+    "mtfjsp_enc_graph_mean_grouped": ([_VP, _VP, C.c_int64, _I, _I, _VP, _VP, _I, _I, _VP], _I),
+    "mtfjsp_enc_head_tf32_grouped": ([_VP, _VP, C.c_int64, _I, _I, _VP, _VP, _I, _I, _VP, _VP, C.c_int64] + [_VP] * 6, _I),
+    "mtfjsp_enc_bn_finalize_grouped": ([_VP, C.c_int64, _I, _I, _VP, _VP, C.c_float, _VP, _VP, _I, _VP], _I),
     "mtfjsp_gae4": ([_VP, _VP, _VP, _VP, _VP, _VP, _I, C.c_int64, C.c_float, C.c_float, _VP], _I),
     "mtfjsp_adv_normalize": ([_VP, _VP, C.c_double, _I, C.c_int64, _VP], _I),
     "mtfjsp_launch_overlap_error": ([_VP], _I),

@@ -20,11 +20,14 @@
 namespace {
 
 // one thread per (row, 4 channels): out[row] = (h[row] + wj*h[row-1] + wm*h[src]) / deg
+// GROUPED: in_scale / in_shift [G,C], the affine of group (env0 + row / N) / epg
+template <bool GROUPED>
 __global__ void __launch_bounds__(256) aggregate_kernel(const float4* __restrict__ h, const float2* __restrict__ adj_w,
                                                         const int16_t* __restrict__ adj_src, float4* __restrict__ out,
                                                         unsigned total, int N, int C4, int c4_shift,
                                                         const float4* __restrict__ in_scale,
-                                                        const float4* __restrict__ in_shift, int in_relu) {
+                                                        const float4* __restrict__ in_shift, int in_relu, long long env0 = 0,
+                                                        int epg = 1) {
     const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;  // one thread per (row, 4 channels); total < 2^31
     if (idx >= total) return;
     const unsigned row = c4_shift >= 0 ? idx >> c4_shift : idx / (unsigned)C4;
@@ -39,7 +42,8 @@ __global__ void __launch_bounds__(256) aggregate_kernel(const float4* __restrict
     float4 xj = hj ? __ldg(h + (idx - (unsigned)C4)) : z4;
     float4 xm = hm ? __ldg(h + ((size_t)(row - v + (unsigned)src) * C4 + c)) : z4;
     if (in_scale) {  // BatchNorm (+ReLU) of the producing layer, folded into the gather
-        const float4 sc = __ldg(in_scale + c), sh = __ldg(in_shift + c);
+        const size_t ga = GROUPED ? (size_t)((env0 + row / (unsigned)N) / epg) * C4 + c : c;
+        const float4 sc = __ldg(in_scale + ga), sh = __ldg(in_shift + ga);
         auto bn = [&](float4& x) {
             x.x = fmaf(x.x, sc.x, sh.x); x.y = fmaf(x.y, sc.y, sh.y); x.z = fmaf(x.z, sc.z, sh.z); x.w = fmaf(x.w, sc.w, sh.w);
             if (in_relu) { x.x = fmaxf(x.x, 0.f); x.y = fmaxf(x.y, 0.f); x.z = fmaxf(x.z, 0.f); x.w = fmaxf(x.w, 0.f); }
@@ -110,13 +114,16 @@ __global__ void __launch_bounds__(256) aggregate_bwd_kernel(const float4* __rest
 }
 
 // per-env mean over the N node rows (graph_pool average): one block per env, thread per channel
+// GROUPED: in_scale / in_shift [G,C], the affine of group b / epg
+template <bool GROUPED>
 __global__ void graph_mean_kernel(const float* __restrict__ h, float* __restrict__ out, int N, int C,
-                                  const float* __restrict__ in_scale, const float* __restrict__ in_shift, int in_relu) {
+                                  const float* __restrict__ in_scale, const float* __restrict__ in_shift, int in_relu, int epg = 1) {
     const long long b = blockIdx.x;
     const float inv = 1.0f / (float)N;  // the reference multiplies each row by the float32 value 1/N and sums
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
         float acc = 0.f;
-        const float sc = in_scale ? in_scale[c] : 1.f, sh = in_scale ? in_shift[c] : 0.f;
+        const long long ga = GROUPED ? (b / epg) * C + c : c;
+        const float sc = in_scale ? in_scale[ga] : 1.f, sh = in_scale ? in_shift[ga] : 0.f;
         for (int v = 0; v < N; v++) {
             float x = h[(b * N + v) * C + c];
             if (in_scale) { x = x * sc + sh; if (in_relu) x = fmaxf(x, 0.f); }
@@ -558,7 +565,7 @@ int mtfjsp_enc_aggregate(const float* h, const float* adj_w, const int16_t* adj_
         const long long nb = B - b0 < chunk ? B - b0 : chunk;
         const unsigned total = (unsigned)(nb * per_env);
         const long long r0 = b0 * N;
-        aggregate_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
+        aggregate_kernel<false><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
             reinterpret_cast<const float4*>(h) + r0 * C4, reinterpret_cast<const float2*>(adj_w) + r0, adj_src + r0,
             reinterpret_cast<float4*>(out) + r0 * C4, total, N, C4, c4_shift, reinterpret_cast<const float4*>(in_scale),
             reinterpret_cast<const float4*>(in_shift), in_relu);
@@ -634,8 +641,41 @@ int mtfjsp_enc_graph_mean(const float* h, float* out, int64_t B, int N, int C, c
                           const float* in_shift, int in_relu, void* stream) {
     if (!h || !out || B < 1 || N < 1 || C < 1) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    graph_mean_kernel<<<(unsigned)B, C < 128 ? 32 * ((C + 31) / 32) : 128, 0, (cudaStream_t)stream>>>(h, out, N, C, in_scale,
+    graph_mean_kernel<false><<<(unsigned)B, C < 128 ? 32 * ((C + 31) / 32) : 128, 0, (cudaStream_t)stream>>>(h, out, N, C, in_scale,
                                                                                                    in_shift, in_relu);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_aggregate_grouped(const float* h, const float* adj_w, const int16_t* adj_src, float* out, int64_t B, int N, int C,
+                                 const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, void* stream) {
+    if (!h || !adj_w || !adj_src || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
+    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
+    const int C4 = C / 4;
+    int c4_shift = -1;
+    for (int k = 0; k < 16; k++)
+        if ((1 << k) == C4) c4_shift = k;
+    const long long per_env = (long long)N * C4;
+    const long long chunk = (long long)0x7fffff00 / per_env;
+    if (chunk < 1) return MTFJSP_E_ARG;
+    for (long long b0 = 0; b0 < B; b0 += chunk) {
+        const long long nb = B - b0 < chunk ? B - b0 : chunk;
+        const unsigned total = (unsigned)(nb * per_env);
+        const long long r0 = b0 * N;
+        aggregate_kernel<true><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
+            reinterpret_cast<const float4*>(h) + r0 * C4, reinterpret_cast<const float2*>(adj_w) + r0, adj_src + r0,
+            reinterpret_cast<float4*>(out) + r0 * C4, total, N, C4, c4_shift, reinterpret_cast<const float4*>(in_scale),
+            reinterpret_cast<const float4*>(in_shift), in_relu, b0, envs_per_group);
+    }
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_graph_mean_grouped(const float* h, float* out, int64_t B, int N, int C, const float* in_scale, const float* in_shift,
+                                  int in_relu, int envs_per_group, void* stream) {
+    if (!h || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 1) return MTFJSP_E_ARG;
+    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
+    graph_mean_kernel<true><<<(unsigned)B, C < 128 ? 32 * ((C + 31) / 32) : 128, 0, (cudaStream_t)stream>>>(h, out, N, C, in_scale,
+                                                                                                         in_shift, in_relu,
+                                                                                                         envs_per_group);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 

@@ -190,6 +190,41 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 
+// Grouped form (per-env BatchNorm statistics, mtfjsp.h "grouped encoder layers"): tiles are env-aligned.  With N <= 128
+// rows per env a tile is rpt = (128 / N) * N rows of whole envs; with N > 128 an env is P = ceil(N / 128) tiles of
+// 128 rows starting at its first row (the last piece owns N - 128 (P - 1) of them).
+__device__ __forceinline__ long long gtile_row0(long long tile, int rpt, int nodes, int P) {
+    return P == 1 ? tile * rpt : (tile / P) * nodes + (tile % P) * 128;
+}
+__device__ __forceinline__ int gtile_rows(long long tile, long long row0, long long rows, int rpt, int nodes, int P) {
+    if (P > 1) return nodes - (int)(tile % P) * 128 < 128 ? nodes - (int)(tile % P) * 128 : 128;
+    return rows - row0 < rpt ? (int)(rows - row0) : rpt;
+}
+// env_stats[env][piece][0|1][c] = column sums of Z and Z^2 over the env rows of one tile, read back from Z (L2) after the
+// epilogue warps stored the tile (bar.sync 3 before the call).  One thread per (env, column) adds the rows in row order
+// in FP64, so the sums depend only on the env's own rows, never on where the env sits in the tile or the batch.
+__device__ __forceinline__ void env_stats_tile(const float* Z, double* __restrict__ env_stats, long long tile, long long row0,
+                                               int nrows, int nodes, int P, int tid) {
+    const int prow = P == 1 ? nodes : nrows;
+    const int nenv = P == 1 ? nrows / nodes : 1;
+    const long long env0 = P == 1 ? row0 / nodes : tile / P;
+    const int piece = P == 1 ? 0 : (int)(tile % P);
+    for (int item = tid; item < nenv * 128; item += NEPI * 32) {
+        const int e = item >> 7, c = item & 127;
+        const float* zp = Z + (row0 + (long long)e * nodes) * 128 + c;
+        double s = 0.0, q = 0.0;
+#pragma unroll 4
+        for (int j = 0; j < prow; j++) {
+            const double v = (double)__ldcg(zp + (long long)j * 128);
+            s += v;
+            q = fma(v, v, q);
+        }
+        double* dst = env_stats + ((env0 + e) * P + piece) * 256 + c;
+        dst[0] = s;
+        dst[128] = q;
+    }
+}
+
 // Warp-specialised.  The A operand streams through a ring of NSTAGE shared-memory stages of 128 rows x KS columns
 // (KS = min(K, 64): a K=128 tile is two stages), NSTAGE-1 of them in flight from HBM while one is transformed and
 // multiplied; the accumulator is double-buffered in TMEM so the epilogue warps drain tile i while tile i+1 is formed.
@@ -198,14 +233,17 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 //   tmem_empty[b] (count 8)  the eight epilogue warps have pulled TMEM[b] into registers
 constexpr int NSTAGE = 4;
 
-template <int KP>
+// GROUPED: env-aligned tiles and per-env statistics (env_stats_tile) in `stats` instead of the batch-wide atomics; no
+// input affine (the grouped K <= 16 first layer has none).
+template <int KP, bool GROUPED>
 __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const float* __restrict__ X, long long rows, int K,
                                                                          const float* __restrict__ W,
                                                                          const float* __restrict__ bias,
                                                                          const float* __restrict__ in_scale,
                                                                          const float* __restrict__ in_shift, int in_relu,
                                                                          float* __restrict__ Z, double* __restrict__ stats,
-                                                                         long long num_tiles, int raw_a) {
+                                                                         long long num_tiles, int raw_a, int g_rpt = 0,
+                                                                         int g_nodes = 0, int g_P = 0) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr int KS = KP > 64 ? 64 : KP, SPT = KP / KS;  // stage width, stages per tile
     constexpr size_t WBYTES = (size_t)TILE_N * KP * 4, SBYTES = (size_t)TILE_M * KS * 4;
@@ -256,7 +294,8 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
         auto issue = [&](long long g) {        // every thread commits one group per stage, empty past the end
             if (g < nst) {
                 const long long tile = blockIdx.x + (g / SPT) * (long long)gridDim.x;
-                tile_issue<KS>(reinterpret_cast<float*>(sRing + (g % NSTAGE) * SBYTES), X, tile * TILE_M, rows, K,
+                tile_issue<KS>(reinterpret_cast<float*>(sRing + (g % NSTAGE) * SBYTES), X,
+                               GROUPED ? gtile_row0(tile, g_rpt, g_nodes, g_P) : tile * TILE_M, rows, K,
                                (int)(g % SPT) * KS, pw, lane);
             }
             asm volatile("cp.async.commit_group;" ::: "memory");
@@ -267,7 +306,7 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
             const int h = (int)(g % SPT), slot = (int)(g % NSTAGE), buf = (int)(i & 1);
             float* sA = reinterpret_cast<float*>(sRing + slot * SBYTES);
             asm volatile("cp.async.wait_group %0;" ::"n"(NSTAGE - 2) : "memory");  // stage g has landed (this thread's pieces)
-            if (affine) tile_transform<KS, true>(sA, tile * TILE_M, rows, K, h * KS, s_scale, s_shift, in_relu != 0, pw, lane);
+            if (!GROUPED && affine) tile_transform<KS, true>(sA, tile * TILE_M, rows, K, h * KS, s_scale, s_shift, in_relu != 0, pw, lane);
             else if (!raw_a) tile_transform<KS, false>(sA, tile * TILE_M, rows, K, h * KS, nullptr, nullptr, false, pw, lane);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the MMA
             // refill the slot stage g-1 used: its MMAs ran while this stage was being transformed
@@ -309,7 +348,10 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
             const int buf = (int)(i & 1);
             mbar_wait(bar_full + buf * 8, (uint32_t)((i >> 1) & 1));
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const long long row0 = tile * TILE_M + quad * 32;
+            const long long trow0 = GROUPED ? gtile_row0(tile, g_rpt, g_nodes, g_P) : tile * TILE_M;
+            const int tnrows = GROUPED ? gtile_rows(tile, trow0, rows, g_rpt, g_nodes, g_P) : 0;
+            const long long rend = GROUPED ? trow0 + tnrows : rows;  // rows past rend belong to another tile (or none)
+            const long long row0 = trow0 + quad * 32;
 #pragma unroll
             for (int c2 = 0; c2 < 2; c2++) {
                 const int cc = half * 2 + c2;
@@ -329,24 +371,32 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
                 const float4 bb = c2 == 0 ? b0 : b1;
                 float* zp = Z + (row0 + sub) * TILE_N + cc * 32 + c4 * 4;
                 float4 s = make_float4(0.f, 0.f, 0.f, 0.f), q = make_float4(0.f, 0.f, 0.f, 0.f);
-                const bool full = row0 + 32 <= rows;
+                const bool full = row0 + 32 <= rend;
 #pragma unroll
                 for (int it = 0; it < 8; it++) {
                     const int rr = it * 4 + sub;
                     float4 v = *reinterpret_cast<const float4*>(stg + rr * STG_W + ((c4 ^ (rr & 7)) << 2));
                     v.x += bb.x; v.y += bb.y; v.z += bb.z; v.w += bb.w;
-                    if (full || row0 + rr < rows) {
+                    if (full || row0 + rr < rend) {
                         *reinterpret_cast<float4*>(zp + (size_t)it * 4 * TILE_N) = v;
-                        s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-                        q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                        if (!GROUPED) {
+                            s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+                            q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                        }
                     }
                 }
-                csum[c2][0] += (double)s.x; csum[c2][1] += (double)s.y; csum[c2][2] += (double)s.z; csum[c2][3] += (double)s.w;
-                csq[c2][0] += (double)q.x; csq[c2][1] += (double)q.y; csq[c2][2] += (double)q.z; csq[c2][3] += (double)q.w;
+                if (!GROUPED) {
+                    csum[c2][0] += (double)s.x; csum[c2][1] += (double)s.y; csum[c2][2] += (double)s.z; csum[c2][3] += (double)s.w;
+                    csq[c2][0] += (double)q.x; csq[c2][1] += (double)q.y; csq[c2][2] += (double)q.z; csq[c2][3] += (double)q.w;
+                }
                 __syncwarp();
             }
+            if (GROUPED) {
+                asm volatile("bar.sync 3, %0;" ::"n"(NEPI * 32) : "memory");  // the tile's rows are stored
+                env_stats_tile(Z, stats, tile, trow0, tnrows, g_nodes, g_P, tid);
+            }
         }
-        if (stats) {  // fold the four row classes, then one atomic per column and warp
+        if (!GROUPED && stats) {  // fold the four row classes, then one atomic per column and warp
 #pragma unroll
             for (int c2 = 0; c2 < 2; c2++)
 #pragma unroll
@@ -390,9 +440,12 @@ __device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap
                  : "memory");
 }
 
-template <bool AFFINE>
+// GROUPED: the affine is per BatchNorm group, g_scale / g_shift [G,128] in global memory, group = (row / nodes) / epg
+template <bool AFFINE, bool GROUPED = false>
 __device__ __forceinline__ void tile_transform_sw(unsigned char* stage, long long row0, long long rows, int kbase,
-                                                  const float* s_scale, const float* s_shift, bool relu, int pw, int lane) {
+                                                  const float* s_scale, const float* s_shift, bool relu, int pw, int lane,
+                                                  const float* g_scale = nullptr, const float* g_shift = nullptr,
+                                                  int nodes = 1, int epg = 1) {
     // stage = two boxes of 128 rows x 128 bytes; this thread owns logical 16-byte piece (q * 4 + c) of rows 8 * grp + r
     const int r = lane & 7, c = lane >> 3, q = pw & 3;
     const int piece = q * 4 + c, box = piece >> 3, pb = piece & 7;
@@ -409,6 +462,11 @@ __device__ __forceinline__ void tile_transform_sw(unsigned char* stage, long lon
         float4 v = x[u];
         if (AFFINE) {
             if (row0 + grp * 8 + r < rows) {
+                if (GROUPED) {
+                    const long long g = (row0 + grp * 8 + r) / nodes / epg;
+                    sc = __ldg(reinterpret_cast<const float4*>(g_scale + g * 128 + k));
+                    sh = __ldg(reinterpret_cast<const float4*>(g_shift + g * 128 + k));
+                }
                 v.x = v.x * sc.x + sh.x; v.y = v.y * sc.y + sh.y; v.z = v.z * sc.z + sh.z; v.w = v.w * sc.w + sh.w;
                 if (relu) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
             }
@@ -424,7 +482,9 @@ __device__ __forceinline__ void tile_transform_sw(unsigned char* stage, long lon
 // through shared memory anyway -- out[r] = (y[r] + w_job y[r-1] + w_mach y[src]) / n + bias, y = act(X) W^T.  Tiles hold
 // whole envs (rpt = (128 / N) * N rows; the TMA box is rpt rows, the rest of the stage is ignored) so that every
 // neighbour is in the tile; the separate aggregation pass (one read and one write of [rows,128]) disappears.
-template <bool AGG>
+// GROUPED: env-aligned tiles (rpt rows of whole envs, or 128-row pieces of an env when nodes > 128: g_P pieces), the
+// input affine per BatchNorm group ([G,128], envs_per_group = g_epg) and per-env statistics (env_stats_tile) in `stats`.
+template <bool AGG, bool GROUPED>
 __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(const __grid_constant__ CUtensorMap tmapX, long long rows,
                                                                              const float* __restrict__ W,
                                                                              const float* __restrict__ bias,
@@ -433,7 +493,8 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
                                                                              float* __restrict__ Z, double* __restrict__ stats,
                                                                              long long num_tiles, int rpt, int nodes,
                                                                              const float2* __restrict__ adj_w,
-                                                                             const int16_t* __restrict__ adj_src) {
+                                                                             const int16_t* __restrict__ adj_src, int g_P = 1,
+                                                                             int g_epg = 1) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr int KP = 128, KS = 64, SPT = 2;
     constexpr int NST = AGG ? 3 : NSTAGE;  // the full-tile epilogue buffer of AGG takes one stage's room
@@ -449,7 +510,7 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(s_bar + 4 + 2 * NST);
     float2* s_adjw = reinterpret_cast<float2*>(s_tmem + 4);        // AGG: [128] (w_job, w_mach) of the tile's rows
     int16_t* s_adjs = reinterpret_cast<int16_t*>(s_adjw + 128);    //      [128] tile row of the machine predecessor, -1 = none
-    const int tile_rows = AGG ? rpt : TILE_M;
+    const int tile_rows = (AGG || GROUPED) ? rpt : TILE_M;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const bool affine = in_scale != nullptr;
@@ -492,7 +553,8 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
                 const int slot = (int)(g % NST);
                 const uint32_t dst = smem_u32(sRing + slot * SBYTES), bar = bar_land + slot * 8;
                 asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t)(tile_rows * 256)) : "memory");
-                const int col = (int)(g % SPT) * KS, row = (int)(tile * tile_rows);
+                const int col = (int)(g % SPT) * KS;
+                const int row = (int)(GROUPED ? gtile_row0(tile, rpt, nodes, g_P) : tile * tile_rows);
                 tma_load_2d(dst, &tmapX, col, row, bar);
                 tma_load_2d(dst + 16384, &tmapX, col + 32, row, bar);
             }
@@ -505,8 +567,10 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
             const int h = (int)(g % SPT), slot = (int)(g % NST), buf = (int)(i & 1);
             unsigned char* sA = sRing + slot * SBYTES;
             mbar_wait(bar_land + slot * 8, (uint32_t)((g / NST) & 1));  // stage g has landed
-            if (affine) tile_transform_sw<true>(sA, tile * tile_rows, rows, h * KS, s_scale, s_shift, in_relu != 0, pw, lane);
-            else tile_transform_sw<false>(sA, tile * tile_rows, rows, h * KS, nullptr, nullptr, false, pw, lane);
+            const long long arow0 = GROUPED ? gtile_row0(tile, rpt, nodes, g_P) : tile * tile_rows;
+            if (affine) tile_transform_sw<true, GROUPED>(sA, arow0, rows, h * KS, s_scale, s_shift, in_relu != 0, pw, lane, in_scale,
+                                                         in_shift, nodes, g_epg);
+            else tile_transform_sw<false>(sA, arow0, rows, h * KS, nullptr, nullptr, false, pw, lane);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the MMA
             if (loader) {  // refill the slot stage g-1 used: its MMAs ran while this stage was being transformed
                 if (g >= 1 && g + NST - 1 < nst)
@@ -617,18 +681,29 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
                         v.x += bb.x; v.y += bb.y; v.z += bb.z; v.w += bb.w;
                         if (prow[it] & (1 << 17)) {
                             *reinterpret_cast<float4*>(Z + (tile * rpt + tr2) * TILE_N + piece * 4) = v;
-                            s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-                            q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                            if (!GROUPED) {
+                                s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+                                q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                            }
                         }
                     }
-                    csum[c2][0] += (Acc)s.x; csum[c2][1] += (Acc)s.y; csum[c2][2] += (Acc)s.z; csum[c2][3] += (Acc)s.w;
-                    csq[c2][0] += (Acc)q.x; csq[c2][1] += (Acc)q.y; csq[c2][2] += (Acc)q.z; csq[c2][3] += (Acc)q.w;
+                    if (!GROUPED) {
+                        csum[c2][0] += (Acc)s.x; csum[c2][1] += (Acc)s.y; csum[c2][2] += (Acc)s.z; csum[c2][3] += (Acc)s.w;
+                        csq[c2][0] += (Acc)q.x; csq[c2][1] += (Acc)q.y; csq[c2][2] += (Acc)q.z; csq[c2][3] += (Acc)q.w;
+                    }
+                }
+                if (GROUPED) {
+                    asm volatile("bar.sync 3, %0;" ::"n"(NEPI * 32) : "memory");  // the tile's rows are stored
+                    env_stats_tile(Z, stats, tile, tile * rpt, gtile_rows(tile, tile * rpt, rows, rpt, nodes, 1), nodes, 1, tid);
                 }
                 continue;
             }
             mbar_wait(bar_full + buf * 8, (uint32_t)((i >> 1) & 1));
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const long long row0 = tile * TILE_M + quad * 32;
+            const long long trow0 = GROUPED ? gtile_row0(tile, rpt, nodes, g_P) : tile * TILE_M;
+            const int tnrows = GROUPED ? gtile_rows(tile, trow0, rows, rpt, nodes, g_P) : 0;
+            const long long rend = GROUPED ? trow0 + tnrows : rows;  // rows past rend belong to another tile (or none)
+            const long long row0 = trow0 + quad * 32;
 #pragma unroll
             for (int c2 = 0; c2 < 2; c2++) {
                 const int cc = half * 2 + c2;
@@ -648,24 +723,34 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_tma_kernel(con
                 const float4 bb = c2 == 0 ? b0 : b1;
                 float* zp = Z + (row0 + sub) * TILE_N + cc * 32 + c4 * 4;
                 float4 s = make_float4(0.f, 0.f, 0.f, 0.f), q = make_float4(0.f, 0.f, 0.f, 0.f);
-                const bool full = row0 + 32 <= rows;
+                const bool full = row0 + 32 <= rend;
 #pragma unroll
                 for (int it = 0; it < 8; it++) {
                     const int rr = it * 4 + sub;
                     float4 v = *reinterpret_cast<const float4*>(stg + rr * STG_W + ((c4 ^ (rr & 7)) << 2));
                     v.x += bb.x; v.y += bb.y; v.z += bb.z; v.w += bb.w;
-                    if (full || row0 + rr < rows) {
+                    if (full || row0 + rr < rend) {
                         *reinterpret_cast<float4*>(zp + (size_t)it * 4 * TILE_N) = v;
-                        s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-                        q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                        if (!GROUPED) {
+                            s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+                            q.x = fmaf(v.x, v.x, q.x); q.y = fmaf(v.y, v.y, q.y); q.z = fmaf(v.z, v.z, q.z); q.w = fmaf(v.w, v.w, q.w);
+                        }
                     }
                 }
-                csum[c2][0] += (Acc)s.x; csum[c2][1] += (Acc)s.y; csum[c2][2] += (Acc)s.z; csum[c2][3] += (Acc)s.w;
-                csq[c2][0] += (Acc)q.x; csq[c2][1] += (Acc)q.y; csq[c2][2] += (Acc)q.z; csq[c2][3] += (Acc)q.w;
+                if (!GROUPED) {
+                    if (!GROUPED) {
+                        csum[c2][0] += (Acc)s.x; csum[c2][1] += (Acc)s.y; csum[c2][2] += (Acc)s.z; csum[c2][3] += (Acc)s.w;
+                        csq[c2][0] += (Acc)q.x; csq[c2][1] += (Acc)q.y; csq[c2][2] += (Acc)q.z; csq[c2][3] += (Acc)q.w;
+                    }
+                }
                 __syncwarp();
             }
+            if (GROUPED) {
+                asm volatile("bar.sync 3, %0;" ::"n"(NEPI * 32) : "memory");  // the tile's rows are stored
+                env_stats_tile(Z, stats, tile, trow0, tnrows, nodes, g_P, tid);
+            }
         }
-        if (stats) {
+        if (!GROUPED && stats) {
 #pragma unroll
             for (int c2 = 0; c2 < 2; c2++)
 #pragma unroll
@@ -697,6 +782,30 @@ __global__ void bn_finalize_kernel(const double* __restrict__ stats, double inv_
     const double sc = (double)gamma[c] / sqrt(var + (double)eps);
     scale[c] = (float)sc;
     shift[c] = (float)((double)beta[c] - mean * sc);
+}
+// grouped: env_stats [B,P,2,C] -> scale, shift [G,C]; a group's sums are its envs' sums (each the sum of its pieces),
+// added in index order
+__global__ void bn_finalize_grouped_kernel(const double* __restrict__ env_stats, long long G, int P, int epg, double inv_rows,
+                                           const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float* scale,
+                                           float* shift, int C) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= G * C) return;
+    const long long g = idx / C;
+    const int c = (int)(idx - g * C);
+    double s = 0.0, q = 0.0;
+    for (int e = 0; e < epg; e++) {
+        const double* st = env_stats + (g * epg + e) * P * 2 * C + c;
+        double es = 0.0, eq = 0.0;
+        for (int p = 0; p < P; p++) { es += st[(size_t)p * 2 * C]; eq += st[(size_t)p * 2 * C + C]; }
+        s += es;
+        q += eq;
+    }
+    const double mean = s * inv_rows;  // as bn_finalize_kernel
+    double var = q * inv_rows - mean * mean;
+    if (var < 0) var = 0;
+    const double sc = (double)gamma[c] / sqrt(var + (double)eps);
+    scale[idx] = (float)sc;
+    shift[idx] = (float)((double)beta[c] - mean * sc);
 }
 
 
@@ -885,11 +994,13 @@ __device__ __forceinline__ float elu_fast(float x) { return x > 0.f ? x : __expf
 
 constexpr int HEAD_WARPS = 16;
 
+// GROUPED: in_scale / in_shift are [G,128], one affine per BatchNorm group of epg envs
+template <bool GROUPED>
 __global__ void __launch_bounds__(HEAD_WARPS * 32, 1) head_tf32_kernel(
     const float* __restrict__ X, const int32_t* __restrict__ cand, long long rows, int rpe, int nodes_per_env,
     const float* __restrict__ in_scale, const float* __restrict__ in_shift, int in_relu, const float* __restrict__ Wa,
     const float* __restrict__ bias_env, long long bias_rows, const float* __restrict__ W1, const float* __restrict__ b1,
-    const float* __restrict__ w2, const float* __restrict__ b2, float* __restrict__ out, long long num_tiles) {
+    const float* __restrict__ w2, const float* __restrict__ b2, float* __restrict__ out, long long num_tiles, int epg = 1) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr size_t WBYTES = (size_t)TILE_N * 128 * 4;
     float* sWa = reinterpret_cast<float*>(smem);
@@ -956,7 +1067,15 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32, 1) head_tf32_kernel(
             const int it = warp + u * HEAD_WARPS, grp = it >> 3, q = it & 7, k = q * 16 + c4 * 4;
             float4 x = v[u];
             if (affine && s_row[slot * 128 + grp * 8 + r8] >= 0) {
-                const float4 sc = *reinterpret_cast<const float4*>(s_scale + k), sh = *reinterpret_cast<const float4*>(s_shift + k);
+                float4 sc, sh;
+                if (GROUPED) {
+                    const int src = s_row[slot * 128 + grp * 8 + r8];
+                    const long long g = (long long)(cand ? src / nodes_per_env : src / rpe) / epg;
+                    sc = __ldg(reinterpret_cast<const float4*>(in_scale + g * 128 + k));
+                    sh = __ldg(reinterpret_cast<const float4*>(in_shift + g * 128 + k));
+                } else {
+                    sc = *reinterpret_cast<const float4*>(s_scale + k); sh = *reinterpret_cast<const float4*>(s_shift + k);
+                }
                 x.x = x.x * sc.x + sh.x; x.y = x.y * sc.y + sh.y; x.z = x.z * sc.z + sh.z; x.w = x.w * sc.w + sh.w;
                 if (in_relu) { x.x = fmaxf(x.x, 0.f); x.y = fmaxf(x.y, 0.f); x.z = fmaxf(x.z, 0.f); x.w = fmaxf(x.w, 0.f); }
             }
@@ -1688,21 +1807,23 @@ __global__ void __launch_bounds__(ESA_HEAD_WARPS * 32, 1) esa_head_tf32_kernel(
 
 }  // namespace
 
-template <int KP>
+// nodes > 0: the grouped form (env-aligned tiles of `nodes`-row envs, per-env statistics; see linear_tf32_kernel)
+template <int KP, bool GROUPED = false>
 static int launch_linear(const float* X, int64_t rows, int K, const float* W, const float* bias, const float* in_scale,
-                         const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream) {
+                         const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream, int nodes = 0) {
     const size_t smem = (size_t)TILE_N * KP * 4 + (size_t)NSTAGE * TILE_M * (KP > 64 ? 64 : KP) * 4 +
                         (size_t)NEPI * 32 * STG_W * 4 + (TILE_N + 256) * 4 + (4 + NSTAGE) * 8 + 16;
     static thread_local bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_kernel<KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(linear_tf32_kernel<KP, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MTFJSP_E_CUDA;
         configured = true;
     }
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const long long tiles = (rows + TILE_M - 1) / TILE_M;
+    const int P = GROUPED ? (nodes + TILE_M - 1) / TILE_M : 1, rpt = GROUPED && P == 1 ? (TILE_M / nodes) * nodes : TILE_M;
+    const long long tiles = GROUPED ? (P == 1 ? (rows + rpt - 1) / rpt : rows / nodes * P) : (rows + TILE_M - 1) / TILE_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
     // MTFJSP_GEMM_RAW_A=1 (opt-in): without a prologue the A operand stays as the FP32 bits cp.async landed -- kind::tf32
     // reads the top 19 bits (truncation) -- and the in-place rounding pass in front of every MMA is skipped: 563 -> 476 us
@@ -1710,8 +1831,12 @@ static int launch_linear(const float* X, int64_t rows, int K, const float* W, co
     // zero, and the PPO update's critic gradient moved visibly away from the FP32 one (cosine 0.982 against > 0.99 with
     // round-to-nearest operands, tests/test_ppo.py); profiles/README.md.
     static const int raw_a = getenv("MTFJSP_GEMM_RAW_A") ? atoi(getenv("MTFJSP_GEMM_RAW_A")) : 0;
-    linear_tf32_kernel<KP><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats,
-                                                                   tiles, raw_a);
+    if constexpr (GROUPED)
+        linear_tf32_kernel<KP, true><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, nullptr, nullptr, 0, Z, stats,
+                                                                             tiles, raw_a, rpt, nodes, P);
+    else
+        linear_tf32_kernel<KP, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z,
+                                                                              stats, tiles, raw_a);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 
@@ -1749,7 +1874,7 @@ static int launch_linear_tma(const float* X, int64_t rows, const float* W, const
                         (TILE_N + 256) * 4 + (4 + 2 * NSTAGE) * 8 + 16 + 128 * 10;
     static thread_local bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MTFJSP_E_CUDA;
         configured = true;
     }
@@ -1758,7 +1883,7 @@ static int launch_linear_tma(const float* X, int64_t rows, const float* W, const
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    linear_tf32_tma_kernel<false><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles,
+    linear_tf32_tma_kernel<false, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles,
                                                                          TILE_M, 0, nullptr, nullptr);
     return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
 }
@@ -1784,7 +1909,7 @@ static int launch_linear_tma_agg(const float* X, int64_t B, int N, const float* 
                         (4 + 2 * 3) * 8 + 16 + 128 * 10;
     static thread_local bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MTFJSP_E_CUDA;
         configured = true;
     }
@@ -1793,8 +1918,51 @@ static int launch_linear_tma_agg(const float* X, int64_t B, int N, const float* 
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long tiles = (rows + rpt - 1) / rpt;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    linear_tf32_tma_kernel<true><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles, rpt,
+    linear_tf32_tma_kernel<true, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles, rpt,
                                                                         N, reinterpret_cast<const float2*>(adj_w), adj_src);
+    return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
+}
+
+// the grouped K = 128 layers (both forms: agg = the aggregation + layer of launch_linear_tma_agg, nodes <= 128); in_scale /
+// in_shift [G,128]; 1 launched, 0 TMA not available, < 0 error
+static int launch_linear_tma_grouped(bool agg, const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
+                                     const float* W, const float* bias, const float* in_scale, const float* in_shift, int in_relu,
+                                     int epg, float* Z, double* env_stats, cudaStream_t stream) {
+    EncodeTiledFn enc = encode_tiled_fn();
+    if (!enc || ((uintptr_t)X & 15)) return 0;
+    const int P = (N + TILE_M - 1) / TILE_M, rpt = P == 1 ? (TILE_M / N) * N : TILE_M;
+    const long long rows = (long long)B * N;
+    CUtensorMap map;
+    const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {512};
+    const cuuint32_t box[2] = {32, (cuuint32_t)rpt};
+    const cuuint32_t estr[2] = {1, 1};
+    if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)X, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        return 0;
+    const size_t smem_agg = (size_t)TILE_N * 128 * 4 + (size_t)3 * TILE_M * 64 * 4 + (size_t)TILE_M * TILE_N * 4 + (TILE_N + 256) * 4 +
+                            (4 + 2 * 3) * 8 + 16 + 128 * 10;
+    const size_t smem_lin = (size_t)TILE_N * 128 * 4 + (size_t)NSTAGE * TILE_M * 64 * 4 + (size_t)NEPI * 32 * STG_W * 4 +
+                            (TILE_N + 256) * 4 + (4 + 2 * NSTAGE) * 8 + 16 + 128 * 10;
+    static thread_local bool configured = false;
+    if (!configured) {
+        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_agg) != cudaSuccess ||
+            cudaFuncSetAttribute(linear_tf32_tma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lin) != cudaSuccess)
+            return MTFJSP_E_CUDA;
+        configured = true;
+    }
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long tiles = P == 1 ? (rows + rpt - 1) / rpt : B * P;
+    const int grid = (int)(tiles < sms ? tiles : sms);
+    if (agg)
+        linear_tf32_tma_kernel<true, true><<<grid, GEMM_WARPS * 32, smem_agg, stream>>>(
+            map, rows, W, bias, in_scale, in_shift, in_relu, Z, env_stats, tiles, rpt, N, reinterpret_cast<const float2*>(adj_w), adj_src,
+            P, epg);
+    else
+        linear_tf32_tma_kernel<false, true><<<grid, GEMM_WARPS * 32, smem_lin, stream>>>(
+            map, rows, W, bias, in_scale, in_shift, in_relu, Z, env_stats, tiles, rpt, N, nullptr, nullptr, P, epg);
     return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
 }
 
@@ -1828,7 +1996,7 @@ int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int row
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (4 * 128 + 4 * 128) * 4 + 256 * 4 + 2 * 8 + 16;
     static thread_local bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(head_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(head_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MTFJSP_E_CUDA;
         configured = true;
     }
@@ -1837,7 +2005,7 @@ int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int row
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    head_tf32_kernel<<<grid, HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(X, cand, rows, rows_per_env, nodes_per_env, in_scale,
+    head_tf32_kernel<false><<<grid, HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(X, cand, rows, rows_per_env, nodes_per_env, in_scale,
                                                                           in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2, b2,
                                                                           out, tiles);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
@@ -1886,6 +2054,72 @@ int mtfjsp_enc_aggregate_linear_tf32(const float* X, int64_t B, int N, const flo
     const int rc = launch_linear_tma_agg(X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, Z, stats, (cudaStream_t)stream);
     if (rc == 0) return MTFJSP_E_STATE;  // not available for this size / driver: the caller runs the two kernels
     return rc < 0 ? rc : MTFJSP_OK;
+}
+
+static bool grouped_args_ok(int64_t B, int N, int epg) { return B >= 1 && N >= 1 && epg >= 1 && B % epg == 0 && B * N <= 0x7fffff00LL; }
+
+int mtfjsp_enc_linear_tf32_grouped(const float* X, int64_t B, int rows_per_env, int K, const float* W, const float* bias,
+                                   const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, float* Z,
+                                   double* env_stats, void* stream) {
+    if (!X || !W || !Z || !env_stats || !grouped_args_ok(B, rows_per_env, envs_per_group)) return MTFJSP_E_ARG;
+    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (K == 128) {
+        const int rc = launch_linear_tma_grouped(false, X, B, rows_per_env, nullptr, nullptr, W, bias, in_scale, in_shift, in_relu,
+                                                 envs_per_group, Z, env_stats, (cudaStream_t)stream);
+        return rc == 0 ? MTFJSP_E_STATE : rc < 0 ? rc : MTFJSP_OK;
+    }
+    if (K < 4 || K > 16 || (K % 4) != 0 || in_scale) return MTFJSP_E_ARG;
+    return launch_linear<16, true>(X, B * rows_per_env, K, W, bias, nullptr, nullptr, 0, Z, env_stats, (cudaStream_t)stream, rows_per_env);
+}
+
+int mtfjsp_enc_aggregate_linear_tf32_grouped(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
+                                             const float* W, const float* bias, const float* in_scale, const float* in_shift,
+                                             int in_relu, int envs_per_group, float* Z, double* env_stats, void* stream) {
+    if (!X || !adj_w || !adj_src || !W || !Z || !env_stats || !grouped_args_ok(B, N, envs_per_group)) return MTFJSP_E_ARG;
+    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (N > TILE_M) return MTFJSP_E_STATE;  // the caller runs mtfjsp_enc_aggregate_grouped + mtfjsp_enc_linear_tf32_grouped
+    const int rc = launch_linear_tma_grouped(true, X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, envs_per_group, Z,
+                                             env_stats, (cudaStream_t)stream);
+    return rc == 0 ? MTFJSP_E_STATE : rc < 0 ? rc : MTFJSP_OK;
+}
+
+int mtfjsp_enc_head_tf32_grouped(const float* X, const int32_t* cand, int64_t B, int rows_per_env, int nodes_per_env,
+                                 const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, const float* Wa,
+                                 const float* bias_env, int64_t bias_rows, const float* W1, const float* b1, const float* w2,
+                                 const float* b2, float* out, void* stream) {
+    if (!X || !in_scale || !in_shift || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1) return MTFJSP_E_ARG;
+    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
+    if (bias_rows != 1 && bias_rows != B) return MTFJSP_E_ARG;
+    if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL)) return MTFJSP_E_ARG;
+    const long long rows = (long long)B * rows_per_env;
+    if (rows > 0x7fffffffLL) return MTFJSP_E_ARG;
+    const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (4 * 128 + 4 * 128) * 4 + 256 * 4 + 2 * 8 + 16;
+    static thread_local bool configured = false;
+    if (!configured) {
+        if (cudaFuncSetAttribute(head_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return MTFJSP_E_CUDA;
+        configured = true;
+    }
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long tiles = (rows + TILE_M - 1) / TILE_M;
+    const int grid = (int)(tiles < sms ? tiles : sms);
+    head_tf32_kernel<true><<<grid, HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(X, cand, rows, rows_per_env, nodes_per_env, in_scale,
+                                                                                in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2,
+                                                                                b2, out, tiles, envs_per_group);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_bn_finalize_grouped(const double* env_stats, int64_t B, int rows_per_env, int envs_per_group, const float* gamma,
+                                   const float* beta, float eps, float* scale, float* shift, int C, void* stream) {
+    if (!env_stats || !gamma || !beta || !scale || !shift || C < 1 || !grouped_args_ok(B, rows_per_env, envs_per_group))
+        return MTFJSP_E_ARG;
+    const long long G = B / envs_per_group;
+    const int P = (rows_per_env + TILE_M - 1) / TILE_M;
+    bn_finalize_grouped_kernel<<<(unsigned)((G * C + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+        env_stats, G, P, envs_per_group, 1.0 / ((double)envs_per_group * rows_per_env), gamma, beta, eps, scale, shift, C);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 
 int mtfjsp_enc_bn_finalize(const double* stats, int64_t rows, const float* gamma, const float* beta, float eps,

@@ -14,7 +14,8 @@ What runs where (round 1): the neighbour aggregation (reference: dense adj -> CO
 SpMM for the degree) is the hand-written `mtfjsp_enc_aggregate` kernel over ELL; graph pooling is
 `mtfjsp_enc_graph_mean`; the 2x2 GAT attention is closed-form elementwise math; the dense per-node projections run
 on the tcgen05 kernel `mtfjsp_enc_linear_tf32` with `precision="tf32"` (BatchNorm statistics in its epilogue, the
-folded BatchNorm + ReLU of the previous layer in its prologue) or on library FP32 GEMMs with `precision="fp32"`;
+folded BatchNorm + ReLU of the previous layer in its prologue; per-env statistics and per-group affines with groups > 1,
+the *_grouped entry points) or on library FP32 GEMMs with `precision="fp32"`;
 BatchNorm uses batch statistics exactly as the reference does (its modules are never put in eval mode, SURVEY.md 3.3).
 """
 from __future__ import annotations
@@ -55,6 +56,11 @@ def _aggregate_raw(h, adj_w, adj_src, in_scale=None, in_shift=None, relu=False):
     B, N, Cc = h.shape
     h = h.contiguous()
     out = torch.empty_like(h)
+    if in_scale is not None and in_scale.dim() == 2:  # per-group affine [G,C] (grouped BatchNorm)
+        check(_lib.lib().mtfjsp_enc_aggregate_grouped(_ptr(h), _ptr(adj_w), _ptr(adj_src), _ptr(out), B, N, Cc, _ptr(in_scale),
+                                                      _ptr(in_shift), int(relu), B // in_scale.shape[0], _stream()),
+              "mtfjsp_enc_aggregate_grouped")
+        return out
     check(_lib.lib().mtfjsp_enc_aggregate(_ptr(h), _ptr(adj_w), _ptr(adj_src), _ptr(out), B, N, Cc, _optr(in_scale),
                                           _optr(in_shift), int(relu), _stream()), "mtfjsp_enc_aggregate")
     return out
@@ -147,8 +153,15 @@ def select(scores, mask, cand, scale, greedy, rng, stream_id):
 
 def head_tf32(x, cand, B, rows_per_env, nodes_per_env, in_scale, in_shift, Wa, bias_env, W1, b1, w2, b2, relu=True):
     """mtfjsp_enc_head_tf32: a whole policy head (gather, BatchNorm + ReLU of the producing layer, Linear, per-env bias,
-    tanh, Linear, tanh, Linear(128, 1)) in one launch -> scores [B, rows_per_env]."""
+    tanh, Linear, tanh, Linear(128, 1)) in one launch -> scores [B, rows_per_env].  in_scale [G,128]: one affine per
+    BatchNorm group of B / G envs (mtfjsp_enc_head_tf32_grouped)."""
     out = torch.empty((B, rows_per_env), dtype=torch.float32, device=x.device)
+    if in_scale is not None and in_scale.dim() == 2:
+        check(_lib.lib().mtfjsp_enc_head_tf32_grouped(_ptr(x), _optr(cand), B, rows_per_env, nodes_per_env, _ptr(in_scale),
+                                                      _ptr(in_shift), 1 if relu else 0, B // in_scale.shape[0], _ptr(Wa),
+                                                      _ptr(bias_env), bias_env.shape[0], _ptr(W1), _optr(b1), _ptr(w2), _optr(b2),
+                                                      _ptr(out), _stream()), "mtfjsp_enc_head_tf32_grouped")
+        return out
     check(_lib.lib().mtfjsp_enc_head_tf32(_ptr(x), _optr(cand), B, rows_per_env, nodes_per_env, _optr(in_scale), _optr(in_shift),
                                           1 if relu else 0, _ptr(Wa), _ptr(bias_env), bias_env.shape[0], _ptr(W1), _optr(b1), _ptr(w2), _optr(b2),
                                           _ptr(out), _stream()), "mtfjsp_enc_head_tf32")
@@ -169,6 +182,10 @@ def _graph_mean_raw(h, in_scale=None, in_shift=None, relu=False):
     B, N, Cc = h.shape
     h = h.contiguous()
     out = torch.empty((B, Cc), dtype=h.dtype, device=h.device)
+    if in_scale is not None and in_scale.dim() == 2:  # per-group affine [G,C]
+        check(_lib.lib().mtfjsp_enc_graph_mean_grouped(_ptr(h), _ptr(out), B, N, Cc, _ptr(in_scale), _ptr(in_shift), int(relu),
+                                                       B // in_scale.shape[0], _stream()), "mtfjsp_enc_graph_mean_grouped")
+        return out
     check(_lib.lib().mtfjsp_enc_graph_mean(_ptr(h), _ptr(out), B, N, Cc, _optr(in_scale), _optr(in_shift), int(relu),
                                            _stream()), "mtfjsp_enc_graph_mean")
     return out
@@ -192,6 +209,51 @@ def linear_tf32(x, weight, bias, in_scale=None, in_shift=None, relu=False, stats
                                             _optr(in_shift), int(relu), _ptr(z), _optr(stats), _stream()),
           "mtfjsp_enc_linear_tf32")
     return z
+
+
+def env_stat_pieces(rows_per_env):
+    """P of the grouped layers' env_stats [B,P,2,128]: 128-row tile pieces per env."""
+    return (rows_per_env + 127) // 128
+
+
+def linear_tf32_grouped(x, rows_per_env, weight, bias, in_scale, in_shift, relu, env_stats):
+    """linear_tf32 over B = rows / rows_per_env envs with env-aligned tiles: in_scale / in_shift [G,128] (one affine per
+    group of B / G envs) or None; env_stats [B,P,2,128] f64 receives each env's column sums of Z and Z^2."""
+    rows, K = x.shape
+    B = rows // rows_per_env
+    z = torch.empty((rows, 128), dtype=torch.float32, device=x.device)
+    epg = 1 if in_scale is None else B // in_scale.shape[0]
+    check(_lib.lib().mtfjsp_enc_linear_tf32_grouped(_ptr(x.contiguous()), B, rows_per_env, K, _ptr(weight), _optr(bias),
+                                                    _optr(in_scale), _optr(in_shift), int(relu), epg, _ptr(z), _ptr(env_stats),
+                                                    _stream()), "mtfjsp_enc_linear_tf32_grouped")
+    return z
+
+
+def aggregate_linear_tf32_grouped(h, adj_w, adj_src, weight, bias, in_scale, in_shift, relu, env_stats):
+    """aggregate_linear_tf32 with [G,128] affines and per-env statistics; None where the form is not available (N > 128)."""
+    B, N = h.shape[0], h.shape[1]
+    if N > 128 or not _FUSED_AGG:
+        return None
+    z = torch.empty((B * N, 128), dtype=torch.float32, device=h.device)
+    epg = 1 if in_scale is None else B // in_scale.shape[0]
+    rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32_grouped(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _optr(bias),
+                                                             _optr(in_scale), _optr(in_shift), int(relu), epg, _ptr(z),
+                                                             _ptr(env_stats), _stream())
+    if rc == -3:  # MTFJSP_E_STATE
+        return None
+    check(rc, "mtfjsp_enc_aggregate_linear_tf32_grouped")
+    return z
+
+
+def bn_finalize_grouped(env_stats, rows_per_env, groups, gamma, beta, eps=1e-5):
+    """env_stats [B,P,2,C] -> scale, shift [groups, C]: BatchNorm with batch statistics per group of B / groups envs."""
+    B = env_stats.shape[0]
+    Cc = gamma.shape[0]
+    scale = torch.empty((groups, Cc), dtype=torch.float32, device=gamma.device)
+    shift = torch.empty_like(scale)
+    check(_lib.lib().mtfjsp_enc_bn_finalize_grouped(_ptr(env_stats), B, rows_per_env, B // groups, _ptr(gamma), _ptr(beta), eps,
+                                                    _ptr(scale), _ptr(shift), Cc, _stream()), "mtfjsp_enc_bn_finalize_grouped")
+    return scale, shift
 
 
 _WGRAD_WS = {}
@@ -531,7 +593,7 @@ class _GraphEncoder:
         h = task_fea.to(torch.float32)
         if self.precision == "tf32":
             if groups != 1:
-                raise ValueError("the tf32 path is the rollout path: one BatchNorm group")
+                return self._encode_tf32_grouped(h, adj_w, adj_src, groups)
             return self._encode_tf32(h, adj_w, adj_src)
         for l in (0, 1):
             pooled = aggregate(h, adj_w, adj_src, adj_dst=adj_dst)                  # gcn_mlp.py:125-149
@@ -573,10 +635,44 @@ class _GraphEncoder:
         self._pending = (sc, sh)  # outer BatchNorm + ReLU of the last layer, applied by the consumers below
         return graph_mean(h, sc, sh, relu=True), h
 
+    def _encode_tf32_grouped(self, h, adj_w, adj_src, groups):
+        """_encode_tf32 with a BatchNorm group per B / groups consecutive envs: the grouped kernels write per-env
+        statistics (summed in a fixed env-local order, so an env's results do not depend on its batch position) and every
+        consumer applies the [groups, 128] affine of its env's group."""
+        w = self.w
+        B, N = h.shape[0], self.N
+        if B % groups:
+            raise ValueError("groups must divide the batch")
+        rows = B * N
+        env_stats = torch.empty((B, env_stat_pieces(N), 2, 128), dtype=torch.float64, device=h.device)
+        fin = lambda name: bn_finalize_grouped(env_stats, N, groups, w[name + "weight"], w[name + "bias"])
+        adj_w, adj_src = adj_w.contiguous(), adj_src.contiguous()
+        sc = sh = None
+        for l in (0, 1):
+            p = "encoder.feature_extract.mlps.%d." % l
+            z = None
+            if l > 0:
+                z = aggregate_linear_tf32_grouped(h, adj_w, adj_src, w[p + "linears.0.weight"], w[p + "linears.0.bias"], sc, sh,
+                                                  True, env_stats)
+            if z is None:
+                pooled = aggregate(h, adj_w, adj_src, sc, sh, relu=sc is not None).reshape(rows, -1)
+                z = linear_tf32_grouped(pooled, N, w[p + "linears.0.weight"], w[p + "linears.0.bias"], None, None, False, env_stats)
+            isc, ish = fin(p + "batch_norms.0.")
+            z = linear_tf32_grouped(z, N, w[p + "linears.1.weight"], w[p + "linears.1.bias"], isc, ish, True, env_stats)
+            isc, ish = fin(p + "batch_norms.1.")
+            z = linear_tf32_grouped(z, N, w[p + "linears.2.weight"], w[p + "linears.2.bias"], isc, ish, True, env_stats)
+            sc, sh = fin("encoder.feature_extract.batch_norms.%d." % l)
+            h = z.reshape(B, N, self.H)
+        self._pending = (sc, sh)  # [groups, 128]
+        return graph_mean(h, sc, sh, relu=True), h
+
     def candidate_features(self, nodes, candidate):
         cf = torch.gather(nodes, 1, candidate.long().unsqueeze(-1).expand(-1, self.J, self.H))   # actor_critic.py:197-207
         if self._pending is not None:
             sc, sh = self._pending
+            if sc.dim() == 2:  # [G,128]: the affine of each env's BatchNorm group
+                epg = cf.shape[0] // sc.shape[0]
+                sc, sh = sc.repeat_interleave(epg, 0).unsqueeze(1), sh.repeat_interleave(epg, 0).unsqueeze(1)
             cf = torch.relu(cf * sc + sh)
         return cf
 
@@ -646,6 +742,8 @@ class _Twin:
         if _FUSED_HEAD:
             return head_tf32(per_row, cand, B, rows_per_env, nodes, in_scale, in_shift, Wa, bias,
                              w[prefix + "linears.1.weight"], w[prefix + "linears.1.bias"], w2, w[prefix + "linears.2.bias"], relu=relu)
+        if in_scale is not None and in_scale.dim() == 2:
+            raise ValueError("per-group BatchNorm affines need the one-launch head (MTFJSP_FUSED_HEAD=1)")
         if cand is not None:
             per_row = torch.gather(per_row, 1, cand.long().unsqueeze(-1).expand(-1, rows_per_env, H)).reshape(-1, H)
         z = linear_tf32(per_row, Wa, None, in_scale, in_shift, relu=relu and in_scale is not None)
@@ -833,7 +931,8 @@ class _MachineTrunk:
 
 
 class MachineActor(_MachineTrunk, _Twin):
-    """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498)."""
+    """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498).  With groups > 1 the tf32
+    path normalises through mtfjsp_enc_bn_fwd: at most 65,535 groups per call (its grid.y)."""
 
     n_values = 2  # width of machine_v
 

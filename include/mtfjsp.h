@@ -312,6 +312,41 @@ int mtfjsp_enc_esa_mach_head_tf32(const float* fea1, const float* fea2, int64_t 
 int mtfjsp_enc_bn_finalize(const double* stats, int64_t rows, const float* gamma, const float* beta, float eps,
                            float* scale, float* shift, int C, void* stream);
 
+/* Grouped encoder layers: per-instance BatchNorm on the tcgen05 path (the reference's test-time rollouts run one instance
+ * at a time with its modules in train mode, so every BatchNorm of model/gcn_mlp.py:154-157, 238-249 normalises with the
+ * statistics of that one instance's rows; trainer/validate.py:60-297, algorithm/agent_func.py:22-63).  B envs of N =
+ * rows_per_env rows each; a group is envs_per_group (epg) consecutive envs, G = B / epg groups (B % epg == 0), and every
+ * affine in_scale / in_shift is [G,C] (C = 128), group of env b = b / epg.
+ *   linear_tf32_grouped / aggregate_linear_tf32_grouped: the layers above with env-aligned tiles -- (128 / N) * N rows of
+ *     whole envs for N <= 128, P = ceil(N / 128) tiles of 128 rows per env otherwise -- and, instead of the batch-wide
+ *     stats, env_stats [B,P,2,128] f64: per env and tile piece the column sums of Z and of Z^2, written (no atomics, no
+ *     zeroing needed), each summed over the env's rows in row order after the tile is stored.  An env's statistics and
+ *     everything computed from them are therefore the same bits whatever its position in the batch.  K = 128 (TMA
+ *     operand, in_scale optional) or 4 <= K <= 16, K % 4 == 0 (no input affine: the first layer); other K -> MTFJSP_E_ARG.
+ *     MTFJSP_E_STATE: no TMA driver entry point, or (aggregate form) N > 128: run mtfjsp_enc_aggregate_grouped +
+ *     mtfjsp_enc_linear_tf32_grouped instead.
+ *   aggregate_grouped / graph_mean_grouped / head_tf32_grouped: mtfjsp_enc_aggregate / _graph_mean / _head_tf32 with the
+ *     [G,C] affine (required here).
+ *   bn_finalize_grouped: env_stats [B,P,2,C] -> scale, shift [G,C]; the pieces of an env, then the envs of a group are
+ *     added in index order in FP64; biased variance over epg * N rows, eps and clamping as mtfjsp_enc_bn_finalize.
+ * Limits: B * N <= 2^31 - 256 rows.  Bad arguments -> MTFJSP_E_ARG. */
+int mtfjsp_enc_linear_tf32_grouped(const float* X, int64_t B, int rows_per_env, int K, const float* W, const float* bias,
+                                   const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, float* Z,
+                                   double* env_stats, void* stream);
+int mtfjsp_enc_aggregate_linear_tf32_grouped(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
+                                             const float* W, const float* bias, const float* in_scale, const float* in_shift,
+                                             int in_relu, int envs_per_group, float* Z, double* env_stats, void* stream);
+int mtfjsp_enc_aggregate_grouped(const float* h, const float* adj_w, const int16_t* adj_src, float* out, int64_t B, int N, int C,
+                                 const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, void* stream);
+int mtfjsp_enc_graph_mean_grouped(const float* h, float* out, int64_t B, int N, int C, const float* in_scale, const float* in_shift,
+                                  int in_relu, int envs_per_group, void* stream);
+int mtfjsp_enc_head_tf32_grouped(const float* X, const int32_t* cand, int64_t B, int rows_per_env, int nodes_per_env,
+                                 const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, const float* Wa,
+                                 const float* bias_env, int64_t bias_rows, const float* W1, const float* b1, const float* w2,
+                                 const float* b2, float* out, void* stream);
+int mtfjsp_enc_bn_finalize_grouped(const double* env_stats, int64_t B, int rows_per_env, int envs_per_group, const float* gamma,
+                                   const float* beta, float eps, float* scale, float* shift, int C, void* stream);
+
 /* replaces: the per-reward GAE of algorithm/ppo_algorithm.py:438-536 (python loop over buffered steps per stream).
  * r, v, v_next, adv: [T,B,4] f32 (streams mk, pt, tt, idle); done [T,B] f32; stats[8] f64 accumulates per-stream
  * sum and sum of squares of the advantages (allreduce it across ranks, then normalise). */
