@@ -2590,7 +2590,8 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
     if (!out) return fail(MTFJSP_E_ARG, "null handle pointer");
     *out = nullptr;
     if (B < 1 || J < 1 || M < 2 || M > 64 || E < 1 || (long long)J * M > 4096)
-        return fail(MTFJSP_E_ARG, "size out of range (need B>=1, J>=1, 2<=M<=64, J*M<=4096, E>=1)");
+        return fail(MTFJSP_E_ARG, "size out of range (need B>=1, J>=1, 2<=M<=64, J*M<=4096, E>=1, and one env's state "
+                                  "within one block's shared memory: J<=48 at M=64, J<=109 at M=32, J<=1678 at M=2)");
     CK(cudaSetDevice(device), "cudaSetDevice");
     mtfjsp_env* h = new (std::nothrow) mtfjsp_env();
     if (!h) return fail(MTFJSP_E_ARG, "out of host memory");
@@ -2624,7 +2625,11 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
     L.smem_per_warp = align_up(off, 16);
     int wpb = 8;
     while (wpb > 1 && (size_t)wpb * L.smem_per_warp > 200 * 1024) wpb >>= 1;
-    if ((size_t)wpb * L.smem_per_warp > 227 * 1024) { delete h; return fail(MTFJSP_E_ARG, "instance too large for shared memory"); }
+    if ((size_t)wpb * L.smem_per_warp > 227 * 1024) {  // about 62 * N + 8 * M * M bytes per env (include/mtfjsp.h)
+        delete h;
+        return fail(MTFJSP_E_ARG, "instance too large: one env's state exceeds one block's shared memory (227 KB); "
+                                  "the largest J is 48 at M=64, 109 at M=32, 1678 at M=2");
+    }
     L.warps_per_block = wpb;
     h->device = device;
     {

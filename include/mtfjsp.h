@@ -43,7 +43,10 @@ enum {
     MTFJSP_E_STATE = -3   /* call order violated (e.g. step before load/reset) */
 };
 
-/* Limits of this build: 2 <= M <= 64 machines, 1 <= J, N = J*M <= 4096 operations. */
+/* Limits of this build: 2 <= M <= 64 machines, 1 <= J, N = J*M <= 4096 operations, and one environment's state must
+ * fit the shared memory of one block (227 KB).  That state takes about 62*N + 8*M*M bytes, so mtfjsp_create returns
+ * MTFJSP_E_ARG well below N = 4096 (no instance of 4096 operations fits).  The largest J it accepts:
+ *   M = 2: J <= 1678,  M = 3: J <= 1152,  M = 7: J <= 510,  M = 32: J <= 109,  M = 33: J <= 106,  M = 64: J <= 48. */
 
 /* replaces: Parallel_env.__init__ (trainer/parallel_env.py:19-36) + the env constructor arguments
  * perform_left_shift_if_possible / reward_function='wrk' (trainer/parallel_env.py:110-118). */

@@ -101,6 +101,16 @@ REPLAYS = [
     # BASELINE.json configs[3]: N = 600 (5 numpy pairwise leaves, the 32-lane kernel with aliased scratch).  One env, one
     # episode = 600 reference steps at ~0.3 s; the bulky dumps are kept at SPARSE_STEPS only
     ("j30m20e5_ls_esa_mixed", 30, 20, 5, 1, True, 1, "mixed", 1.0, 1, 110),
+    # the edges of the size range: M = 64 (more machines than a warp has lanes, 64-bit machine masks), one edge group
+    # per machine (E = M), a single job (the ESA mask's one-job branches), M = 2, J = 70 (three 32-job chunks), and
+    # N = 143 (an odd size above one numpy pairwise leaf)
+    ("j2m64e4_ls_esa_mixed", 2, 64, 4, 1, True, 1, "mixed", 1.0, 1, 111),
+    ("j2m64e64_ls_fin_mixed", 2, 64, 64, 1, True, 0, "mixed", 1.0, 1, 112),
+    ("j1m5e2_ls_esa_mixed", 1, 5, 2, 3, True, 1, "mixed", 1.0, 2, 113),
+    ("j1m2e1_nols_fin_lowest", 1, 2, 1, 3, False, 0, "lowest", 1.0, 1, 114),
+    ("j70m2e1_ls_esa_mixed", 70, 2, 1, 2, True, 1, "mixed", 1.0, 1, 115),
+    ("j4m8e8_ls_esa_random", 4, 8, 8, 2, True, 1, "random", 1.0, 1, 116),
+    ("j13m11e3_nols_esa_mixed", 13, 11, 3, 2, False, 1, "mixed", 1.0, 1, 117),
 ]
 # steps whose full observation / schedule state a large fixture keeps (all steps below N = 200)
 SPARSE_STEPS = sorted(set(range(0, 24)) | set(range(24, 600, 24)) | set(range(585, 600)))
