@@ -1373,10 +1373,15 @@ __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk_tf32_kernel(
 // Second form of the trunk kernel: 128 machines per tile, the two node sets as TWO products per layer (t1 = h1 W into TMEM
 // columns 0..127, t2 = h2 W into 128..255), so that the thread that owns a machine's TMEM lane holds both of its rows:
 // no exchange of node-2 rows through shared memory, every thread does the same work, half the barriers per machine.
+// GROUPED (per-env BatchNorm statistics): a tile is rpt = (128 / M) * M machines of whole envs (lanes >= rpt idle), and
+// instead of the batch-wide atomics `stats` is env_stats [B,1,2,128]: the last layer also parks the output rows in the
+// (then free) first A buffer, and one thread per (env, column) adds the env's rows from there in row order in FP64, so
+// an env's statistics are the same bits at any batch position.
+template <bool GROUPED>
 __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
     const float* __restrict__ f1, const float* __restrict__ f2, const float* __restrict__ W1p, const float* __restrict__ W2p,
     const float* __restrict__ Wt, const float* __restrict__ a_src, const float* __restrict__ a_dst, float* __restrict__ out,
-    double* __restrict__ stats, long long R, long long num_tiles) {
+    double* __restrict__ stats, long long R, long long num_tiles, int rpt, int M) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr size_t WBYTES = (size_t)TILE_N * 128 * 4;
     float* sW = reinterpret_cast<float*>(smem);
@@ -1416,8 +1421,8 @@ __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
     uint32_t phase = 0;
     double st_sum = 0.0, st_sq = 0.0;
     for (long long tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const long long m = tile * 128 + mloc;
-        const bool mok = m < R;
+        const long long m = tile * (GROUPED ? rpt : 128) + mloc;
+        const bool mok = m < R && (!GROUPED || mloc < rpt);
         {   // input projections on the CUDA cores, straight into the two A operands
             float fa[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, fb[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             if (mok) {
@@ -1517,7 +1522,13 @@ __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
 #pragma unroll
                     for (int j = 0; j < 8; j++) op[j] = make_float4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
                 }
-                if (stats) {  // recursive halving over the warp's 32 machines: lane l ends up with column cg * 32 + l
+                if (GROUPED) {  // row mloc of the tile, 16-byte pieces XOR-swizzled by the row (the products are done with sA1)
+#pragma unroll
+                    for (int j = 0; j < 8; j++)
+                        *reinterpret_cast<float4*>(sA1 + mloc * 128 + (((cg * 8 + j) ^ (mloc & 7)) << 2)) =
+                            make_float4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
+                }
+                if (!GROUPED && stats) {  // recursive halving over the warp's 32 machines: lane l ends up with column cg * 32 + l
                     float q[32];
 #pragma unroll
                     for (int j = 0; j < 32; j++) q[j] = o[j] * o[j];
@@ -1538,8 +1549,25 @@ __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
             }
         }
         __syncthreads();  // s_dot and the A buffers are rewritten by the next tile
+        if (GROUPED) {    // the tile's rows are parked in sA1 (the barrier above): per-env sums in row order, FP64
+            const long long row0 = tile * rpt, env0 = row0 / M;
+            const int nenv = (int)(R - row0 < rpt ? R - row0 : rpt) / M;
+            for (int item = tid; item < nenv * 128; item += TRUNK_WARPS * 32) {
+                const int e = item >> 7, c = item & 127;
+                double sum = 0.0, sq = 0.0;
+                for (int j = 0; j < M; j++) {
+                    const int r = e * M + j;
+                    const double v = (double)sA1[r * 128 + ((((c >> 2) ^ (r & 7))) << 2) + (c & 3)];
+                    sum += v;
+                    sq = fma(v, v, sq);
+                }
+                stats[(env0 + e) * 256 + c] = sum;
+                stats[(env0 + e) * 256 + 128 + c] = sq;
+            }
+            __syncthreads();  // sA1 is the next tile's operand
+        }
     }
-    if (stats) {
+    if (!GROUPED && stats) {
         atomicAdd(stats + cg * 32 + lane, st_sum);
         atomicAdd(stats + 128 + cg * 32 + lane, st_sq);
     }
@@ -2022,14 +2050,14 @@ int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float*
         const size_t smem2 = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
         static thread_local bool configured2 = false;
         if (!configured2) {
-            if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess)
+            if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess)
                 return MTFJSP_E_CUDA;
             configured2 = true;
         }
         const long long tiles2 = (R + 127) / 128;
         const int grid2 = (int)(tiles2 < sms ? tiles2 : sms);
-        gat_trunk2_tf32_kernel<<<grid2, TRUNK_WARPS * 32, smem2, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out, stats,
-                                                                                     R, tiles2);
+        gat_trunk2_tf32_kernel<false><<<grid2, TRUNK_WARPS * 32, smem2, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
+                                                                                            stats, R, tiles2, 128, 1);
         return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
     }
     const size_t smem = 2 * (size_t)TILE_N * 128 * 4 + (64 * 128 + 3 * 4 * 64 + 256 + 128 * 14) * 4 + 8 + 16;
@@ -2043,6 +2071,30 @@ int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float*
     const int grid = (int)(tiles < sms ? tiles : sms);
     gat_trunk_tf32_kernel<<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out, stats, R,
                                                                                 tiles);
+    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+}
+
+int mtfjsp_enc_gat_trunk_tf32_grouped(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
+                                      const float* a_src, const float* a_dst, float* out, double* env_stats, int64_t B, int M,
+                                      void* stream) {
+    if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || !env_stats || B < 1 || M < 1 || M > 128 ||
+        B * M > 0x7fffff00LL)
+        return MTFJSP_E_ARG;
+    const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
+    static thread_local bool configured = false;
+    if (!configured) {
+        if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            return MTFJSP_E_CUDA;
+        configured = true;
+    }
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int epT = 128 / M;  // whole envs per tile
+    const long long tiles = (B + epT - 1) / epT;
+    const int grid = (int)(tiles < sms ? tiles : sms);
+    gat_trunk2_tf32_kernel<true><<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
+                                                                                         env_stats, B * M, tiles, epT * M, M);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 

@@ -178,6 +178,17 @@ def gat_trunk_tf32(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, stats=None):
     return out
 
 
+def gat_trunk_tf32_grouped(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, env_stats, M):
+    """mtfjsp_enc_gat_trunk_tf32_grouped: gat_trunk_tf32 over B = R / M envs with env-aligned tiles -> [R,128];
+    env_stats [B,1,2,128] f64 receives each env's column sums of the result and of its squares."""
+    R = fea1.shape[0]
+    out = torch.empty((R, 128), dtype=torch.float32, device=fea1.device)
+    check(_lib.lib().mtfjsp_enc_gat_trunk_tf32_grouped(_ptr(fea1), _ptr(fea2), _ptr(W1p), _ptr(W2p), _ptr(Wt), _ptr(a_src),
+                                                       _ptr(a_dst), _ptr(out), _ptr(env_stats), R // M, M, _stream()),
+          "mtfjsp_enc_gat_trunk_tf32_grouped")
+    return out
+
+
 def _graph_mean_raw(h, in_scale=None, in_shift=None, relu=False):
     B, N, Cc = h.shape
     h = h.contiguous()
@@ -818,15 +829,17 @@ class JobActor(_GraphEncoder, _Twin):
         prob = F.softmax(s, dim=-1)
         return prob, pooled, job_v
 
-    def forward(self, task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation, greedy=False, generator=None, rng=None):
+    def forward(self, task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation, greedy=False, generator=None, rng=None,
+                groups=1):
         """-> task_index [B], action_index [B] (job), log_a [B], prob [B,J], h_g_o_pooled [B,H], job_v [B,2].
         rng = (seed, device step counter): sampling by the one-launch selection kernel (`select`) instead of
-        torch.multinomial on `generator`."""
+        torch.multinomial on `generator`.  groups: BatchNorm groups of B / groups consecutive envs (see `encode`)."""
         if rng is not None and not greedy:
-            s, pooled, job_v = self.evaluate(task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation, return_logits=True)
+            s, pooled, job_v = self.evaluate(task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation, groups=groups,
+                                             return_logits=True)
             prob, a, log_a, task_index = select(s, mask_operation, candidate.to(torch.int32).contiguous(), 1.0, False, rng, 0)
             return task_index, a, log_a, prob, pooled, job_v
-        prob, pooled, job_v = self.evaluate(task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation)
+        prob, pooled, job_v = self.evaluate(task_fea, adj_w, adj_src, candidate, h_g_m_pooled, mask_operation, groups=groups)
         if greedy:                                                                       # agent_func.py greedy / sample
             a = prob.argmax(dim=-1)
         else:
@@ -913,6 +926,11 @@ class _MachineTrunk:
             sc, sh = bn_finalize(stats, R, w["bn.weight"], w["bn.bias"])
             self._pending_m = (sc, sh)
             return buf.view(B, self.M, H), _graph_mean_raw(buf.view(B, self.M, H), sc, sh, relu=False)
+        if _FUSED_TRUNK and _FUSED_HEAD and B > groups:
+            # groups of several envs (training rollouts, Rollout(bn_group_envs=...)): per-env statistics from the trunk
+            # kernel; groups of one env (per-instance validation) keep the separate BatchNorm pass below, whose decisions
+            # tests/test_grouped_bn.py pins bit for bit against one-instance batches
+            return self._trunk_tf32_grouped(f1, f2, Wt, a_src, a_dst, groups)
         if _FUSED_TRUNK:
             buf = gat_trunk_tf32(f1, f2, w["m_fea_1_fcl.weight"], w["m_fea_2_fcl.weight"], Wt, a_src, a_dst)
         else:
@@ -923,6 +941,20 @@ class _MachineTrunk:
         nodes = _bn_train(buf, w["bn.weight"], w["bn.bias"], groups=groups).reshape(B, self.M, H)
         return nodes, nodes.mean(dim=1)
 
+    def _trunk_tf32_grouped(self, f1, f2, Wt, a_src, a_dst, groups):
+        """_trunk_tf32 with a BatchNorm group per B / groups envs: per-env statistics from the grouped trunk kernel (an
+        env's are the same bits at any batch position), the [groups, 128] affines applied by the pooling and the policy
+        head's prologue.  f1 [B*M,6], f2 [B*M,8] f32."""
+        w, H = self.w, self.H
+        B = f1.shape[0] // self.M
+        if B % groups:
+            raise ValueError("groups must divide the batch")
+        env_stats = torch.empty((B, 1, 2, 128), dtype=torch.float64, device=f1.device)
+        buf = gat_trunk_tf32_grouped(f1, f2, w["m_fea_1_fcl.weight"], w["m_fea_2_fcl.weight"], Wt, a_src, a_dst, env_stats, self.M)
+        sc, sh = bn_finalize_grouped(env_stats, self.M, groups, w["bn.weight"], w["bn.bias"])
+        self._pending_m = (sc, sh)
+        return buf.view(B, self.M, H), _graph_mean_raw(buf.view(B, self.M, H), sc, sh, relu=False)
+
     def parameters(self):
         return self.w.parameters()
 
@@ -931,8 +963,10 @@ class _MachineTrunk:
 
 
 class MachineActor(_MachineTrunk, _Twin):
-    """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498).  With groups > 1 the tf32
-    path normalises through mtfjsp_enc_bn_fwd: at most 65,535 groups per call (its grid.y)."""
+    """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498).  With 1 < groups < B the
+    tf32 path takes per-env statistics from the grouped trunk kernel and applies the [groups, 128] affines in the pooling
+    and the policy head.  With one env per group (or MTFJSP_FUSED_TRUNK=0 / MTFJSP_FUSED_HEAD=0) it normalises through
+    mtfjsp_enc_bn_fwd, which takes at most 65,535 groups per call (its grid.y)."""
 
     n_values = 2  # width of machine_v
 

@@ -55,6 +55,13 @@ class PPOConfig:
     encoder_tf32: bool = False  # every [rows,128] x [128,<=128] product of the update (graph encoders, GAT projections,
                                 # policy heads; > 95 % of its FLOPs) forward + backward on the hand-written tcgen05 TF32
                                 # kernels instead of library FP32 GEMMs under autograd
+    bn_group_envs: int | None = None  # BatchNorm statistics per buffered step AND per group of this many consecutive envs
+                                      # (the rollout's Rollout(bn_group_envs=...)): B envs train as B / bn_group_envs
+                                      # reference-sized batches side by side; None = per step over all B envs
+
+
+# grid.y limit of mtfjsp_enc_bn_fwd, the BatchNorm of the update's training path: BatchNorm groups per call
+_MAX_BN_GROUPS = 65535
 
 
 def _obs(bt, name, idx, nxt=False):
@@ -121,6 +128,22 @@ class MAPPOUpdate:
         self.allreduce_events = []   # (start, end) CUDA events of every gradient allreduce, for the time-share report
         self._shard_weight = {}      # B_local -> B_local * world / B_total (one tiny allreduce per batch size)
 
+    def _groups_per_step(self, B):
+        """BatchNorm groups in one buffered step of B envs."""
+        ge = self.cfg.bn_group_envs
+        if ge is None:
+            return 1
+        if ge < 1 or B % ge or B // ge > _MAX_BN_GROUPS:
+            raise ValueError("bn_group_envs must divide the env batch into at most %d groups" % _MAX_BN_GROUPS)
+        return B // ge
+
+    def _steps_per_chunk(self, steps, B, extra=0):
+        """`steps` capped so that (steps + extra) x groups-per-step stays within one BatchNorm call (grouped BatchNorm only:
+        with one group per step the chunking is as it always was)."""
+        if self.cfg.bn_group_envs is None:
+            return steps
+        return max(1, min(steps, _MAX_BN_GROUPS // self._groups_per_step(B) - extra))
+
     def _grad_weight(self, B, device):
         ws = _world()
         if ws == 1:
@@ -135,14 +158,15 @@ class MAPPOUpdate:
     def _critic_all(self, task_fea, adj_w, adj_src, mf1, mf2):
         """Global critic over all T buffered steps, T BatchNorm groups, chunked by whole steps."""
         T, B, N = task_fea.shape[:3]
-        per = max(1, (2 * self.max_rows) // (B * N))
+        per = self._steps_per_chunk(max(1, (2 * self.max_rows) // (B * N)), B)
+        gps = self._groups_per_step(B)
         out = []
         for t0 in range(0, T, per):
             t1 = min(T, t0 + per)
             g = t1 - t0
             v = self.critic.forward(task_fea[t0:t1].reshape(g * B, N, -1), adj_w[t0:t1].reshape(g * B, N, 2),
                                     adj_src[t0:t1].reshape(g * B, N), mf1[t0:t1].reshape(g * B, -1, 6),
-                                    mf2[t0:t1].reshape(g * B, -1, 8), groups=g)
+                                    mf2[t0:t1].reshape(g * B, -1, 8), groups=g * gps)
             out.append(v.reshape(g, B, 4))
         return torch.cat(out, dim=0)
 
@@ -181,7 +205,8 @@ class MAPPOUpdate:
         B = bt["candidate"].shape[1]
         J, M, H = self.job.J, self.job.M, self.job.H
         N = J * M
-        cs = max(1, min(S, self.max_rows // (B * N)))
+        cs = self._steps_per_chunk(max(1, min(S, self.max_rows // (B * N))), B, extra=1)  # the trunk takes one step more
+        gps = self._groups_per_step(B)
         take = lambda name, i=idx: bt[name].index_select(0, i)
         mse_sum = lambda a, b: ((a - b) ** 2).sum()
         inv = 1.0 / (S * B)
@@ -205,7 +230,7 @@ class MAPPOUpdate:
             p0 = max(s0 - 1, 0)
             ti = idx[p0:s1]
             nodes_m, pooled_m = self.mch.trunk(take("mach_fea1", ti).reshape(-1, M, 6), _obs(bt, "mach_fea2", ti).reshape(-1, M, 8),
-                                               groups=s1 - p0)
+                                               groups=(s1 - p0) * gps)
             pm = pooled_m.reshape(s1 - p0, B, H)
             gm = (torch.cat((inp, pm[:-1]), dim=0) if s0 == 0 else pm[:-1]).reshape(g * B, H)
             if s0 > 0:
@@ -215,7 +240,7 @@ class MAPPOUpdate:
             adst = _enc.ell_invert(asrc)
             chunks.append((ci, tf, aw, asrc, adst))
             prob_j, pooled_o, job_v = self.job.evaluate(tf, aw, asrc, take("candidate", ci).reshape(g * B, J), gm,
-                                                        take("job_mask", ci).reshape(g * B, J), groups=g, adj_dst=adst)
+                                                        take("job_mask", ci).reshape(g * B, J), groups=g * gps, adj_dst=adst)
             prob_m, mch_v = self.mch.heads(nodes_m, pooled_m, pooled_o, take("mach_mask", ci).reshape(g * B, M))
             prob_j, prob_m = prob_j.reshape(g, B, J), prob_m.reshape(g, B, M)
             job_v, mch_v = job_v.reshape(g, B, 2), mch_v.reshape(g, B, 2)
@@ -255,7 +280,7 @@ class MAPPOUpdate:
         for ci, tf, aw, asrc, adst in chunks:
             g = ci.numel()
             v_s = self.critic.forward(tf, aw, asrc, take("mach_fea1", ci).reshape(g * B, M, 6),
-                                      _obs(bt, "mach_fea2", ci).reshape(g * B, M, 8), groups=g, adj_dst=adst).reshape(g, B, 4)
+                                      _obs(bt, "mach_fea2", ci).reshape(g * B, M, 8), groups=g * gps, adj_dst=adst).reshape(g, B, 4)
             tg = adv["tgt_glob"].index_select(0, ci)
             rw = take("rw", ci)
             w_mk, w_ec, w_tt = rw[..., 0], rw[..., 1], rw[..., 2]
@@ -300,7 +325,8 @@ class MAPPOUpdate:
         T, B = bt["candidate"].shape[:2]
         J, M, H = self.job.J, self.job.M, self.job.H
         N = J * M
-        cs = max(1, self.max_rows // (B * N))
+        cs = self._steps_per_chunk(max(1, self.max_rows // (B * N)), B)
+        gps = self._groups_per_step(B)
         ep0 = bt.get("episode_start")
         dev = bt["candidate"].device
         with torch.no_grad():
@@ -311,7 +337,7 @@ class MAPPOUpdate:
                 g = s1 - s0
                 ii = torch.arange(s0, s1, device=dev)
                 nodes_m, pooled_m = self.mch.trunk(bt["mach_fea1"][s0:s1].reshape(-1, M, 6),
-                                                   _obs(bt, "mach_fea2", ii).reshape(-1, M, 8), groups=g)
+                                                   _obs(bt, "mach_fea2", ii).reshape(-1, M, 8), groups=g * gps)
                 pm = pooled_m.reshape(g, B, H)
                 gm = torch.cat((inp if prev is None else prev, pm[:-1]), dim=0).clone()
                 for t in range(s0, s1):
@@ -322,7 +348,7 @@ class MAPPOUpdate:
                 prob_j, pooled_o, _ = self.job.evaluate(
                     _obs(bt, "task_fea", ii).reshape(g * B, N, -1), _obs(bt, "adj_w", ii).reshape(g * B, N, 2),
                     _obs(bt, "adj_src", ii).reshape(g * B, N), bt["candidate"][s0:s1].reshape(g * B, J), gm.reshape(g * B, H),
-                    bt["job_mask"][s0:s1].reshape(g * B, J), groups=g)
+                    bt["job_mask"][s0:s1].reshape(g * B, J), groups=g * gps)
                 prob_m, _ = self.mch.heads(nodes_m, pooled_m, pooled_o, bt["mach_mask"][s0:s1].reshape(g * B, M))
                 la = torch.log(prob_j.gather(1, bt["a_job"][s0:s1].reshape(-1, 1).long()).squeeze(-1))
                 mla = torch.log(prob_m.gather(1, bt["a_mach"][s0:s1].reshape(-1, 1).long()).squeeze(-1))
@@ -367,33 +393,44 @@ def collect(rollout, weights_per_episode):
     """Runs len(weights_per_episode) episodes with `rollout` (Run.py:290-545) into a `buffer.RolloutBuffer` (each
     observation stored once; T = episodes * N buffered steps) and returns it: the batch `MAPPOUpdate.update` takes."""
     env = rollout.env
-    N = env.N
     job, mch = rollout.job, rollout.mch
     if isinstance(job, _enc.EsaJobActor) or isinstance(mch, _enc.EsaMachineActor):
         raise TypeError("the ESA-PPO actors are an evaluation baseline (the reference never trains them): roll them out "
                         "with rollout.Rollout / validate.greedy_validate, not into a PPO buffer")
     buf = RolloutBuffer(len(weights_per_episode), env)
     for w in weights_per_episode:
-        rollout.begin_episode(w)
-        wt = torch.as_tensor(w, dtype=torch.float32, device=env.device)
-        for s in range(N):
-            buf.store_pre(env, rollout)
-            rollout.step()
-            buf.store_post(env, rollout, wt)
-        t = buf.t
-        with torch.no_grad():                                                                        # Run.py:452-475
-            _, h_o, jv = job.evaluate(env.task_fea, env.adj_w, env.adj_src, env.candidate, rollout.h_mch, buf["job_mask"][t - 1])
-            _, _, mv = mch.forward(buf["mach_fea1"][t - 1], env.mach_fea, h_o, buf["mach_mask"][t - 1])
-        buf.store_bootstrap(jv, mv)
+        collect_episode(rollout, buf, w)
     return buf
 
 
-def train_iteration(rollout, updater, weights_per_episode, mini_bs=None):
-    """One buffer of experience followed by one PPO update (the body of the reference's training loop, Run.py:530-560).
-    `update` refreshes the rollout's inference twins afterwards, so the next call rolls out with the new weights.  When
-    the rollout runs on a different arithmetic path than the update (TF32 twin vs FP32 / tcgen05 training path), the
-    behaviour log-probabilities are re-evaluated on the update's path first (MAPPOUpdate.recompute_old_logp)."""
-    bt = collect(rollout, weights_per_episode)
+def collect_episode(rollout, buf, weights):
+    """One episode of `rollout` appended to `buf` (a RolloutBuffer with room for it); weights [B,3] per-env reward weights."""
+    env = rollout.env
+    job, mch = rollout.job, rollout.mch
+    rollout.begin_episode(weights)
+    wt = torch.as_tensor(weights, dtype=torch.float32, device=env.device)
+    for s in range(env.N):
+        buf.store_pre(env, rollout)
+        rollout.step()
+        buf.store_post(env, rollout, wt)
+    t = buf.t
+    with torch.no_grad():                                                                            # Run.py:452-475
+        _, h_o, jv = job.evaluate(env.task_fea, env.adj_w, env.adj_src, env.candidate, rollout.h_mch, buf["job_mask"][t - 1],
+                                  groups=rollout.groups)
+        _, _, mv = mch.forward(buf["mach_fea1"][t - 1], env.mach_fea, h_o, buf["mach_mask"][t - 1], groups=rollout.groups)
+    buf.store_bootstrap(jv, mv)
+
+
+def update_from_buffer(rollout, updater, bt, mini_bs=None, generator=None):
+    """The PPO update on a filled buffer.  `update` refreshes the rollout's inference twins afterwards, so the next episode
+    rolls out with the new weights.  When the rollout runs on a different arithmetic path than the update (TF32 twin vs
+    FP32 / tcgen05 training path), the behaviour log-probabilities are re-evaluated on the update's path first
+    (MAPPOUpdate.recompute_old_logp).  generator: draws the minibatch orders (MAPPOUpdate.update)."""
     if getattr(rollout.job, "precision", "fp32") != "fp32" and not updater.cfg.recompute_old_logp:
         updater.recompute_old_logp(bt)
-    return updater.update(bt, mini_bs or rollout.env.N)
+    return updater.update(bt, mini_bs or rollout.env.N, generator=generator)
+
+
+def train_iteration(rollout, updater, weights_per_episode, mini_bs=None):
+    """One buffer of experience followed by one PPO update (the body of the reference's training loop, Run.py:530-560)."""
+    return update_from_buffer(rollout, updater, collect(rollout, weights_per_episode), mini_bs)

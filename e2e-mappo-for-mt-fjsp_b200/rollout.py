@@ -27,9 +27,16 @@ def nvtx_range(name):
 
 
 class Rollout:
-    def __init__(self, env: BatchedMTFJSPEnv, job_actor, machine_actor, greedy=False, use_cuda_graph=False, seed=0):
+    def __init__(self, env: BatchedMTFJSPEnv, job_actor, machine_actor, greedy=False, use_cuda_graph=False, seed=0,
+                 bn_group_envs=None):
+        """bn_group_envs: every BatchNorm of both actors normalises over groups of this many consecutive envs (the
+        reference's env_batch), so B = G * bn_group_envs envs roll out as G independent reference-sized batches; None =
+        statistics over the whole batch."""
         assert env.obs_dtype == torch.float32, "the actors consume F32 observations"
         self.env, self.job, self.mch = env, job_actor, machine_actor
+        if bn_group_envs is not None and (bn_group_envs < 1 or env.B % bn_group_envs):
+            raise ValueError("bn_group_envs must divide the env batch")
+        self.groups = 1 if bn_group_envs is None else env.B // bn_group_envs
         self.greedy = greedy
         self.gen = torch.Generator(device=env.device)
         self.gen.manual_seed(seed)
@@ -70,12 +77,13 @@ class Rollout:
             rng = (self._rng_seed, self._rng_step) if self.fused_select else None
             with nvtx_range("mtfjsp/job_actor"):
                 ti, ai, la, prob, h_o, jv = self.job.forward(env.task_fea, env.adj_w, env.adj_src, env.candidate, h_in,
-                                                             env.job_mask, greedy=self.greedy, generator=self._g(), rng=rng)
+                                                             env.job_mask, greedy=self.greedy, generator=self._g(), rng=rng,
+                                                             groups=self.groups)
                 env.op.copy_(ti.to(torch.int32))
             with nvtx_range("mtfjsp/mfea1"):
                 m1, mmask = env.mfea1(env.op)
             with nvtx_range("mtfjsp/machine_actor"):
-                mp, h_m, mv = self.mch.forward(m1, env.mach_fea, h_o, mmask, return_logits=rng is not None)
+                mp, h_m, mv = self.mch.forward(m1, env.mach_fea, h_o, mmask, groups=self.groups, return_logits=rng is not None)
             if rng is not None:
                 mp, ma, mla, _ = enc_select(mp, mmask, None, 1.0, False, rng, 1)
                 self._rng_step.add_(1)

@@ -26,6 +26,38 @@ def load_actor_state_dicts(npz_path_or_dict, tag):
     return pick("op"), pick("mch")
 
 
+def load_checkpoint(job_pth, mch_pth, n_job, n_machine, precision="fp32", device=None, hidden=128):
+    """(JobActor, MachineActor) from two `torch.save`d state_dicts with the reference's key names: the
+    `PPO_job_actor_*.pth` / `PPO_machine_actor_*.pth` files `train.Trainer` writes, or the reference's own checkpoints
+    (Run.py:773-814).  The pair plugs straight into `greedy_validate` / `sampled_validate`."""
+    from .encoder import JobActor, MachineActor
+
+    ld = lambda f: torch.load(f, map_location="cpu", weights_only=True)
+    return (JobActor(ld(job_pth), n_job, n_machine, hidden=hidden, device=device, precision=precision),
+            MachineActor(ld(mch_pth), n_machine, hidden=hidden, device=device, precision=precision))
+
+
+def read_mip_csv(path):
+    """The MIP result CSV of the reference's solver runs (tester/Solver_seed*/MO_FJSP_MIP_result_(...).csv, parsed as
+    trainer/validate.py:14-58 does): a header row, then one row per instance of runtime, best_objective, Makespan,
+    MachineEC, MachineIdleT, TransEC -> dict of [S] float64 arrays under those names."""
+    import csv
+
+    with open(path, newline="") as f:
+        rows = list(csv.reader(f))
+    names = ("runtime", "best_objective", "Makespan", "MachineEC", "MachineIdleT", "TransEC")
+    data = np.array([[float(v) for v in r] for r in rows[1:] if r], dtype=np.float64).reshape(-1, len(names))
+    return {n: data[:, i] for i, n in enumerate(names)}
+
+
+def mip_gaps(final4, mip, weights=(0.4, 0.4, 0.2)):
+    """Relative gaps to the MIP solutions (Run.py:708-716): per instance (cost - mip) / mip of makespan, processing
+    energy, transport time and idle time [S,4], and their weighted sum w_mk g_mk + w_ec (g_pt + g_idle) + w_tt g_tt [S]."""
+    ref = np.stack((mip["Makespan"], mip["MachineEC"], mip["TransEC"], mip["MachineIdleT"]), axis=-1)[: len(final4)]
+    g = (np.asarray(final4) - ref) / ref
+    return g, _objective(g, weights)
+
+
 def _objective(final4, weights):
     w = weights
     return w[0] * final4[..., 0] + w[1] * (final4[..., 1] + final4[..., 3]) + w[2] * final4[..., 2]

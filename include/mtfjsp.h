@@ -349,6 +349,14 @@ int mtfjsp_enc_head_tf32_grouped(const float* X, const int32_t* cand, int64_t B,
                                  const float* b2, float* out, void* stream);
 int mtfjsp_enc_bn_finalize_grouped(const double* env_stats, int64_t B, int rows_per_env, int envs_per_group, const float* gamma,
                                    const float* beta, float eps, float* scale, float* shift, int C, void* stream);
+/* mtfjsp_enc_gat_trunk_tf32 over B envs of M machines (M <= 128) with per-env statistics: tiles of (128 / M) * M machines
+ * of whole envs, out [B*M,128] as there, and instead of `stats` env_stats [B,1,2,128] f64 = per env the column sums of
+ * out and of out^2 (written, no atomics; each env's rows added in row order in FP64, so the same bits at any batch
+ * position).  mtfjsp_enc_bn_finalize_grouped(env_stats, B, M, ...) turns them into the [G,128] affines that
+ * graph_mean_grouped and head_tf32_grouped apply: the machine trunk with per-group BatchNorm and no normalisation pass. */
+int mtfjsp_enc_gat_trunk_tf32_grouped(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
+                                      const float* a_src, const float* a_dst, float* out, double* env_stats, int64_t B, int M,
+                                      void* stream);
 
 /* replaces: the per-reward GAE of algorithm/ppo_algorithm.py:438-536 (python loop over buffered steps per stream).
  * r, v, v_next, adv: [T,B,4] f32 (streams mk, pt, tt, idle); done [T,B] f32; stats[8] f64 accumulates per-stream
