@@ -142,7 +142,8 @@ __global__ void graph_mean_kernel(const float* __restrict__ h, float* __restrict
 constexpr int BN_ROWS = 512;  // rows of one group per block
 
 // column sums of (a, b) over this block's rows -> FP64 atomics into acc[g][0][C], acc[g][1][C]
-// MODE 0: a = x, b = x*x (statistics);  MODE 1: a = g', b = g' * xhat (backward sums), g' = gy * [y > 0]
+// MODE 0: a = x - p, b = (x - p)^2 with p the group's first row (statistics, shifted so that E[a^2] - E[a]^2 does not
+//         cancel when |mean| >> std);  MODE 1: a = g', b = g' * xhat (backward sums), g' = gy * [y > 0]
 template <int MODE>
 __global__ void __launch_bounds__(256) bn_reduce_kernel(const float4* __restrict__ x, const float4* __restrict__ gy,
                                                         const float* __restrict__ w, const float* __restrict__ b,
@@ -156,6 +157,7 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const float4* __restrict
     const int C = C4 * 4;
     float4 sa = make_float4(0.f, 0.f, 0.f, 0.f), sb = sa;
     float4 mu = sa, rs = sa, ww = sa, bb = sa;
+    if (MODE == 0) mu = __ldg(x + (size_t)g * R * C4 + cq);  // the shift p
     if (MODE == 1) {
         mu = reinterpret_cast<const float4*>(mean + (size_t)g * C)[cq];
         rs = reinterpret_cast<const float4*>(rstd + (size_t)g * C)[cq];
@@ -167,8 +169,9 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const float4* __restrict
             const size_t i = ((size_t)g * R + r) * C4 + cq;
             const float4 v = __ldg(x + i);
             if (MODE == 0) {
-                sa.x += v.x; sa.y += v.y; sa.z += v.z; sa.w += v.w;
-                sb.x = fmaf(v.x, v.x, sb.x); sb.y = fmaf(v.y, v.y, sb.y); sb.z = fmaf(v.z, v.z, sb.z); sb.w = fmaf(v.w, v.w, sb.w);
+                const float4 d = make_float4(v.x - mu.x, v.y - mu.y, v.z - mu.z, v.w - mu.w);
+                sa.x += d.x; sa.y += d.y; sa.z += d.z; sa.w += d.w;
+                sb.x = fmaf(d.x, d.x, sb.x); sb.y = fmaf(d.y, d.y, sb.y); sb.z = fmaf(d.z, d.z, sb.z); sb.w = fmaf(d.w, d.w, sb.w);
             } else {
                 float4 d = __ldg(gy + i);
                 const float4 xh = make_float4((v.x - mu.x) * rs.x, (v.y - mu.y) * rs.y, (v.z - mu.z) * rs.z, (v.w - mu.w) * rs.w);
@@ -196,15 +199,16 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const float4* __restrict
     }
 }
 
-__global__ void bn_stats_finalize_kernel(const double* __restrict__ acc, double inv_rows, float eps, float* mean, float* rstd,
-                                         int G, int C) {
+// acc holds the sums of x - p and (x - p)^2 with p = x[g, 0, c] (bn_reduce_kernel<0>)
+__global__ void bn_stats_finalize_kernel(const double* __restrict__ acc, const float* __restrict__ x, long long R, double inv_rows,
+                                         float eps, float* mean, float* rstd, int G, int C) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= G * C) return;
     const int g = i / C, c = i - g * C;
     const double m = acc[((size_t)g * 2) * C + c] * inv_rows;
     double var = acc[((size_t)g * 2 + 1) * C + c] * inv_rows - m * m;  // biased, as torch normalises in training mode
     if (var < 0) var = 0;
-    mean[i] = (float)m;
+    mean[i] = (float)((double)__ldg(x + (size_t)g * R * C + c) + m);
     rstd[i] = (float)(1.0 / sqrt(var + (double)eps));
 }
 
@@ -615,7 +619,8 @@ int mtfjsp_enc_bn_fwd(const float* x, const float* w, const float* b, float eps,
     if (cudaMemsetAsync(workspace, 0, (size_t)G * 2 * C * sizeof(double), s) != cudaSuccess) return MTFJSP_E_CUDA;
     bn_reduce_kernel<0><<<grid, threads, smem, s>>>(reinterpret_cast<const float4*>(x), nullptr, w, b, nullptr, nullptr, workspace,
                                                     R, C4, 0);
-    bn_stats_finalize_kernel<<<(unsigned)((G * C + 255) / 256), 256, 0, s>>>(workspace, 1.0 / (double)R, eps, mean, rstd, (int)G, C);
+    bn_stats_finalize_kernel<<<(unsigned)((G * C + 255) / 256), 256, 0, s>>>(workspace, x, R, 1.0 / (double)R, eps, mean, rstd,
+                                                                          (int)G, C);
     bn_apply_kernel<0><<<grid, threads, 0, s>>>(reinterpret_cast<const float4*>(x), nullptr, w, b, mean, rstd, nullptr,
                                                 reinterpret_cast<float4*>(y), R, C4, relu, 0.f);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;

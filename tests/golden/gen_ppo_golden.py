@@ -48,7 +48,10 @@ def load():
     return ppo_algorithm, actor_critic, g_pool_cal, replaybuffer
 
 
-def main():
+def run_update(before_update=None):
+    """Fills the reference ReplayBuffer along the recorded trajectory and runs the reference update once.
+    before_update(ppo): called with the PPOAlgorithm object right before the update (e.g. to wrap its optimisers).
+    -> (out, nets): the arrays of ppo_golden.npz without the updated parameters, and the three reference modules."""
     pa, ac, g_pool_cal, rb = load()
     g = np.load(os.path.join(HERE, "replay_j6m6_ls_esa.npz"))
     J, M = int(g["J"]), int(g["M"])
@@ -137,6 +140,8 @@ def main():
             return iter(idx)
 
     pa.SubsetRandomSampler = Recording
+    if before_update is not None:
+        before_update(ppo)
     torch.manual_seed(2024)
     with contextlib.redirect_stdout(io.StringIO()):
         loss_mean, loss_std = ppo.global_update_JointActions_GAT_selfCritic(buf, EP * N, gp, args, N)
@@ -146,7 +151,12 @@ def main():
            "log_a": buf.a_logprob_operation.numpy(), "m_log_a": buf.a_logprob.numpy(),
            "job_v": buf.job_v.numpy(), "mch_v": buf.machine_v.numpy(), "job_v_n": buf.job_v_.numpy(),
            "mch_v_n": buf.machine_v_.numpy(), "mach_mask": buf.mask_machine_.numpy().reshape(EP * N, B, M)}
-    for tag, net in (("job", job), ("mch", mch), ("crit", crit)):
+    return out, (("job", job), ("mch", mch), ("crit", crit))
+
+
+def main():
+    out, nets = run_update()
+    for tag, net in nets:
         for k, v in net.state_dict().items():
             if enc._Params.is_parameter(k):
                 out["%s/%s" % (tag, k)] = v.detach().numpy().astype(np.float32)
