@@ -84,12 +84,9 @@ SIGNATURES = {
     "mtfjsp_enc_aggregate_bwd": ([_VP, _VP, _VP, _VP, _VP, C.c_int64, _I, _I, _VP], _I),
     "mtfjsp_enc_graph_mean": ([_VP, _VP, C.c_int64, _I, _I, _VP, _VP, _I, _VP], _I),
     "mtfjsp_enc_linear_tf32": ([_VP, C.c_int64, _I, _VP, _VP, _VP, _VP, _I, _VP, _VP, _VP], _I),
-    "mtfjsp_enc_mach_proj": ([_VP, _VP, _VP, _VP, _VP, C.c_int64, _VP], _I),
     "mtfjsp_enc_gat_attend": ([_VP, _VP, _VP, _VP, C.c_int64, _I, _VP], _I),
     "mtfjsp_enc_gat_attend_bwd": ([_VP, _VP, _VP, _VP, _VP, _VP, C.c_int64, _I, _VP], _I),
     "mtfjsp_enc_gat_attend_bwd_blocks": ([C.c_int64], _I),
-    "mtfjsp_enc_bias_tanh": ([_VP, _VP, C.c_int64, _I, C.c_int64, _VP], _I),
-    "mtfjsp_enc_tanh_dot": ([_VP, _VP, _VP, _VP, C.c_int64, _VP], _I),
     "mtfjsp_enc_gat_trunk_tf32": ([_VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, C.c_int64, _VP], _I),
     "mtfjsp_enc_aggregate_linear_tf32": ([_VP, C.c_int64, _I, _VP, _VP, _VP, _VP, _VP, _VP, _I, _VP, _VP, _VP], _I),
     "mtfjsp_enc_select": ([_VP, _VP, _VP, C.c_float, _I, C.c_int64, _I, _U64, _VP, _I, _VP, _VP, _VP, _VP, _VP], _I),

@@ -315,36 +315,6 @@ __device__ __forceinline__ float warp_sum(float v) {
 __device__ __forceinline__ float dot4(const float4 a, const float4 b) { return a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w; }
 __device__ __forceinline__ float elu1(float x) { return x > 0.f ? x : expm1f(x); }
 
-// m_fea_1_fcl / m_fea_2_fcl (actor_critic.py:381-392, bias-free Linear(6,128) and Linear(8,128)) written as the two row
-// blocks of ONE [2R,128] buffer -- the layout the GAT projection reads, so no torch.cat.
-__global__ void __launch_bounds__(256) mach_proj_kernel(const float* __restrict__ f1, const float* __restrict__ f2,
-                                                        const float* __restrict__ W1, const float* __restrict__ W2,
-                                                        float4* __restrict__ out, long long R) {
-    // blockIdx.y picks the projection; a lane keeps its four weight rows in registers and the warp walks rows
-    const bool second = blockIdx.y == 1;
-    const int K = second ? 8 : 6;
-    const float* __restrict__ f = second ? f2 : f1;
-    const float* __restrict__ W = second ? W2 : W1;  // [128, K]
-    const int lane = threadIdx.x & 31;
-    float wr[4][8];
-#pragma unroll
-    for (int j = 0; j < 4; j++)
-#pragma unroll
-        for (int k = 0; k < 8; k++) wr[j][k] = k < K ? __ldg(W + (lane * 4 + j) * K + k) : 0.f;
-    const long long nw = (long long)gridDim.x * (blockDim.x >> 5);
-    for (long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); row < R; row += nw) {
-        const float xl = lane < K ? __ldg(f + row * K + lane) : 0.f;  // one coalesced load, broadcast by shuffle
-        float o[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-            const float xk = __shfl_sync(0xffffffffu, xl, k);
-#pragma unroll
-            for (int j = 0; j < 4; j++) o[j] = fmaf(xk, wr[j][k], o[j]);
-        }
-        out[((second ? R : 0) + row) * 32 + lane] = make_float4(o[0], o[1], o[2], o[3]);
-    }
-}
-
 // GATLayer.forward on the fixed 2-node graph after the projection (model/gat.py:82-159): t = [t1; t2] ([2R,128]),
 //   e11 = lrelu(t1.a_src + t1.a_dst), e12 = lrelu(t1.a_src + t2.a_dst), att = softmax(e11, e12),
 //   h1' = att0 t1 + att1 t2, h2' = t2.
@@ -439,32 +409,6 @@ __global__ void __launch_bounds__(256) gat_attend_bwd_kernel(const float4* __res
         }
         reinterpret_cast<float4*>(dparts)[((size_t)blockIdx.x * 2 + which) * 32 + lane] = a;
     }
-}
-
-// first layer of a policy head after its per-row product (encoder._head_tf32): z[r] = tanh(z[r] + bias[r / rows_per_env]),
-// in place; bias [B,128] or a single row (bias_rows == 1)
-__global__ void __launch_bounds__(256) bias_tanh_kernel(float4* __restrict__ z, const float4* __restrict__ bias, long long rows,
-                                                        int rows_per_env, long long bias_rows) {
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= rows * 32) return;
-    const long long row = idx >> 5;
-    const int c = (int)(idx & 31);
-    const long long e = bias_rows == 1 ? 0 : row / rows_per_env;
-    float4 v = z[idx];
-    const float4 b = __ldg(bias + e * 32 + c);
-    z[idx] = make_float4(tanhf(v.x + b.x), tanhf(v.y + b.y), tanhf(v.z + b.z), tanhf(v.w + b.w));
-}
-
-// last two steps of a policy head: out[r] = tanh(z[r]) . w + b   (tanh of the second layer, then Linear(128, 1))
-__global__ void __launch_bounds__(256) tanh_dot_kernel(const float4* __restrict__ z, const float4* __restrict__ w,
-                                                       const float* __restrict__ b, float* __restrict__ out, long long rows) {
-    const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (row >= rows) return;
-    const float4 v = __ldg(z + row * 32 + lane);
-    const float4 t = make_float4(tanhf(v.x), tanhf(v.y), tanhf(v.z), tanhf(v.w));
-    const float s = warp_sum(dot4(t, __ldg(w + lane)));
-    if (lane == 0) out[row] = s + (b ? __ldg(b) : 0.f);
 }
 
 
@@ -684,15 +628,6 @@ int mtfjsp_enc_graph_mean_grouped(const float* h, float* out, int64_t B, int N, 
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 
-int mtfjsp_enc_mach_proj(const float* fea1, const float* fea2, const float* W1, const float* W2, float* out, int64_t R,
-                         void* stream) {
-    if (!fea1 || !fea2 || !W1 || !W2 || !out || R < 1) return MTFJSP_E_ARG;
-    const long long blocks = (R + 7) / 8;
-    mach_proj_kernel<<<dim3((unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), 2), 256, 0, (cudaStream_t)stream>>>(
-        fea1, fea2, W1, W2, reinterpret_cast<float4*>(out), R);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
-}
-
 int mtfjsp_enc_gat_attend(const float* t, const float* a_src, const float* a_dst, float* out, int64_t R, int mode,
                           void* stream) {
     if (!t || !a_src || !a_dst || !out || R < 1 || mode < 0 || mode > 2) return MTFJSP_E_ARG;
@@ -713,21 +648,6 @@ int mtfjsp_enc_gat_attend_bwd(const float* t, const float* a_src, const float* a
     gat_attend_bwd_kernel<<<mtfjsp_enc_gat_attend_bwd_blocks(R), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4*>(t), reinterpret_cast<const float4*>(a_src), reinterpret_cast<const float4*>(a_dst),
         reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(dt), dparts, R, mode);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
-}
-
-int mtfjsp_enc_bias_tanh(float* z, const float* bias, int64_t rows, int rows_per_env, int64_t bias_rows, void* stream) {
-    if (!z || !bias || rows < 1 || rows_per_env < 1 || (bias_rows != 1 && bias_rows * rows_per_env != rows)) return MTFJSP_E_ARG;
-    const long long total = rows * 32;
-    bias_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<float4*>(z), reinterpret_cast<const float4*>(bias), rows, rows_per_env, bias_rows);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
-}
-
-int mtfjsp_enc_tanh_dot(const float* z, const float* w, const float* b, float* out, int64_t rows, void* stream) {
-    if (!z || !w || !out || rows < 1) return MTFJSP_E_ARG;
-    tanh_dot_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
-        reinterpret_cast<const float4*>(z), reinterpret_cast<const float4*>(w), b, out, rows);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 

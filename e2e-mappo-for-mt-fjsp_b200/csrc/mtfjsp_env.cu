@@ -762,21 +762,10 @@ struct Spec {
         const int b = by_smem < by_threads ? by_smem : by_threads;
         return b < 32 ? b : 32;
     }
-    static constexpr int BTT_FULL = NOTT ? 0 : TT * 8;
-    // TTG (G = 8, compile with -DMTFJSP_SPEC_TTG=1; off): the transport table is read through L1 (prefetched when the block
-    // starts) instead of being staged, together with the two-chunk idle buffer, where that puts one more block on an SM
-    // (J6M6: 6 -> 7 blocks, 4.6 -> 3.95 waves of 65,536 envs).  Measured and rejected: the 72-register cap that seven
-    // 128-thread blocks need spills 64 bytes in the observation modes and the table reads lengthen the step's dependent
-    // chain -- one-launch random step 72.5 us against 64.5, transition alone 49.2 against 44.2 (profiles/README.md, r3w)
-#ifndef MTFJSP_SPEC_TTG
-#define MTFJSP_SPEC_TTG 0
-#endif
-    static constexpr bool TTG = MTFJSP_SPEC_TTG && !NOTT && G_ == 8 && minb(NPT_CHUNK, 0) > minb(NPT_FULL, BTT_FULL) &&
-                                minb(NPT_CHUNK, 0) > minb(NPT_CHUNK, BTT_FULL);
-    static constexpr int B_TT = TTG ? 0 : BTT_FULL;
+    static constexpr int B_TT = NOTT ? 0 : TT * 8;
     // CHUNK: the idle terms pass through the two-chunk buffer.  Always with COLD; without it wherever the smaller scratch
     // lets one more block onto an SM (J10M10: 18 -> 19 blocks, 3.07 -> 2.91 waves of 16,384 envs)
-    static constexpr bool CHUNK = COLD_ || TTG || minb(NPT_CHUNK, B_TT) > minb(NPT_FULL, B_TT);
+    static constexpr bool CHUNK = COLD_ || minb(NPT_CHUNK, B_TT) > minb(NPT_FULL, B_TT);
     static constexpr int NPT = CHUNK ? NPT_CHUNK : NPT_FULL;
     static_assert(NPT >= 3 * M, "the random-step mode parks three compacted machine rows in the idle-term scratch");
     static constexpr int B_PT = NPT * 8;
@@ -1032,12 +1021,6 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
         if (gl == 0) bulk_g2s(s_pt, g_sd + SC0, (S::SD - SC0) * 8, bar);
         if (gl < 3) wv = P.weights[(size_t)bc * 3 + gl];
     }
-    if constexpr (S::TTG) {  // the transport table (M * M doubles) into L1: the step reads a few entries of it
-        if (gl < 4) {
-            const int o = gl * 16 < M * M - 1 ? gl * 16 : M * M - 1;
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(g_xs + S::O_TT + o));
-        }
-    }
     double tr = 0.0, pr = 0.0;  // MODE_POLICY, lane k < M: t[op][k], p[op][k]
     int nsel = 1;
     if constexpr ((MODE & MODE_POLICY) != 0) {
@@ -1132,7 +1115,7 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     // duration / selected power of op v: shared memory, or (COLD) straight from the state record in HBM.  The stepped
     // op's own values are in registers (d, pa): its HBM words are written by this very launch.
     auto TT = [&](const int i, const int j) -> double {
-        if constexpr (S::NOTT || S::TTG) return __ldg(g_xs + S::O_TT + i * M + j);
+        if constexpr (S::NOTT) return __ldg(g_xs + S::O_TT + i * M + j);
         else return s_tt[i * M + j];
     };
     bool stepped = false;  // set once the action is known to be valid
@@ -2254,15 +2237,13 @@ struct mtfjsp_env {
     const void* obs_ptrs[4];
     int obs_dtype;
     int host_zerocopy;             // MTFJSP_HOST_ZEROCOPY: packed host step writes records straight to mapped host memory
-    int host_chunks, fuse_policy;  // tuning knobs read from the environment at create time (tests compare the settings)
-    int alternate_order, flip;     // MTFJSP_ALTERNATE_ORDER (default on): successive step launches walk the batch in
-                                   // opposite directions for L2 reuse
-    // MTFJSP_L2_PERSIST (default on): the small records every launch starts from -- job masks, candidates, the si record
-    // (route order, counters) -- live in one slab that step launches mark as an L2-persisting access window, so the loads
-    // at the head of a warp's dependent chain hit L2 instead of DRAM although the batch's working set is larger than L2
+    int fuse_policy;  // MTFJSP_FUSE_POLICY, read from the environment at create time (tests compare the settings)
+    int flip;         // successive eager step launches walk the batch in opposite directions for L2 reuse (Params::rev)
+    // The small records every launch starts from -- job masks, candidates, the si record (route order, counters) -- live
+    // in one slab that step launches mark as an L2-persisting access window, so the loads at the head of a warp's
+    // dependent chain hit L2 instead of DRAM although the batch's working set is larger than L2
     unsigned char* slab;
     size_t slab_bytes, window_bytes;
-    int l2_persist;
     int64_t launches;
     // MTFJSP_LAUNCH_OVERLAP (default on): whole-batch step launches of the size-specialised kernel may start while the
     // previous one finishes (programmatic dependent launch; see ovl_wait).  done_ep: one completion epoch per warp-sized
@@ -2281,10 +2262,10 @@ struct mtfjsp_env {
 // streams -- copy-in c -> kernel c -> copy-out c, kernels in chunk order on ONE stream -- so that chunk c's copy-out
 // overlaps chunk c+1's kernel.  (Round 1 gave every chunk its own stream: the block scheduler then interleaves the blocks
 // of all chunk kernels, every chunk finishes near the end and no copy-out can start early: 161 us per 65,536-env step
-// against 174 us unchunked.  `MTFJSP_HOST_PIPE=0` restores that form.)  The whole fan-out is captured once per set of
-// buffer addresses into a CUDA graph and replayed with a single launch call per step.
+// against 174 us unchunked.)  The whole fan-out is captured once per set of buffer addresses into a CUDA graph and
+// replayed with a single launch call per step.
 struct HostPipe {
-    static constexpr int MAXC = 8;
+    static constexpr int MAXC = 8, CHUNKS = 4;  // most chunks, and the chunk count aimed at
     cudaStream_t ms, cs[MAXC];
     cudaEvent_t fork, join[MAXC], hev[MAXC], kev[MAXC];
     struct Entry {
@@ -2384,8 +2365,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
         const int rc = flush_reset(h, s);
         if (rc != MTFJSP_OK) return rc;
     }
-    static const size_t extra = getenv("MTFJSP_EXTRA_SMEM") ? (size_t)atoi(getenv("MTFJSP_EXTRA_SMEM")) : 0;  // occupancy experiments
-    const size_t smem = (size_t)S::WARPS * S::EPW * S::ENV_BYTES + (S::BAR_IN_PAD ? 0 : 16 * ((S::WARPS * 8 + 15) / 16)) + extra;
+    const size_t smem = (size_t)S::WARPS * S::EPW * S::ENV_BYTES + (S::BAR_IN_PAD ? 0 : 16 * ((S::WARPS * 8 + 15) / 16));
     static thread_local int configured_dev = -1;
     if (configured_dev != h->device) {
         CK(cudaFuncSetAttribute(env_kernel_s<S, MODE, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
@@ -2395,7 +2375,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     const int per_block = S::WARPS * S::EPW;
     const int blocks = (P.b1 - P.b0 + per_block - 1) / per_block;
     Params Q = P;
-    if (h->alternate_order && (MODE & MODE_STEP)) {  // eager step launches alternate direction (see Params::rev)
+    if (MODE & MODE_STEP) {  // eager step launches alternate direction (see Params::rev)
         Q.rev = h->flip;
         h->flip ^= 1;
     }
@@ -2635,11 +2615,9 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
     {
         const char* fg = getenv("MTFJSP_FORCE_GENERIC");  // test hook: run the generic kernel on every size
         h->force_generic = fg && fg[0] == '1';
-        h->host_chunks = getenv("MTFJSP_HOST_CHUNKS") ? atoi(getenv("MTFJSP_HOST_CHUNKS")) : 4;
         // default: records zero-copy; the actions too from 16,384 envs up (below that the explicit copy is as fast)
         h->host_zerocopy = getenv("MTFJSP_HOST_ZEROCOPY") ? atoi(getenv("MTFJSP_HOST_ZEROCOPY")) : (B >= 16384 ? 2 : 1);
         h->fuse_policy = getenv("MTFJSP_FUSE_POLICY") ? atoi(getenv("MTFJSP_FUSE_POLICY")) : 1;
-        h->alternate_order = getenv("MTFJSP_ALTERNATE_ORDER") ? atoi(getenv("MTFJSP_ALTERNATE_ORDER")) : 1;
         h->obs_inc_allowed = !(getenv("MTFJSP_OBS_INCREMENTAL") && atoi(getenv("MTFJSP_OBS_INCREMENTAL")) == 0);  // test hook
         h->fused_reset = getenv("MTFJSP_FUSED_RESET") ? atoi(getenv("MTFJSP_FUSED_RESET")) : 1;
         h->launch_overlap = getenv("MTFJSP_LAUNCH_OVERLAP") ? atoi(getenv("MTFJSP_LAUNCH_OVERLAP")) : 1;
@@ -2664,20 +2642,17 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
         h->si = reinterpret_cast<int16_t*>(h->slab + 2 * b_jm + b_cd);
         h->xs = reinterpret_cast<double*>(h->slab + 2 * b_jm + b_cd + b_si);  // static tables (transport table, min durations)
         h->window_bytes = 0;
-        h->l2_persist = getenv("MTFJSP_L2_PERSIST") ? atoi(getenv("MTFJSP_L2_PERSIST")) : 1;  // 2: the static tables as well
-        if (h->l2_persist) {
-            cudaDeviceProp prop;
-            if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
-                size_t want = h->l2_persist >= 2 ? h->slab_bytes : h->slab_bytes - b_xs;
-                if (want > (size_t)prop.accessPolicyMaxWindowSize) want = (size_t)prop.accessPolicyMaxWindowSize;
-                size_t carve = want < (size_t)prop.persistingL2CacheMaxSize ? want : (size_t)prop.persistingL2CacheMaxSize;
-                size_t cur = 0;
-                cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize);
-                if (cur < carve) cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve);
-                h->window_bytes = want;
-            }
-            cudaGetLastError();
+        cudaDeviceProp prop;
+        if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
+            size_t want = h->slab_bytes - b_xs;  // the window leaves out the static tables
+            if (want > (size_t)prop.accessPolicyMaxWindowSize) want = (size_t)prop.accessPolicyMaxWindowSize;
+            size_t carve = want < (size_t)prop.persistingL2CacheMaxSize ? want : (size_t)prop.persistingL2CacheMaxSize;
+            size_t cur = 0;
+            cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize);
+            if (cur < carve) cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve);
+            h->window_bytes = want;
         }
+        cudaGetLastError();
     }
     ALLOC(h->t, Bs * N * M * 8);
     ALLOC(h->p, Bs * N * M * 8);
@@ -2807,11 +2782,9 @@ int mtfjsp_reset(mtfjsp_env* h, const double* weights, void* stream) {
     int rc = launch_env<MODE_RESET, double>(h, P, s);
     if (rc != MTFJSP_OK) return rc;
     h->reset_done = true;
-    if (!getenv("MTFJSP_RESET_SNAPSHOT") || atoi(getenv("MTFJSP_RESET_SNAPSHOT")) != 0) {
-        CK(cudaMemcpyAsync(h->sd0, h->sd, (size_t)L.B * L.sd_stride * 8, cudaMemcpyDeviceToDevice, s), "snapshot sd");
-        CK(cudaMemcpyAsync(h->si0, h->si, (size_t)L.B * L.si_stride * 2, cudaMemcpyDeviceToDevice, s), "snapshot si");
-        h->reset_snap = true;
-    }
+    CK(cudaMemcpyAsync(h->sd0, h->sd, (size_t)L.B * L.sd_stride * 8, cudaMemcpyDeviceToDevice, s), "snapshot sd");
+    CK(cudaMemcpyAsync(h->si0, h->si, (size_t)L.B * L.si_stride * 2, cudaMemcpyDeviceToDevice, s), "snapshot si");
+    h->reset_snap = true;
     return MTFJSP_OK;
 }
 
@@ -3082,10 +3055,9 @@ static int host_step_impl(mtfjsp_env* h, const HostIO& io, void* task_fea, void*
         if (rc == MTFJSP_OK) rc = copy_out(b0, b1, q);
         return rc;
     };
-    const int want_chunks = h->host_chunks;  // MTFJSP_HOST_CHUNKS, 0: no graph
     const bool pinned = is_pinned(io.op) && is_pinned(io.mach) && is_pinned(io.act) && is_pinned(io.info6) &&
                         is_pinned(io.jm) && is_pinned(io.cand) && is_pinned(io.rec);
-    if (!pinned || want_chunks <= 0) {
+    if (!pinned) {
         // pageable buffers: the copies are staged by the driver and cannot overlap; plain in-order sequence
         int rc = chunk(0, L.B, s);
         if (rc) return rc;
@@ -3149,11 +3121,10 @@ static int host_step_impl(mtfjsp_env* h, const HostIO& io, void* task_fea, void*
     }
     HostPipe* hp = h->pipe;
     // chunks of whole 256-env groups, at least 4,096 envs each (below that one launch does not fill the GPU)
-    int chunks = want_chunks > HostPipe::MAXC ? HostPipe::MAXC : want_chunks;
+    int chunks = HostPipe::CHUNKS;
     while (chunks > 1 && L.B / chunks < 4096) chunks--;
     int per = ((L.B + chunks - 1) / chunks + 255) / 256 * 256;
-    static const int ordered = getenv("MTFJSP_HOST_PIPE") ? atoi(getenv("MTFJSP_HOST_PIPE")) : 1;
-    if (ordered && !h->force_generic && chunks > 1) {  // whole waves per chunk (the chunk kernels run one after the other)
+    if (!h->force_generic && chunks > 1) {  // whole waves per chunk (the chunk kernels run one after the other)
         static thread_local int wave_J = -1, wave_M = -1, wave_dev = -1, wave = 0;
         if (wave_J != L.J || wave_M != L.M || wave_dev != h->device) {
             wave = envs_per_wave(L.J, L.M, h->device);
@@ -3182,42 +3153,28 @@ static int host_step_impl(mtfjsp_env* h, const HostIO& io, void* task_fea, void*
         CK(cudaStreamBeginCapture(hp->ms, cudaStreamCaptureModeRelaxed), "cudaStreamBeginCapture");
         int rc = MTFJSP_OK;
         cudaError_t ce = cudaEventRecord(hp->fork, hp->ms);
-        if (ordered) {
-            cudaStream_t qi = hp->cs[0], qk = hp->cs[1], qo = hp->cs[2];  // copies in, kernels (in chunk order), copies out
-            for (int k = 0; k < 3 && ce == cudaSuccess; k++) ce = cudaStreamWaitEvent(hp->cs[k], hp->fork, 0);
-            auto range = [&](int c, int& b0, int& b1) { b0 = c * per; b1 = (c + 1) * per < L.B ? (c + 1) * per : L.B; return b0 < b1; };
-            int b0, b1;
-            for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-                rc = copy_in(b0, b1, qi);
-                if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->hev[c], qi);
-            }
-            for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-                ce = cudaStreamWaitEvent(qk, hp->hev[c], 0);
-                if (ce != cudaSuccess) break;
-                rc = kernel(b0, b1, qk);
-                if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->kev[c], qk);
-            }
-            for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-                ce = cudaStreamWaitEvent(qo, hp->kev[c], 0);
-                if (ce != cudaSuccess) break;
-                rc = copy_out(b0, b1, qo);
-            }
-            for (int k = 0; k < 3 && rc == MTFJSP_OK && ce == cudaSuccess; k++) {
-                ce = cudaEventRecord(hp->join[k], hp->cs[k]);
-                if (ce == cudaSuccess) ce = cudaStreamWaitEvent(hp->ms, hp->join[k], 0);
-            }
-        } else {
-            for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess; c++) {
-                const int b0 = c * per, b1 = (c + 1) * per < L.B ? (c + 1) * per : L.B;
-                if (b0 >= b1) break;
-                cudaStream_t q = hp->cs[c];
-                ce = cudaStreamWaitEvent(q, hp->fork, 0);
-                if (ce != cudaSuccess) break;
-                rc = chunk(b0, b1, q);
-                if (rc) break;
-                ce = cudaEventRecord(hp->join[c], q);
-                if (ce == cudaSuccess) ce = cudaStreamWaitEvent(hp->ms, hp->join[c], 0);
-            }
+        cudaStream_t qi = hp->cs[0], qk = hp->cs[1], qo = hp->cs[2];  // copies in, kernels (in chunk order), copies out
+        for (int k = 0; k < 3 && ce == cudaSuccess; k++) ce = cudaStreamWaitEvent(hp->cs[k], hp->fork, 0);
+        auto range = [&](int c, int& b0, int& b1) { b0 = c * per; b1 = (c + 1) * per < L.B ? (c + 1) * per : L.B; return b0 < b1; };
+        int b0, b1;
+        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
+            rc = copy_in(b0, b1, qi);
+            if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->hev[c], qi);
+        }
+        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
+            ce = cudaStreamWaitEvent(qk, hp->hev[c], 0);
+            if (ce != cudaSuccess) break;
+            rc = kernel(b0, b1, qk);
+            if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->kev[c], qk);
+        }
+        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
+            ce = cudaStreamWaitEvent(qo, hp->kev[c], 0);
+            if (ce != cudaSuccess) break;
+            rc = copy_out(b0, b1, qo);
+        }
+        for (int k = 0; k < 3 && rc == MTFJSP_OK && ce == cudaSuccess; k++) {
+            ce = cudaEventRecord(hp->join[k], hp->cs[k]);
+            if (ce == cudaSuccess) ce = cudaStreamWaitEvent(hp->ms, hp->join[k], 0);
         }
         cudaError_t ee = cudaStreamEndCapture(hp->ms, &g);
         const int kernels = (int)(h->launches - l0);

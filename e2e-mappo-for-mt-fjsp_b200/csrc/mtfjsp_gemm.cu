@@ -242,7 +242,7 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
                                                                          const float* __restrict__ in_scale,
                                                                          const float* __restrict__ in_shift, int in_relu,
                                                                          float* __restrict__ Z, double* __restrict__ stats,
-                                                                         long long num_tiles, int raw_a, int g_rpt = 0,
+                                                                         long long num_tiles, int g_rpt = 0,
                                                                          int g_nodes = 0, int g_P = 0) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr int KS = KP > 64 ? 64 : KP, SPT = KP / KS;  // stage width, stages per tile
@@ -307,7 +307,7 @@ __global__ void __launch_bounds__(GEMM_WARPS * 32, 1) linear_tf32_kernel(const f
             float* sA = reinterpret_cast<float*>(sRing + slot * SBYTES);
             asm volatile("cp.async.wait_group %0;" ::"n"(NSTAGE - 2) : "memory");  // stage g has landed (this thread's pieces)
             if (!GROUPED && affine) tile_transform<KS, true>(sA, tile * TILE_M, rows, K, h * KS, s_scale, s_shift, in_relu != 0, pw, lane);
-            else if (!raw_a) tile_transform<KS, false>(sA, tile * TILE_M, rows, K, h * KS, nullptr, nullptr, false, pw, lane);
+            else tile_transform<KS, false>(sA, tile * TILE_M, rows, K, h * KS, nullptr, nullptr, false, pw, lane);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the MMA
             // refill the slot stage g-1 used: its MMAs ran while this stage was being transformed
             if (g >= 1 && g + NSTAGE - 1 < nst)
@@ -982,8 +982,7 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ parts, const float
 // staged as the A operand; `tcgen05.mma` -> TMEM; the first epilogue adds the per-env bias (the per-env column blocks of
 // the first weight matrix, applied once per env by the caller), takes tanh and writes the result back INTO the A buffer
 // (the first product has finished reading it) as the second product's operand; the second epilogue takes tanh, dots the
-// row with w2 and writes one float per row.  Replaces gather + 2 GEMM launches + bias_tanh + tanh_dot: five passes over
-// [rows,128] tensors become one gathered read.  Both weight matrices stay in shared memory (2 x 64 KB), one CTA per SM.
+// row with w2 and writes one float per row: one gathered read of [rows,128] in all.  Both weight matrices stay in shared memory (2 x 64 KB), one CTA per SM.
 // tanh / ELU for operands that are rounded to TF32 next (or summed into a score next to TF32 products): one ex2.approx
 // and one fast division instead of the ~25-instruction accurate routines; absolute error < 3e-7
 __device__ __forceinline__ float tanh_fast(float x) {
@@ -1172,211 +1171,17 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32, 1) head_tf32_kernel(
 // GAT layer model/gat.py:82-159 on the fixed 2-node graph with ELU between them, mean over the two node sets):
 //     h1 = f1 W1p^T, h2 = f2 W2p^T;   3 x { t = [h1; h2] W;  att = softmax(lrelu(t1.a_src + t1.a_dst), lrelu(t1.a_src + t2.a_dst));
 //                                          h1 = att0 t1 + att1 t2, h2 = t2;  (ELU on both between layers) };   out = (h1 + h2) / 2
-// Nothing couples machines before the BatchNorm that follows, so 64 machines (tile rows 0..63 = their node-1 rows,
-// 64..127 = their node-2 rows) run through all three layers on one SM: the input projections (K = 6 / 8) on the CUDA
-// cores straight into the A operand, each layer's product on `tcgen05.mma` into TMEM, the attention / combination / ELU in
-// the epilogue, written back into the A buffer for the next layer.  Replaces mach_proj + 3 x (GEMM launch + gat_attend):
-// thirteen passes over [2R,128] tensors become one [R,128] write.
-constexpr int TRUNK_WARPS = 16;
-
-__global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk_tf32_kernel(
-    const float* __restrict__ f1, const float* __restrict__ f2, const float* __restrict__ W1p, const float* __restrict__ W2p,
-    const float* __restrict__ Wt, const float* __restrict__ a_src, const float* __restrict__ a_dst, float* __restrict__ out,
-    double* __restrict__ stats, long long R, long long num_tiles) {
-    extern __shared__ __align__(1024) unsigned char smem[];
-    constexpr size_t WBYTES = (size_t)TILE_N * 128 * 4;
-    float* sW = reinterpret_cast<float*>(smem);
-    float* sA = reinterpret_cast<float*>(smem + WBYTES);
-    float* sT2 = reinterpret_cast<float*>(smem + 2 * WBYTES);           // [64][128] raw t2 rows, 16-byte pieces XOR-swizzled
-    float* s_dot = sT2 + 64 * 128;                                       // [3][4][64]: s1, d1, d2 partials per column group
-    float* s_as = s_dot + 3 * 4 * 64;
-    float* s_ad = s_as + 128;
-    float* s_w1p = s_ad + 128;                                           // [128][6]
-    float* s_w2p = s_w1p + 128 * 6;                                      // [128][8]
-    uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_w2p + 128 * 8);
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(s_bar + 1);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid < 128) { s_as[tid] = a_src[tid]; s_ad[tid] = a_dst[tid]; }
-    for (int i = tid; i < 128 * 6; i += blockDim.x) s_w1p[i] = W1p[i];
-    for (int i = tid; i < 128 * 8; i += blockDim.x) s_w2p[i] = W2p[i];
-    if (tid == 0) {
-        mbar_init(smem_u32(s_bar), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(s_tmem)), "r"(128));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    stage_block<false, TRUNK_WARPS>(sW, Wt, 0, TILE_N, 128, 128, 128, nullptr, nullptr, false, warp, lane);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem_base = *s_tmem;
-    const uint32_t bar = smem_u32(s_bar);
-
-    const int quad = warp & 3, cg = warp >> 2;   // TMEM lanes 32 quad .., columns 32 cg ..
-    const int trow = quad * 32 + lane;           // tile row of this thread: < 64 node 1, >= 64 node 2
-    const bool node2 = quad >= 2;
-    const int mloc = trow & 63;                  // machine within the tile
-    char* const a_dst_row = reinterpret_cast<char*>(sA) + (trow >> 3) * 4096 + (cg * 8) * 128 + (trow & 7) * 16;
-    uint32_t phase = 0;
-    double st_sum = 0.0, st_sq = 0.0;  // node-1 threads: column cg * 32 + lane of `out`, for the BatchNorm that follows
-    for (long long tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const long long m = tile * 64 + mloc;
-        const bool mok = m < R;
-        {   // input projections on the CUDA cores, straight into the A operand
-            float f[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-            if (mok) {
-                if (node2) {
-                    const float4 u0 = __ldg(reinterpret_cast<const float4*>(f2 + m * 8)), u1 = __ldg(reinterpret_cast<const float4*>(f2 + m * 8) + 1);
-                    f[0] = u0.x; f[1] = u0.y; f[2] = u0.z; f[3] = u0.w; f[4] = u1.x; f[5] = u1.y; f[6] = u1.z; f[7] = u1.w;
-                } else {
-                    const float2* p2 = reinterpret_cast<const float2*>(f1 + m * 6);
-                    const float2 u0 = __ldg(p2), u1 = __ldg(p2 + 1), u2 = __ldg(p2 + 2);
-                    f[0] = u0.x; f[1] = u0.y; f[2] = u1.x; f[3] = u1.y; f[4] = u2.x; f[5] = u2.y;
-                }
-            }
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-                float o[4];
-#pragma unroll
-                for (int c = 0; c < 4; c++) {
-                    const int col = cg * 32 + j * 4 + c;
-                    float acc;
-                    if (node2) {
-                        const float4 wa = *reinterpret_cast<const float4*>(s_w2p + col * 8), wb = *reinterpret_cast<const float4*>(s_w2p + col * 8 + 4);
-                        acc = fmaf(f[7], wb.w, fmaf(f[6], wb.z, fmaf(f[5], wb.y, fmaf(f[4], wb.x,
-                              fmaf(f[3], wa.w, fmaf(f[2], wa.z, fmaf(f[1], wa.y, f[0] * wa.x)))))));
-                    } else {
-                        const float2 wa = *reinterpret_cast<const float2*>(s_w1p + col * 6), wb = *reinterpret_cast<const float2*>(s_w1p + col * 6 + 2),
-                                     wc = *reinterpret_cast<const float2*>(s_w1p + col * 6 + 4);
-                        acc = fmaf(f[5], wc.y, fmaf(f[4], wc.x, fmaf(f[3], wb.y, fmaf(f[2], wb.x, fmaf(f[1], wa.y, f[0] * wa.x)))));
-                    }
-                    o[c] = to_tf32(acc);
-                }
-                *reinterpret_cast<float4*>(a_dst_row + j * 128) = make_float4(o[0], o[1], o[2], o[3]);
-            }
-        }
-#pragma unroll 1
-        for (int layer = 0; layer < 3; layer++) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncthreads();
-            if (tid == 0) {
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t aA = smem_u32(sA), aW = smem_u32(sW);
-#pragma unroll
-                for (int k = 0; k < 16; k++)
-                    umma_tf32(tmem_base, make_desc(aA + k * 256, 128, 4096), make_desc(aW + k * 256, 128, 4096), k > 0 ? 1u : 0u);
-                asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            uint32_t r[32];
-            TMEM_LD32(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(cg * 32), r);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            // partial dots over this thread's 32 columns; node-2 rows also park their raw values for the node-1 threads
-            float pa = 0.f, pb = 0.f;
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-                const float4 va = *reinterpret_cast<const float4*>(s_as + cg * 32 + 4 * j), vd = *reinterpret_cast<const float4*>(s_ad + cg * 32 + 4 * j);
-                const float x0 = __uint_as_float(r[4 * j]), x1 = __uint_as_float(r[4 * j + 1]), x2 = __uint_as_float(r[4 * j + 2]),
-                            x3 = __uint_as_float(r[4 * j + 3]);
-                pa = fmaf(x3, va.w, fmaf(x2, va.z, fmaf(x1, va.y, fmaf(x0, va.x, pa))));
-                pb = fmaf(x3, vd.w, fmaf(x2, vd.z, fmaf(x1, vd.y, fmaf(x0, vd.x, pb))));
-            }
-            if (node2) {
-                s_dot[(2 * 4 + cg) * 64 + mloc] = pb;
-#pragma unroll
-                for (int j = 0; j < 8; j++)
-                    *reinterpret_cast<uint4*>(sT2 + mloc * 128 + (((cg * 8 + j) ^ (mloc & 7)) << 2)) =
-                        make_uint4(r[4 * j], r[4 * j + 1], r[4 * j + 2], r[4 * j + 3]);
-            } else {
-                s_dot[(0 * 4 + cg) * 64 + mloc] = pa;
-                s_dot[(1 * 4 + cg) * 64 + mloc] = pb;
-            }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncthreads();
-            float a0 = 0.f, a1 = 1.f;  // node-2 rows: h2' = t2
-            if (!node2) {
-                const float s1 = (s_dot[0 * 64 + mloc] + s_dot[1 * 64 + mloc]) + (s_dot[2 * 64 + mloc] + s_dot[3 * 64 + mloc]);
-                const float d1 = (s_dot[4 * 64 + mloc] + s_dot[5 * 64 + mloc]) + (s_dot[6 * 64 + mloc] + s_dot[7 * 64 + mloc]);
-                const float d2 = (s_dot[8 * 64 + mloc] + s_dot[9 * 64 + mloc]) + (s_dot[10 * 64 + mloc] + s_dot[11 * 64 + mloc]);
-                float e11 = s1 + d1, e12 = s1 + d2;
-                e11 = e11 > 0.f ? e11 : 0.2f * e11;
-                e12 = e12 > 0.f ? e12 : 0.2f * e12;
-                const float mx = fmaxf(e11, e12);
-                const float p1 = expf(e11 - mx), p2 = expf(e12 - mx);
-                a0 = p1 / (p1 + p2); a1 = p2 / (p1 + p2);
-            }
-            if (layer < 2) {  // next layer's operand: elu(h') of every row, back into the A buffer (the product is done with it)
-#pragma unroll
-                for (int j = 0; j < 8; j++) {
-                    float4 x = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
-                                           __uint_as_float(r[4 * j + 3]));
-                    if (!node2) {
-                        const float4 y = *reinterpret_cast<const float4*>(sT2 + mloc * 128 + (((cg * 8 + j) ^ (mloc & 7)) << 2));
-                        x.x = a0 * x.x + a1 * y.x; x.y = a0 * x.y + a1 * y.y; x.z = a0 * x.z + a1 * y.z; x.w = a0 * x.w + a1 * y.w;
-                    }
-                    x.x = to_tf32(elu_fast(x.x)); x.y = to_tf32(elu_fast(x.y)); x.z = to_tf32(elu_fast(x.z)); x.w = to_tf32(elu_fast(x.w));
-                    *reinterpret_cast<float4*>(a_dst_row + j * 128) = x;
-                }
-            } else if (!node2) {  // mean over the two node sets (warp-uniform branch: the shuffles below need every lane)
-                float4* op = reinterpret_cast<float4*>(out + m * 128 + cg * 32);
-                float o[32];
-#pragma unroll
-                for (int j = 0; j < 8; j++) {
-                    const float4 y = *reinterpret_cast<const float4*>(sT2 + mloc * 128 + (((cg * 8 + j) ^ (mloc & 7)) << 2));
-                    float4 x = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
-                                           __uint_as_float(r[4 * j + 3]));
-                    x.x = 0.5f * ((a0 * x.x + a1 * y.x) + y.x); x.y = 0.5f * ((a0 * x.y + a1 * y.y) + y.y);
-                    x.z = 0.5f * ((a0 * x.z + a1 * y.z) + y.z); x.w = 0.5f * ((a0 * x.w + a1 * y.w) + y.w);
-                    if (mok) op[j] = x;
-                    else x = make_float4(0.f, 0.f, 0.f, 0.f);
-                    o[4 * j] = x.x; o[4 * j + 1] = x.y; o[4 * j + 2] = x.z; o[4 * j + 3] = x.w;
-                }
-                if (stats) {  // column sums over the warp's 32 rows by recursive halving: lane l ends up with column l
-                    float q[32];
-#pragma unroll
-                    for (int j = 0; j < 32; j++) q[j] = o[j] * o[j];
-#pragma unroll
-                    for (int off = 16, n = 16; off >= 1; off >>= 1, n >>= 1) {
-                        const bool up = (lane & off) != 0;
-#pragma unroll
-                        for (int j = 0; j < n; j++) {
-                            const float so = up ? o[j] : o[j + n], ko = up ? o[j + n] : o[j];
-                            const float sq = up ? q[j] : q[j + n], kq = up ? q[j + n] : q[j];
-                            o[j] = ko + __shfl_xor_sync(0xffffffffu, so, off);
-                            q[j] = kq + __shfl_xor_sync(0xffffffffu, sq, off);
-                        }
-                    }
-                    st_sum += (double)o[0];
-                    st_sq += (double)q[0];
-                }
-            }
-        }
-        __syncthreads();  // sT2 / s_dot / the A buffer are rewritten by the next tile
-    }
-    if (stats && !node2) {
-        atomicAdd(stats + cg * 32 + lane, st_sum);
-        atomicAdd(stats + 128 + cg * 32 + lane, st_sq);
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128));
-}
-
-
-// Second form of the trunk kernel: 128 machines per tile, the two node sets as TWO products per layer (t1 = h1 W into TMEM
-// columns 0..127, t2 = h2 W into 128..255), so that the thread that owns a machine's TMEM lane holds both of its rows:
-// no exchange of node-2 rows through shared memory, every thread does the same work, half the barriers per machine.
+// Nothing couples machines before the BatchNorm that follows, so 128 machines run through all three layers on one SM: the
+// input projections (K = 6 / 8) on the CUDA cores straight into the A operands, each layer's product on `tcgen05.mma` into
+// TMEM, the attention / combination / ELU in the epilogue, written back into the A buffers for the next layer; one [R,128]
+// write in all.  The two node sets are TWO products per layer (t1 = h1 W into TMEM columns 0..127, t2 = h2 W into
+// 128..255), so that the thread that owns a machine's TMEM lane holds both of its rows: no exchange of node-2 rows through
+// shared memory, every thread does the same work.
 // GROUPED (per-env BatchNorm statistics): a tile is rpt = (128 / M) * M machines of whole envs (lanes >= rpt idle), and
 // instead of the batch-wide atomics `stats` is env_stats [B,1,2,128]: the last layer also parks the output rows in the
 // (then free) first A buffer, and one thread per (env, column) adds the env's rows from there in row order in FP64, so
 // an env's statistics are the same bits at any batch position.
+constexpr int TRUNK_WARPS = 16;
 template <bool GROUPED>
 __global__ void __launch_bounds__(TRUNK_WARPS * 32, 1) gat_trunk2_tf32_kernel(
     const float* __restrict__ f1, const float* __restrict__ f2, const float* __restrict__ W1p, const float* __restrict__ W2p,
@@ -1853,18 +1658,12 @@ static int launch_linear(const float* X, int64_t rows, int K, const float* W, co
     const int P = GROUPED ? (nodes + TILE_M - 1) / TILE_M : 1, rpt = GROUPED && P == 1 ? (TILE_M / nodes) * nodes : TILE_M;
     const long long tiles = GROUPED ? (P == 1 ? (rows + rpt - 1) / rpt : rows / nodes * P) : (rows + TILE_M - 1) / TILE_M;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    // MTFJSP_GEMM_RAW_A=1 (opt-in): without a prologue the A operand stays as the FP32 bits cp.async landed -- kind::tf32
-    // reads the top 19 bits (truncation) -- and the in-place rounding pass in front of every MMA is skipped: 563 -> 476 us
-    // per 2.36 M-row K = 128 layer (65 -> 77 % of the measured HBM peak).  Not the default: truncation is biased towards
-    // zero, and the PPO update's critic gradient moved visibly away from the FP32 one (cosine 0.982 against > 0.99 with
-    // round-to-nearest operands, tests/test_ppo.py); profiles/README.md.
-    static const int raw_a = getenv("MTFJSP_GEMM_RAW_A") ? atoi(getenv("MTFJSP_GEMM_RAW_A")) : 0;
     if constexpr (GROUPED)
         linear_tf32_kernel<KP, true><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, nullptr, nullptr, 0, Z, stats,
-                                                                             tiles, raw_a, rpt, nodes, P);
+                                                                             tiles, rpt, nodes, P);
     else
         linear_tf32_kernel<KP, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z,
-                                                                              stats, tiles, raw_a);
+                                                                              stats, tiles);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 
@@ -1887,8 +1686,7 @@ static EncodeTiledFn encode_tiled_fn() {
 
 static int launch_linear_tma(const float* X, int64_t rows, const float* W, const float* bias, const float* in_scale,
                              const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream) {
-    static const int enabled = getenv("MTFJSP_GEMM_TMA") ? atoi(getenv("MTFJSP_GEMM_TMA")) : 1;
-    EncodeTiledFn enc = enabled ? encode_tiled_fn() : nullptr;
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc || ((uintptr_t)X & 15)) return 0;
     CUtensorMap map;
     const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
@@ -1920,8 +1718,7 @@ static int launch_linear_tma(const float* X, int64_t rows, const float* W, const
 static int launch_linear_tma_agg(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src, const float* W,
                                  const float* bias, const float* in_scale, const float* in_shift, int in_relu, float* Z,
                                  double* stats, cudaStream_t stream) {
-    static const int enabled = getenv("MTFJSP_GEMM_TMA") ? atoi(getenv("MTFJSP_GEMM_TMA")) : 1;
-    EncodeTiledFn enc = enabled ? encode_tiled_fn() : nullptr;
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc || ((uintptr_t)X & 15) || N > TILE_M) return 0;
     const int rpt = (TILE_M / N) * N;
     const long long rows = (long long)B * N;
@@ -2042,35 +1839,20 @@ int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int row
 int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
                               const float* a_src, const float* a_dst, float* out, double* stats, int64_t R, void* stream) {
     if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || R < 1) return MTFJSP_E_ARG;
-    static const int form = getenv("MTFJSP_TRUNK_FORM") ? atoi(getenv("MTFJSP_TRUNK_FORM")) : 2;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (form == 2) {  // 128 machines per tile, two products per layer
-        const size_t smem2 = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
-        static thread_local bool configured2 = false;
-        if (!configured2) {
-            if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2) != cudaSuccess)
-                return MTFJSP_E_CUDA;
-            configured2 = true;
-        }
-        const long long tiles2 = (R + 127) / 128;
-        const int grid2 = (int)(tiles2 < sms ? tiles2 : sms);
-        gat_trunk2_tf32_kernel<false><<<grid2, TRUNK_WARPS * 32, smem2, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
-                                                                                            stats, R, tiles2, 128, 1);
-        return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
-    }
-    const size_t smem = 2 * (size_t)TILE_N * 128 * 4 + (64 * 128 + 3 * 4 * 64 + 256 + 128 * 14) * 4 + 8 + 16;
+    const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
     static thread_local bool configured = false;
     if (!configured) {
-        if (cudaFuncSetAttribute(gat_trunk_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
             return MTFJSP_E_CUDA;
         configured = true;
     }
-    const long long tiles = (R + 63) / 64;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long tiles = (R + 127) / 128;
     const int grid = (int)(tiles < sms ? tiles : sms);
-    gat_trunk_tf32_kernel<<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out, stats, R,
-                                                                                tiles);
+    gat_trunk2_tf32_kernel<false><<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
+                                                                                          stats, R, tiles, 128, 1);
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 

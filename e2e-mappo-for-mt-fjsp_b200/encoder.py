@@ -27,17 +27,8 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-import os
-
 from . import _lib
 from ._lib import check
-
-# MTFJSP_FUSED_HEAD=0: the policy heads of the rollout path as separate launches (gather, GEMM, bias + tanh, GEMM,
-# tanh + dot) instead of the one-launch head kernel -- kept for A/B measurements
-_FUSED_HEAD = os.environ.get("MTFJSP_FUSED_HEAD", "1") != "0"
-_FUSED_TRUNK = os.environ.get("MTFJSP_FUSED_TRUNK", "1") != "0"  # likewise for the machine-node trunk
-_FUSED_AGG = os.environ.get("MTFJSP_FUSED_AGG", "1") != "0"      # likewise aggregation + first layer of a GIN MLP
-_FUSED_ESA = os.environ.get("MTFJSP_FUSED_ESA", "1") != "0"      # likewise the ESA machine actor (EsaMachineActor)
 
 
 def _ptr(t):
@@ -120,7 +111,7 @@ def aggregate_linear_tf32(h, adj_w, adj_src, weight, bias, in_scale=None, in_shi
     neighbourhood mean is applied to the product rows in the epilogue).  h [B,N,128] -> [B*N,128], or None when this
     form is not available for the size (the caller then runs aggregate + linear_tf32)."""
     B, N = h.shape[0], h.shape[1]
-    if N > 128 or h.shape[2] != 128 or not _FUSED_AGG:
+    if N > 128 or h.shape[2] != 128:
         return None
     z = torch.empty((B * N, 128), dtype=torch.float32, device=h.device)
     rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _optr(bias),
@@ -243,7 +234,7 @@ def linear_tf32_grouped(x, rows_per_env, weight, bias, in_scale, in_shift, relu,
 def aggregate_linear_tf32_grouped(h, adj_w, adj_src, weight, bias, in_scale, in_shift, relu, env_stats):
     """aggregate_linear_tf32 with [G,128] affines and per-env statistics; None where the form is not available (N > 128)."""
     B, N = h.shape[0], h.shape[1]
-    if N > 128 or not _FUSED_AGG:
+    if N > 128:
         return None
     z = torch.empty((B * N, 128), dtype=torch.float32, device=h.device)
     epg = 1 if in_scale is None else B // in_scale.shape[0]
@@ -286,20 +277,10 @@ def wgrad_tf32(gz, x, want_bias=True):
     return dW, db
 
 
-def mach_proj(fea1, fea2, W1, W2):
-    """[fea1 @ W1.T ; fea2 @ W2.T] as one [2R,128] buffer (mtfjsp_enc_mach_proj); fea1 [R,6], fea2 [R,8] f32."""
-    R = fea1.shape[0]
-    out = torch.empty((2 * R, 128), dtype=torch.float32, device=fea1.device)
-    check(_lib.lib().mtfjsp_enc_mach_proj(_ptr(fea1), _ptr(fea2), _ptr(W1), _ptr(W2), _ptr(out), R, _stream()),
-          "mtfjsp_enc_mach_proj")
-    return out
-
-
-def gat_attend(t, a_src, a_dst, mode, out=None):
+def gat_attend(t, a_src, a_dst, mode):
     """Attention + combination (+ELU / node-set mean) of the closed-form 2-node GAT layer, see include/mtfjsp.h."""
     R = t.shape[0] // 2
-    if out is None:
-        out = torch.empty((R if mode == 2 else 2 * R, 128), dtype=torch.float32, device=t.device)
+    out = torch.empty((R if mode == 2 else 2 * R, 128), dtype=torch.float32, device=t.device)
     check(_lib.lib().mtfjsp_enc_gat_attend(_ptr(t), _ptr(a_src), _ptr(a_dst), _ptr(out), R, mode, _stream()),
           "mtfjsp_enc_gat_attend")
     return out
@@ -332,20 +313,6 @@ class _GatAttendFn(torch.autograd.Function):
 
 def gat_attend_train(t, a_src, a_dst, mode):
     return _GatAttendFn.apply(t, a_src, a_dst, mode)
-
-
-def bias_tanh_(z, bias, rows_per_env):
-    """z[r] = tanh(z[r] + bias[r // rows_per_env]) in place; bias [B,128] or [1,128]."""
-    check(_lib.lib().mtfjsp_enc_bias_tanh(_ptr(z), _ptr(bias), z.shape[0], rows_per_env, bias.shape[0], _stream()),
-          "mtfjsp_enc_bias_tanh")
-    return z
-
-
-def tanh_dot(z, w, b):
-    """tanh(z) @ w + b for z [rows,128], w [128], b [1] -> [rows]."""
-    out = torch.empty(z.shape[0], dtype=torch.float32, device=z.device)
-    check(_lib.lib().mtfjsp_enc_tanh_dot(_ptr(z), _ptr(w), _optr(b), _ptr(out), z.shape[0], _stream()), "mtfjsp_enc_tanh_dot")
-    return out
 
 
 class _LinearTF32Fn(torch.autograd.Function):
@@ -750,17 +717,8 @@ class _Twin:
             B, nodes = per_row.shape[0], per_row.shape[1]
         else:
             B, nodes = per_row.shape[0] // rows_per_env, 0
-        if _FUSED_HEAD:
-            return head_tf32(per_row, cand, B, rows_per_env, nodes, in_scale, in_shift, Wa, bias,
-                             w[prefix + "linears.1.weight"], w[prefix + "linears.1.bias"], w2, w[prefix + "linears.2.bias"], relu=relu)
-        if in_scale is not None and in_scale.dim() == 2:
-            raise ValueError("per-group BatchNorm affines need the one-launch head (MTFJSP_FUSED_HEAD=1)")
-        if cand is not None:
-            per_row = torch.gather(per_row, 1, cand.long().unsqueeze(-1).expand(-1, rows_per_env, H)).reshape(-1, H)
-        z = linear_tf32(per_row, Wa, None, in_scale, in_shift, relu=relu and in_scale is not None)
-        bias_tanh_(z, bias, rows_per_env)
-        z = linear_tf32(z, w[prefix + "linears.1.weight"], w[prefix + "linears.1.bias"])
-        return tanh_dot(z, w2, w[prefix + "linears.2.bias"]).view(B, rows_per_env)
+        return head_tf32(per_row, cand, B, rows_per_env, nodes, in_scale, in_shift, Wa, bias,
+                         w[prefix + "linears.1.weight"], w[prefix + "linears.1.bias"], w2, w[prefix + "linears.2.bias"], relu=relu)
 
 
 def _head_train(self, prefix, per_row, env_terms, rows_per_env):
@@ -906,9 +864,8 @@ class _MachineTrunk:
         return nodes, nodes.mean(dim=1)
 
     def _trunk_tf32(self, machine_fea_1, machine_fea_2, groups):
-        """Rollout path: input projections written as one [2R,128] buffer, then per GAT layer ONE tensor-core
-        projection of both node sets and ONE kernel for attention + combination + ELU (the last one emits the
-        node-set mean); every [rows,128] tensor is written once and read once."""
+        """Rollout path: input projections, three GAT layers and the node-set mean in one tcgen05 launch
+        (gat_trunk_tf32); one BatchNorm group, groups of several envs, or one env per group."""
         w, H = self.w, self.H
         B = machine_fea_1.shape[0]
         R = B * self.M
@@ -918,7 +875,7 @@ class _MachineTrunk:
         a_src = self._derived("gat_a_src", lambda: self.w["gat_layer.a"][0, :H, 0])
         a_dst = self._derived("gat_a_dst", lambda: self.w["gat_layer.a"][0, H:, 0])
         self._pending_m = None
-        if _FUSED_TRUNK and groups == 1:
+        if groups == 1:
             # the trunk kernel leaves the BatchNorm statistics behind; the normalisation itself is applied by the consumers
             # (the policy head's prologue; the mean over machines commutes with the per-column affine)
             stats = torch.zeros(256, dtype=torch.float64, device=f1.device)
@@ -926,18 +883,12 @@ class _MachineTrunk:
             sc, sh = bn_finalize(stats, R, w["bn.weight"], w["bn.bias"])
             self._pending_m = (sc, sh)
             return buf.view(B, self.M, H), _graph_mean_raw(buf.view(B, self.M, H), sc, sh, relu=False)
-        if _FUSED_TRUNK and _FUSED_HEAD and B > groups:
+        if B > groups:
             # groups of several envs (training rollouts, Rollout(bn_group_envs=...)): per-env statistics from the trunk
             # kernel; groups of one env (per-instance validation) keep the separate BatchNorm pass below, whose decisions
             # tests/test_grouped_bn.py pins bit for bit against one-instance batches
             return self._trunk_tf32_grouped(f1, f2, Wt, a_src, a_dst, groups)
-        if _FUSED_TRUNK:
-            buf = gat_trunk_tf32(f1, f2, w["m_fea_1_fcl.weight"], w["m_fea_2_fcl.weight"], Wt, a_src, a_dst)
-        else:
-            buf = mach_proj(f1, f2, w["m_fea_1_fcl.weight"], w["m_fea_2_fcl.weight"])
-            for layer in range(3):
-                t = linear_tf32(buf, Wt, None)
-                buf = gat_attend(t, a_src, a_dst, 1, out=buf) if layer < 2 else gat_attend(t, a_src, a_dst, 2)
+        buf = gat_trunk_tf32(f1, f2, w["m_fea_1_fcl.weight"], w["m_fea_2_fcl.weight"], Wt, a_src, a_dst)
         nodes = _bn_train(buf, w["bn.weight"], w["bn.bias"], groups=groups).reshape(B, self.M, H)
         return nodes, nodes.mean(dim=1)
 
@@ -965,8 +916,8 @@ class _MachineTrunk:
 class MachineActor(_MachineTrunk, _Twin):
     """Forward of Machine_Actor_JointAction_selfGAT_selfCritic (model/actor_critic.py:359-498).  With 1 < groups < B the
     tf32 path takes per-env statistics from the grouped trunk kernel and applies the [groups, 128] affines in the pooling
-    and the policy head.  With one env per group (or MTFJSP_FUSED_TRUNK=0 / MTFJSP_FUSED_HEAD=0) it normalises through
-    mtfjsp_enc_bn_fwd, which takes at most 65,535 groups per call (its grid.y)."""
+    and the policy head.  With one env per group it normalises through mtfjsp_enc_bn_fwd, which takes at most 65,535
+    groups per call (its grid.y)."""
 
     n_values = 2  # width of machine_v
 
@@ -1024,7 +975,7 @@ class EsaMachineActor(_Twin):
     precision "fp32": that chain literally on library FP32 GEMMs (per-instance BatchNorm groups work);
     "tf32": BatchNorm and both projections folded into the first m_policy layer (K = 14 on the raw features), the
     statistics from the feature moments -- mtfjsp_enc_esa_mach_stats + mtfjsp_enc_esa_mach_fold + mtfjsp_enc_esa_mach_head_tf32,
-    no [B*M,128] intermediate; one BatchNorm group.  MTFJSP_FUSED_ESA=0 runs the tf32 path layer by layer instead."""
+    no [B*M,128] intermediate; one BatchNorm group."""
 
     n_values = 2
 
@@ -1045,7 +996,7 @@ class EsaMachineActor(_Twin):
         if self.precision == "tf32":
             if groups != 1:
                 raise ValueError("the tf32 ESA machine actor is the rollout path: one BatchNorm group")
-            s, pooled = (self._scores_fused if _FUSED_ESA else self._scores_layers)(f1, f2, h_pooled_o.contiguous(), B)
+            s, pooled = self._scores_fused(f1, f2, h_pooled_o.contiguous(), B)
             machine_v = _mlp3_tanh_tf32(w, "machine_critic.", pooled)
         else:
             s, pooled = self._scores_fp32(f1, f2, h_pooled_o, B, groups)
@@ -1097,24 +1048,6 @@ class EsaMachineActor(_Twin):
                                                 _ptr(w["m_policy.linears.1.bias"]), _ptr(w2), _ptr(w["m_policy.linears.2.bias"]),
                                                 _ptr(s), _stream()), "mtfjsp_enc_esa_mach_head_tf32")
         return s, pooled
-
-    def _scores_layers(self, f1, f2, h_pooled_o, B):
-        """The tf32 path one layer per launch (A/B reference for the fused form): both projections and BatchNorms
-        materialised, the first m_policy layer's per-row block split in two products."""
-        w, M, H = self.w, self.M, self.H
-        W1p = self._derived("esa_W1p", lambda: F.pad(w["m_fea_1_fcl.weight"], (0, 2)))  # K = 8: the kernel takes K % 4 == 0
-        h1 = _bn_train(linear_tf32(F.pad(f1, (0, 2)), W1p, None), w["bn.weight"], w["bn.bias"])
-        h2 = _bn_train(linear_tf32(f2, w["m_fea_2_fcl.weight"], None), w["bn.weight"], w["bn.bias"])
-        pooled = (_graph_mean_raw(h1.view(B, M, H)) + _graph_mean_raw(h2.view(B, M, H))) / 2
-        W0 = w["m_policy.linears.0.weight"]
-        Wa = self._derived("esa_W0a", lambda: W0[:, :H])
-        Wb = self._derived("esa_W0b", lambda: W0[:, H:2 * H])
-        bias = self._env_bias(pooled, h_pooled_o, w["m_policy.linears.0.bias"])
-        z = linear_tf32(h1, Wa, None) + linear_tf32(h2, Wb, None)
-        bias_tanh_(z, bias, M)
-        z = linear_tf32(z, w["m_policy.linears.1.weight"], w["m_policy.linears.1.bias"])
-        w2 = self._derived("esa_w2", lambda: w["m_policy.linears.2.weight"].reshape(-1))
-        return tanh_dot(z, w2, w["m_policy.linears.2.bias"]).view(B, M) * 10, pooled
 
 
 def global_critic_keys(hidden=128, in_dim=12):

@@ -2,7 +2,7 @@
 
 One rollout step = job actor (GIN encoder + head) -> candidate-machine features -> machine actor (GAT + head) ->
 fused env step + observation.  Everything stays on the GPU: sampling is one selection kernel per actor (masked softmax,
-counter-based draw, log-probability; `torch.multinomial` with MTFJSP_FUSED_SELECT=0), the
+counter-based draw, log-probability; `torch.multinomial` above 32 jobs or machines), the
 candidate -> op mapping, masks and rewards never visit the host, so there is no host synchronisation inside an
 episode (the reference crosses the host/device boundary four times per step).  The whole step can be captured in a
 CUDA graph and replayed (`Rollout(..., use_cuda_graph=True)`)."""
@@ -54,8 +54,7 @@ class Rollout:
         self._warm = 0
         # sampling by the one-launch selection kernel (encoder.select): counter-based draws keyed by (seed, step counter,
         # env); the counter lives on the device and is advanced inside the step, so CUDA-graph replays draw fresh numbers
-        self.fused_select = ((not greedy) and os.environ.get("MTFJSP_FUSED_SELECT", "1") != "0"
-                             and env.J <= 32 and env.M <= 32)  # one warp lane per job / machine
+        self.fused_select = (not greedy) and env.J <= 32 and env.M <= 32  # one warp lane per job / machine
         self._rng_seed = seed
         self._rng_step = torch.zeros(1, dtype=torch.int64, device=dev)
 

@@ -178,7 +178,7 @@ int mtfjsp_step_host(mtfjsp_env* h, const int32_t* op_host, const int32_t* mach_
  * size-specialised kernel, the step is ONE launch whose warps write their finished records straight into
  * `records_host` over PCIe while the rest of the batch is still being stepped -- no staging buffer, no copy engine
  * (MTFJSP_HOST_ZEROCOPY: 1 = records, 2 = the actions are read from `actions_host` in place as well; default 2 from
- * 16,384 envs up, else 1; 0 = the staged form).  Staged form: the batch is cut into MTFJSP_HOST_CHUNKS (default 4) chunks
+ * 16,384 envs up, else 1; 0 = the staged form).  Staged form: the batch is cut into 4 chunks
  * whose copy-in -> kernel -> copy-out chains run on three streams, replayed as one CUDA graph per step, so that the
  * copy-out of chunk c overlaps the kernel of chunk c+1; pageable buffers take the plain in-order path.  mtfjsp_step_host
  * with NULL job_mask_host / candidate_host writes its [B,6] step info the same zero-copy way.  Synchronises `stream`
@@ -215,25 +215,18 @@ int mtfjsp_enc_bn_bwd(const float* x, const float* gy, const float* w, const flo
  * (gcn_mlp.py:154-157) folded into its consumer.  in_scale / in_shift [C] f32 or both NULL. */
 int mtfjsp_enc_graph_mean(const float* h, float* out, int64_t B, int N, int C, const float* in_scale,
                           const float* in_shift, int in_relu, void* stream);
-/* Rollout-path fusions of the machine actor and the policy heads (hidden = 128, every pointer 16-byte aligned):
- * mach_proj   replaces m_fea_1_fcl / m_fea_2_fcl (actor_critic.py:381-392) + the concatenation: fea1 [R,6], fea2 [R,8],
- *             W1 [128,6], W2 [128,8] -> out [2R,128] = [fea1 W1^T ; fea2 W2^T];
- * gat_attend  replaces everything of GATLayer.forward after the projection (model/gat.py:82-159, closed form on the
- *             2-node graph) and the ELU / node-set mean around it (actor_critic.py:400-420): t [2R,128] = [t1; t2] ->
- *             mode 0: [h1'; h2'], mode 1: [elu(h1'); elu(h2')], mode 2: out [R,128] = (h1' + h2') / 2;
- * bias_tanh   z[r] = tanh(z[r] + bias[r / rows_per_env]) in place (first layer of MLPActor, gcn_mlp.py:305-320, with the
- *             per-env part of its input applied as a bias), bias [bias_rows,128], bias_rows = rows / rows_per_env or 1;
- * tanh_dot    out[r] = tanh(z[r]) . w + b (second tanh and the Linear(128,1) of the same MLP). */
-int mtfjsp_enc_mach_proj(const float* fea1, const float* fea2, const float* W1, const float* W2, float* out, int64_t R,
-                         void* stream);
 /* The machine-node trunk up to the mean over the two node sets (actor_critic.py:381-420) in one launch, hidden = 128:
  * input projections fea1 [R,6] W1p[128,6]^T and fea2 [R,8] W2p[128,8]^T, three GAT layers (projection by Wt = gat_layer.W^T
  * [128 out,128 in] on tcgen05.mma kind::tf32, attention with a_src / a_dst, ELU between layers) and the node-set mean ->
  * out [R,128]; stats (may be NULL) [256] f64 += column sums of out and of out^2 for the BatchNorm that follows
- * (actor_critic.py:434; mtfjsp_enc_bn_finalize turns them into the affine its consumers apply).  64 machines stay on one
- * SM through all three layers; replaces mtfjsp_enc_mach_proj + 3 x (mtfjsp_enc_linear_tf32 + mtfjsp_enc_gat_attend). */
+ * (actor_critic.py:434; mtfjsp_enc_bn_finalize turns them into the affine its consumers apply).  128 machines stay on one
+ * SM through all three layers. */
 int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
                               const float* a_src, const float* a_dst, float* out, double* stats, int64_t R, void* stream);
+/* One GAT layer after its projection, as the PPO update's forward runs it (hidden = 128, every pointer 16-byte aligned):
+ * everything of GATLayer.forward after the projection (model/gat.py:82-159, closed form on the 2-node graph) and the
+ * ELU / node-set mean around it (actor_critic.py:400-420): t [2R,128] = [t1; t2] ->
+ * mode 0: [h1'; h2'], mode 1: [elu(h1'); elu(h2')], mode 2: out [R,128] = (h1' + h2') / 2. */
 int mtfjsp_enc_gat_attend(const float* t, const float* a_src, const float* a_dst, float* out, int64_t R, int mode,
                           void* stream);
 /* Backward of mtfjsp_enc_gat_attend for the PPO update: g = gradient of its output, dt [2R,128] = gradient of t,
@@ -241,8 +234,6 @@ int mtfjsp_enc_gat_attend(const float* t, const float* a_src, const float* a_dst
 int mtfjsp_enc_gat_attend_bwd(const float* t, const float* a_src, const float* a_dst, const float* g, float* dt, float* dparts,
                               int64_t R, int mode, void* stream);
 int mtfjsp_enc_gat_attend_bwd_blocks(int64_t R);
-int mtfjsp_enc_bias_tanh(float* z, const float* bias, int64_t rows, int rows_per_env, int64_t bias_rows, void* stream);
-int mtfjsp_enc_tanh_dot(const float* z, const float* w, const float* b, float* out, int64_t rows, void* stream);
 /* Action selection of a rollout step (algorithm/agent_func.py:22-63): prob [B,R] = softmax over the entries with
  * mask == 0 of scores * scale (R <= 32), action [B] = a draw from it (counter-based uniform keyed by seed, *counter -- a
  * device step counter the caller advances, so that CUDA-graph replays draw fresh numbers --, env and stream_id) or the
@@ -257,8 +248,7 @@ int mtfjsp_enc_select(const float* scores, const uint8_t* mask, const int32_t* c
  * src(r) = (r / rows_per_env) * nodes_per_env + cand[r] when cand != NULL (the candidate op of each job gathered from the
  * node embeddings), else r; act = x * in_scale + in_shift (then ReLU if in_relu) when in_scale != NULL (the producing
  * layer's BatchNorm), else identity; bias_env [bias_rows,128] with bias_rows = B or 1 = the first layer's bias plus its per-env column blocks
- * applied to the per-env inputs; b1 / b2 may be NULL.  Replaces torch.gather + mtfjsp_enc_linear_tf32 +
- * mtfjsp_enc_bias_tanh + mtfjsp_enc_linear_tf32 + mtfjsp_enc_tanh_dot. */
+ * applied to the per-env inputs; b1 / b2 may be NULL. */
 int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int rows_per_env, int nodes_per_env,
                          const float* in_scale, const float* in_shift, int in_relu, const float* Wa, const float* bias_env,
                          int64_t bias_rows, const float* W1, const float* b1, const float* w2, const float* b2, float* out,

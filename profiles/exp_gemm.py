@@ -33,5 +33,5 @@ t_plain = timeit(lambda: enc.linear_tf32(x, W, b))
 stats = torch.zeros(256, dtype=torch.float64, device="cuda")
 t_aff = timeit(lambda: enc.linear_tf32(x, W, b, sc, sh, relu=True, stats=stats))
 t_wg = timeit(lambda: enc.wgrad_tf32(gz, x))
-print("rows %d raw_a=%s: plain %.1f us (%.2f TB/s, max err %.2e)  affine+stats %.1f us (%.2f TB/s)  wgrad %.1f us (%.2f TB/s)"
-      % (rows, os.environ.get("MTFJSP_GEMM_RAW_A", "0"), t_plain, gb / t_plain * 1e3, err, t_aff, gb / t_aff * 1e3, t_wg, gb / t_wg * 1e3))
+print("rows %d: plain %.1f us (%.2f TB/s, max err %.2e)  affine+stats %.1f us (%.2f TB/s)  wgrad %.1f us (%.2f TB/s)"
+      % (rows, t_plain, gb / t_plain * 1e3, err, t_aff, gb / t_aff * 1e3, t_wg, gb / t_wg * 1e3))

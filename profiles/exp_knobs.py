@@ -1,7 +1,7 @@
 """Knob experiments for the env kernel and the host-step pipeline (one process per setting; the knobs are read from
 the environment when the handle is created):
 
-    MTFJSP_HOST_CHUNKS=0|1|2|4|8  MTFJSP_FUSE_POLICY=0|1  MTFJSP_OBS_INCREMENTAL=0|1  python profiles/exp_knobs.py [workload] [reps]
+    MTFJSP_HOST_ZEROCOPY=0|1|2  MTFJSP_FUSE_POLICY=0|1  MTFJSP_OBS_INCREMENTAL=0|1  python profiles/exp_knobs.py [workload] [reps]
 
 Prints one JSON line: fused-kernel time per launch (CUDA events around each launch, recorded actions replayed),
 whole random-rollout step time, and the host-buffer step rate."""

@@ -3,7 +3,6 @@
   forward   one machine-actor forward (scores, pooled, values) on the features of a live env batch, CUDA events around
             each call, the 126 MB L2 overwritten (256 MB memset) before every timed call; median of 60 calls:
               esa_fused   EsaMachineActor tf32 (stats + fold + head kernels, three small tcgen05 layers for pooled / bias)
-              esa_layers  the same with MTFJSP_FUSED_ESA=0 (projections, BatchNorms, split first layer as separate launches)
               esa_fp32    EsaMachineActor fp32 (library FP32 GEMMs, the reference's arithmetic)
               mappo_tf32  MachineActor tf32 (GAT trunk in one launch + head in one launch), for comparison
   rollout   sampled rollouts under CUDA-graph replay (the configuration of bench.py's actor-driven rollout): env-steps/s
@@ -71,21 +70,15 @@ def forward_times():
     sd_map = enc.seeded_state_dict(enc.machine_actor_keys(128), 12)
     out = {}
     with torch.no_grad():
-        for name, mk, fused in (("esa_fused", lambda: enc.EsaMachineActor(sd_esa, M, precision="tf32"), True),
-                                ("esa_layers", lambda: enc.EsaMachineActor(sd_esa, M, precision="tf32"), False),
-                                ("esa_fp32", lambda: enc.EsaMachineActor(sd_esa, M, precision="fp32"), True),
-                                ("mappo_tf32", lambda: enc.MachineActor(sd_map, M, precision="tf32"), True)):
-            enc._FUSED_ESA = fused
+        for name, mk in (("esa_fused", lambda: enc.EsaMachineActor(sd_esa, M, precision="tf32")),
+                         ("esa_fp32", lambda: enc.EsaMachineActor(sd_esa, M, precision="fp32")),
+                         ("mappo_tf32", lambda: enc.MachineActor(sd_map, M, precision="tf32"))):
             a = mk()
             out[name] = time_calls(lambda: a.forward(m1, m2, h_o, mmask, return_logits=True))
             print(name, out[name], flush=True)
-        enc._FUSED_ESA = True
         ref = enc.EsaMachineActor(sd_esa, M, precision="fp32").forward(m1, m2, h_o, mmask, return_logits=True)[0]
-        for fused in (True, False):
-            enc._FUSED_ESA = fused
-            s = enc.EsaMachineActor(sd_esa, M, precision="tf32").forward(m1, m2, h_o, mmask, return_logits=True)[0]
-            out["max_abs_dev_scores_vs_fp32_" + ("fused" if fused else "layers")] = float((s - ref).abs().max())
-        enc._FUSED_ESA = True
+        s = enc.EsaMachineActor(sd_esa, M, precision="tf32").forward(m1, m2, h_o, mmask, return_logits=True)[0]
+        out["max_abs_dev_scores_vs_fp32_fused"] = float((s - ref).abs().max())
     out["scores_abs_max_fp32"] = float(ref.abs().max())
     out["fused_kernels_us_per_call"] = kernel_breakdown(lambda: enc.EsaMachineActor(sd_esa, M, precision="tf32"), (m1, m2, h_o, mmask))
     return out

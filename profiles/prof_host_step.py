@@ -1,6 +1,5 @@
-"""Host-buffer step (mtfjsp_step_host_packed, bench.py's e2e) against the chunk count of its copy / kernel pipeline, and
-its parts alone: the packed H2D copy, the fused kernel over the whole batch, the packed D2H copy, an empty graph launch +
-synchronize.    python profiles/prof_host_step.py [A|B|C]"""
+"""Host-buffer step (mtfjsp_step_host_packed, bench.py's e2e) and its parts alone: the packed H2D copy, the fused kernel
+over the whole batch, the packed D2H copy, an empty graph launch + synchronize.    python profiles/prof_host_step.py [A|B|C]"""
 import importlib
 import os
 import sys
@@ -20,16 +19,10 @@ d = pkg.instances.synthetic_instances(0, B, J, M, E, wl["seed"])
 w = pkg.instances.random_weights(0, B, wl["seed"])
 
 
-def make(chunks):
-    os.environ["MTFJSP_HOST_CHUNKS"] = str(chunks)
-    env = envm.BatchedMTFJSPEnv(B, J, M, E, obs_dtype=torch.float32)
-    env.load(d["t"], d["p"], d["transT"], d["edge"])
-    env.scaler_init()
-    env.reset(w)
-    return env
-
-
-env = make(4)
+env = envm.BatchedMTFJSPEnv(B, J, M, E, obs_dtype=torch.float32)
+env.load(d["t"], d["p"], d["transT"], d["edge"])
+env.scaler_init()
+env.reset(w)
 rec_op = torch.empty((N, B), dtype=torch.int32, device="cuda")
 rec_mc = torch.empty((N, B), dtype=torch.int32, device="cuda")
 for s in range(N):
@@ -38,20 +31,18 @@ for s in range(N):
 h_act = torch.stack([rec_op.cpu(), rec_mc.cpu()], dim=2).contiguous().pin_memory()
 act_ptr = [h_act[s].data_ptr() for s in range(N)]
 
-for chunks in (1, 2, 3, 4, 6, 8):
-    env = make(chunks)
-    _, h_rec = env.host_buffers()
-    step = env.host_stepper(h_rec)
-    best = 1e9
-    for rep in range(4):
-        env.reset(w); env.scaler_reset()
-        torch.cuda.synchronize()
-        t0 = time.perf_counter()
-        for s in range(N):
-            step(act_ptr[s])
-        torch.cuda.synchronize()
-        best = min(best, (time.perf_counter() - t0) / N)
-    print("chunks %d: %.1f us per %d-env step -> %.3e env-steps/s" % (chunks, best * 1e6, B, B / best), flush=True)
+_, h_rec = env.host_buffers()
+step = env.host_stepper(h_rec)
+best = 1e9
+for rep in range(4):
+    env.reset(w); env.scaler_reset()
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for s in range(N):
+        step(act_ptr[s])
+    torch.cuda.synchronize()
+    best = min(best, (time.perf_counter() - t0) / N)
+print("host step: %.1f us per %d-env step -> %.3e env-steps/s" % (best * 1e6, B, B / best), flush=True)
 
 # the parts alone
 nbytes = int(env._lib.mtfjsp_host_record_bytes(env._h))

@@ -46,15 +46,10 @@ if what in ("enc", "all"):
         enc.linear_tf32(x, W, b, sc, sh, relu=True, stats=stats)
         enc.wgrad_tf32(torch.randn(rows, 128, device="cuda", generator=g), x)
     R = 50
-    enc.mach_proj(torch.randn(R, 6, device="cuda"), torch.randn(R, 8, device="cuda"), torch.randn(128, 6, device="cuda"),
-                  torch.randn(128, 8, device="cuda"))
     t = torch.randn(2 * R, 128, device="cuda")
     for mode in (0, 1, 2):
         enc.gat_attend(t, torch.randn(128, device="cuda"), torch.randn(128, device="cuda"), mode)
-    z = torch.randn(R * 6, 128, device="cuda")
-    enc.bias_tanh_(z, torch.randn(R, 128, device="cuda"), 6)
-    enc.tanh_dot(z, torch.randn(128, device="cuda"), torch.randn(1, device="cuda"))
-    # round-2 kernels: TMA layer (rows >= 4096), aggregation in the epilogue, one-launch head / trunk (both forms), selection
+    # round-2 kernels: TMA layer (rows >= 4096), aggregation in the epilogue, one-launch head / trunk, selection
     rows = 4096 + 77
     x = torch.randn(rows, 128, device="cuda", generator=g)
     W = torch.randn(128, 128, device="cuda", generator=g) / 11.3
@@ -76,10 +71,8 @@ if what in ("enc", "all"):
     enc.head_tf32(nodes, cand, Bq, 6, 36, sc, sh, W, bias, W, b, b, b[:1].contiguous())
     enc.head_tf32(nodes.reshape(-1, 128)[: Bq * 6].contiguous(), None, Bq, 6, 0, None, None, W, bias[:1].contiguous(), W, b, b,
                   b[:1].contiguous(), relu=False)
-    for form in ("2", "1"):
-        os.environ["MTFJSP_TRUNK_FORM"] = form  # read once per process: the second value only matters in a fresh process
-        enc.gat_trunk_tf32(torch.randn(777, 6, device="cuda"), torch.randn(777, 8, device="cuda"), torch.randn(128, 6, device="cuda"),
-                           torch.randn(128, 8, device="cuda"), W, b, b, stats)
+    enc.gat_trunk_tf32(torch.randn(777, 6, device="cuda"), torch.randn(777, 8, device="cuda"), torch.randn(128, 6, device="cuda"),
+                       torch.randn(128, 8, device="cuda"), W, b, b, stats)
     counter = torch.zeros(1, dtype=torch.int64, device="cuda")
     for R_ in (6, 20, 32):
         sco = torch.randn(501, R_, device="cuda", generator=g)

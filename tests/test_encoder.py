@@ -267,10 +267,10 @@ def test_selection_kernel_softmax_draws_and_log_probabilities(R):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("R", [5, 64, 1000, 64 * 148 * 2 + 17])
-def test_fused_machine_trunk_matches_the_layerwise_path(R):
-    """mtfjsp_enc_gat_trunk_tf32 (input projections + three GAT layers + node-set mean, one launch, 64 machines per SM)
-    against the same chain in FP64 with TF32-rounded GEMM operands (tight), the layer-by-layer kernels (TF32 noise) and
-    plain FP32 (TF32 tolerance over three layers)."""
+def test_fused_machine_trunk_matches_the_fp64_chain_on_tf32_operands(R):
+    """mtfjsp_enc_gat_trunk_tf32 (input projections + three GAT layers + node-set mean, one launch, 128 machines per SM)
+    against the same chain in FP64 with TF32-rounded GEMM operands (tight) and plain FP32 (TF32 tolerance over three
+    layers)."""
     torch = pytest.importorskip("torch")
     F = torch.nn.functional
     enc = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.encoder")
@@ -308,11 +308,6 @@ def test_fused_machine_trunk_matches_the_layerwise_path(R):
 
     np.testing.assert_allclose(out.cpu().numpy(), chain(tf32).cpu().numpy(), rtol=3e-3, atol=3e-3)  # a flipped TF32 rounding = 5e-4
     np.testing.assert_allclose(out.cpu().numpy(), chain(lambda t: t).cpu().numpy(), rtol=3e-2, atol=3e-2)
-    buf = enc.mach_proj(f1, f2, W1p, W2p)
-    for layer in range(3):
-        t = enc.linear_tf32(buf, Wt, None)
-        buf = enc.gat_attend(t, a_src, a_dst, 1 if layer < 2 else 2)
-    np.testing.assert_allclose(out.cpu().numpy(), buf.cpu().numpy(), rtol=3e-3, atol=3e-3)
 
 
 @pytest.mark.gpu
@@ -367,9 +362,9 @@ def test_tcgen05_training_linear_gradients_match_autograd(K):
 
 
 @pytest.mark.gpu
-def test_machine_trunk_and_head_fusion_kernels_match_torch():
-    """mach_proj / gat_attend / bias_tanh / tanh_dot (rollout-path fusions) against the torch expressions they replace
-    (actor_critic.py:381-420, model/gat.py:82-159, gcn_mlp.py:305-320), FP32 tolerance."""
+def test_gat_attend_kernel_matches_torch():
+    """gat_attend (the GAT layer after its projection) against the torch expression it replaces
+    (actor_critic.py:400-420, model/gat.py:82-159), FP32 tolerance."""
     torch = pytest.importorskip("torch")
     F = torch.nn.functional
     enc = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.encoder")
@@ -377,8 +372,6 @@ def test_machine_trunk_and_head_fusion_kernels_match_torch():
     rn = lambda *sh: torch.randn(*sh, device="cuda", generator=g)
     close = lambda a, b, tol=2e-5: np.testing.assert_allclose(a.cpu().numpy(), b.cpu().numpy(), rtol=tol, atol=tol)
     R = 1003
-    f1, f2, W1, W2 = rn(R, 6), rn(R, 8), rn(128, 6), rn(128, 8)
-    close(enc.mach_proj(f1, f2, W1, W2), torch.cat((F.linear(f1, W1), F.linear(f2, W2)), 0))
     t, a_src, a_dst = rn(2 * R, 128), rn(128) * 0.1, rn(128) * 0.1
     t1, t2 = t[:R], t[R:]
     e11 = F.leaky_relu(t1 @ a_src + t1 @ a_dst, 0.2)
@@ -388,13 +381,6 @@ def test_machine_trunk_and_head_fusion_kernels_match_torch():
     close(enc.gat_attend(t, a_src, a_dst, 0), torch.cat((h1, h2), 0), 1e-4)
     close(enc.gat_attend(t, a_src, a_dst, 1), torch.cat((F.elu(h1), F.elu(h2)), 0), 1e-4)
     close(enc.gat_attend(t, a_src, a_dst, 2), torch.stack((h1, h2), 1).mean(1), 1e-4)
-    B, r = 167, 6
-    z, bias = rn(B * r, 128), rn(B, 128)
-    ref = torch.tanh(z.view(B, r, 128) + bias.unsqueeze(1)).view(-1, 128)
-    close(enc.bias_tanh_(z.clone(), bias, r), ref)
-    close(enc.bias_tanh_(z.clone(), bias[:1].contiguous(), r), torch.tanh(z + bias[:1]))
-    w2, b2 = rn(128) * 0.1, rn(1)
-    close(enc.tanh_dot(z, w2, b2), torch.tanh(z) @ w2 + b2, 1e-4)
 
 
 @pytest.mark.gpu

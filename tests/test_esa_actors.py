@@ -223,10 +223,8 @@ def test_esa_kernels_match_fp64(B, M, const_col):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("B,M", [(4, 6), (1000, 6), (300, 10), (700, 20)])
-def test_fused_machine_actor_matches_layer_by_layer(B, M, monkeypatch):
-    """The fused tf32 machine actor (stats + fold + head) against MTFJSP_FUSED_ESA=0 (projections, BatchNorms and the
-    split first layer as separate launches) and against the FP32 actor.  The two tf32 forms round different operands
-    to TF32 (raw features vs. normalised embeddings), so they agree to TF32 accuracy, not bit for bit."""
+def test_fused_machine_actor_matches_the_fp32_actor(B, M):
+    """The fused tf32 machine actor (stats + fold + head) against the FP32 actor, to TF32 accuracy."""
     sd = enc.seeded_state_dict(enc.esa_machine_actor_keys(128), 31)
     f1, f2 = _features(B, M, 7 * B + M, True)
     f1, f2 = f1.view(B, M, 6), f2.view(B, M, 8)
@@ -234,14 +232,12 @@ def test_fused_machine_actor_matches_layer_by_layer(B, M, monkeypatch):
     mask = torch.zeros((B, M), dtype=torch.bool, device="cuda")
     res = {}
     with torch.no_grad():
-        for name, prec, fused in (("fused", "tf32", True), ("layers", "tf32", False), ("fp32", "fp32", True)):
-            monkeypatch.setattr(enc, "_FUSED_ESA", fused)
+        for prec in ("tf32", "fp32"):
             mch = enc.EsaMachineActor(sd, M, precision=prec)
-            res[name] = [t.cpu().numpy() for t in mch.forward(f1, f2, h_o, mask, return_logits=True)]
-    for other in ("layers", "fp32"):
-        for i, name in enumerate(("scores", "pooled", "machine_v")):
-            a, b = res["fused"][i], res[other][i]
-            np.testing.assert_allclose(a, b, rtol=1e-2, atol=1e-2 * max(1.0, np.abs(b).max()), err_msg="%s vs %s" % (name, other))
+            res[prec] = [t.cpu().numpy() for t in mch.forward(f1, f2, h_o, mask, return_logits=True)]
+    for i, name in enumerate(("scores", "pooled", "machine_v")):
+        a, b = res["tf32"][i], res["fp32"][i]
+        np.testing.assert_allclose(a, b, rtol=1e-2, atol=1e-2 * max(1.0, np.abs(b).max()), err_msg=name)
 
 
 @pytest.mark.gpu
