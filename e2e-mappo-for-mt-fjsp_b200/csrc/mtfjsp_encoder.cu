@@ -468,6 +468,12 @@ __global__ void __launch_bounds__(256) select_kernel(const float* __restrict__ s
     }
 }
 
+// Operand alignment, checked on the host before any launch: the kernels read and write 16 bytes (float4) or 8 bytes
+// (float2: adj_w) at a time.  NULL passes (optional pointers are checked for presence separately).
+template <class... P>
+bool al16(P... p) { return ((((uintptr_t)p & 15) == 0) && ...); }
+bool al8(const void* p) { return ((uintptr_t)p & 7) == 0; }
+
 }  // namespace
 
 extern "C" {
@@ -501,6 +507,7 @@ int mtfjsp_enc_aggregate(const float* h, const float* adj_w, const int16_t* adj_
                          int C, const float* in_scale, const float* in_shift, int in_relu, void* stream) {
     if (!h || !adj_w || !adj_src || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return MTFJSP_E_ARG;
     const int C4 = C / 4;
     int c4_shift = -1;
     for (int k = 0; k < 16; k++)
@@ -532,6 +539,7 @@ int mtfjsp_enc_ell_invert(const int16_t* adj_src, int16_t* adj_dst, int64_t B, i
 int mtfjsp_enc_aggregate_bwd(const float* g, const float* adj_w, const int16_t* adj_src, const int16_t* adj_dst, float* out,
                              int64_t B, int N, int C, void* stream) {
     if (!g || !adj_w || !adj_src || !adj_dst || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
+    if (!al16(g, out) || !al8(adj_w)) return MTFJSP_E_ARG;
     const int C4 = C / 4;
     int c4_shift = -1;
     for (int k = 0; k < 16; k++)
@@ -555,6 +563,7 @@ static bool bn_args_ok(int64_t G, int64_t R, int C) { return G >= 1 && G <= 6553
 int mtfjsp_enc_bn_fwd(const float* x, const float* w, const float* b, float eps, int64_t G, int64_t R, int C, int relu, float* y,
                       float* mean, float* rstd, double* workspace, void* stream) {
     if (!x || !w || !b || !y || !mean || !rstd || !workspace || !bn_args_ok(G, R, C)) return MTFJSP_E_ARG;
+    if (!al16(x, w, b, y, mean, rstd) || !al8(workspace)) return MTFJSP_E_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     const int C4 = C / 4, ny = 256 / C4 > 0 ? 256 / C4 : 1;
     const int threads = C4 * ny > 256 ? C4 : 256;
@@ -573,6 +582,7 @@ int mtfjsp_enc_bn_fwd(const float* x, const float* w, const float* b, float eps,
 int mtfjsp_enc_bn_bwd(const float* x, const float* gy, const float* w, const float* b, const float* mean, const float* rstd,
                       int64_t G, int64_t R, int C, int relu, float* dx, double* sums, void* stream) {
     if (!x || !gy || !w || !b || !mean || !rstd || !dx || !sums || !bn_args_ok(G, R, C)) return MTFJSP_E_ARG;
+    if (!al16(x, gy, w, b, mean, rstd, dx) || !al8(sums)) return MTFJSP_E_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     const int C4 = C / 4, ny = 256 / C4 > 0 ? 256 / C4 : 1;
     const int threads = C4 * ny > 256 ? C4 : 256;
@@ -599,6 +609,7 @@ int mtfjsp_enc_aggregate_grouped(const float* h, const float* adj_w, const int16
                                  const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, void* stream) {
     if (!h || !adj_w || !adj_src || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
     if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
+    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return MTFJSP_E_ARG;
     const int C4 = C / 4;
     int c4_shift = -1;
     for (int k = 0; k < 16; k++)
@@ -631,6 +642,7 @@ int mtfjsp_enc_graph_mean_grouped(const float* h, float* out, int64_t B, int N, 
 int mtfjsp_enc_gat_attend(const float* t, const float* a_src, const float* a_dst, float* out, int64_t R, int mode,
                           void* stream) {
     if (!t || !a_src || !a_dst || !out || R < 1 || mode < 0 || mode > 2) return MTFJSP_E_ARG;
+    if (!al16(t, a_src, a_dst, out)) return MTFJSP_E_ARG;
     gat_attend_kernel<<<(unsigned)((R + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4*>(t), reinterpret_cast<const float4*>(a_src), reinterpret_cast<const float4*>(a_dst),
         reinterpret_cast<float4*>(out), R, mode);
@@ -645,6 +657,7 @@ int mtfjsp_enc_gat_attend_bwd_blocks(int64_t R) {
 int mtfjsp_enc_gat_attend_bwd(const float* t, const float* a_src, const float* a_dst, const float* g, float* dt, float* dparts,
                               int64_t R, int mode, void* stream) {
     if (!t || !a_src || !a_dst || !g || !dt || !dparts || R < 1 || mode < 0 || mode > 2) return MTFJSP_E_ARG;
+    if (!al16(t, a_src, a_dst, g, dt, dparts)) return MTFJSP_E_ARG;
     gat_attend_bwd_kernel<<<mtfjsp_enc_gat_attend_bwd_blocks(R), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4*>(t), reinterpret_cast<const float4*>(a_src), reinterpret_cast<const float4*>(a_dst),
         reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(dt), dparts, R, mode);

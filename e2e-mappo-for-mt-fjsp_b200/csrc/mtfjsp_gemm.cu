@@ -1638,6 +1638,12 @@ __global__ void __launch_bounds__(ESA_HEAD_WARPS * 32, 1) esa_head_tf32_kernel(
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256));
 }
 
+// Operand alignment, checked on the host before any launch: cp.async, TMA and the float4 loads / stores move 16 bytes at a
+// time, adj_w and fea1 are read as float2.  NULL passes (optional pointers are checked for presence separately).
+template <class... P>
+bool al16(P... p) { return ((((uintptr_t)p & 15) == 0) && ...); }
+bool al8(const void* p) { return ((uintptr_t)p & 7) == 0; }
+
 }  // namespace
 
 // nodes > 0: the grouped form (env-aligned tiles of `nodes`-row envs, per-env statistics; see linear_tf32_kernel)
@@ -1667,7 +1673,8 @@ static int launch_linear(const float* X, int64_t rows, int K, const float* W, co
     return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
 }
 
-// K = 128 through the TMA kernel; returns 1 if launched, 0 if the driver entry point is not available (caller falls back)
+// K = 128 through the TMA kernel (X 16-byte aligned, checked by the caller); returns 1 if launched, 0 if the driver entry
+// point is not available (caller falls back)
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1687,7 +1694,7 @@ static EncodeTiledFn encode_tiled_fn() {
 static int launch_linear_tma(const float* X, int64_t rows, const float* W, const float* bias, const float* in_scale,
                              const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream) {
     EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc || ((uintptr_t)X & 15)) return 0;
+    if (!enc) return 0;
     CUtensorMap map;
     const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
     const cuuint64_t strides[1] = {512};
@@ -1719,7 +1726,7 @@ static int launch_linear_tma_agg(const float* X, int64_t B, int N, const float* 
                                  const float* bias, const float* in_scale, const float* in_shift, int in_relu, float* Z,
                                  double* stats, cudaStream_t stream) {
     EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc || ((uintptr_t)X & 15) || N > TILE_M) return 0;
+    if (!enc || N > TILE_M) return 0;
     const int rpt = (TILE_M / N) * N;
     const long long rows = (long long)B * N;
     CUtensorMap map;
@@ -1754,7 +1761,7 @@ static int launch_linear_tma_grouped(bool agg, const float* X, int64_t B, int N,
                                      const float* W, const float* bias, const float* in_scale, const float* in_shift, int in_relu,
                                      int epg, float* Z, double* env_stats, cudaStream_t stream) {
     EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc || ((uintptr_t)X & 15)) return 0;
+    if (!enc) return 0;
     const int P = (N + TILE_M - 1) / TILE_M, rpt = P == 1 ? (TILE_M / N) * N : TILE_M;
     const long long rows = (long long)B * N;
     CUtensorMap map;
@@ -1797,6 +1804,7 @@ int mtfjsp_enc_linear_tf32(const float* X, int64_t rows, int K, const float* W, 
                            const float* in_shift, int in_relu, float* Z, double* stats, void* stream) {
     if (!X || !W || !Z || rows < 1 || K < 4 || K > 128 || (K % 4) != 0) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(X, W, Z) || !al8(stats)) return MTFJSP_E_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     if (K == 128 && rows >= 4096) {  // the big layers: A operand by TMA (falls through when the driver lacks the entry point)
         const int rc = launch_linear_tma(X, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
@@ -1814,6 +1822,7 @@ int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int row
                          void* stream) {
     if (!X || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(X, Wa, bias_env, W1)) return MTFJSP_E_ARG;
     if (bias_rows != 1 && bias_rows != B) return MTFJSP_E_ARG;
     if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL)) return MTFJSP_E_ARG;
     const long long rows = (long long)B * rows_per_env;
@@ -1839,6 +1848,7 @@ int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int row
 int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
                               const float* a_src, const float* a_dst, float* out, double* stats, int64_t R, void* stream) {
     if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || R < 1) return MTFJSP_E_ARG;
+    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(stats)) return MTFJSP_E_ARG;
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
     static thread_local bool configured = false;
     if (!configured) {
@@ -1862,6 +1872,7 @@ int mtfjsp_enc_gat_trunk_tf32_grouped(const float* fea1, const float* fea2, cons
     if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || !env_stats || B < 1 || M < 1 || M > 128 ||
         B * M > 0x7fffff00LL)
         return MTFJSP_E_ARG;
+    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(env_stats)) return MTFJSP_E_ARG;
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
     static thread_local bool configured = false;
     if (!configured) {
@@ -1885,6 +1896,7 @@ int mtfjsp_enc_aggregate_linear_tf32(const float* X, int64_t B, int N, const flo
                                      double* stats, void* stream) {
     if (!X || !adj_w || !adj_src || !W || !Z || B < 1 || N < 1) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(X, W, Z) || !al8(adj_w) || !al8(stats)) return MTFJSP_E_ARG;
     const int rc = launch_linear_tma_agg(X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, Z, stats, (cudaStream_t)stream);
     if (rc == 0) return MTFJSP_E_STATE;  // not available for this size / driver: the caller runs the two kernels
     return rc < 0 ? rc : MTFJSP_OK;
@@ -1897,6 +1909,7 @@ int mtfjsp_enc_linear_tf32_grouped(const float* X, int64_t B, int rows_per_env, 
                                    double* env_stats, void* stream) {
     if (!X || !W || !Z || !env_stats || !grouped_args_ok(B, rows_per_env, envs_per_group)) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(X, W, Z, in_scale, in_shift) || !al8(env_stats)) return MTFJSP_E_ARG;
     if (K == 128) {
         const int rc = launch_linear_tma_grouped(false, X, B, rows_per_env, nullptr, nullptr, W, bias, in_scale, in_shift, in_relu,
                                                  envs_per_group, Z, env_stats, (cudaStream_t)stream);
@@ -1911,6 +1924,7 @@ int mtfjsp_enc_aggregate_linear_tf32_grouped(const float* X, int64_t B, int N, c
                                              int in_relu, int envs_per_group, float* Z, double* env_stats, void* stream) {
     if (!X || !adj_w || !adj_src || !W || !Z || !env_stats || !grouped_args_ok(B, N, envs_per_group)) return MTFJSP_E_ARG;
     if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!al16(X, W, Z, in_scale, in_shift) || !al8(adj_w) || !al8(env_stats)) return MTFJSP_E_ARG;
     if (N > TILE_M) return MTFJSP_E_STATE;  // the caller runs mtfjsp_enc_aggregate_grouped + mtfjsp_enc_linear_tf32_grouped
     const int rc = launch_linear_tma_grouped(true, X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, envs_per_group, Z,
                                              env_stats, (cudaStream_t)stream);
@@ -1924,6 +1938,7 @@ int mtfjsp_enc_head_tf32_grouped(const float* X, const int32_t* cand, int64_t B,
     if (!X || !in_scale || !in_shift || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1) return MTFJSP_E_ARG;
     if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
     if (bias_rows != 1 && bias_rows != B) return MTFJSP_E_ARG;
+    if (!al16(X, Wa, bias_env, W1, in_scale, in_shift)) return MTFJSP_E_ARG;
     if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL)) return MTFJSP_E_ARG;
     const long long rows = (long long)B * rows_per_env;
     if (rows > 0x7fffffffLL) return MTFJSP_E_ARG;
@@ -1989,6 +2004,7 @@ int mtfjsp_enc_esa_mach_fold(const double* moments, int64_t rows, const float* W
 int mtfjsp_enc_esa_mach_head_tf32(const float* fea1, const float* fea2, int64_t B, int M, const float* W0f, const float* bias_env,
                                   const float* W1, const float* b1, const float* w2, const float* b2, float* out, void* stream) {
     if (!fea1 || !fea2 || !W0f || !bias_env || !W1 || !w2 || !out || B < 1 || M < 1) return MTFJSP_E_ARG;
+    if (!al16(W0f, bias_env, W1)) return MTFJSP_E_ARG;
     const long long rows = (long long)B * M;
     const size_t smem = 2 * (size_t)TILE_N * 128 * 4 + 2 * (size_t)TILE_M * 16 * 4 + (4 * 128 + 2 * 128) * 4 + 2 * 8 + 16;
     static thread_local bool configured = false;
@@ -2047,6 +2063,7 @@ int64_t mtfjsp_enc_wgrad_workspace_floats(int K) {
 int mtfjsp_enc_wgrad_tf32(const float* dY, const float* X, int64_t rows, int K, float* dW, float* db, float* workspace,
                           void* stream) {
     if (!dY || !X || !dW || !workspace || rows < 1 || K < 4 || K > 128 || (K % 4) != 0) return MTFJSP_E_ARG;
+    if (!al16(dY, X, workspace)) return MTFJSP_E_ARG;
     cudaStream_t s = (cudaStream_t)stream;
     const int sms = wgrad_sms();
     switch (wgrad_np(K)) {

@@ -190,7 +190,16 @@ int mtfjsp_host_record_bytes(const mtfjsp_env* h);
 /* ---- encoder side (SURVEY.md 8 a13) --------------------------------------------------------------------------
  * replaces: actor_critic.py:139-140 (dense adj -> sparse COO), gcn_mlp.py:125 (FP64 SpMM A*h) and :133-149 (degree
  * SpMM): out[b,v,:] = (h[b,v,:] + adj_w[b,v,0]*h[b,v-1,:] + adj_w[b,v,1]*h[b,adj_src[b,v],:]) / in_degree, FP32
- * fused multiply-adds.  h, out: [B,N,C] f32 (C % 4 == 0); adj_w / adj_src as written by mtfjsp_obs. */
+ * fused multiply-adds.  h, out: [B,N,C] f32 (C % 4 == 0); adj_w / adj_src as written by mtfjsp_obs.
+ *
+ * Alignment (every mtfjsp_enc_* entry point below): the kernels move activations, weights and affines 16 bytes at a
+ * time (float4, cp.async, TMA), so these pointers must be 16-byte aligned: h / g / x / gy / out / y / dx / mean / rstd /
+ * t / dt / dparts and the BatchNorm w / b of aggregate, aggregate_bwd, bn_fwd, bn_bwd and gat_attend(_bwd); in_scale /
+ * in_shift of aggregate(_grouped) and of every *_grouped layer and head; X, W, Z of the linear layers; X, Wa, W1,
+ * bias_env of the heads; dY, X, workspace of wgrad; fea2, Wt, out of the GAT trunks; W0f, W1, bias_env of the ESA head.
+ * adj_w, fea1 and the f64 stats / workspace / env_stats / sums buffers must be 8-byte aligned.  A misaligned pointer
+ * returns MTFJSP_E_ARG before anything is launched.  Every torch allocation and every row slice of a [rows, C % 4 == 0]
+ * tensor satisfies this. */
 int mtfjsp_enc_aggregate(const float* h, const float* adj_w, const int16_t* adj_src, float* out, int64_t B, int N,
                          int C, const float* in_scale, const float* in_shift, int in_relu, void* stream);
 /* Backward of mtfjsp_enc_aggregate for the PPO update (ppo_algorithm.py:739-775 re-runs the encoder with gradients;

@@ -101,10 +101,16 @@ def test_aggregate_kernel_matches_dense_fp64_reference():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("K,rows,affine", [(128, 128, False), (128, 1000, True), (12, 333, False), (12, 4096 + 17, True),
-                                           (128, 128 * 300 + 5, True), (64, 777, True)])
+                                           (128, 128 * 300 + 5, True), (64, 777, True),
+                                           # every K class (16, 32, 64, 128), K below the class, K not a multiple of 8
+                                           (4, 1, True), (8, 127, False), (16, 129, True), (20, 333, False), (32, 127, True),
+                                           (36, 1, False), (60, 129, True), (68, 777, False), (100, 127, True), (124, 4096 + 17, True),
+                                           # one row either side of the switch to the TMA operand at K = 128
+                                           (128, 4095, True), (128, 4096, False), (128, 4096, True)])
 def test_tcgen05_linear_matches_fp32_matmul(K, rows, affine):
     """Fused linear layer on the tensor cores (TF32 operands, FP32 accumulate) against an FP64 matmul of the
-    TF32-rounded operands (tight) and against plain FP32 (TF32 tolerance, 10-bit mantissa)."""
+    TF32-rounded operands (tight) and against plain FP32 (TF32 tolerance, 10-bit mantissa).  Every instantiation of the
+    cp.async kernel (K padded to 16, 32, 64, 128, the padding zero-filled) and the TMA kernel (K = 128, rows >= 4,096)."""
     torch = pytest.importorskip("torch")
     enc = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.encoder")
     g = torch.Generator(device="cuda").manual_seed(K * 1000 + rows)
@@ -131,6 +137,8 @@ def test_tcgen05_linear_matches_fp32_matmul(K, rows, affine):
     np.testing.assert_allclose(z.double().cpu().numpy(), ref_f.cpu().numpy(), rtol=5e-3, atol=5e-3)
     np.testing.assert_allclose(stats[:128].cpu().numpy(), z.double().sum(0).cpu().numpy(), rtol=1e-5, atol=1e-3)
     np.testing.assert_allclose(stats[128:].cpu().numpy(), (z.double() ** 2).sum(0).cpu().numpy(), rtol=1e-5, atol=1e-3)
+    if rows == 1:  # torch's batch_norm needs two rows per channel
+        return
     scale, shift = enc.bn_finalize(stats, rows, torch.ones(128, device="cuda"), torch.zeros(128, device="cuda"))
     bn = torch.nn.functional.batch_norm(z, None, None, None, None, True, 0.0, 1e-5)
     np.testing.assert_allclose((z * scale + shift).cpu().numpy(), bn.cpu().numpy(), rtol=1e-3, atol=1e-4)
@@ -312,7 +320,9 @@ def test_fused_machine_trunk_matches_the_fp64_chain_on_tf32_operands(R):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("K,rows", [(128, 64), (128, 1000), (12, 333), (12, 64 * 200 + 17), (128, 64 * 148 * 3 + 5),
-                                    (64, 777), (32, 4096)])
+                                    (64, 777), (32, 4096),
+                                    # K below its class (4 / 16, 20 / 32, 36 / 64, 100 / 128), one partial 64-row stage
+                                    (4, 1), (16, 63), (20, 65), (36, 1), (100, 63), (100, 65), (4, 64 * 148 + 3)])
 def test_tcgen05_weight_gradient_matches_fp64_product(K, rows):
     """dW = dY^T X and db = column sums of dY on the tensor cores (TF32 operands, FP32 accumulate over the rows of a
     CTA, fixed-order FP32 sum of the CTA partials) against the FP64 product of the TF32-rounded operands (tight:
@@ -335,7 +345,11 @@ def test_tcgen05_weight_gradient_matches_fp64_product(K, rows):
     ref_f = gz.double().T @ x.double()
     scale = float(rows) ** 0.5  # entries are sums of `rows` products of unit normals
     np.testing.assert_allclose(dW.double().cpu().numpy() / scale, ref_t.cpu().numpy() / scale, rtol=0, atol=2e-5)
-    np.testing.assert_allclose(dW.double().cpu().numpy() / scale, ref_f.cpu().numpy() / scale, rtol=0, atol=3e-3)
+    if rows >= 64:
+        np.testing.assert_allclose(dW.double().cpu().numpy() / scale, ref_f.cpu().numpy() / scale, rtol=0, atol=3e-3)
+    else:  # too few rows to average the operand rounding: each operand within 2^-11 of its TF32 value
+        bound = 2.0 ** -10 * (gz.double().abs().T @ x.double().abs()) + 1e-6
+        assert bool(((dW.double() - ref_f).abs() <= bound).all())
     np.testing.assert_allclose(db.double().cpu().numpy() / scale, gz.double().sum(0).cpu().numpy() / scale, rtol=0, atol=1e-5)
 
 

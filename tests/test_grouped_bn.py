@@ -74,8 +74,8 @@ def _env(J, M, E, B, seed=77, steps=0):
 @pytest.mark.parametrize("N", [36, 100, 120, 150, 200, 600])
 @pytest.mark.parametrize("epg", [1, 3, 16])
 def test_grouped_kernels_against_fp64(N, epg):
-    """linear (K = 12 and K = 128 with a per-group affine), aggregation + layer, finalize, aggregation, pooling and the
-    policy head against FP64 torch, B = 5 epg envs (not a multiple of the envs per tile for N = 36 with epg != 3)."""
+    """linear (K = 4, 8, 12, 16 and K = 128 with a per-group affine), aggregation + layer, finalize, aggregation, pooling
+    and the policy head against FP64 torch, B = 5 epg envs (not a multiple of the envs per tile for N = 36 with epg != 3)."""
     torch.manual_seed(N * 31 + epg)
     dev = torch.device("cuda")
     B = 5 * epg
@@ -90,6 +90,14 @@ def test_grouped_kernels_against_fp64(N, epg):
     z = enc.linear_tf32_grouped(x12, N, W12, b, None, None, False, es)
     ref = _tf32(x12).double() @ _tf32(W12).double().T + b.double()
     np.testing.assert_allclose(z.double().cpu().numpy(), ref.cpu().numpy(), rtol=2e-5, atol=2e-5)
+    for K in (4, 8, 16):  # the other widths the grouped first layer accepts
+        xk, Wk = torch.randn(rows, K, device=dev), torch.randn(128, K, device=dev) / K ** 0.5
+        esk = torch.full_like(es, float("nan"))
+        zk = enc.linear_tf32_grouped(xk, N, Wk, b, None, None, False, esk)
+        refk = _tf32(xk).double() @ _tf32(Wk).double().T + b.double()
+        np.testing.assert_allclose(zk.double().cpu().numpy(), refk.cpu().numpy(), rtol=2e-5, atol=2e-5, err_msg="K=%d" % K)
+        zd = zk.double().view(B, N, 128)
+        np.testing.assert_allclose(esk[:, 0, 0].cpu().numpy(), zd[:, :128].sum(1).cpu().numpy(), rtol=1e-12, atol=1e-9)
 
     def check_stats(z, es):
         zd = z.double().view(B, N, 128)

@@ -224,41 +224,76 @@ def _bn64(x, w, b, groups):
     return ((xs - mean) / torch.sqrt(var + 1e-5) * w + b).reshape(x.shape)
 
 
-def _mlp3_tanh64(w, p, x):                                          # MLPActor / MLPCritic, gcn_mlp.py:322-434
-    h = torch.tanh(F.linear(x, w[p + "linears.0.weight"], w[p + "linears.0.bias"]))
-    h = torch.tanh(F.linear(h, w[p + "linears.1.weight"], w[p + "linears.1.bias"]))
+def _linear64(rnd):
+    """F.linear, or with rnd (the operand rounding of the tcgen05 path, e.g. to TF32) applied to both GEMM operands."""
+    return F.linear if rnd is None else (lambda x, W, b=None: F.linear(rnd(x), rnd(W), b))
+
+
+def _mlp3_tanh64(w, p, x, rnd=None):                                # MLPActor / MLPCritic, gcn_mlp.py:322-434
+    """rnd: see f64_graph_cnn; the tcgen05 path runs the two 128 -> 128 layers on rounded operands, the last in FP32."""
+    lin = _linear64(rnd)
+    h = torch.tanh(lin(x, w[p + "linears.0.weight"], w[p + "linears.0.bias"]))
+    h = torch.tanh(lin(h, w[p + "linears.1.weight"], w[p + "linears.1.bias"]))
     return F.linear(h, w[p + "linears.2.weight"], w[p + "linears.2.bias"])
 
 
-def f64_graph_cnn(w, task_fea, A, groups):
+def f64_graph_cnn(w, task_fea, A, groups, rnd=None, trace=None, feed=None):
     """GraphCNN.forward (gcn_mlp.py:160-197) with next_layer (:109-158): dense neighbourhood mean (bmm, then division by
     the in-degree = non-zeros of the row, :125-149), MLP (:238-249: Linear -> BN -> ReLU twice, then Linear), BN, ReLU;
-    then the graph mean (:192).  BatchNorm statistics per group of consecutive envs."""
+    then the graph mean (:192).  BatchNorm statistics per group of consecutive envs.
+    rnd: None = the reference's arithmetic order.  Otherwise the shadow of the tcgen05 path (encoder._encode_tf32 and its
+    grouped form): rnd rounds both operands of every Linear, and the first Linear of the second round forms the product
+    first and then the weighted neighbourhood mean of the product rows when N <= 128 (the fused aggregation + layer,
+    DESIGN.md section 6), the mean first above 128 nodes.  trace: a list that receives the six pre-BatchNorm Linear outputs.
+    feed: six tensors that replace those outputs once traced, so that each layer starts from given values (a device run's
+    layer outputs: the restatement then checks one layer at a time)."""
     B, N, _ = task_fea.shape
     deg = (A != 0).sum(-1, keepdim=True).double()
+    lin = _linear64(rnd)
     h = task_fea.double()
     for l in (0, 1):
-        x = (torch.bmm(A, h) / deg).reshape(B * N, -1)
         p = "encoder.feature_extract.mlps.%d." % l
-        for i in (0, 1):
-            x = F.relu(_bn64(F.linear(x, w[p + "linears.%d.weight" % i], w[p + "linears.%d.bias" % i]),
-                             w[p + "batch_norms.%d.weight" % i], w[p + "batch_norms.%d.bias" % i], groups))
-        x = F.linear(x, w[p + "linears.2.weight"], w[p + "linears.2.bias"])
+        x = h
+        for i in (0, 1, 2):
+            W, b = w[p + "linears.%d.weight" % i], w[p + "linears.%d.bias" % i]
+            if i > 0:
+                x = lin(x, W, b)
+            elif rnd is not None and l == 1 and N <= 128:
+                x = (torch.bmm(A, lin(x, W).reshape(B, N, -1)) / deg).reshape(B * N, -1) + b
+            else:
+                x = lin((torch.bmm(A, x) / deg).reshape(B * N, -1), W, b)
+            if trace is not None:
+                trace.append(x)
+            if feed is not None:
+                x = feed[3 * l + i].double()
+            if i < 2:
+                x = F.relu(_bn64(x, w[p + "batch_norms.%d.weight" % i], w[p + "batch_norms.%d.bias" % i], groups))
         x = F.relu(_bn64(x, w["encoder.feature_extract.batch_norms.%d.weight" % l], w["encoder.feature_extract.batch_norms.%d.bias" % l],
                          groups))
         h = x.reshape(B, N, -1)
     return h.mean(dim=1), h
 
 
-def f64_job_evaluate(w, task_fea, A, candidate, h_g_m_pooled, mask, groups):
-    """Operation_Actor_JointAction_selfCritic.forward (actor_critic.py:180-296) without the draw -> prob, pooled, job_v."""
-    pooled, nodes = f64_graph_cnn(w, task_fea, A, groups)
+def f64_job_evaluate(w, task_fea, A, candidate, h_g_m_pooled, mask, groups, rnd=None, trace=None, feed=None):
+    """Operation_Actor_JointAction_selfCritic.forward (actor_critic.py:180-296) without the draw -> prob, pooled, job_v.
+    rnd / trace / feed: see f64_graph_cnn.  With rnd, the policy head's first Linear is split into the column blocks of
+    encoder._head_tf32: the candidate rows times the first block, plus (pooled, h_g_m_pooled) times the other two applied
+    per env as a bias, each product on rounded operands."""
+    pooled, nodes = f64_graph_cnn(w, task_fea, A, groups, rnd, trace, feed)
     J, H = candidate.shape[1], nodes.shape[-1]
     cf = torch.gather(nodes, 1, candidate.long().unsqueeze(-1).expand(-1, J, H))             # :197-207
     gm = w["_input"][None, None, :].expand_as(cf) if h_g_m_pooled is None else h_g_m_pooled.unsqueeze(1).expand_as(cf)  # :230-240
-    x = torch.cat((cf, pooled.unsqueeze(1).expand_as(cf), gm), dim=-1)                      # :244-247
-    s = _mlp3_tanh64(w, "o_policy.", x).squeeze(-1).masked_fill(mask.bool(), float("-inf"))   # :256, :266-268
-    return F.softmax(s, dim=-1), pooled, _mlp3_tanh64(w, "job_critic.", pooled)               # :278, :293
+    if rnd is None:
+        x = torch.cat((cf, pooled.unsqueeze(1).expand_as(cf), gm), dim=-1)                  # :244-247
+        s = _mlp3_tanh64(w, "o_policy.", x)
+    else:
+        lin, W0, p = _linear64(rnd), w["o_policy.linears.0.weight"], "o_policy."
+        env_bias = lin(pooled, W0[:, H:2 * H], w[p + "linears.0.bias"]) + lin(gm[:, 0], W0[:, 2 * H:])
+        h = torch.tanh(lin(cf, W0[:, :H]) + env_bias.unsqueeze(1))
+        h = torch.tanh(lin(h, w[p + "linears.1.weight"], w[p + "linears.1.bias"]))
+        s = F.linear(h, w[p + "linears.2.weight"], w[p + "linears.2.bias"])
+    s = s.squeeze(-1).masked_fill(mask.bool(), float("-inf"))                                # :256, :266-268
+    return F.softmax(s, dim=-1), pooled, _mlp3_tanh64(w, "job_critic.", pooled, rnd)          # :278, :293
 
 
 def _gat64(w, h1, h2):
