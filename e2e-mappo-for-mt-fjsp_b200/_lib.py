@@ -72,6 +72,7 @@ SIGNATURES = {
     "mtfjsp_costs": ([_VP, _VP, _VP, _VP], _I),
     "mtfjsp_export_state": ([_VP] + [_VP] * 4 + [_VP], _I),
     "mtfjsp_export_scaler": ([_VP] + [_VP] * 4 + [_VP], _I),
+    "mtfjsp_gather": ([_VP, _VP, _VP, _VP], _I),
     "mtfjsp_policy_random": ([_VP, _U64, _U64, _I, _VP, _VP, _VP], _I),
     "mtfjsp_random_step": ([_VP, _U64, _U64] + [_VP] * 14 + [_I, _I, _VP], _I),
     "mtfjsp_step_host": ([_VP] + [_VP] * 9 + [_I, _I, _VP], _I),
@@ -111,6 +112,7 @@ SIGNATURES = {
     "mtfjsp_launch_count": ([_VP], C.c_int64),
     "mtfjsp_bytes_per_step": ([_VP, _I], C.c_int64),
     "mtfjsp_bytes_per_random_step": ([_VP, _I], C.c_int64),
+    "mtfjsp_bytes_per_gather": ([_VP], C.c_int64),
     "mtfjsp_random_step_is_fused": ([_VP], _I),
     "mtfjsp_last_error": ([], C.c_char_p),
     "mtfjsp_version": ([], C.c_char_p),

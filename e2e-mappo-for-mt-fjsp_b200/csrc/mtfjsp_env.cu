@@ -2175,6 +2175,75 @@ __global__ void reset_copy_kernel(Layout L, const double* __restrict__ sd0, cons
     }
 }
 
+// Env gather (mtfjsp_gather): destination env b becomes a copy of source env idx[b] -- every per-env record and table the
+// handle keeps.  The two handles share (J, M, E), so they share every stride.
+struct GatherArgs {
+    Layout L;
+    int src_B;
+    const int32_t* idx;
+    const double *sd, *sd0, *xs, *t, *p;
+    const int16_t *si, *si0;
+    const int8_t* edge_id;
+    const uint8_t *jm_fin, *jm_esa, *dn, *inv;
+    const int32_t* cand;
+    double *d_sd, *d_sd0, *d_xs, *d_t, *d_p;
+    int16_t *d_si, *d_si0;
+    int8_t* d_edge_id;
+    uint8_t *d_jm_fin, *d_jm_esa, *d_dn, *d_inv;
+    int32_t* d_cand;
+};
+
+template <typename W>
+__device__ __forceinline__ void copy_words(void* dst, const void* src, size_t n) {
+    for (size_t k = threadIdx.x; k < n; k += blockDim.x) reinterpret_cast<W*>(dst)[k] = reinterpret_cast<const W*>(src)[k];
+}
+
+// One block per destination env, 16 bytes per thread (every record is 16-byte aligned; the t / p tables of one env are
+// too when N*M is even, 8-byte words otherwise), as reset_copy_kernel.  A source index outside the batch is input from
+// outside the program: that env gets its invalid flag and nothing else.
+__global__ void __launch_bounds__(128) gather_kernel(const __grid_constant__ GatherArgs A) {
+    const Layout& L = A.L;
+    const size_t b = blockIdx.x;
+    const int src = A.idx[b];
+    if (src < 0 || src >= A.src_B) {
+#ifdef MTFJSP_DEBUG_BOUNDS  // debug builds: an out-of-range source env is a caller bug worth stopping at
+        assert(src >= 0 && src < A.src_B);
+#endif
+        if (threadIdx.x == 0) A.d_inv[b] = 1;
+        return;
+    }
+    const size_t a = (size_t)src;
+    copy_words<double2>(A.d_sd + b * L.sd_stride, A.sd + a * L.sd_stride, L.sd_stride / 2);
+    copy_words<double2>(A.d_sd0 + b * L.sd_stride, A.sd0 + a * L.sd_stride, L.sd_stride / 2);
+    copy_words<double2>(A.d_xs + b * L.xs_stride, A.xs + a * L.xs_stride, L.xs_stride / 2);
+    copy_words<int4>(A.d_si + b * L.si_stride, A.si + a * L.si_stride, L.si_stride / 8);
+    copy_words<int4>(A.d_si0 + b * L.si_stride, A.si0 + a * L.si_stride, L.si_stride / 8);
+    const size_t nm = (size_t)L.N * L.M;
+    if (nm % 2 == 0) {
+        copy_words<double2>(A.d_t + b * nm, A.t + a * nm, nm / 2);
+        copy_words<double2>(A.d_p + b * nm, A.p + a * nm, nm / 2);
+    } else {
+        copy_words<double>(A.d_t + b * nm, A.t + a * nm, nm);
+        copy_words<double>(A.d_p + b * nm, A.p + a * nm, nm);
+    }
+    for (int k = threadIdx.x; k < L.M; k += blockDim.x) A.d_edge_id[b * L.M + k] = A.edge_id[a * L.M + k];
+    for (int j = threadIdx.x; j < L.J; j += blockDim.x) {
+        A.d_jm_fin[b * L.J + j] = A.jm_fin[a * L.J + j];
+        A.d_jm_esa[b * L.J + j] = A.jm_esa[a * L.J + j];
+        A.d_cand[b * L.J + j] = A.cand[a * L.J + j];
+    }
+    if (threadIdx.x == 0) {
+        A.d_dn[b] = A.dn[a];
+        A.d_inv[b] = A.inv[a];
+    }
+}
+
+// bytes gather_kernel copies per env (each read once and written once)
+size_t gather_env_bytes(const Layout& L) {
+    return (size_t)2 * L.sd_stride * 8 + (size_t)L.xs_stride * 8 + (size_t)2 * L.si_stride * 2 + (size_t)2 * L.N * L.M * 8 +
+           (size_t)L.M + (size_t)2 * L.J + (size_t)4 * L.J + 2;
+}
+
 thread_local char g_err[512] = "";
 
 int fail(int code, const char* msg, cudaError_t e = cudaSuccess) {
@@ -2941,6 +3010,43 @@ int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int6
     return MTFJSP_OK;
 }
 
+int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, void* stream) {
+    if (!dst || !src || !idx) return fail(MTFJSP_E_ARG, "mtfjsp_gather: bad argument");
+    if (dst == src) return fail(MTFJSP_E_ARG, "mtfjsp_gather: src and dst are the same handle (no in-place gather)");
+    if (dst->device != src->device) return fail(MTFJSP_E_ARG, "mtfjsp_gather: src and dst live on different devices");
+    const Layout &Ld = dst->L, &Ls = src->L;
+    if (Ld.J != Ls.J || Ld.M != Ls.M || Ld.E != Ls.E || Ld.left_shift != Ls.left_shift)
+        return fail(MTFJSP_E_ARG, "mtfjsp_gather: src and dst differ in (J, M, E, left_shift)");
+    if (dst->cfgw[0] != src->cfgw[0] || dst->cfgw[1] != src->cfgw[1] || dst->cfgw[2] != src->cfgw[2] ||
+        dst->divisor != src->divisor || dst->gamma != src->gamma)
+        return fail(MTFJSP_E_ARG, "mtfjsp_gather: src and dst differ in mtfjsp_set_params (weights, divisor, gamma)");
+    if (!src->loaded) return fail(MTFJSP_E_STATE, "mtfjsp_gather from a handle that was never loaded");
+    cudaStream_t s = (cudaStream_t)stream;
+    // a non-step call on both handles: recorded resets run now (src's belongs to the copied state; dst's next step would
+    // otherwise perform its own on the copy), and the next step of either waits for the copy in full
+    mtfjsp_env* hs = const_cast<mtfjsp_env*>(src);
+    int rc = enter(hs, s);
+    if (rc) return rc;
+    rc = enter(dst, s);
+    if (rc) return rc;
+    GatherArgs A;
+    memset(&A, 0, sizeof A);
+    A.L = Ld; A.src_B = Ls.B; A.idx = idx;
+    A.sd = hs->sd; A.sd0 = hs->sd0; A.xs = hs->xs; A.t = hs->t; A.p = hs->p; A.si = hs->si; A.si0 = hs->si0;
+    A.edge_id = hs->edge_id; A.jm_fin = hs->jm_fin; A.jm_esa = hs->jm_esa; A.dn = hs->dn; A.inv = hs->inv; A.cand = hs->cand;
+    A.d_sd = dst->sd; A.d_sd0 = dst->sd0; A.d_xs = dst->xs; A.d_t = dst->t; A.d_p = dst->p; A.d_si = dst->si; A.d_si0 = dst->si0;
+    A.d_edge_id = dst->edge_id; A.d_jm_fin = dst->jm_fin; A.d_jm_esa = dst->jm_esa; A.d_dn = dst->dn; A.d_inv = dst->inv;
+    A.d_cand = dst->cand;
+    gather_kernel<<<Ld.B, 128, 0, s>>>(A);
+    dst->launches++;
+    CK(cudaGetLastError(), "gather_kernel");
+    dst->loaded = true;
+    dst->reset_done = hs->reset_done;
+    dst->reset_snap = hs->reset_snap;
+    dst->obs_synced = false;  // the caller's observation buffers no longer mirror dst's state
+    return MTFJSP_OK;
+}
+
 int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int mask_mode, int32_t* op,
                          int32_t* mach, void* stream) {
     if (!h || !op || !mach) return fail(MTFJSP_E_ARG, "mtfjsp_policy_random: bad argument");
@@ -3226,6 +3332,8 @@ int mtfjsp_host_record_bytes(const mtfjsp_env* h) { return h ? h->rec_stride : 0
 int mtfjsp_launch_overlap_error(const mtfjsp_env* h) { return h ? (int)*(volatile unsigned*)h->ovl_err : 0; }
 
 int64_t mtfjsp_launch_count(const mtfjsp_env* h) { return h ? h->launches : 0; }
+
+int64_t mtfjsp_bytes_per_gather(const mtfjsp_env* h) { return h ? (int64_t)(2 * gather_env_bytes(h->L) + 4) : 0; }
 
 int64_t mtfjsp_bytes_per_step(const mtfjsp_env* h, int dtype) {
     if (!h) return 0;

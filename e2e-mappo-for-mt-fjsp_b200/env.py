@@ -224,6 +224,37 @@ class BatchedMTFJSPEnv:
 
         return step
 
+    # buffers this class owns and hands to the library: what gather_from copies besides the handle's own state
+    _OWNED = ("task_fea", "mach_fea", "adj_w", "adj_src", "job_mask", "candidate", "reward5", "scaled4", "done", "invalid",
+              "op", "mach", "mfea1_buf", "mach_mask")
+
+    def gather_from(self, src, idx):
+        """Env b of this object becomes a copy of env idx[b] of `src` (idx [B] integers; duplicates and permutations are
+        allowed, src.B may differ).  The handle's state -- records, static tables, reset snapshot, masks, candidates,
+        reward-scaler state -- goes through mtfjsp_gather; the buffers this object owns (observation, masks, candidates,
+        step outputs, last actions, candidate-machine features) are copied by index on the device.  Afterwards the object
+        is indistinguishable from one that stepped there itself.  An idx entry outside [0, src.B) leaves env b as it was
+        and sets its invalid flag.  src and this object must have the same sizes, left_shift, reward parameters and
+        observation dtype (MTFJSPError / ValueError otherwise); src must have been loaded."""
+        if not isinstance(src, BatchedMTFJSPEnv):
+            raise TypeError("gather_from needs a BatchedMTFJSPEnv")
+        if src.obs_dtype != self.obs_dtype:
+            raise ValueError("gather_from between environments of different observation dtypes")
+        idx = _to_dev(idx, self.device, torch.int32)
+        if tuple(idx.shape) != (self.B,):
+            raise ValueError("idx must have shape [%d]" % self.B)
+        check(self._lib.mtfjsp_gather(self._h, src._h, _ptr(idx), _stream()), "mtfjsp_gather")
+        ok = (idx >= 0) & (idx < src.B)
+        i = torch.where(ok, idx, 0).long()
+        # two launches per buffer, written in place (the library tracks the observation pointers)
+        for name in self._OWNED:
+            d = getattr(self, name)
+            if name == "invalid":
+                torch.index_select(src.invalid, 0, i, out=d)
+                d.masked_fill_(~ok, 1)
+            else:
+                torch.where(ok.view((-1,) + (1,) * (d.dim() - 1)), getattr(src, name).index_select(0, i), d, out=d)
+
     # ---- views ---------------------------------------------------------------------------------------------------
     def dense_adj(self, dtype=torch.float64):
         adj = torch.empty((self.B, self.N, self.N), dtype=dtype, device=self.device)

@@ -201,3 +201,142 @@ def sampled_validate(job_actor, machine_actor, instances, samples, seed=0, weigh
         out["actions"] = acts.reshape(N, K, S, 2)
         out["best_actions"] = acts[:, best * S + cols]
     return out
+
+
+# per-call BatchNorm group limit of the per-group paths (mtfjsp_enc_bn_fwd's grid.y)
+_MAX_GROUPS = 65535
+
+
+def beam_select(score, width):
+    """One beam step's selection.  score [S, C] f64: the children of an instance in flat order (w * J + j) * M + m, -inf for
+    the impossible ones.  Children rank by (score descending, flat index ascending) and slot w takes the child ranked w; a
+    slot whose child scores -inf is dead and takes the rank-0 child instead (so that every env steps validly).
+    -> child [S, width] int64 flat index, slot score [S, width] f64 (-inf for a dead slot), alive [S, width] bool."""
+    val, order = torch.sort(score, dim=1, descending=True, stable=True)
+    val, order = val[:, :width], order[:, :width]
+    alive = val > float("-inf")
+    return torch.where(alive, order, order[:, :1]), val, alive
+
+
+def _beam_chunk(job_actor, machine_actor, inst, W, weights, left_shift, per_instance_batchnorm, envs, want_actions):
+    """Beam search over one chunk of S instances on the env pair `envs` (two handles of S * W envs, env s * W + w).
+    -> final4 [S,W,4], log_prob [S,W], actions [N,S*W,2] (or None), all on the device."""
+    S, N, M = inst["t"].shape
+    J = N // M
+    B = S * W
+    A, Bn = envs
+    A.load(*(np.repeat(inst[k], W, axis=0) for k in ("t", "p", "transT", "edge")))
+    A.scaler_init()
+    A.reset(np.tile(np.asarray(weights, dtype=np.float64), (B, 1)))
+    A.obs(MASK_ESA)
+    dev = A.device
+    ninf = float("-inf")
+    score = torch.full((S, W), ninf, dtype=torch.float64, device=dev)
+    score[:, 0] = 0.0
+    job_groups, mach_groups = (B, B * J) if per_instance_batchnorm else (1, 1)
+    base = (torch.arange(S, device=dev) * W).unsqueeze(1)
+    parents = torch.empty((N, B), dtype=torch.int64, device=dev) if want_actions else None
+    acts = torch.empty((N, B, 2), dtype=torch.int32, device=dev) if want_actions else None
+    h_mch = None
+    with torch.no_grad():
+        for step in range(N):
+            pj, pooled, _ = job_actor.evaluate(A.task_fea, A.adj_w, A.adj_src, A.candidate, h_mch, A.job_mask, groups=job_groups)
+            # the (env, job) children: candidate-machine features of each job's candidate op, child = env * J + j
+            f1, mm = [], []
+            for j in range(J):
+                a, b = A.mfea1(A.candidate[:, j].contiguous())
+                f1.append(a.clone())
+                mm.append(b.clone())
+            f1 = torch.stack(f1, 1).view(B * J, M, -1)
+            mm = torch.stack(mm, 1).view(B * J, M)
+            pm, hm, _ = machine_actor.forward(f1, A.mach_fea.repeat_interleave(J, 0), pooled.repeat_interleave(J, 0), mm,
+                                              groups=mach_groups)
+            child = (score.reshape(B, 1, 1) + torch.log(pj).double().reshape(B, J, 1)) + torch.log(pm).double().reshape(B, J, M)
+            bad = A.job_mask.bool().reshape(B, J, 1) | mm.bool().reshape(B, J, M)
+            child = torch.where(bad, ninf, child)
+            pick, score, _ = beam_select(child.view(S, W * J * M), W)
+            parent = (base + pick // (J * M)).view(-1)
+            job = ((pick // M) % J).view(-1)
+            Bn.gather_from(A, parent)
+            Bn.op.copy_(Bn.candidate.gather(1, job.unsqueeze(1)).squeeze(1))
+            Bn.mach.copy_((pick % M).view(-1))
+            h_mch = hm.index_select(0, parent * J + job)
+            if want_actions:
+                parents[step] = parent
+                acts[step, :, 0] = Bn.op
+                acts[step, :, 1] = Bn.mach
+            Bn.step_obs(Bn.op, Bn.mach, MASK_ESA)
+            A, Bn = Bn, A
+    if not (bool(A.done.all()) and not bool(A.invalid.any())):
+        raise RuntimeError("beam search ended with an unfinished or invalid env")
+    final4 = A.costs().view(S, W, 4)
+    actions = None
+    if want_actions:  # follow every final slot's parents back to the start
+        actions = torch.empty_like(acts)
+        cur = torch.arange(B, device=dev)
+        for step in range(N - 1, -1, -1):
+            actions[step] = acts[step].index_select(0, cur)
+            cur = parents[step].index_select(0, cur)
+    return final4, score, actions
+
+
+def beam_validate(job_actor, machine_actor, instances, width, weights=(0.4, 0.4, 0.2), left_shift=True,
+                  per_instance_batchnorm=True, max_envs=32768, return_actions=False):
+    """Deterministic beam search of width W = `width` over joint (job, machine) actions for every instance of `instances`
+    ({"t","p","transT","edge"} arrays, [S,...]), on the same actor pairs, precisions and BatchNorm semantics as
+    `greedy_validate`.
+
+    Each instance keeps W partial schedules (slots; slot 0 starts live, the others dead at score -inf).  Per step the job
+    actor runs on every slot's env, and the machine actor on every (slot, job) child -- with per_instance_batchnorm each
+    child is its own BatchNorm group, as a batch-1 validation of that env would be.  A (slot, job, machine) child scores
+    parent + log p_job + log p_mach (torch.log of the FP32 probabilities greedy arg-maxes, summed in FP64; masked jobs and
+    infeasible machines -inf), and the W best children of the instance become its next slots (`beam_select`: ties to the
+    lowest flat index (w * J + j) * M + m; a slot without a finite child is dead and copies the best one).  The envs of the
+    chosen parents are copied into a second env batch (`BatchedMTFJSPEnv.gather_from`) and stepped there; the two batches
+    swap roles every step.  Instances run in chunks of at most `max_envs` envs (and of at most 65,535 children, the
+    per-group BatchNorm limit of one machine-actor call).  With per_instance_batchnorm and tf32 actors an instance's
+    result does not depend on the chunking or on the other instances.
+    per_instance_batchnorm=False gives each actor call one BatchNorm group over its whole batch, as greedy_validate does,
+    but the batch here is not greedy's: the job actor's statistics run over the S_chunk * W slot envs, dead slots (copies
+    of their instance's best child) included, and the machine actor's over all S_chunk * W * J (slot, job) children, those
+    of masked and finished jobs included.  The result then depends on W, on `max_envs` and on the other instances of the
+    chunk; it is not the whole-batch greedy semantics at W = 1 either.
+    -> dict: final4 [W,S,4], objective [W,S], log_prob [W,S] (the slot's score), alive [W,S], best_index [S] (the live
+             slot of the lowest objective, lowest w on ties), best_final4 [S,4], best_objective [S] and, with
+             return_actions, actions [N,W,S,2] (op, machine) and best_actions [N,S,2]."""
+    inst = {k: np.asarray(instances[k]) for k in ("t", "p", "transT", "edge")}
+    S, N, M = inst["t"].shape
+    J, E = N // M, inst["edge"].shape[1]
+    W = int(width)
+    if W < 1 or max_envs < W:
+        raise ValueError("width must be >= 1 and max_envs >= width")
+    if W * J > _MAX_GROUPS:
+        raise ValueError("width * J = %d children per instance exceed the %d BatchNorm groups of one machine-actor call"
+                         % (W * J, _MAX_GROUPS))
+    chunk = max(1, min(max_envs // W, _MAX_GROUPS // (W * J)))
+    final4 = np.zeros((W, S, 4))
+    log_prob = np.zeros((W, S))
+    acts = np.zeros((N, W, S, 2), dtype=np.int32) if return_actions else None
+    envs = None
+    for s0 in range(0, S, chunk):
+        s1 = min(S, s0 + chunk)
+        B = (s1 - s0) * W
+        if envs is None or envs[0].B != B:
+            envs = tuple(BatchedMTFJSPEnv(B, J, M, E, left_shift=left_shift, weights=weights, obs_dtype=torch.float32,
+                                          mask_mode=MASK_ESA) for _ in range(2))
+        f4, lp, ac = _beam_chunk(job_actor, machine_actor, {k: v[s0:s1] for k, v in inst.items()}, W, weights, left_shift,
+                                 per_instance_batchnorm, envs, return_actions)
+        final4[:, s0:s1] = f4.transpose(0, 1).cpu().numpy()
+        log_prob[:, s0:s1] = lp.t().cpu().numpy()
+        if acts is not None:
+            acts[:, :, s0:s1] = ac.view(N, s1 - s0, W, 2).transpose(1, 2).cpu().numpy()
+    obj = _objective(final4, weights)
+    alive = log_prob > -np.inf
+    best = np.argmin(np.where(alive, obj, np.inf), axis=0)
+    cols = np.arange(S)
+    out = {"final4": final4, "objective": obj, "log_prob": log_prob, "alive": alive, "best_index": best,
+           "best_final4": final4[best, cols], "best_objective": obj[best, cols]}
+    if acts is not None:
+        out["actions"] = acts
+        out["best_actions"] = acts[:, best, cols]
+    return out

@@ -134,6 +134,24 @@ int mtfjsp_costs(mtfjsp_env* h, double* cost4, double* total_e1, void* stream);
 int mtfjsp_export_state(mtfjsp_env* h, int32_t* mach, double* st, double* ft, int32_t* routes, void* stream);
 int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int64_t* n, void* stream);
 
+/* Copies environments between handles: afterwards env b of `dst` is in exactly the state env idx[b] of `src` was in,
+ * and every later call on dst env b returns the same bits as on a fresh env that replayed idx[b]'s whole history --
+ * steps, observations, masks, candidates, rewards, scaled rewards, costs, export_state / export_scaler, and later
+ * resets back to that instance.  Per env it copies the state records, the static tables (t, p, transport table,
+ * minimum durations, edge groups), the reset snapshot, both job-mask forms, the candidates and the done / invalid
+ * flags; dst takes src's loaded / reset status.  idx: [dst.B] int32 on the device; duplicates and permutations are
+ * allowed and dst.B may differ from src.B.  The reward scaler's state travels with the env.
+ * Both handles first perform a recorded reset (mtfjsp_reset): one recorded on src is in the copied state, and one
+ * recorded on dst is performed before the copy overwrites it (a later step of dst would otherwise perform it on the
+ * copied state).  The next step of either handle waits for the copy in full, and dst's next observation-writing step
+ * rewrites every row.
+ * MTFJSP_E_ARG, nothing written: src == dst, a NULL argument, different devices, (J, M, E, left_shift) differ, or the
+ * mtfjsp_set_params values differ.  MTFJSP_E_STATE, nothing written: src was never loaded.  An idx[b] outside [0, src.B)
+ * cannot be checked on the host without a synchronisation: for such a b the kernel writes only dst's invalid flag of
+ * env b (1) and leaves the rest of that env as it was (the convention of an invalid action); debug builds
+ * (MTFJSP_DEBUG_BOUNDS) assert.  src and dst must be used on the same stream, or ordered by the caller. */
+int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, void* stream);
+
 /* Uniform random valid action from the env's current masks: a selectable job (under mask_mode), its candidate
  * op, and a feasible machine for it; counter-based, keyed by (seed, env_offset + env, ops scheduled so far).
  * Mirrors tester/pdrs.py Random_task / Random_m (:75-86, :139-156).  op, mach [B] int32 (-1 when done). */
@@ -377,6 +395,8 @@ int64_t mtfjsp_bytes_per_step(const mtfjsp_env* h, int dtype);
  * bytes plus the policy / candidate-machine-feature traffic (job mask, candidates, t / p rows, edge ids in; action,
  * [M,6] features, machine mask out).  mtfjsp_random_step_is_fused: 1 if mtfjsp_random_step is that single launch. */
 int64_t mtfjsp_bytes_per_random_step(const mtfjsp_env* h, int dtype);
+/* Bytes mtfjsp_gather reads and writes per destination env (the records and tables it copies, counted once each way). */
+int64_t mtfjsp_bytes_per_gather(const mtfjsp_env* h);
 int mtfjsp_random_step_is_fused(const mtfjsp_env* h);
 const char* mtfjsp_last_error(void);
 const char* mtfjsp_version(void);
