@@ -73,6 +73,7 @@ SIGNATURES = {
     "mtfjsp_export_state": ([_VP] + [_VP] * 4 + [_VP], _I),
     "mtfjsp_export_scaler": ([_VP] + [_VP] * 4 + [_VP], _I),
     "mtfjsp_gather": ([_VP, _VP, _VP, _VP], _I),
+    "mtfjsp_peek": ([_VP, _VP, _VP, _I, _VP, _VP, _VP], _I),
     "mtfjsp_policy_random": ([_VP, _U64, _U64, _I, _VP, _VP, _VP], _I),
     "mtfjsp_random_step": ([_VP, _U64, _U64] + [_VP] * 14 + [_I, _I, _VP], _I),
     "mtfjsp_step_host": ([_VP] + [_VP] * 9 + [_I, _I, _VP], _I),
@@ -113,6 +114,7 @@ SIGNATURES = {
     "mtfjsp_bytes_per_step": ([_VP, _I], C.c_int64),
     "mtfjsp_bytes_per_random_step": ([_VP, _I], C.c_int64),
     "mtfjsp_bytes_per_gather": ([_VP], C.c_int64),
+    "mtfjsp_bytes_per_peek": ([_VP, _I], C.c_int64),
     "mtfjsp_random_step_is_fused": ([_VP], _I),
     "mtfjsp_last_error": ([], C.c_char_p),
     "mtfjsp_version": ([], C.c_char_p),

@@ -2244,6 +2244,297 @@ size_t gather_env_bytes(const Layout& L) {
            (size_t)L.M + (size_t)2 * L.J + (size_t)4 * L.J + 2;
 }
 
+// One-step lookahead (mtfjsp_peek): what mtfjsp_step would return for each of K (op, machine) pairs per env, computed
+// from a read-only copy of the env's records.  One block per env stages the records once; then, per chunk of
+// PEEK_CHUNK pairs, warps evaluate one pair each (placement scan, makespan, energy) and threads finish one pair each
+// (the sequential idle sum and the reward).  Every quantity is the step's own FP64 expression in the step's operand
+// order (env_kernel above), restated on the read-only copy by deltas:
+//   placement  the step's scan over machine m's route, unchanged;
+//   makespan   max over every op of its finish time, job a/M's remaining chain re-derived from a's new finish;
+//   energy     numpy's pairwise sum of the per-op estimate with a's term d*p in place of minpt[a]: only the leaf that
+//              holds a is re-added, the other leaves are the env's (computed once per block), then the leaves are
+//              combined by the plan's postfix program;
+//   idle time  the flat-order sequential sum: the unchanged prefix in front of a's slot (prefix sums computed once per
+//              block), a's term, its route follower's term against a's new finish, then the unchanged rest.
+struct PeekArgs {
+    Layout L;
+    PwPlan pw;
+    const double *sd, *xs, *t, *p;
+    const int16_t* si;
+    const int32_t *op, *mach;
+    int K;
+    double cfgw[3], divisor;
+    double* reward5;
+    uint8_t* invalid;
+};
+
+constexpr int PEEK_CHUNK = 128, PEEK_STK = 16;
+
+// shared-memory plan of peek_kernel (bytes): the staged record prefix st ft dur psel scal, the static doubles, the idle
+// prefix sums, the base leaf results, the si record up to the counters and nsched, the route offsets, the per-warp leaf
+// combine stacks and the per-pair results of one chunk
+struct PeekSmem {
+    int sd, xs, pre, leaf, stk, si, off, c_d, c_i, total;
+};
+__host__ __device__ inline PeekSmem peek_smem(const Layout& L, int nleaves, int warps) {
+    PeekSmem s;
+    int o = 0;
+    s.sd = o; o += (L.o_scal + 4 + 1) / 2 * 16;
+    s.xs = o; o += L.xs_stride * 8;
+    s.pre = o; o += (L.N + 1) * 8;
+    s.leaf = o; o += nleaves * 8;
+    s.stk = o; o += warps * PEEK_STK * 8;
+    s.c_d = o; o += PEEK_CHUNK * 5 * 8;  // st, d, mk, env, trans per pair
+    s.c_i = o; o += PEEK_CHUNK * 4 * 4;  // valid, slot, next, prev per pair
+    s.si = o; o += (L.o_misc + 3) * 2;
+    s.off = (o + 3) / 4 * 4; o = s.off + L.M * 4;
+    s.total = (o + 15) / 16 * 16;
+    return s;
+}
+
+// one leaf of numpy's pairwise sum (pairwise_sum's leaf pass) over est(off .. off + n - 1); every 8-lane segment
+// computes it, lane k == 0 of a segment holds the result
+template <class Est>
+__device__ __forceinline__ double peek_leaf(const Est& est, int off, int n, int k) {
+    const int nb = (n >= 8) ? n - (n & 7) : 0;
+    double r = 0.0;
+    if (n >= 8) {
+        r = est(off + k);
+        for (int i = 8 + k; i < nb; i += 8) r += est(off + i);
+    }
+    r = r + __shfl_down_sync(FULL, r, 1, 8);
+    r = r + __shfl_down_sync(FULL, r, 2, 8);
+    r = r + __shfl_down_sync(FULL, r, 4, 8);
+    double res = r;
+    if (k == 0)
+        for (int i = nb; i < n; i++) res += est(off + i);
+    return res;
+}
+
+__global__ void __launch_bounds__(128) peek_kernel(const __grid_constant__ PeekArgs A) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const Layout& L = A.L;
+    const PwPlan& pw = A.pw;
+    const int N = L.N, M = L.M, K = A.K;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const size_t b = blockIdx.x;
+    const PeekSmem S = peek_smem(L, pw.nleaves, nwarps);
+    double* s_sd = reinterpret_cast<double*>(smem_raw + S.sd);
+    double* s_xs = reinterpret_cast<double*>(smem_raw + S.xs);
+    double* s_pre = reinterpret_cast<double*>(smem_raw + S.pre);
+    double* s_leaf = reinterpret_cast<double*>(smem_raw + S.leaf);
+    double* s_stk = reinterpret_cast<double*>(smem_raw + S.stk) + warp * PEEK_STK;
+    double* c_d = reinterpret_cast<double*>(smem_raw + S.c_d);
+    int* c_i = reinterpret_cast<int*>(smem_raw + S.c_i);
+    int16_t* s_si = reinterpret_cast<int16_t*>(smem_raw + S.si);
+    int* s_off = reinterpret_cast<int*>(smem_raw + S.off);
+
+    // ---- stage the record prefix (st ft dur psel scal), the static doubles and the si record ----
+    {
+        const double* g_sd = A.sd + b * L.sd_stride;
+        for (int i = threadIdx.x; i < L.o_scal + 4; i += blockDim.x) s_sd[i] = g_sd[i];
+        const uint4* src = reinterpret_cast<const uint4*>(A.xs + b * L.xs_stride);
+        uint4* dst = reinterpret_cast<uint4*>(s_xs);
+        for (int i = threadIdx.x; i < L.xs_stride / 2; i += blockDim.x) dst[i] = __ldg(src + i);
+        const int16_t* g_si = A.si + b * L.si_stride;
+        for (int i = threadIdx.x; i < L.o_misc + 3; i += blockDim.x) s_si[i] = g_si[i];
+    }
+    __syncthreads();
+    const double* s_st = s_sd + L.o_st;
+    const double* s_ft = s_sd + L.o_ft;
+    const double* s_dur = s_sd + L.o_dur;
+    const double* s_psel = s_sd + L.o_psel;
+    const double* s_scal = s_sd + L.o_scal;  // mk_prev, e_prev, trans, idle_prev
+    const int16_t* s_mach = s_si + L.o_mach;
+    const int16_t* s_ord = s_si + L.o_ord;
+    const int16_t* s_rpred = s_si + L.o_rpred;
+    const int16_t* s_cnt = s_si + L.o_cnt;
+    const int nsched0 = s_si[L.o_misc + 2];
+    const double* s_mind = s_xs + L.o_mind;
+    const double* s_minpt = s_xs + L.o_minpt;
+    const double* s_tt = s_xs + L.o_tt;
+    // the env's per-op energy estimate (env_kernel's s_pt)
+    const auto est = [&](int v) { return (s_mach[v] >= 0) ? s_dur[v] * s_psel[v] : s_minpt[v]; };
+    if (warp == 0) {  // base leaf results, four leaves at a time as pairwise_sum
+        for (int L0 = 0; L0 < pw.nleaves; L0 += 4) {
+            const int Lx = L0 + (lane >> 3);
+            const bool act = Lx < pw.nleaves;
+            const double r = peek_leaf(est, act ? pw.leaf_off[Lx] : 0, act ? pw.leaf_len[Lx] : 0, lane & 7);
+            if (act && (lane & 7) == 0) s_leaf[Lx] = r;
+        }
+    } else if (warp == 1) {  // route offsets: machine m's route is ord[off[m], off[m] + cnt[m])
+        if (lane == 0) {
+            int o = 0;
+            for (int mm = 0; mm < M; mm++) { s_off[mm] = o; o += s_cnt[mm]; }
+        }
+    }
+    if (threadIdx.x == 0) {  // idle prefix sums over the flat order: s_pre[g] = the step's running sum in front of term g
+        double idle = 0.0;
+        for (int g = 0; g < nsched0; g++) {
+            s_pre[g] = idle;
+            const int v = s_ord[g], rp = s_rpred[v];
+            const double term = (rp < 0) ? (s_st[v] - 0.0) : (s_st[v] - s_ft[rp]);
+            idle = idle + term * 1.0;
+        }
+        s_pre[nsched0] = idle;
+    }
+    __syncthreads();
+
+    for (int k0 = 0; k0 < K; k0 += PEEK_CHUNK) {
+        const int kn = min(PEEK_CHUNK, K - k0);
+        // ---- phase 1: one warp per pair ----
+        for (int c = warp; c < kn; c += nwarps) {
+            const int a = A.op[b * K + k0 + c], m = A.mach[b * K + k0 + c];
+            double d = 0.0, pa = 0.0;
+            bool valid = (a >= 0) && (a < N) && (m >= 0) && (m < M) && (nsched0 < N);
+            if (valid) valid = (s_mach[a] < 0) && (((a % M) == 0) || (s_mach[a - 1] >= 0));
+            if (valid) {
+                d = __ldg(A.t + (b * N + a) * M + m);
+                pa = __ldg(A.p + (b * N + a) * M + m);
+                valid = !(d < 0);
+            }
+            if (!valid) {
+                if (lane == 0) c_i[c * 4] = 0;
+                continue;
+            }
+            const bool first = (a % M) == 0;
+            const int ja = a / M;
+            // placement: env_kernel's scan over machine m's route (SS:1548-1601, 1689-1775)
+            const double arr_a = first ? 0.0 : s_ft[a - 1] + s_tt[s_mach[a - 1] * M + m];
+            const int len = s_cnt[m];
+            const double ttmm = s_tt[m * M + m];
+            const int offm = s_off[m];
+            double st = arr_a;
+            int where = 0, prev = -1, next = -1;
+            if (len > 0) {
+                const double lbft = arr_a + d;
+                unsigned best = 0xffffffffu;
+                const int lastop = s_ord[offm + len - 1];
+                if (L.left_shift) {
+                    for (int kk0 = 0; kk0 < len; kk0 += 32) {
+                        const int kk = kk0 + lane;
+                        unsigned key = 0xffffffffu;
+                        if (kk < len) {
+                            const int v = s_ord[offm + kk];
+                            const bool vfirst = (v % M) == 0;
+                            double nst = vfirst ? 0.0 : s_ft[v - 1] + s_tt[s_mach[v - 1] * M + m];
+                            bool ok;
+                            if (kk == 0) {
+                                ok = (lbft <= nst);
+                            } else {
+                                const int rp = s_ord[offm + kk - 1];
+                                double val = s_ft[rp] + ((rp / M == v / M) ? ttmm : 0.0);
+                                nst = fmax(nst, val);
+                                ok = !(lbft > nst) && !((nst - s_ft[rp]) < d);
+                            }
+                            if (ok) key = ((unsigned)kk << 16) | (unsigned)v;
+                        }
+                        best = min(best, __reduce_min_sync(FULL, key));
+                    }
+                }
+                if (best != 0xffffffffu) {
+                    where = (int)(best >> 16);
+                    next = (int)(best & 0xffffu);
+                    if (where > 0) {
+                        prev = s_rpred[next];
+                        double y = s_ft[prev] + ((prev / M == ja) ? ttmm : 0.0);
+                        st = (y > arr_a) ? y : arr_a;
+                    }
+                } else {
+                    where = len;
+                    prev = lastop;
+                    double y = s_ft[prev] + ((prev / M == ja) ? ttmm : 0.0);
+                    st = (y > arr_a) ? y : arr_a;
+                }
+            }
+            // makespan estimate: a's job from a on is the re-derived chain (SS:1964-1995), every other op as it stands
+            double cur = st + d, mx = cur;
+            for (int cc = (a % M) + 1; cc < M; cc++) {
+                cur = cur + s_mind[ja * M + cc];
+                mx = fmax(mx, cur);
+            }
+            for (int v = lane; v < N; v += 32)
+                if (v < a || v >= (ja + 1) * M) mx = fmax(mx, s_ft[v]);
+            const double mkv = warp_max(mx);
+            // energy estimate: re-add the leaf holding a, combine the leaves with the plan's postfix program
+            const double ea = d * pa;
+            const auto est_a = [&](int v) { return v == a ? ea : est(v); };
+            int La = 0;
+            while (La + 1 < pw.nleaves && pw.leaf_off[La + 1] <= a) La++;
+            const double leaf_a = peek_leaf(est_a, pw.leaf_off[La], pw.leaf_len[La], lane & 7);
+            double env = leaf_a;
+            if (lane == 0 && pw.nleaves > 1) {
+                int sp = 0;
+                for (int i = 0; i < pw.nprog; i++) {
+                    const int q = pw.prog[i];
+                    if (q >= 0) {
+                        s_stk[sp++] = (q == La) ? leaf_a : s_leaf[q];
+                    } else {
+                        s_stk[sp - 2] = s_stk[sp - 2] + s_stk[sp - 1];
+                        sp--;
+                    }
+                }
+                env = s_stk[0];
+            }
+            if (lane == 0) {
+                const double nt = first ? 0.0 : s_tt[s_mach[a - 1] * M + m];  // SS:872-877
+                double* r = c_d + c * 5;
+                r[0] = st; r[1] = d; r[2] = mkv; r[3] = env; r[4] = s_scal[2] + nt;
+                int* q = c_i + c * 4;
+                q[0] = 1; q[1] = offm + where; q[2] = next; q[3] = prev;
+            }
+            __syncwarp();
+        }
+        __syncthreads();
+        // ---- phase 2: one thread per pair: idle sum, reward (wrk_reward_function, SS:1066-1132) ----
+        for (int c = threadIdx.x; c < kn; c += blockDim.x) {
+            const size_t o = b * K + k0 + c;
+            const int* q = c_i + c * 4;
+            if (!q[0]) {
+                if (A.reward5)
+                    for (int i = 0; i < 5; i++) A.reward5[o * 5 + i] = 0.0;
+                if (A.invalid) A.invalid[o] = 1;
+                continue;
+            }
+            const double* r = c_d + c * 5;
+            const double st = r[0], ft = st + r[1];
+            const int slot = q[1], next = q[2], prev = q[3];
+            double idle = s_pre[slot];
+            idle = idle + ((prev < 0) ? (st - 0.0) : (st - s_ft[prev])) * 1.0;
+            int g = slot;
+            if (next >= 0) {
+                idle = idle + (s_st[next] - ft) * 1.0;
+                g++;
+            }
+            for (; g < nsched0; g++) {
+                const int v = s_ord[g], rp = s_rpred[v];
+                const double term = (rp < 0) ? (s_st[v] - 0.0) : (s_st[v] - s_ft[rp]);
+                idle = idle + term * 1.0;
+            }
+            const double mk_prev = s_scal[0], e_prev = s_scal[1], trans_prev = s_scal[2], idle_prev = s_scal[3];
+            const double r_t = 1.0 * mk_prev - r[2];
+            double r_pt = 1.0 * e_prev - r[3];
+            r_pt = r_pt / (double)N;
+            const double r_tt = 1.0 * trans_prev - r[4];
+            const double r_idle = 1.0 * idle_prev - idle;
+            const double total = A.cfgw[0] * r_t + A.cfgw[1] * (r_pt + 1.0 * r_idle) + A.cfgw[2] * r_tt * 1.0;
+            if (A.reward5) {
+                double* r5 = A.reward5 + o * 5;
+                r5[0] = total / A.divisor; r5[1] = r_t; r5[2] = r_idle; r5[3] = r_pt; r5[4] = r_tt;
+            }
+            if (A.invalid) A.invalid[o] = 0;
+        }
+        __syncthreads();
+    }
+}
+
+// bytes peek_kernel reads and writes for one env and K pairs: the staged records once, per pair the pair, its t / p
+// entries, 5 rewards and the flag
+size_t peek_env_bytes(const Layout& L, int K) {
+    return (size_t)(L.o_scal + 4) * 8 + (size_t)L.xs_stride * 8 + (size_t)(L.o_misc + 3) * 2 +
+           (size_t)K * (8 + 16 + 5 * 8 + 1);
+}
+
 thread_local char g_err[512] = "";
 
 int fail(int code, const char* msg, cudaError_t e = cudaSuccess) {
@@ -3047,6 +3338,38 @@ int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, vo
     return MTFJSP_OK;
 }
 
+int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, double* reward5, uint8_t* invalid,
+                void* stream) {
+    if (!h || !op || !mach || K < 1) return fail(MTFJSP_E_ARG, "mtfjsp_peek: bad argument");
+    if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_peek before mtfjsp_reset");
+    const Layout& L = h->L;
+    const int warps = 4;
+    const size_t smem = (size_t)peek_smem(L, h->pw.nleaves, warps).total;
+    if (smem > 227 * 1024) return fail(MTFJSP_E_ARG, "mtfjsp_peek: one env's records exceed one block's shared memory");
+    cudaStream_t s = (cudaStream_t)stream;
+    // a non-step call: a recorded reset runs now, and the next step waits for the peek in full
+    int rc = enter(h, s);
+    if (rc) return rc;
+    static thread_local int configured_dev = -1;
+    static thread_local size_t configured_smem = 0;
+    if (smem > 48 * 1024 && (configured_dev != h->device || configured_smem < smem)) {
+        CK(cudaFuncSetAttribute(peek_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute");
+        configured_dev = h->device;
+        configured_smem = smem;
+    }
+    PeekArgs A;
+    memset(&A, 0, sizeof A);
+    A.L = L; A.pw = h->pw;
+    A.sd = h->sd; A.xs = h->xs; A.t = h->t; A.p = h->p; A.si = h->si;
+    A.op = op; A.mach = mach; A.K = K;
+    A.cfgw[0] = h->cfgw[0]; A.cfgw[1] = h->cfgw[1]; A.cfgw[2] = h->cfgw[2]; A.divisor = h->divisor;
+    A.reward5 = reward5; A.invalid = invalid;
+    peek_kernel<<<L.B, warps * 32, smem, s>>>(A);
+    h->launches++;
+    CK(cudaGetLastError(), "peek_kernel");
+    return MTFJSP_OK;
+}
+
 int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int mask_mode, int32_t* op,
                          int32_t* mach, void* stream) {
     if (!h || !op || !mach) return fail(MTFJSP_E_ARG, "mtfjsp_policy_random: bad argument");
@@ -3334,6 +3657,8 @@ int mtfjsp_launch_overlap_error(const mtfjsp_env* h) { return h ? (int)*(volatil
 int64_t mtfjsp_launch_count(const mtfjsp_env* h) { return h ? h->launches : 0; }
 
 int64_t mtfjsp_bytes_per_gather(const mtfjsp_env* h) { return h ? (int64_t)(2 * gather_env_bytes(h->L) + 4) : 0; }
+
+int64_t mtfjsp_bytes_per_peek(const mtfjsp_env* h, int K) { return h && K > 0 ? (int64_t)peek_env_bytes(h->L, K) : 0; }
 
 int64_t mtfjsp_bytes_per_step(const mtfjsp_env* h, int dtype) {
     if (!h) return 0;

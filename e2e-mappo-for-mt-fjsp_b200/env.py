@@ -255,6 +255,50 @@ class BatchedMTFJSPEnv:
             else:
                 torch.where(ok.view((-1,) + (1,) * (d.dim() - 1)), getattr(src, name).index_select(0, i), d, out=d)
 
+    # ---- one-step lookahead ----------------------------------------------------------------------------------------
+    def peek(self, op, mach):
+        """What `step` would return for each of K (op, machine) pairs per env, without changing the env (mtfjsp_peek).
+        op, mach: [B,K] integer tensors on this env's device.  Returns (reward5 [B,K,5] f64 = (r, r_mk, r_idle, r_pt,
+        r_tt), bit for bit the step's; invalid [B,K] u8, the step's invalid flag, zeros in reward5 where set), in new
+        buffers.  No scaled rewards: the reward scaler does not advance."""
+        _on(self.device, op, mach)
+        if op.dim() != 2 or op.shape[0] != self.B or tuple(mach.shape) != tuple(op.shape):
+            raise ValueError("op and mach must both have shape [%d, K]" % self.B)
+        op = op.to(torch.int32).contiguous()
+        mach = mach.to(torch.int32).contiguous()
+        K = op.shape[1]
+        r5 = torch.empty((self.B, K, 5), dtype=torch.float64, device=self.device)
+        inv = torch.empty((self.B, K), dtype=torch.uint8, device=self.device)
+        check(self._lib.mtfjsp_peek(self._h, _ptr(op), _ptr(mach), K, _ptr(r5), _ptr(inv), _stream()), "mtfjsp_peek")
+        return r5, inv
+
+    def candidate_ops(self):
+        """[B,J] int32: the next op of every job from the env's current schedule (j*M + the number of its scheduled ops,
+        the job's last op once it is finished).  Read from the handle's state, so it is current after any call -- unlike
+        the `candidate` buffer, which follows observation-writing steps only."""
+        mach = torch.empty((self.B, self.N), dtype=torch.int32, device=self.device)
+        check(self._lib.mtfjsp_export_state(self._h, _ptr(mach), None, None, None, _stream()), "mtfjsp_export_state")
+        nx = (mach.view(self.B, self.J, self.M) >= 0).sum(dim=2, dtype=torch.int32)  # a job's scheduled ops are a prefix
+        base = torch.arange(self.J, dtype=torch.int32, device=self.device) * self.M
+        return base + torch.clamp(nx, max=self.M - 1)
+
+    def peek_candidates(self, machines=None):
+        """peek over the candidate op of every job.  machines=None: every (candidate op of job j, machine m) pair,
+        returns reward5 [B,J,M,5] and invalid [B,J,M].  machines [B,N] integers (a machine for every op, as the machine
+        rules produce): the pair (candidate op of job j, machines[b, op]), returns reward5 [B,J,5] and invalid [B,J].
+        The candidate of a finished job is its last op, already scheduled: reported invalid."""
+        B, J, M = self.B, self.J, self.M
+        cand = self.candidate_ops()
+        if machines is None:
+            op = cand.unsqueeze(2).expand(B, J, M).reshape(B, J * M)
+            mach = torch.arange(M, dtype=torch.int32, device=self.device).repeat(J).expand(B, J * M)
+            r5, inv = self.peek(op, mach)
+            return r5.view(B, J, M, 5), inv.view(B, J, M)
+        _on(self.device, machines)
+        if tuple(machines.shape) != (B, self.N):
+            raise ValueError("machines must have shape [%d, %d]" % (B, self.N))
+        return self.peek(cand, torch.gather(machines, 1, cand.long()))
+
     # ---- views ---------------------------------------------------------------------------------------------------
     def dense_adj(self, dtype=torch.float64):
         adj = torch.empty((self.B, self.N, self.N), dtype=dtype, device=self.device)

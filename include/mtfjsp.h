@@ -152,6 +152,24 @@ int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int6
  * (MTFJSP_DEBUG_BOUNDS) assert.  src and dst must be used on the same stream, or ordered by the caller. */
 int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, void* stream);
 
+/* One-step lookahead: for K (op, machine) pairs per env, what mtfjsp_step would return for that action from the current
+ * state, without changing the state.  op, mach: [B,K] int32 on the device.  reward5 [B,K,5] f64 receives, bit for bit,
+ * what the step would write for env b and action (op[b,k], mach[b,k]): r (the mtfjsp_set_params-weighted sum over the
+ * divisor), then r_mk, r_idle, r_pt, r_tt.  invalid [B,K] u8 receives the step's invalid flag for the pair (the op is
+ * not the next op of its job, the machine is out of range or infeasible (t < 0), or the env is done); an invalid pair
+ * gets zeros in reward5, as the step writes.  Either output may be NULL.  No scaled rewards: the reward scaler does not
+ * advance.
+ * Read-only: nothing of the handle is written -- state records, reward-scaler state, reset snapshot, both job-mask forms,
+ * candidates, done / invalid flags -- and a fused step after a peek still rewrites only the observation rows it changes.
+ * A non-step call: a recorded reset (mtfjsp_reset) is performed first, so a peek right after mtfjsp_reset sees the reset
+ * state, and the next step waits for the peek in full.
+ * Replaces the reference's lookahead by replay (tester/pdrs.py:425-433, 495-510: reset, replay the chosen prefix, step
+ * one candidate, read r_idle -- once per candidate per decision).
+ * MTFJSP_E_ARG, nothing written: a NULL handle, op or mach, or K < 1.  MTFJSP_E_STATE, nothing written: before the first
+ * mtfjsp_reset.  op / mach entries are data: out-of-range values make that pair invalid. */
+int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, double* reward5, uint8_t* invalid,
+                void* stream);
+
 /* Uniform random valid action from the env's current masks: a selectable job (under mask_mode), its candidate
  * op, and a feasible machine for it; counter-based, keyed by (seed, env_offset + env, ops scheduled so far).
  * Mirrors tester/pdrs.py Random_task / Random_m (:75-86, :139-156).  op, mach [B] int32 (-1 when done). */
@@ -397,6 +415,9 @@ int64_t mtfjsp_bytes_per_step(const mtfjsp_env* h, int dtype);
 int64_t mtfjsp_bytes_per_random_step(const mtfjsp_env* h, int dtype);
 /* Bytes mtfjsp_gather reads and writes per destination env (the records and tables it copies, counted once each way). */
 int64_t mtfjsp_bytes_per_gather(const mtfjsp_env* h);
+/* Bytes mtfjsp_peek reads and writes per env for K pairs (the record prefix it stages once, per pair the pair, its t / p
+ * entries and the outputs). */
+int64_t mtfjsp_bytes_per_peek(const mtfjsp_env* h, int K);
 int mtfjsp_random_step_is_fused(const mtfjsp_env* h);
 const char* mtfjsp_last_error(void);
 const char* mtfjsp_version(void);
