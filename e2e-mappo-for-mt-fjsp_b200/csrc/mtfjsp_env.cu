@@ -40,7 +40,6 @@
 #include <string.h>
 
 #include <new>
-#include <vector>
 
 #include "../../include/mtfjsp.h"
 
@@ -103,7 +102,6 @@ struct Params {
     unsigned char* rec;    // optional packed step records, rec_stride bytes per env (include/mtfjsp.h, mtfjsp_step_host_packed):
                            // f64 r | f64 scaled[4] | u8 done | u8 mask_bits[ceil(J/8)] | u8 next_op[J] | padding to 8
     int rec_stride;
-    int b0, b1;     // env range [b0, b1) of this launch (host-step pipeline launches sub-ranges)
     int rev;        // blocks walk the env range from its END (alternate launches: what the previous launch touched last is
                     // still in L2 when this one starts -- a batch's working set is larger than the 126 MB L2, and a
                     // forward walk every launch evicts each line just before it is needed again)
@@ -234,8 +232,8 @@ __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const Layout& L = P.L;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int b = P.b0 + blockIdx.x * L.warps_per_block + warp;
-    if (b >= P.b1) return;
+    const int b = blockIdx.x * L.warps_per_block + warp;
+    if (b >= L.B) return;
     const int N = L.N, M = L.M, J = L.J;
     unsigned char* base = smem_raw + (size_t)warp * L.smem_per_warp;
     double* s_sd = reinterpret_cast<double*>(base + L.sm_sd);
@@ -893,9 +891,12 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int gl = lane & (G - 1), ge = lane / G;
     const unsigned gmask = S::GMASK << (ge * G);  // member mask of this lane's group
-    const int B = P.b1;
-    const int blk = P.rev ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x;
-    const int wb0 = P.b0 + (blk * S::WARPS + warp) * EPW;
+    const int B = P.L.B;
+    // reversed walk without a branch: ~blockIdx.x + gridDim.x = gridDim.x - 1 - blockIdx.x.  The branchless form keeps
+    // the per-step instantiations at the register allocation (or better) they had when wb0 carried a run-time offset
+    const unsigned flip = P.rev ? ~0u : 0u;
+    const int blk = (int)((blockIdx.x ^ flip) + (gridDim.x & flip));
+    const int wb0 = (blk * S::WARPS + warp) * EPW;
     // launch overlap (ovl_wait): the next launch may become resident as soon as every block of this one has started
     constexpr bool OVL = S::OVL && (MODE & MODE_STEP) && !(MODE & MODE_HOST);
     if (OVL && P.ep) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
@@ -1728,7 +1729,7 @@ __global__ void __launch_bounds__(S::WARPS * 32, S::MINB) env_kernel_s(const __g
 #pragma unroll 1
         for (int i = gl; i < S::SI / 8; i += G) g4[i] = s4[i];
     }
-    if (OVL && P.ep) {  // the entry index is recomputed rather than kept live through the step (whole batch: b0 = 0)
+    if (OVL && P.ep) {  // the entry index wb0 / EPW is recomputed rather than kept live through the step
         __syncwarp();
         if ((threadIdx.x & 31) == 0) {
             const unsigned bk = P.rev ? gridDim.x - 1 - blockIdx.x : blockIdx.x;
@@ -2596,7 +2597,7 @@ struct mtfjsp_env {
     bool obs_inc_enabled, obs_inc_allowed, obs_synced;
     const void* obs_ptrs[4];
     int obs_dtype;
-    int host_zerocopy;             // MTFJSP_HOST_ZEROCOPY: packed host step writes records straight to mapped host memory
+    bool host_act_in_place;  // host step: actions read from mapped host memory in place (MTFJSP_HOST_ZEROCOPY=2), else copied in
     int fuse_policy;  // MTFJSP_FUSE_POLICY, read from the environment at create time (tests compare the settings)
     int flip;         // successive eager step launches walk the batch in opposite directions for L2 reuse (Params::rev)
     // The small records every launch starts from -- job masks, candidates, the si record (route order, counters) -- live
@@ -2615,25 +2616,6 @@ struct mtfjsp_env {
     unsigned long long* done_ep;
     unsigned long long ep;
     unsigned *ovl_err, *ovl_err_d;
-    struct HostPipe* pipe;  // host-step pipeline (streams, events, instantiated graphs), created on first use
-};
-
-// Host-step pipeline: the batch is cut into chunks; the copies in, the kernels and the copies out run on three
-// streams -- copy-in c -> kernel c -> copy-out c, kernels in chunk order on ONE stream -- so that chunk c's copy-out
-// overlaps chunk c+1's kernel.  (Round 1 gave every chunk its own stream: the block scheduler then interleaves the blocks
-// of all chunk kernels, every chunk finishes near the end and no copy-out can start early: 161 us per 65,536-env step
-// against 174 us unchunked.)  The whole fan-out is captured once per set of buffer addresses into a CUDA graph and
-// replayed with a single launch call per step.
-struct HostPipe {
-    static constexpr int MAXC = 8, CHUNKS = 4;  // most chunks, and the chunk count aimed at
-    cudaStream_t ms, cs[MAXC];
-    cudaEvent_t fork, join[MAXC], hev[MAXC], kev[MAXC];
-    struct Entry {
-        const void* key[11];
-        int mask_mode, dtype, chunks, kernels, inc;
-        cudaGraphExec_t exec;
-    };
-    std::vector<Entry> cache;
 };
 
 #define CK(call, msg)                                            \
@@ -2651,7 +2633,6 @@ static Params make_params(mtfjsp_env* h) {
     P.cfgw[0] = h->cfgw[0]; P.cfgw[1] = h->cfgw[1]; P.cfgw[2] = h->cfgw[2];
     P.divisor = h->divisor; P.gamma = h->gamma;
     P.jm_fin = h->jm_fin; P.jm_esa = h->jm_esa; P.cand_int = h->cand;
-    P.b0 = 0; P.b1 = h->L.B;
     return P;
 }
 
@@ -2699,7 +2680,7 @@ static int launch_env(mtfjsp_env* h, const Params& P, cudaStream_t s) {
         configured_dev = h->device;
         configured_smem = smem;
     }
-    int blocks = (P.b1 - P.b0 + L.warps_per_block - 1) / L.warps_per_block;
+    int blocks = (L.B + L.warps_per_block - 1) / L.warps_per_block;
     env_kernel<MODE, OutT><<<blocks, L.warps_per_block * 32, smem, s>>>(P);
     h->launches++;
     h->ovl_chain = false;
@@ -2733,7 +2714,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
         configured_dev = h->device;
     }
     const int per_block = S::WARPS * S::EPW;
-    const int blocks = (P.b1 - P.b0 + per_block - 1) / per_block;
+    const int blocks = (L.B + per_block - 1) / per_block;
     Params Q = P;
     if (MODE & MODE_STEP) {  // eager step launches alternate direction (see Params::rev)
         Q.rev = h->flip;
@@ -2748,7 +2729,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     // another call on the handle wait for their predecessor in full.  A launch being captured into a graph takes no
     // part: its epoch would be released only when the graph runs.
     bool pdl = false;
-    if (S::OVL && (MODE & MODE_STEP) && !(MODE & MODE_HOST) && P.b0 == 0 && P.b1 == L.B && h->launch_overlap) {
+    if (S::OVL && (MODE & MODE_STEP) && !(MODE & MODE_HOST) && h->launch_overlap) {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         if (cudaStreamIsCapturing(s, &cs) != cudaSuccess) {
             cudaGetLastError();
@@ -2801,18 +2782,6 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
 #define MTFJSP_SPEC_SIZES(X) \
     X(6, 6, 8, 4, false) X(10, 6, 16, 1, false) X(20, 6, 32, 1, false) X(10, 10, 16, 1, false) X(15, 10, 32, 1, true) \
     X(20, 10, 32, 1, true) X(30, 20, 32, 1, true)
-
-// envs that ONE wave of resident blocks of the size's specialised kernel covers on this device (0: no specialisation).
-// The host-step pipeline cuts the batch into whole waves: a chunk of 1.15 waves costs two block lifetimes, one wave one.
-static int envs_per_wave(int J, int M, int device) {
-    int sms = 0;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) return 0;
-#define X(JJ, MM, GG, WW, CC) \
-    if (J == JJ && M == MM) return sms * Spec<JJ, MM, GG, WW, CC>::MINB * WW * Spec<JJ, MM, GG, WW, CC>::EPW;
-    MTFJSP_SPEC_SIZES(X)
-#undef X
-    return 0;
-}
 
 static bool has_spec(int J, int M) {
 #define X(JJ, MM, GG, WW, CC) if (J == JJ && M == MM) return true;
@@ -2903,14 +2872,14 @@ static void obs_mark(mtfjsp_env* h, const void* tfea, const void* mfea, const vo
     h->obs_ptrs[0] = tfea; h->obs_ptrs[1] = mfea; h->obs_ptrs[2] = adj_w; h->obs_ptrs[3] = adj_src;
 }
 
-// fused step + observation over the env range [b0, b1) (the whole batch, or one chunk of the host-step pipeline)
-static int step_obs_range(mtfjsp_env* h, const int32_t* op, const int32_t* mach, double* reward5, double* scaled4,
-                          uint8_t* done, uint8_t* invalid, double* info6, void* task_fea, void* mach_fea, float* adj_w,
-                          int16_t* adj_src, uint8_t* job_mask, int32_t* candidate, int mask_mode, int dtype, int b0, int b1,
-                          cudaStream_t s, const int2* act2 = nullptr, unsigned char* rec = nullptr, int obs_inc = 0) {
+// fused step + observation over the whole batch
+static int launch_step_obs(mtfjsp_env* h, const int32_t* op, const int32_t* mach, double* reward5, double* scaled4,
+                           uint8_t* done, uint8_t* invalid, double* info6, void* task_fea, void* mach_fea, float* adj_w,
+                           int16_t* adj_src, uint8_t* job_mask, int32_t* candidate, int mask_mode, int dtype,
+                           cudaStream_t s, const int2* act2 = nullptr, unsigned char* rec = nullptr, int obs_inc = 0) {
     Params P = make_params(h);
     P.op = op; P.mach = mach; P.reward5 = reward5; P.scaled4 = scaled4; P.done = done; P.invalid = invalid;
-    P.info6 = info6; P.b0 = b0; P.b1 = b1; P.act2 = act2; P.rec = rec; P.rec_stride = h->rec_stride;
+    P.info6 = info6; P.act2 = act2; P.rec = rec; P.rec_stride = h->rec_stride;
     P.obs_inc = obs_inc;
     int rc = fill_obs(h, P, task_fea, mach_fea, adj_w, adj_src, job_mask, candidate, mask_mode, dtype);
     if (rc) return rc;
@@ -2975,8 +2944,8 @@ int mtfjsp_create(mtfjsp_env** out, int B, int J, int M, int E, int left_shift, 
     {
         const char* fg = getenv("MTFJSP_FORCE_GENERIC");  // test hook: run the generic kernel on every size
         h->force_generic = fg && fg[0] == '1';
-        // default: records zero-copy; the actions too from 16,384 envs up (below that the explicit copy is as fast)
-        h->host_zerocopy = getenv("MTFJSP_HOST_ZEROCOPY") ? atoi(getenv("MTFJSP_HOST_ZEROCOPY")) : (B >= 16384 ? 2 : 1);
+        // test hook (1 | 2); default: from 16,384 envs up (below that the explicit copy is as fast)
+        h->host_act_in_place = getenv("MTFJSP_HOST_ZEROCOPY") ? atoi(getenv("MTFJSP_HOST_ZEROCOPY")) >= 2 : B >= 16384;
         h->fuse_policy = getenv("MTFJSP_FUSE_POLICY") ? atoi(getenv("MTFJSP_FUSE_POLICY")) : 1;
         h->obs_inc_allowed = !(getenv("MTFJSP_OBS_INCREMENTAL") && atoi(getenv("MTFJSP_OBS_INCREMENTAL")) == 0);  // test hook
         h->fused_reset = getenv("MTFJSP_FUSED_RESET") ? atoi(getenv("MTFJSP_FUSED_RESET")) : 1;
@@ -3050,16 +3019,6 @@ int mtfjsp_destroy(mtfjsp_env* h) {
     for (void* q : ptrs)
         if (q) cudaFree(q);
     if (h->ovl_err) cudaFreeHost(h->ovl_err);
-    if (h->pipe) {
-        for (auto& e : h->pipe->cache) cudaGraphExecDestroy(e.exec);
-        cudaStreamDestroy(h->pipe->ms);
-        cudaEventDestroy(h->pipe->fork);
-        for (int c = 0; c < HostPipe::MAXC; c++) {
-            cudaStreamDestroy(h->pipe->cs[c]); cudaEventDestroy(h->pipe->join[c]);
-            cudaEventDestroy(h->pipe->hev[c]); cudaEventDestroy(h->pipe->kev[c]);
-        }
-        delete h->pipe;
-    }
     delete h;
     return MTFJSP_OK;
 }
@@ -3186,8 +3145,8 @@ int mtfjsp_step_obs(mtfjsp_env* h, const int32_t* op, const int32_t* mach, doubl
     int rc = enter(h, (cudaStream_t)stream, true);
     if (rc) return rc;
     const int inc = obs_inc_now(h, task_fea, mach_fea, adj_w, adj_src, dtype);
-    rc = step_obs_range(h, op, mach, reward5, scaled4, done, invalid, nullptr, task_fea, mach_fea, adj_w, adj_src,
-                            job_mask, candidate, mask_mode, dtype, 0, h->L.B, (cudaStream_t)stream, nullptr, nullptr, inc);
+    rc = launch_step_obs(h, op, mach, reward5, scaled4, done, invalid, nullptr, task_fea, mach_fea, adj_w, adj_src,
+                         job_mask, candidate, mask_mode, dtype, (cudaStream_t)stream, nullptr, nullptr, inc);
     if (rc == MTFJSP_OK) obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
     return rc;
 }
@@ -3424,17 +3383,10 @@ int mtfjsp_random_step(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int32_
                            candidate, mask_mode, dtype, stream);
 }
 
-static bool is_pinned(const void* p) {
-    if (!p) return true;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-    return a.type == cudaMemoryTypeHost;
-}
-
 }  // extern "C"
 
-// Host-buffer step behind both entry points.  Packed form: act_host [B,2] i32 in, rec_host [B] records out (one copy
-// each way per chunk); split form: op / mach in, info6 / job_mask / candidate out (five copies per chunk).
+// Host-buffer step behind both entry points.  Packed form: act [B,2] i32 in, rec [B] records out; split form: op / mach
+// in, info6 / job_mask / candidate out (each may be NULL).
 struct HostIO {
     const int32_t *op, *mach, *act;
     double* info6;
@@ -3447,181 +3399,55 @@ static int host_step_impl(mtfjsp_env* h, const HostIO& io, void* task_fea, void*
                           int mask_mode, int dtype, cudaStream_t s) {
     const Layout& L = h->L;
     const bool packed = io.act != nullptr;
-    const int inc = obs_inc_now(h, task_fea, mach_fea, adj_w, adj_src, dtype);  // one decision for all chunks of the step
-    const uint8_t* jm_dev = mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin;
-    const size_t rs = (size_t)h->rec_stride;
-    // the three parts of one chunk [b0, b1): copy-in, kernel, copy-out
-    auto copy_in = [&](int b0, int b1, cudaStream_t q) -> int {
-        const size_t n = (size_t)(b1 - b0);
+    const int inc = obs_inc_now(h, task_fea, mach_fea, adj_w, adj_src, dtype);
+    // In place: when every buffer the call passes is pinned and mapped into the device's address space, ONE launch over
+    // the whole batch reads and writes them through their device addresses, so the PCIe writes of the first warps run
+    // under the rest of the kernel -- no staging buffer, no copy engine.
+    bool mapped = true;
+    auto dev = [&](const void* p) -> void* {
+        void* d = nullptr;
+        if (p && mapped && (cudaHostGetDevicePointer(&d, const_cast<void*>(p), 0) != cudaSuccess || !d)) {
+            cudaGetLastError();  // pageable, or not mapped for this device
+            mapped = false;
+        }
+        return d;
+    };
+    const int2* act = reinterpret_cast<const int2*>(dev(io.act));
+    const int32_t* op = reinterpret_cast<const int32_t*>(dev(io.op));
+    const int32_t* mach = reinterpret_cast<const int32_t*>(dev(io.mach));
+    double* info6 = reinterpret_cast<double*>(dev(io.info6));
+    uint8_t* jm = reinterpret_cast<uint8_t*>(dev(io.jm));
+    int32_t* cand = reinterpret_cast<int32_t*>(dev(io.cand));
+    unsigned char* rec = reinterpret_cast<unsigned char*>(dev(io.rec));
+    if (!mapped) {  // staged: copy in, one launch into the handle's device scratch, copy out, in order on `s`
+        info6 = io.info6 ? h->info6 : nullptr;
+        rec = io.rec ? h->rec : nullptr;
+        jm = nullptr;  // copied out of the kernel's own mask / candidate buffers
+        cand = nullptr;
+    }
+    // the actions are read in place from 16,384 envs up; below that the explicit copy is as fast
+    if (!mapped || !h->host_act_in_place) {
         if (packed) {
-            CK(cudaMemcpyAsync(h->act2 + b0, io.act + (size_t)b0 * 2, n * 8, cudaMemcpyHostToDevice, q), "H2D actions");
+            CK(cudaMemcpyAsync(h->act2, io.act, (size_t)L.B * 8, cudaMemcpyHostToDevice, s), "H2D actions");
+            act = h->act2;
         } else {
-            CK(cudaMemcpyAsync(h->a_op + b0, io.op + b0, n * 4, cudaMemcpyHostToDevice, q), "H2D op");
-            CK(cudaMemcpyAsync(h->a_mach + b0, io.mach + b0, n * 4, cudaMemcpyHostToDevice, q), "H2D mach");
-        }
-        return MTFJSP_OK;
-    };
-    auto kernel = [&](int b0, int b1, cudaStream_t q) -> int {
-        return step_obs_range(h, h->a_op, h->a_mach, nullptr, nullptr, h->dn, h->inv, io.info6 ? h->info6 : nullptr,
-                              task_fea, mach_fea, adj_w, adj_src, nullptr, nullptr, mask_mode, dtype, b0, b1, q,
-                              packed ? h->act2 : nullptr, io.rec ? h->rec : nullptr, inc);
-    };
-    auto copy_out = [&](int b0, int b1, cudaStream_t q) -> int {
-        const size_t n = (size_t)(b1 - b0);
-        if (io.rec) CK(cudaMemcpyAsync(io.rec + b0 * rs, h->rec + b0 * rs, n * rs, cudaMemcpyDeviceToHost, q), "D2H records");
-        if (io.info6)
-            CK(cudaMemcpyAsync(io.info6 + (size_t)b0 * 6, h->info6 + (size_t)b0 * 6, n * 48, cudaMemcpyDeviceToHost, q), "D2H info6");
-        if (io.jm)
-            CK(cudaMemcpyAsync(io.jm + (size_t)b0 * L.J, jm_dev + (size_t)b0 * L.J, n * L.J, cudaMemcpyDeviceToHost, q), "D2H job_mask");
-        if (io.cand)
-            CK(cudaMemcpyAsync(io.cand + (size_t)b0 * L.J, h->cand + (size_t)b0 * L.J, n * L.J * 4, cudaMemcpyDeviceToHost, q),
-               "D2H candidate");
-        return MTFJSP_OK;
-    };
-    auto chunk = [&](int b0, int b1, cudaStream_t q) -> int {  // everything one chunk does, in order, on stream q
-        int rc = copy_in(b0, b1, q);
-        if (rc == MTFJSP_OK) rc = kernel(b0, b1, q);
-        if (rc == MTFJSP_OK) rc = copy_out(b0, b1, q);
-        return rc;
-    };
-    const bool pinned = is_pinned(io.op) && is_pinned(io.mach) && is_pinned(io.act) && is_pinned(io.info6) &&
-                        is_pinned(io.jm) && is_pinned(io.cand) && is_pinned(io.rec);
-    if (!pinned) {
-        // pageable buffers: the copies are staged by the driver and cannot overlap; plain in-order sequence
-        int rc = chunk(0, L.B, s);
-        if (rc) return rc;
-        obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
-        CK(cudaStreamSynchronize(s), "cudaStreamSynchronize");
-        return MTFJSP_OK;
-    }
-    // Zero-copy form (packed records in pinned, device-mapped host memory; MTFJSP_HOST_ZEROCOPY, default on): ONE launch over
-    // the whole batch whose warps write their finished records straight into the caller's buffer, so the PCIe writes of
-    // the first blocks run under the rest of the kernel -- no staging buffer, no copy engine, no cross-stream dependencies.
-    // Level 2 also reads the packed actions from the caller's buffer instead of copying them in first.
-    if (packed && h->host_zerocopy > 0 && !h->force_generic && has_spec(L.J, L.M)) {
-        void* drec = nullptr;
-        void* dact = nullptr;
-        if (cudaHostGetDevicePointer(&drec, io.rec, 0) == cudaSuccess && drec &&
-            (h->host_zerocopy < 2 || (cudaHostGetDevicePointer(&dact, const_cast<int32_t*>(io.act), 0) == cudaSuccess && dact))) {
-            if (!dact) CK(cudaMemcpyAsync(h->act2, io.act, (size_t)L.B * 8, cudaMemcpyHostToDevice, s), "H2D actions");
-            int rc = step_obs_range(h, h->a_op, h->a_mach, nullptr, nullptr, h->dn, h->inv, nullptr, task_fea, mach_fea, adj_w,
-                                    adj_src, nullptr, nullptr, mask_mode, dtype, 0, L.B, s,
-                                    dact ? reinterpret_cast<const int2*>(dact) : h->act2, reinterpret_cast<unsigned char*>(drec), inc);
-            if (rc) return rc;
-            obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
-            CK(cudaStreamSynchronize(s), "cudaStreamSynchronize");
-            return MTFJSP_OK;
-        }
-        cudaGetLastError();  // not mapped for this device: the copy pipeline below
-    }
-    // the split form when only the [B,6] step info comes back (job mask / candidates stay on the device): same idea
-    if (!packed && io.info6 && !io.jm && !io.cand && h->host_zerocopy > 0 && !h->force_generic && has_spec(L.J, L.M)) {
-        void *dinfo = nullptr, *dop = nullptr, *dmach = nullptr;
-        if (cudaHostGetDevicePointer(&dinfo, io.info6, 0) == cudaSuccess && dinfo &&
-            (h->host_zerocopy < 2 || (cudaHostGetDevicePointer(&dop, const_cast<int32_t*>(io.op), 0) == cudaSuccess && dop &&
-                                      cudaHostGetDevicePointer(&dmach, const_cast<int32_t*>(io.mach), 0) == cudaSuccess && dmach))) {
-            if (!dop) {
-                CK(cudaMemcpyAsync(h->a_op, io.op, (size_t)L.B * 4, cudaMemcpyHostToDevice, s), "H2D op");
-                CK(cudaMemcpyAsync(h->a_mach, io.mach, (size_t)L.B * 4, cudaMemcpyHostToDevice, s), "H2D mach");
-            }
-            int rc = step_obs_range(h, dop ? reinterpret_cast<const int32_t*>(dop) : h->a_op,
-                                    dop ? reinterpret_cast<const int32_t*>(dmach) : h->a_mach, nullptr, nullptr, h->dn, h->inv,
-                                    reinterpret_cast<double*>(dinfo), task_fea, mach_fea, adj_w, adj_src, nullptr, nullptr, mask_mode,
-                                    dtype, 0, L.B, s, nullptr, nullptr, inc);
-            if (rc) return rc;
-            obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
-            CK(cudaStreamSynchronize(s), "cudaStreamSynchronize");
-            return MTFJSP_OK;
-        }
-        cudaGetLastError();
-    }
-    if (!h->pipe) {
-        HostPipe* hp = new (std::nothrow) HostPipe();
-        if (!hp) return fail(MTFJSP_E_ARG, "out of host memory");
-        CK(cudaStreamCreateWithFlags(&hp->ms, cudaStreamNonBlocking), "cudaStreamCreate");
-        CK(cudaEventCreateWithFlags(&hp->fork, cudaEventDisableTiming), "cudaEventCreate");
-        for (int c = 0; c < HostPipe::MAXC; c++) {
-            CK(cudaStreamCreateWithFlags(&hp->cs[c], cudaStreamNonBlocking), "cudaStreamCreate");
-            CK(cudaEventCreateWithFlags(&hp->join[c], cudaEventDisableTiming), "cudaEventCreate");
-            CK(cudaEventCreateWithFlags(&hp->hev[c], cudaEventDisableTiming), "cudaEventCreate");
-            CK(cudaEventCreateWithFlags(&hp->kev[c], cudaEventDisableTiming), "cudaEventCreate");
-        }
-        h->pipe = hp;
-    }
-    HostPipe* hp = h->pipe;
-    // chunks of whole 256-env groups, at least 4,096 envs each (below that one launch does not fill the GPU)
-    int chunks = HostPipe::CHUNKS;
-    while (chunks > 1 && L.B / chunks < 4096) chunks--;
-    int per = ((L.B + chunks - 1) / chunks + 255) / 256 * 256;
-    if (!h->force_generic && chunks > 1) {  // whole waves per chunk (the chunk kernels run one after the other)
-        static thread_local int wave_J = -1, wave_M = -1, wave_dev = -1, wave = 0;
-        if (wave_J != L.J || wave_M != L.M || wave_dev != h->device) {
-            wave = envs_per_wave(L.J, L.M, h->device);
-            wave_J = L.J; wave_M = L.M; wave_dev = h->device;
-        }
-        if (wave > 0 && L.B > wave) {
-            int k = (L.B / chunks + wave / 2) / wave;
-            if (k < 1) k = 1;
-            while ((L.B + k * wave - 1) / (k * wave) > HostPipe::MAXC) k++;
-            per = k * wave;
-            chunks = (L.B + per - 1) / per;
+            CK(cudaMemcpyAsync(h->a_op, io.op, (size_t)L.B * 4, cudaMemcpyHostToDevice, s), "H2D op");
+            CK(cudaMemcpyAsync(h->a_mach, io.mach, (size_t)L.B * 4, cudaMemcpyHostToDevice, s), "H2D mach");
+            op = h->a_op;
+            mach = h->a_mach;
         }
     }
-    const void* key[11] = {io.op, io.mach, io.act, io.info6, io.jm, io.cand, io.rec, task_fea, mach_fea, adj_w, adj_src};
-    HostPipe::Entry* ent = nullptr;
-    for (auto& e : hp->cache)
-        if (!memcmp(e.key, key, sizeof key) && e.mask_mode == mask_mode && e.dtype == dtype && e.chunks == chunks && e.inc == inc) { ent = &e; break; }
-    if (!ent) {
-        if (hp->cache.size() >= 256) {  // addresses keep changing: start over rather than grow without bound
-            for (auto& e : hp->cache) cudaGraphExecDestroy(e.exec);
-            hp->cache.clear();
-        }
-
-        const int64_t l0 = h->launches;
-        cudaGraph_t g = nullptr;
-        CK(cudaStreamBeginCapture(hp->ms, cudaStreamCaptureModeRelaxed), "cudaStreamBeginCapture");
-        int rc = MTFJSP_OK;
-        cudaError_t ce = cudaEventRecord(hp->fork, hp->ms);
-        cudaStream_t qi = hp->cs[0], qk = hp->cs[1], qo = hp->cs[2];  // copies in, kernels (in chunk order), copies out
-        for (int k = 0; k < 3 && ce == cudaSuccess; k++) ce = cudaStreamWaitEvent(hp->cs[k], hp->fork, 0);
-        auto range = [&](int c, int& b0, int& b1) { b0 = c * per; b1 = (c + 1) * per < L.B ? (c + 1) * per : L.B; return b0 < b1; };
-        int b0, b1;
-        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-            rc = copy_in(b0, b1, qi);
-            if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->hev[c], qi);
-        }
-        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-            ce = cudaStreamWaitEvent(qk, hp->hev[c], 0);
-            if (ce != cudaSuccess) break;
-            rc = kernel(b0, b1, qk);
-            if (rc == MTFJSP_OK) ce = cudaEventRecord(hp->kev[c], qk);
-        }
-        for (int c = 0; c < chunks && rc == MTFJSP_OK && ce == cudaSuccess && range(c, b0, b1); c++) {
-            ce = cudaStreamWaitEvent(qo, hp->kev[c], 0);
-            if (ce != cudaSuccess) break;
-            rc = copy_out(b0, b1, qo);
-        }
-        for (int k = 0; k < 3 && rc == MTFJSP_OK && ce == cudaSuccess; k++) {
-            ce = cudaEventRecord(hp->join[k], hp->cs[k]);
-            if (ce == cudaSuccess) ce = cudaStreamWaitEvent(hp->ms, hp->join[k], 0);
-        }
-        cudaError_t ee = cudaStreamEndCapture(hp->ms, &g);
-        const int kernels = (int)(h->launches - l0);
-        h->launches = l0;  // the capture launched nothing; replays are counted below
-        if (rc) { if (g) cudaGraphDestroy(g); return rc; }
-        if (ce != cudaSuccess) { if (g) cudaGraphDestroy(g); return fail(MTFJSP_E_CUDA, "host-step capture", ce); }
-        CK(ee, "cudaStreamEndCapture");
-        HostPipe::Entry e;
-        memcpy(e.key, key, sizeof key);
-        e.mask_mode = mask_mode; e.dtype = dtype; e.chunks = chunks; e.kernels = kernels; e.inc = inc;
-        cudaError_t ie = cudaGraphInstantiate(&e.exec, g, 0);
-        cudaGraphDestroy(g);
-        CK(ie, "cudaGraphInstantiate");
-        hp->cache.push_back(e);
-        ent = &hp->cache.back();
+    int rc = launch_step_obs(h, op, mach, nullptr, nullptr, h->dn, h->inv, info6, task_fea, mach_fea, adj_w, adj_src, jm,
+                             cand, mask_mode, dtype, s, act, rec, inc);
+    if (rc) return rc;
+    if (!mapped) {
+        const size_t B = (size_t)L.B;
+        const uint8_t* jm_dev = mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin;
+        if (io.rec) CK(cudaMemcpyAsync(io.rec, h->rec, B * h->rec_stride, cudaMemcpyDeviceToHost, s), "D2H records");
+        if (io.info6) CK(cudaMemcpyAsync(io.info6, h->info6, B * 48, cudaMemcpyDeviceToHost, s), "D2H info6");
+        if (io.jm) CK(cudaMemcpyAsync(io.jm, jm_dev, B * L.J, cudaMemcpyDeviceToHost, s), "D2H job_mask");
+        if (io.cand) CK(cudaMemcpyAsync(io.cand, h->cand, B * L.J * 4, cudaMemcpyDeviceToHost, s), "D2H candidate");
     }
-    CK(cudaGraphLaunch(ent->exec, s), "cudaGraphLaunch");
-    h->launches += ent->kernels;
     obs_mark(h, task_fea, mach_fea, adj_w, adj_src, dtype);
     CK(cudaStreamSynchronize(s), "cudaStreamSynchronize");
     return MTFJSP_OK;

@@ -210,15 +210,13 @@ int mtfjsp_step_host(mtfjsp_env* h, const int32_t* op_host, const int32_t* mach_
  *     u8  mask_bits[(J+7)/8]   bit (j & 7) of byte (j >> 3) set = job j not selectable   algorithm/ppo_algorithm.py:202-317
  *     u8  next_op[J]           candidate op of job j = j * M + next_op[j]; then zero padding to a multiple of 8
  * (48 bytes at J = 6: the step's D2H traffic is what bounds the call, see DESIGN.md section 5).
- * With pinned buffers (cudaHostAlloc / cudaHostRegister'd, hence mapped into the device's address space) and a
- * size-specialised kernel, the step is ONE launch whose warps write their finished records straight into
- * `records_host` over PCIe while the rest of the batch is still being stepped -- no staging buffer, no copy engine
- * (MTFJSP_HOST_ZEROCOPY: 1 = records, 2 = the actions are read from `actions_host` in place as well; default 2 from
- * 16,384 envs up, else 1; 0 = the staged form).  Staged form: the batch is cut into 4 chunks
- * whose copy-in -> kernel -> copy-out chains run on three streams, replayed as one CUDA graph per step, so that the
- * copy-out of chunk c overlaps the kernel of chunk c+1; pageable buffers take the plain in-order path.  mtfjsp_step_host
- * with NULL job_mask_host / candidate_host writes its [B,6] step info the same zero-copy way.  Synchronises `stream`
- * before returning: the host buffers are complete when the call returns. */
+ * With pinned buffers (cudaHostAlloc / cudaHostRegister'd, hence mapped into the device's address space) the step is
+ * ONE launch whose warps write their finished records straight into `records_host` over PCIe while the rest of the
+ * batch is still being stepped -- no staging buffer, no copy engine; from 16,384 envs up the actions are read from
+ * `actions_host` in place as well (below that they are copied in first).  mtfjsp_step_host writes its step info, job
+ * mask and candidates into mapped buffers the same way.  If any buffer is pageable (not mapped), the call copies in,
+ * steps into device scratch and copies out, in order on `stream`.  Synchronises `stream` before returning: the host
+ * buffers are complete when the call returns. */
 int mtfjsp_step_host_packed(mtfjsp_env* h, const int32_t* actions_host, void* records_host, void* task_fea, void* mach_fea,
                             float* adj_w, int16_t* adj_src, int mask_mode, int dtype, void* stream);
 int mtfjsp_host_record_bytes(const mtfjsp_env* h);

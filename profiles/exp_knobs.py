@@ -1,7 +1,7 @@
-"""Knob experiments for the env kernel and the host-step pipeline (one process per setting; the knobs are read from
-the environment when the handle is created):
+"""Knob experiments for the env kernel and the host-buffer step (one process per setting; the knobs are read from
+the environment when the handle is created; MTFJSP_HOST_ZEROCOPY=2 reads the host step's actions in place, 1 copies them):
 
-    MTFJSP_HOST_ZEROCOPY=0|1|2  MTFJSP_FUSE_POLICY=0|1  MTFJSP_OBS_INCREMENTAL=0|1  python profiles/exp_knobs.py [workload] [reps]
+    MTFJSP_HOST_ZEROCOPY=1|2  MTFJSP_FUSE_POLICY=0|1  MTFJSP_OBS_INCREMENTAL=0|1  python profiles/exp_knobs.py [workload] [reps]
 
 Prints one JSON line: fused-kernel time per launch (CUDA events around each launch, recorded actions replayed),
 whole random-rollout step time, and the host-buffer step rate."""
@@ -81,7 +81,7 @@ torch.cuda.synchronize()
 h_us = (time.perf_counter() - t0) * 1e6 / (reps * N)
 assert float(info6[:, 1].sum()) == B and torch.equal(env.costs(), costs_ref)
 
-# packed host-buffer step: one copy each way per chunk
+# packed host-buffer step
 p_act, p_rec = env.host_buffers()
 p_acts = torch.stack([rec_op.cpu(), rec_mc.cpu()], dim=2).contiguous().pin_memory()  # [N,B,2]
 

@@ -1,5 +1,6 @@
-"""Does a device->host copy overlap a running kernel on this box?  (The host-step pipeline of mtfjsp_step_host_packed
-assumes it does.)  A ~100 us memory-bound kernel on one stream, a 4.7 MB pinned D2H copy on another."""
+"""Does a device->host copy overlap a running kernel on this box?  (The chunked copy pipeline mtfjsp_step_host_packed
+used before its kernel wrote the records into mapped host memory assumed it did.)  A ~100 us memory-bound kernel on one
+stream, a 4.7 MB pinned D2H copy on another."""
 import time
 
 import torch

@@ -1,7 +1,10 @@
-"""Host-buffer packed step (mtfjsp_step_host_packed, bench.py's e2e) by MTFJSP_HOST_ZEROCOPY level:
-0 = staged copy pipeline (H2D actions, chunk kernels, D2H records through the copy engine), 1 = one launch whose warps
-write the records straight into the mapped pinned host buffer, 2 = the actions are read from mapped host memory too.
-    python profiles/prof_zerocopy.py [A|B|C]"""
+"""Host-buffer packed step (mtfjsp_step_host_packed, bench.py's e2e) with pinned buffers, by MTFJSP_HOST_ZEROCOPY level:
+1 = one launch whose warps write the records straight into the mapped pinned host buffer, the actions copied in first,
+2 = the actions are read from mapped host memory in place too.  The checksum of the last records lets two builds of the
+library (MTFJSP_LIB) be compared on the same inputs.
+    python profiles/prof_zerocopy.py [A|B|C]     a bench.WORKLOADS key
+    python profiles/prof_zerocopy.py J M E B     any size (synthetic instances, seed 0)"""
+import hashlib
 import importlib
 import os
 import sys
@@ -12,13 +15,17 @@ import torch  # noqa: E402
 
 import bench  # noqa: E402
 
-wl = bench.WORKLOADS[sys.argv[1] if len(sys.argv) > 1 else "A"]
+if len(sys.argv) == 5:
+    J, M, E, B = (int(x) for x in sys.argv[1:])
+    seed = 0
+else:
+    wl = bench.WORKLOADS[sys.argv[1] if len(sys.argv) > 1 else "A"]
+    J, M, E, B, seed = wl["J"], wl["M"], wl["E"], wl["B"], wl["seed"]
 pkg = importlib.import_module("e2e-mappo-for-mt-fjsp_b200")
 envm = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.env")
-J, M, E, B = wl["J"], wl["M"], wl["E"], wl["B"]
 N = J * M
-d = pkg.instances.synthetic_instances(0, B, J, M, E, wl["seed"])
-w = pkg.instances.random_weights(0, B, wl["seed"])
+d = pkg.instances.synthetic_instances(0, B, J, M, E, seed)
+w = pkg.instances.random_weights(0, B, seed)
 
 
 def make(level):
@@ -30,7 +37,7 @@ def make(level):
     return env
 
 
-env = make(0)
+env = make(1)
 rec_op = torch.empty((N, B), dtype=torch.int32, device="cuda")
 rec_mc = torch.empty((N, B), dtype=torch.int32, device="cuda")
 for s in range(N):
@@ -39,8 +46,9 @@ for s in range(N):
 h_act = torch.stack([rec_op.cpu(), rec_mc.cpu()], dim=2).contiguous().pin_memory()
 act_ptr = [h_act[s].data_ptr() for s in range(N)]
 
+print("J%dM%dE%d x %d envs, %s" % (J, M, E, B, torch.cuda.get_device_name()), flush=True)
 ref = None
-for level in (0, 1, 2, 1, 0):
+for level in (1, 2, 2, 1):
     env = make(level)
     _, h_rec = env.host_buffers()
     step = env.host_stepper(h_rec)
@@ -59,5 +67,6 @@ for level in (0, 1, 2, 1, 0):
     if ref is None:
         ref = final
     same = bool(torch.equal(final, ref))
-    print("zerocopy %d: median %.1f us (min %.1f) per %d-env step -> %.3e env-steps/s; last records identical to level 0: %s"
-          % (level, med * 1e6, ts[0] * 1e6, B, B / med, same), flush=True)
+    print("zerocopy %d: median %.1f us (min %.1f) per %d-env step -> %.3e env-steps/s; last records identical to level 1: "
+          "%s, sha1 %s" % (level, med * 1e6, ts[0] * 1e6, B, B / med, same, hashlib.sha1(final.numpy().tobytes()).hexdigest()[:16]),
+          flush=True)

@@ -229,17 +229,18 @@ def test_step_before_reset_is_a_state_error():
 
 
 @pytest.mark.parametrize("B", [4096 + 77, 3 * 4096 + 77])
-@pytest.mark.parametrize("pinned", [True, False, "copy", "zerocopy_actions"])
+@pytest.mark.parametrize("pinned", [True, False, "mixed", "zerocopy_actions"])
 def test_host_step_equals_device_step(pinned, B, kernel_path, monkeypatch):
-    """mtfjsp_step_host with pinned (graph-replayed chunk pipeline; 1 chunk and 3 ragged chunks) and with pageable
-    host buffers (in-order copies) must equal the device-pointer call bit for bit, including the all-invalid step
-    after the episode has ended.  The packed form with pinned buffers writes its records straight into the mapped host
-    buffer (default); "copy" = the staged copy pipeline instead (MTFJSP_HOST_ZEROCOPY=0), "zerocopy_actions" = the actions
-    are read from the mapped host buffer as well (=2)."""
+    """mtfjsp_step_host and mtfjsp_step_host_packed with pinned host buffers (one launch that writes step info, job mask,
+    candidates and records straight into the mapped host buffers; with the generic kernel under kernel_path "generic")
+    and with pageable ones (copy in, launch, copy out) must equal the device-pointer call bit for bit, including the
+    all-invalid step after the episode has ended.  "mixed" = pageable actions with pinned outputs: one pageable buffer
+    sends the whole call the staged way.  "zerocopy_actions" = the actions are read from the mapped host buffers in
+    place as well (MTFJSP_HOST_ZEROCOPY=2; by default only from 16,384 envs up)."""
     if kernel_path == "unfused":
         pytest.skip("no random_step here, 'auto' covers it")
-    if pinned in ("copy", "zerocopy_actions"):
-        monkeypatch.setenv("MTFJSP_HOST_ZEROCOPY", "0" if pinned == "copy" else "2")  # read by mtfjsp_create
+    if pinned == "zerocopy_actions":
+        monkeypatch.setenv("MTFJSP_HOST_ZEROCOPY", "2")  # read by mtfjsp_create
         pinned = True
     envm = importlib.import_module("e2e-mappo-for-mt-fjsp_b200.env")
     J, M, E = 6, 6, 2
@@ -263,9 +264,13 @@ def test_host_step_equals_device_step(pinned, B, kernel_path, monkeypatch):
     io_env.scaler_init()
     io_env.reset(w)
     pk_act, pk_rec = pk_env.host_buffers()
+    if pinned is not True:
+        pk_act = pk_act.clone()
     if not pinned:
-        pk_act, pk_rec = pk_act.clone(), pk_rec.clone()
+        pk_rec = pk_rec.clone()
+    assert pk_act.is_pinned() == (pinned is True) and pk_rec.is_pinned() == bool(pinned)
     pk_rec.fill_(0xAB)
+    pin_in = (lambda x: x.pin_memory()) if pinned is True else (lambda x: x)
     pin = (lambda x: x.pin_memory()) if pinned else (lambda x: x)
     info6 = pin(torch.full((B, 6), -7.0, dtype=torch.float64))
     h_jm = pin(torch.full((B, J), 9, dtype=torch.uint8))
@@ -275,7 +280,7 @@ def test_host_step_equals_device_step(pinned, B, kernel_path, monkeypatch):
         op, mach = dev_env.policy_random(seed=5)
         if s == N:
             op, mach = torch.zeros_like(op), torch.zeros_like(mach)
-        h_op, h_mc = pin(op.cpu()), pin(mach.cpu())
+        h_op, h_mc = pin_in(op.cpu()), pin_in(mach.cpu())
         dev_env.step_obs(op, mach)
         host_env.step_host(h_op, h_mc, info6, h_jm, h_cd)
         eq(info6[:, 0].numpy(), dev_env.reward5[:, 0].cpu().numpy())

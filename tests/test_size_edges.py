@@ -279,17 +279,15 @@ def test_views_at_large_n(size):
 # ---------------------------------------------------------------------------------------------------------------------
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("zerocopy", [None, "0"])
+@pytest.mark.parametrize("pinned", [True, False])
 @pytest.mark.parametrize("size", [(1678, 2, 1, 3), (48, 64, 4, 3), (1, 64, 8, 5), (1, 2, 1, 2)])
-def test_packed_host_records_at_the_edges(size, zerocopy, monkeypatch):
+def test_packed_host_records_at_the_edges(size, pinned, monkeypatch):
     """Records of ~2 KB (J = 1678: 210 mask bytes), J = 48 at M = 64, and J = 1: the decoded records equal the
-    device-pointer step, the padding is zero, and canary rows behind the batch stay untouched; with the records written
-    into the mapped host buffer (default) and through the staged copy (MTFJSP_HOST_ZEROCOPY=0)."""
+    device-pointer step, the padding is zero, and canary rows behind the batch stay untouched; with pinned buffers
+    (the generic kernel writes the records straight into the mapped host buffer) and with pageable ones (staged copy)."""
     torch = _torch()
-    if zerocopy is None:
-        monkeypatch.delenv("MTFJSP_HOST_ZEROCOPY", raising=False)
-    else:
-        monkeypatch.setenv("MTFJSP_HOST_ZEROCOPY", zerocopy)
+    monkeypatch.delenv("MTFJSP_HOST_ZEROCOPY", raising=False)
+    pin = (lambda x: x.pin_memory()) if pinned else (lambda x: x)
     J, M, E, B = size
     N = J * M
     envm = _envm()
@@ -306,8 +304,8 @@ def test_packed_host_records_at_the_edges(size, zerocopy, monkeypatch):
     nbytes = int(pk_env.host_buffers()[1].shape[1])
     used = 41 + (J + 7) // 8 + J
     assert nbytes == (used + 7) // 8 * 8
-    pk_act = torch.zeros((B, 2), dtype=torch.int32).pin_memory()
-    guard = torch.full((B + 4, nbytes), 0x5A, dtype=torch.uint8).pin_memory()   # four records of canary behind the batch
+    pk_act = pin(torch.zeros((B, 2), dtype=torch.int32))
+    guard = pin(torch.full((B + 4, nbytes), 0x5A, dtype=torch.uint8))   # four records of canary behind the batch
     pk_rec = guard[:B]
     check_obs = set(_checkpoints(N))
     for s in range(N):
