@@ -74,6 +74,7 @@ SIGNATURES = {
     "mtfjsp_export_scaler": ([_VP] + [_VP] * 4 + [_VP], _I),
     "mtfjsp_gather": ([_VP, _VP, _VP, _VP], _I),
     "mtfjsp_peek": ([_VP, _VP, _VP, _I, _VP, _VP, _VP], _I),
+    "mtfjsp_replay": ([_VP, _VP, _I, _VP, _I, _VP, _VP, _VP, _VP], _I),
     "mtfjsp_policy_random": ([_VP, _U64, _U64, _I, _VP, _VP, _VP], _I),
     "mtfjsp_random_step": ([_VP, _U64, _U64] + [_VP] * 14 + [_I, _I, _VP], _I),
     "mtfjsp_step_host": ([_VP] + [_VP] * 9 + [_I, _I, _VP], _I),

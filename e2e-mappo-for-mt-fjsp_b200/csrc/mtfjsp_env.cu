@@ -227,6 +227,247 @@ __device__ double pairwise_sum(const double* a, const PwPlan& pw, double* s_leaf
     return top;
 }
 
+// One env's records staged in shared memory at the Layout::sm_* offsets of its warp's slice `base`: the state the generic
+// kernel steps (env_kernel) and the replay kernel runs whole episodes on (replay_kernel)
+struct EnvSmem {
+    double *sd, *xs, *pt, *v, *leaf;
+    int16_t *si, *nxt;
+    double *st, *ft, *dur, *psel, *scal, *macc, *ipre, *eacc, *eleaf;
+    int16_t *mach, *ord, *rpred, *cnt, *misc;
+    const double *mind, *minpt, *tt;
+    __device__ __forceinline__ EnvSmem(const Layout& L, unsigned char* base) {
+        sd = reinterpret_cast<double*>(base + L.sm_sd);
+        xs = reinterpret_cast<double*>(base + L.sm_xs);
+        pt = reinterpret_cast<double*>(base + L.sm_pt);  // idle terms, then est_pt
+        v = reinterpret_cast<double*>(base + L.sm_v);    // per-job ESA key
+        leaf = reinterpret_cast<double*>(base + L.sm_leaf);
+        si = reinterpret_cast<int16_t*>(base + L.sm_si);
+        nxt = reinterpret_cast<int16_t*>(base + L.sm_nxt);
+        st = sd + L.o_st; ft = sd + L.o_ft; dur = sd + L.o_dur; psel = sd + L.o_psel;
+        scal = sd + L.o_scal;  // mk_prev, e_prev, trans, idle_prev
+        macc = sd + L.o_macc; ipre = sd + L.o_ipre; eacc = sd + L.o_eacc; eleaf = sd + L.o_eleaf;
+        mach = si + L.o_mach; ord = si + L.o_ord; rpred = si + L.o_rpred; cnt = si + L.o_cnt;
+        misc = si + L.o_misc;  // removed_head, fresh_co, nsched
+        mind = xs + L.o_mind; minpt = xs + L.o_minpt; tt = xs + L.o_tt;
+    }
+};
+
+// what one transition leaves for the step's reward epilogue and incremental observation
+struct StepOut {
+    bool valid, done;
+    double idle, nt, trans, ec;
+    int o_next, o_tail;  // machine follower and route tail of the stepped op
+};
+
+// One transition of action (a, m) on the staged env (SS:716-974, 1476-1809; trainer/DGenv_func.py:46-170): validity,
+// placement with or without left shift, the move into the flat order, the flat-order idle-time sum and the step's
+// transport and energy terms.  tp: the env's row of the instance tables t / p.  WB: also write what changed to the env's
+// records g_sd / g_si (the generic step kernel); the replay kernel runs on the staged copy only.
+template <bool WB>
+__device__ __forceinline__ StepOut env_transition(const Layout& L, const EnvSmem& S, const double* t, const double* p,
+                                                  size_t tp, int a, int m, double* g_sd, int16_t* g_si, int lane) {
+    const int N = L.N, M = L.M;
+    StepOut o;
+    o.valid = false; o.done = false; o.idle = 0.0; o.nt = 0.0; o.trans = 0.0; o.ec = 0.0; o.o_next = -1; o.o_tail = -1;
+    const int nsched0 = S.misc[2];
+    double d = 0.0, pa = 0.0;
+    bool valid = (a >= 0) && (a < N) && (m >= 0) && (m < M) && (nsched0 < N);
+    if (valid) valid = (S.mach[a] < 0) && (((a % M) == 0) || (S.mach[a - 1] >= 0));
+    if (valid) {
+        d = __ldg(t + (tp * N + a) * M + m);
+        pa = __ldg(p + (tp * N + a) * M + m);
+        valid = !(d < 0);
+    }
+    o.valid = valid;
+    if (valid) {
+        const bool first = (a % M) == 0;
+        const int ja = a / M;
+        // job-arc refresh at step start (SS:1502): transient markers of the previous step expire
+        int rem_head = -1, fresh = -1;
+        const double arr_a = first ? 0.0 : S.ft[a - 1] + S.tt[S.mach[a - 1] * M + m];  // DGenv_func.py:46-66
+        const int len = S.cnt[m];
+        const double ttmm = S.tt[m * M + m];
+        double st = arr_a;
+        int where = 0, prev = -1, next = -1;
+        // machine m's route is ord[offm, offm + len)
+        int offm = 0;
+        for (int m0 = 0; m0 < m; m0 += 32) offm += __reduce_add_sync(FULL, (m0 + lane < m) ? (int)S.cnt[m0 + lane] : 0);
+        if (len > 0) {
+            // one pass over the route of machine m: arrival of each op, first feasible slot (SS:1548-1601)
+            const double lbft = arr_a + d;
+            unsigned best = 0xffffffffu;
+            const int lastop = S.ord[offm + len - 1];
+            if (L.left_shift) {
+                for (int k0 = 0; k0 < len; k0 += 32) {
+                    const int k = k0 + lane;
+                    unsigned key = 0xffffffffu;
+                    if (k < len) {
+                        const int v = S.ord[offm + k];
+                        const bool vfirst = (v % M) == 0;
+                        double nst = vfirst ? 0.0 : S.ft[v - 1] + S.tt[S.mach[v - 1] * M + m];
+                        bool ok;
+                        if (k == 0) {
+                            ok = (lbft <= nst);  // SS:1548 (route head has no machine in-arc)
+                        } else {
+                            const int rp = S.ord[offm + k - 1];
+                            double val = S.ft[rp] + ((rp / M == v / M) ? ttmm : 0.0);
+                            nst = fmax(nst, val);
+                            ok = !(lbft > nst) && !((nst - S.ft[rp]) < d);  // SS:1597-1601
+                        }
+                        if (ok) key = ((unsigned)k << 16) | (unsigned)v;
+                    }
+                    best = min(best, __reduce_min_sync(FULL, key));
+                }
+            }
+            if (best != 0xffffffffu) {
+                where = (int)(best >> 16);
+                next = (int)(best & 0xffffu);
+                if (where > 0) {
+                    prev = S.rpred[next];
+                    double y = S.ft[prev] + ((prev / M == ja) ? ttmm : 0.0);  // SS:1619
+                    st = (y > arr_a) ? y : arr_a;
+                    if (next == prev + 1 && (next % M) != 0) rem_head = next;  // SS:1660
+                }
+            } else {  // _append_at_the_end, SS:1689-1775
+                where = len;
+                prev = lastop;
+                double y = S.ft[prev] + ((prev / M == ja) ? ttmm : 0.0);
+                st = (y > arr_a) ? y : arr_a;
+            }
+            if (prev >= 0 && prev == a - 1 && !first) fresh = a;
+            o.o_tail = (where == len) ? a : lastop;
+        } else {
+            o.o_tail = a;
+        }
+        o.o_next = next;
+        __syncwarp();
+        // ---- apply: open slot p of the flat order (entries behind it move up by one), link the op in ----
+        const int p_ = offm + where;
+        for (int g0 = ((nsched0 > 0 ? nsched0 - 1 : 0) / 32) * 32; g0 >= 0 && g0 + 31 >= p_; g0 -= 32) {
+            const int g = g0 + lane;
+            const bool mv_ = g >= p_ && g < nsched0;
+            const int16_t x = mv_ ? S.ord[g] : (int16_t)0;
+            __syncwarp();
+            if (mv_) {
+                S.ord[g + 1] = x;
+                if (WB) g_si[L.o_ord + g + 1] = x;
+            }
+            __syncwarp();
+        }
+        if (lane == 0) {
+            S.mach[a] = (int16_t)m; S.ord[p_] = (int16_t)a; S.rpred[a] = (int16_t)prev;
+            if (next >= 0) S.rpred[next] = (int16_t)a;
+            S.cnt[m] = (int16_t)(len + 1);
+            S.misc[0] = (int16_t)rem_head; S.misc[1] = (int16_t)fresh; S.misc[2] = (int16_t)(nsched0 + 1);
+            S.st[a] = st; S.ft[a] = st + d; S.dur[a] = d; S.psel[a] = pa;
+            if (WB) {
+                g_si[L.o_mach + a] = (int16_t)m; g_si[L.o_ord + p_] = (int16_t)a; g_si[L.o_rpred + a] = (int16_t)prev;
+                if (next >= 0) g_si[L.o_rpred + next] = (int16_t)a;
+                g_si[L.o_cnt + m] = (int16_t)(len + 1);
+                g_si[L.o_misc + 0] = (int16_t)rem_head; g_si[L.o_misc + 1] = (int16_t)fresh;
+                g_si[L.o_misc + 2] = (int16_t)(nsched0 + 1);
+                g_si[L.o_nxt + ja] = (int16_t)((a % M) + 1);
+                g_sd[L.o_st + a] = st; g_sd[L.o_ft + a] = st + d; g_sd[L.o_dur + a] = d; g_sd[L.o_psel + a] = pa;
+                double cur = st + d;  // estimator chain of the remaining ops of this job (SS:1964-1995)
+                for (int c = (a % M) + 1; c < M; c++) {
+                    g_sd[L.o_st + ja * M + c] = cur;
+                    cur = cur + S.mind[ja * M + c];
+                    g_sd[L.o_ft + ja * M + c] = cur;
+                }
+            }
+        }
+        __syncwarp();
+        const int nsched = nsched0 + 1;
+        o.done = (nsched == N);
+        // ---- idle time: sequential sum in (machine, route) order = flat order, DGenv_func.py:144-170 ----
+        for (int g = lane; g < nsched; g += 32) {
+            const int v = S.ord[g], rp = S.rpred[v];
+            const double term = (rp < 0) ? (S.st[v] - 0.0) : (S.st[v] - S.ft[rp]);
+            S.pt[g] = term * 1.0;
+        }
+        __syncwarp();
+        double idle = 0.0;
+        if (L.nich) {  // large instances: running sum in front of every 32nd term (the specialised kernel restarts there)
+            for (int g = 0; g <= nsched; g++) {
+                if ((g & 31) == 0 && (g >> 5) < L.nich && lane == 0) S.ipre[g >> 5] = idle;
+                if (g < nsched) idle = idle + S.pt[g];
+            }
+        } else {
+#pragma unroll 4
+            for (int g = 0; g < nsched; g++) idle = idle + S.pt[g];
+        }
+        __syncwarp();
+        o.idle = idle;
+        o.nt = first ? 0.0 : S.tt[S.mach[a - 1] * M + m];  // SS:872-877
+        o.trans = S.scal[2] + o.nt;
+        o.ec = pa * d;
+    }
+    __syncwarp();
+    return o;
+}
+
+// Per-job walk over the staged env: scheduled prefix, estimator chain (SS:1964-1995), ESA key (ppo_algorithm.py:280),
+// est_pt; with SUMS the makespan estimate (*mkv) and the energy estimate (*env, numpy's pairwise sum) (SS:894-896)
+template <bool SUMS>
+__device__ __forceinline__ void env_estimates(const Layout& L, const PwPlan& pw, const EnvSmem& S, int lane, double* mkv,
+                                              double* env) {
+    const int N = L.N, M = L.M, J = L.J;
+    for (int j = lane; j < J; j += 32) {
+        const int jb = j * M;
+        double cur = 0.0, rm = 0.0;
+        int nx = 0;
+        while (nx < M && S.mach[jb + nx] >= 0) {
+            cur = S.ft[jb + nx];
+            rm = fmax(rm, cur);
+            nx++;
+        }
+        for (int c = nx; c < M; c++) {
+            S.st[jb + c] = (c == 0) ? 0.0 : cur;
+            cur = ((c == 0) ? 0.0 : cur) + S.mind[jb + c];
+            S.ft[jb + c] = cur;
+        }
+        S.nxt[j] = (int16_t)nx;
+        S.v[j] = (nx == M) ? INFINITY : rm;
+    }
+    __syncwarp();
+    double mx = -INFINITY;
+    for (int v = lane; v < N; v += 32) {
+        S.pt[v] = (S.mach[v] >= 0) ? S.dur[v] * S.psel[v] : S.minpt[v];
+        mx = fmax(mx, S.ft[v]);
+    }
+    __syncwarp();
+    if (SUMS) {
+        *mkv = warp_max(mx);
+        *env = pairwise_sum(S.pt, pw, S.leaf, lane, S.eacc, S.eleaf);
+    }
+}
+
+// step reward of a valid transition (wrk_reward_function, SS:1066-1132): (total before the divisor, r_mk, r_idle, r_pt,
+// r_tt); lane 0 then advances the machine accumulators (SS:2323-2338) and the previous-step scalars (SS:932-936)
+struct StepReward {
+    double total, r_t, r_idle, r_pt, r_tt;
+};
+__device__ __forceinline__ StepReward env_reward(const Layout& L, const EnvSmem& S, const double* cfgw, int m, double mkv,
+                                                 double env, const StepOut& o, int lane) {
+    const int N = L.N;
+    const double mk_prev = S.scal[0], e_prev = S.scal[1], trans_prev = S.scal[2], idle_prev = S.scal[3];
+    StepReward w;
+    w.r_t = 1.0 * mk_prev - mkv;
+    double r_pt = 1.0 * e_prev - env;
+    w.r_pt = r_pt / (double)N;
+    w.r_tt = 1.0 * trans_prev - o.trans;
+    w.r_idle = 1.0 * idle_prev - o.idle;
+    w.total = cfgw[0] * w.r_t + cfgw[1] * (w.r_pt + 1.0 * w.r_idle) + cfgw[2] * w.r_tt * 1.0;
+    __syncwarp();
+    if (lane == 0) {
+        S.macc[m * 3 + 0] += o.ec / (double)N;
+        S.macc[m * 3 + 1] += o.nt;
+        S.macc[m * 3 + 2] += o.idle - idle_prev;
+        S.scal[0] = mkv; S.scal[1] = env; S.scal[2] = o.trans; S.scal[3] = o.idle;
+    }
+    return w;
+}
+
 template <int MODE, typename OutT>
 __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -236,13 +477,13 @@ __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params
     if (b >= L.B) return;
     const int N = L.N, M = L.M, J = L.J;
     unsigned char* base = smem_raw + (size_t)warp * L.smem_per_warp;
-    double* s_sd = reinterpret_cast<double*>(base + L.sm_sd);
-    double* s_xs = reinterpret_cast<double*>(base + L.sm_xs);
-    double* s_pt = reinterpret_cast<double*>(base + L.sm_pt);  // idle terms, then est_pt
-    double* s_v = reinterpret_cast<double*>(base + L.sm_v);    // per-job ESA key
-    double* s_leaf = reinterpret_cast<double*>(base + L.sm_leaf);
-    int16_t* s_si = reinterpret_cast<int16_t*>(base + L.sm_si);
-    int16_t* s_nxt = reinterpret_cast<int16_t*>(base + L.sm_nxt);
+    const EnvSmem S(L, base);
+    double* s_sd = S.sd;
+    double* s_xs = S.xs;
+    double* s_pt = S.pt;
+    double* s_v = S.v;
+    int16_t* s_si = S.si;
+    int16_t* s_nxt = S.nxt;
     int16_t* s_tail = reinterpret_cast<int16_t*>(base + L.sm_tail);
 
     double* g_sd = P.sd + (size_t)b * L.sd_stride;
@@ -263,24 +504,21 @@ __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params
             for (int i = lane; i < L.si_stride / 8; i += 32) dst[i] = src[i];
         }
     }
-    double* s_st = s_sd + L.o_st;
-    double* s_ft = s_sd + L.o_ft;
-    double* s_dur = s_sd + L.o_dur;
-    double* s_psel = s_sd + L.o_psel;
-    double* s_scal = s_sd + L.o_scal;  // mk_prev, e_prev, trans, idle_prev
-    double* s_macc = s_sd + L.o_macc;
+    double* s_st = S.st;
+    double* s_ft = S.ft;
+    double* s_dur = S.dur;
+    double* s_psel = S.psel;
+    double* s_scal = S.scal;
+    double* s_macc = S.macc;
     double* s_w = s_sd + L.o_w;
     double* s_sc = s_sd + L.o_sc;  // R[4] mean[4] S[4] n
-    int16_t* s_mach = s_si + L.o_mach;
-    int16_t* s_ord = s_si + L.o_ord;
-    int16_t* s_rpred = s_si + L.o_rpred;
-    int16_t* s_cnt = s_si + L.o_cnt;
-    int16_t* s_misc = s_si + L.o_misc;  // removed_head, fresh_co, nsched
-    const double* s_mind = s_xs + L.o_mind;
-    const double* s_minpt = s_xs + L.o_minpt;
-    const double* s_tt = s_xs + L.o_tt;
-    double* s_eacc = s_sd + L.o_eacc;    // cached pairwise-sum accumulators / leaf results of the energy estimate
-    double* s_eleaf = s_sd + L.o_eleaf;
+    int16_t* s_mach = S.mach;
+    int16_t* s_ord = S.ord;
+    int16_t* s_rpred = S.rpred;
+    int16_t* s_cnt = S.cnt;
+    int16_t* s_misc = S.misc;
+    const double* s_minpt = S.minpt;
+    const double* s_tt = S.tt;
 
     if (MODE & MODE_RESET) {  // load_instance + reset, SS:397-714, 1183-1245
         __syncwarp();
@@ -297,177 +535,23 @@ __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params
     __syncwarp();
 
     int a = -1, m = -1;
-    bool valid = false, done = false;
     double mkv = 0.0, env = 0.0;
-    double idle = 0.0, nt = 0.0, trans = 0.0, ec = 0.0;  // step results kept in registers for the reward epilogue
-    // incremental observation (see env_kernel_s): machine follower and route tail of the stepped op, previous transients
-    int o_next = -1, o_tail = -1, rem_prev = -1, fresh_prev = -1;
+    StepOut so;  // step results kept in registers for the reward epilogue and the incremental observation
+    so.valid = false; so.done = false; so.o_next = -1; so.o_tail = -1;
+    // incremental observation (see env_kernel_s): previous transients
+    int rem_prev = -1, fresh_prev = -1;
 
     if (MODE & MODE_STEP) {
         if (P.act2) { const int2 am = P.act2[b]; a = am.x; m = am.y; }
         else { a = P.op[b]; m = P.mach[b]; }
-        const int nsched0 = s_misc[2];
         rem_prev = s_misc[0];
         fresh_prev = s_misc[1];
-        double d = 0.0, pa = 0.0;
-        valid = (a >= 0) && (a < N) && (m >= 0) && (m < M) && (nsched0 < N);
-        if (valid) valid = (s_mach[a] < 0) && (((a % M) == 0) || (s_mach[a - 1] >= 0));
-        if (valid) {
-            d = __ldg(P.t + ((size_t)b * N + a) * M + m);
-            pa = __ldg(P.p + ((size_t)b * N + a) * M + m);
-            valid = !(d < 0);
-        }
-        if (valid) {
-            const bool first = (a % M) == 0;
-            const int ja = a / M;
-            // job-arc refresh at step start (SS:1502): transient markers of the previous step expire
-            int rem_head = -1, fresh = -1;
-            const double arr_a = first ? 0.0 : s_ft[a - 1] + s_tt[s_mach[a - 1] * M + m];  // DGenv_func.py:46-66
-            const int len = s_cnt[m];
-            const double ttmm = s_tt[m * M + m];
-            double st = arr_a;
-            int where = 0, prev = -1, next = -1;
-            // machine m's route is ord[offm, offm + len)
-            int offm = 0;
-            for (int m0 = 0; m0 < m; m0 += 32) offm += __reduce_add_sync(FULL, (m0 + lane < m) ? (int)s_cnt[m0 + lane] : 0);
-            if (len > 0) {
-                // one pass over the route of machine m: arrival of each op, first feasible slot (SS:1548-1601)
-                const double lbft = arr_a + d;
-                unsigned best = 0xffffffffu;
-                const int lastop = s_ord[offm + len - 1];
-                if (L.left_shift) {
-                    for (int k0 = 0; k0 < len; k0 += 32) {
-                        const int k = k0 + lane;
-                        unsigned key = 0xffffffffu;
-                        if (k < len) {
-                            const int v = s_ord[offm + k];
-                            const bool vfirst = (v % M) == 0;
-                            double nst = vfirst ? 0.0 : s_ft[v - 1] + s_tt[s_mach[v - 1] * M + m];
-                            bool ok;
-                            if (k == 0) {
-                                ok = (lbft <= nst);  // SS:1548 (route head has no machine in-arc)
-                            } else {
-                                const int rp = s_ord[offm + k - 1];
-                                double val = s_ft[rp] + ((rp / M == v / M) ? ttmm : 0.0);
-                                nst = fmax(nst, val);
-                                ok = !(lbft > nst) && !((nst - s_ft[rp]) < d);  // SS:1597-1601
-                            }
-                            if (ok) key = ((unsigned)k << 16) | (unsigned)v;
-                        }
-                        best = min(best, __reduce_min_sync(FULL, key));
-                    }
-                }
-                if (best != 0xffffffffu) {
-                    where = (int)(best >> 16);
-                    next = (int)(best & 0xffffu);
-                    if (where > 0) {
-                        prev = s_rpred[next];
-                        double y = s_ft[prev] + ((prev / M == ja) ? ttmm : 0.0);  // SS:1619
-                        st = (y > arr_a) ? y : arr_a;
-                        if (next == prev + 1 && (next % M) != 0) rem_head = next;  // SS:1660
-                    }
-                } else {  // _append_at_the_end, SS:1689-1775
-                    where = len;
-                    prev = lastop;
-                    double y = s_ft[prev] + ((prev / M == ja) ? ttmm : 0.0);
-                    st = (y > arr_a) ? y : arr_a;
-                }
-                if (prev >= 0 && prev == a - 1 && !first) fresh = a;
-                o_tail = (where == len) ? a : lastop;
-            } else {
-                o_tail = a;
-            }
-            o_next = next;
-            __syncwarp();
-            // ---- apply: open slot p of the flat order (entries behind it move up by one), link the op in ----
-            const int p = offm + where;
-            for (int g0 = ((nsched0 > 0 ? nsched0 - 1 : 0) / 32) * 32; g0 >= 0 && g0 + 31 >= p; g0 -= 32) {
-                const int g = g0 + lane;
-                const bool mv_ = g >= p && g < nsched0;
-                const int16_t x = mv_ ? s_ord[g] : (int16_t)0;
-                __syncwarp();
-                if (mv_) { s_ord[g + 1] = x; g_si[L.o_ord + g + 1] = x; }
-                __syncwarp();
-            }
-            if (lane == 0) {
-                s_mach[a] = (int16_t)m; s_ord[p] = (int16_t)a; s_rpred[a] = (int16_t)prev;
-                if (next >= 0) s_rpred[next] = (int16_t)a;
-                s_cnt[m] = (int16_t)(len + 1);
-                s_misc[0] = (int16_t)rem_head; s_misc[1] = (int16_t)fresh; s_misc[2] = (int16_t)(nsched0 + 1);
-                s_st[a] = st; s_ft[a] = st + d; s_dur[a] = d; s_psel[a] = pa;
-                g_si[L.o_mach + a] = (int16_t)m; g_si[L.o_ord + p] = (int16_t)a; g_si[L.o_rpred + a] = (int16_t)prev;
-                if (next >= 0) g_si[L.o_rpred + next] = (int16_t)a;
-                g_si[L.o_cnt + m] = (int16_t)(len + 1);
-                g_si[L.o_misc + 0] = (int16_t)rem_head; g_si[L.o_misc + 1] = (int16_t)fresh;
-                g_si[L.o_misc + 2] = (int16_t)(nsched0 + 1);
-                g_si[L.o_nxt + ja] = (int16_t)((a % M) + 1);
-                g_sd[L.o_st + a] = st; g_sd[L.o_ft + a] = st + d; g_sd[L.o_dur + a] = d; g_sd[L.o_psel + a] = pa;
-                double cur = st + d;  // estimator chain of the remaining ops of this job (SS:1964-1995)
-                for (int c = (a % M) + 1; c < M; c++) {
-                    g_sd[L.o_st + ja * M + c] = cur;
-                    cur = cur + s_mind[ja * M + c];
-                    g_sd[L.o_ft + ja * M + c] = cur;
-                }
-            }
-            __syncwarp();
-            const int nsched = nsched0 + 1;
-            done = (nsched == N);
-            // ---- idle time: sequential sum in (machine, route) order = flat order, DGenv_func.py:144-170 ----
-            for (int g = lane; g < nsched; g += 32) {
-                const int v = s_ord[g], rp = s_rpred[v];
-                const double term = (rp < 0) ? (s_st[v] - 0.0) : (s_st[v] - s_ft[rp]);
-                s_pt[g] = term * 1.0;
-            }
-            __syncwarp();
-            if (L.nich) {  // large instances: running sum in front of every 32nd term (the specialised kernel restarts there)
-                for (int g = 0; g <= nsched; g++) {
-                    if ((g & 31) == 0 && (g >> 5) < L.nich && lane == 0) s_sd[L.o_ipre + (g >> 5)] = idle;
-                    if (g < nsched) idle = idle + s_pt[g];
-                }
-            } else {
-#pragma unroll 4
-                for (int g = 0; g < nsched; g++) idle = idle + s_pt[g];
-            }
-            __syncwarp();
-            nt = first ? 0.0 : s_tt[s_mach[a - 1] * M + m];  // SS:872-877
-            trans = s_scal[2] + nt;
-            ec = pa * d;
-        }
-        __syncwarp();
+        so = env_transition<true>(L, S, P.t, P.p, (size_t)b, a, m, g_sd, g_si, lane);
     }
+    const bool valid = so.valid, done = so.done;
+    const int o_next = so.o_next, o_tail = so.o_tail;
 
-    // ---- per-job walk: scheduled prefix, estimator chain (SS:1964-1995), ESA key (ppo_algorithm.py:280) ----
-    for (int j = lane; j < J; j += 32) {
-        const int jb = j * M;
-        double cur = 0.0, rm = 0.0;
-        int nx = 0;
-        while (nx < M && s_mach[jb + nx] >= 0) {
-            cur = s_ft[jb + nx];
-            rm = fmax(rm, cur);
-            nx++;
-        }
-        for (int c = nx; c < M; c++) {
-            s_st[jb + c] = (c == 0) ? 0.0 : cur;
-            cur = ((c == 0) ? 0.0 : cur) + s_mind[jb + c];
-            s_ft[jb + c] = cur;
-        }
-        s_nxt[j] = (int16_t)nx;
-        s_v[j] = (nx == M) ? INFINITY : rm;
-    }
-    __syncwarp();
-    // est_pt, makespan estimate, energy estimate (SS:894-896)
-    {
-        double mx = -INFINITY;
-        for (int v = lane; v < N; v += 32) {
-            s_pt[v] = (s_mach[v] >= 0) ? s_dur[v] * s_psel[v] : s_minpt[v];
-            mx = fmax(mx, s_ft[v]);
-        }
-        __syncwarp();
-        if (MODE & (MODE_STEP | MODE_RESET)) {
-            mkv = warp_max(mx);
-            env = pairwise_sum(s_pt, P.pw, s_leaf, lane, s_eacc, s_eleaf);
-        }
-    }
+    env_estimates<(MODE & (MODE_STEP | MODE_RESET)) != 0>(L, P.pw, S, lane, &mkv, &env);
 
     if (MODE & MODE_RESET) {
         if (lane == 0) { s_scal[0] = mkv; s_scal[1] = env; s_scal[2] = 0.0; s_scal[3] = 0.0; }  // SS:697-705
@@ -488,22 +572,8 @@ __global__ void __launch_bounds__(256) env_kernel(const __grid_constant__ Params
 
     if ((MODE & MODE_STEP)) {
         if (valid) {
-            const double mk_prev = s_scal[0], e_prev = s_scal[1], trans_prev = s_scal[2], idle_prev = s_scal[3];
-            // wrk_reward_function, SS:1066-1132
-            const double r_t = 1.0 * mk_prev - mkv;
-            double r_pt = 1.0 * e_prev - env;
-            r_pt = r_pt / (double)N;
-            const double r_tt = 1.0 * trans_prev - trans;
-            const double r_idle = 1.0 * idle_prev - idle;
-            const double total = P.cfgw[0] * r_t + P.cfgw[1] * (r_pt + 1.0 * r_idle) + P.cfgw[2] * r_tt * 1.0;
-            __syncwarp();
-            if (lane == 0) {
-                // machine accumulators, SS:2323-2338
-                s_macc[m * 3 + 0] += ec / (double)N;
-                s_macc[m * 3 + 1] += nt;
-                s_macc[m * 3 + 2] += idle - idle_prev;
-                s_scal[0] = mkv; s_scal[1] = env; s_scal[2] = trans; s_scal[3] = idle;  // SS:932-936
-            }
+            const StepReward rw = env_reward(L, S, P.cfgw, m, mkv, env, so, lane);
+            const double r_t = rw.r_t, r_idle = rw.r_idle, r_pt = rw.r_pt, r_tt = rw.r_tt, total = rw.total;
             // reward scaling, ppo_trick.py:73-88,115-119 (lanes 0..3 own one component each)
             double scaled = 0.0;
             if (lane < 4) {
@@ -2536,6 +2606,85 @@ size_t peek_env_bytes(const Layout& L, int K) {
            (size_t)K * (8 + 16 + 5 * 8 + 1);
 }
 
+// Whole-episode replay (mtfjsp_replay): candidate r runs T (op, machine) actions from the episode start of env src[r]
+// (the reset snapshot sd0 / si0) and leaves the costs, the summed rewards and the index of its first invalid action.
+// One warp per candidate, in env_kernel's lane layout and shared-memory slice (Layout::sm_*), so every size the handle
+// accepts fits: the warp stages the snapshot records and the static doubles once, then runs every transition on that
+// copy with env_kernel's own device code (env_transition, env_estimates, env_reward) and writes 4 + 5 doubles and an int.
+// The actions are read 32 at a time, one (op, machine) pair per lane in one coalesced 256-byte read, and broadcast by
+// shuffle.  Nothing of the handle is written.
+struct ReplayArgs {
+    Layout L;
+    PwPlan pw;
+    const double *sd0, *xs, *t, *p;
+    const int16_t* si0;
+    const int32_t *src, *actions;
+    int R, T;
+    double cfgw[3], divisor;
+    double *cost4, *return5;
+    int32_t* first_invalid;
+};
+
+__global__ void __launch_bounds__(256) replay_kernel(const __grid_constant__ ReplayArgs A) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const Layout& L = A.L;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int r = blockIdx.x * L.warps_per_block + warp;
+    if (r >= A.R) return;
+    const int src = A.src[r];
+    if (src < 0 || src >= L.B) {  // a source index is data: this candidate gets -2 and zero rows, the others run
+        if (A.cost4 && lane < 4) A.cost4[(size_t)r * 4 + lane] = 0.0;
+        if (A.return5 && lane < 5) A.return5[(size_t)r * 5 + lane] = 0.0;
+        if (A.first_invalid && lane == 0) A.first_invalid[r] = -2;
+        return;
+    }
+    const EnvSmem S(L, smem_raw + (size_t)warp * L.smem_per_warp);
+    {
+        const uint4* g = reinterpret_cast<const uint4*>(A.sd0 + (size_t)src * L.sd_stride);
+        uint4* d = reinterpret_cast<uint4*>(S.sd);
+        for (int i = lane; i < L.sd_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.xs + (size_t)src * L.xs_stride);
+        d = reinterpret_cast<uint4*>(S.xs);
+        for (int i = lane; i < L.xs_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.si0 + (size_t)src * L.si_stride);
+        d = reinterpret_cast<uint4*>(S.si);
+        for (int i = lane; i < L.si_stride / 8; i += 32) d[i] = __ldg(g + i);
+    }
+    __syncwarp();
+    const int32_t* act = A.actions + (size_t)r * A.T * 2;
+    double ret[5] = {0.0, 0.0, 0.0, 0.0, 0.0};  // lane 0: the step-order sums of the step's reward5
+    int bad = -1, op_l = 0, mach_l = 0;
+    for (int s = 0; s < A.T; s++) {
+        if ((s & 31) == 0) {
+            op_l = s + lane < A.T ? __ldg(act + 2 * (s + lane)) : 0;
+            mach_l = s + lane < A.T ? __ldg(act + 2 * (s + lane) + 1) : 0;
+        }
+        const int a = __shfl_sync(FULL, op_l, s & 31), m = __shfl_sync(FULL, mach_l, s & 31);
+        const StepOut so = env_transition<false>(L, S, A.t, A.p, (size_t)src, a, m, nullptr, nullptr, lane);
+        double r5[5] = {0.0, 0.0, 0.0, 0.0, 0.0};  // what the step writes for an invalid action
+        if (so.valid) {
+            double mkv, env;
+            env_estimates<true>(L, A.pw, S, lane, &mkv, &env);
+            const StepReward rw = env_reward(L, S, A.cfgw, m, mkv, env, so, lane);
+            r5[0] = rw.total / A.divisor; r5[1] = rw.r_t; r5[2] = rw.r_idle; r5[3] = rw.r_pt; r5[4] = rw.r_tt;
+            __syncwarp();
+        } else if (bad < 0) {
+            bad = s;
+        }
+#pragma unroll
+        for (int k = 0; k < 5; k++) ret[k] += r5[k];
+    }
+    if (lane == 0) {
+        if (A.cost4) {  // costs_kernel's expressions
+            double* c = A.cost4 + (size_t)r * 4;
+            c[0] = S.scal[0]; c[1] = S.scal[1] / (double)L.N; c[2] = S.scal[2]; c[3] = S.scal[3];
+        }
+        if (A.return5)
+            for (int k = 0; k < 5; k++) A.return5[(size_t)r * 5 + k] = ret[k];
+        if (A.first_invalid) A.first_invalid[r] = bad;
+    }
+}
+
 thread_local char g_err[512] = "";
 
 int fail(int code, const char* msg, cudaError_t e = cudaSuccess) {
@@ -3326,6 +3475,37 @@ int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, do
     peek_kernel<<<L.B, warps * 32, smem, s>>>(A);
     h->launches++;
     CK(cudaGetLastError(), "peek_kernel");
+    return MTFJSP_OK;
+}
+
+int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, double* cost4, double* return5,
+                  int32_t* first_invalid, void* stream) {
+    if (!h || !src || !actions || R < 1 || T < 1 || T > h->L.N) return fail(MTFJSP_E_ARG, "mtfjsp_replay: bad argument");
+    if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_replay before mtfjsp_reset");
+    const Layout& L = h->L;
+    cudaStream_t s = (cudaStream_t)stream;
+    // a non-step call: a recorded reset runs now, and the next step waits for the replay in full
+    int rc = enter(h, s);
+    if (rc) return rc;
+    const size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
+    static thread_local int configured_dev = -1;
+    static thread_local size_t configured_smem = 0;
+    if (configured_dev != h->device || configured_smem < smem) {
+        CK(cudaFuncSetAttribute(replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute");
+        configured_dev = h->device;
+        configured_smem = smem;
+    }
+    ReplayArgs A;
+    memset(&A, 0, sizeof A);
+    A.L = L; A.pw = h->pw;
+    A.sd0 = h->sd0; A.xs = h->xs; A.t = h->t; A.p = h->p; A.si0 = h->si0;
+    A.src = src; A.actions = actions; A.R = R; A.T = T;
+    A.cfgw[0] = h->cfgw[0]; A.cfgw[1] = h->cfgw[1]; A.cfgw[2] = h->cfgw[2]; A.divisor = h->divisor;
+    A.cost4 = cost4; A.return5 = return5; A.first_invalid = first_invalid;
+    const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
+    replay_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
+    h->launches++;
+    CK(cudaGetLastError(), "replay_kernel");
     return MTFJSP_OK;
 }
 

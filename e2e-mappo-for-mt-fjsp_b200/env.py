@@ -299,6 +299,33 @@ class BatchedMTFJSPEnv:
             raise ValueError("machines must have shape [%d, %d]" % (B, self.N))
         return self.peek(cand, torch.gather(machines, 1, cand.long()))
 
+    # ---- whole-episode replay ----------------------------------------------------------------------------------------
+    def replay(self, actions, src=None):
+        """What T steps of each of R action sequences leave, each from the episode start of env src[r], without changing
+        the env (mtfjsp_replay).  actions: [T,R,2] integer (op, machine) tensor on this env's device, 1 <= T <= N -- the
+        [N,S,2] layout greedy_validate, beam_validate and the rules' rollouts return.  src: [R] integers (duplicates and
+        permutations allowed); None means arange(B) and needs R == B.  Returns new tensors final4 [R,4] f64 (what `costs`
+        would return), return5 [R,5] f64 (the step-order sum of the steps' reward5) and first_invalid [R] int32 (-1, or the
+        index of the first invalid action, which was a no-op; -2 where src is outside [0, B), with zero rows)."""
+        _on(self.device, actions, src)
+        if actions.dim() != 3 or actions.shape[2] != 2:
+            raise ValueError("actions must have shape [T, R, 2]")
+        T, R = int(actions.shape[0]), int(actions.shape[1])
+        if src is None:
+            if R != self.B:
+                raise ValueError("src=None replays env r from row r: needs R == B = %d" % self.B)
+            src = torch.arange(R, dtype=torch.int32, device=self.device)
+        elif tuple(src.shape) != (R,):
+            raise ValueError("src must have shape [%d]" % R)
+        src = src.to(torch.int32).contiguous()
+        act = actions.to(torch.int32).transpose(0, 1).contiguous()  # [R,T,2]: one contiguous run per candidate
+        final4 = torch.empty((R, 4), dtype=torch.float64, device=self.device)
+        ret5 = torch.empty((R, 5), dtype=torch.float64, device=self.device)
+        finv = torch.empty((R,), dtype=torch.int32, device=self.device)
+        check(self._lib.mtfjsp_replay(self._h, _ptr(src), R, _ptr(act), T, _ptr(final4), _ptr(ret5), _ptr(finv),
+                                      _stream()), "mtfjsp_replay")
+        return final4, ret5, finv
+
     # ---- views ---------------------------------------------------------------------------------------------------
     def dense_adj(self, dtype=torch.float64):
         adj = torch.empty((self.B, self.N, self.N), dtype=dtype, device=self.device)

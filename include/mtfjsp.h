@@ -170,6 +170,23 @@ int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, vo
 int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, double* reward5, uint8_t* invalid,
                 void* stream);
 
+/* Whole-episode replay: for R candidate action sequences, what T steps from an episode start would leave, without
+ * changing the handle.  src [R] int32: candidate r starts from the episode start (the reset snapshot, which travels with
+ * mtfjsp_gather) of env src[r]; actions [R,T,2] int32 (op, machine), contiguous per candidate; 1 <= T <= N.  All on the
+ * device.  Outputs, any of which may be NULL: cost4 [R,4] f64 receives what mtfjsp_costs would return after the T
+ * actions; return5 [R,5] f64 the step-order FP64 sum, from 0.0, of the reward5 every step would write; first_invalid [R]
+ * int32 -1 if every action was valid, else the index of the first invalid one (an invalid action is a no-op, as in
+ * mtfjsp_step, and the replay goes on).  The bits equal those of a fresh copy of env src[r] taken at its episode start
+ * and stepped T times by mtfjsp_step, then read by mtfjsp_costs.  Rewards use the mtfjsp_set_params values; the reward
+ * scaler takes no part.  A src[r] outside [0, B) is data: that candidate gets -2 in first_invalid and zero rows in
+ * cost4 / return5, and the others are unaffected.
+ * Read-only: nothing of the handle is written.  A non-step call: a recorded reset (mtfjsp_reset) is performed first, and
+ * the next step waits for the replay in full.
+ * MTFJSP_E_ARG, nothing written: a NULL handle, src or actions, R < 1, T < 1 or T > N.  MTFJSP_E_STATE, nothing written:
+ * before the first mtfjsp_reset since mtfjsp_load. */
+int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, double* cost4, double* return5,
+                  int32_t* first_invalid, void* stream);
+
 /* Uniform random valid action from the env's current masks: a selectable job (under mask_mode), its candidate
  * op, and a feasible machine for it; counter-based, keyed by (seed, env_offset + env, ops scheduled so far).
  * Mirrors tester/pdrs.py Random_task / Random_m (:75-86, :139-156).  op, mach [B] int32 (-1 when done). */
