@@ -14,10 +14,11 @@ SRC_DIR = os.path.join(_HERE, "csrc")
 # MTFJSP_LIB: load another build of the same library (A/B runs of kernel variants on the GPU box); default in-tree .so
 LIB_PATH = os.environ.get("MTFJSP_LIB") or os.path.join(_HERE, "libmtfjsp_b200.so")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "mtfjsp.h")
-SOURCES = ["mtfjsp_env.cu", "mtfjsp_encoder.cu", "mtfjsp_gemm.cu"]
+SOURCES = ["mtfjsp_env.cu", "mtfjsp_encoder.cu", "mtfjsp_gemm.cu", "mtfjsp_pareto.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
-# the env kernels restate the reference's FP64 arithmetic operation by operation: no FMA contraction there
-EXTRA_FLAGS = {"mtfjsp_env.cu": ["-fmad=false"]}
+# the env kernels restate the reference's FP64 arithmetic operation by operation, and the hypervolume its numpy
+# specification: no FMA contraction there
+EXTRA_FLAGS = {"mtfjsp_env.cu": ["-fmad=false"], "mtfjsp_pareto.cu": ["-fmad=false"]}
 
 
 def _stale() -> bool:
@@ -110,6 +111,8 @@ SIGNATURES = {
     "mtfjsp_enc_gat_trunk_tf32_grouped": ([_VP] * 9 + [C.c_int64, _I, _VP], _I),
     "mtfjsp_gae4": ([_VP, _VP, _VP, _VP, _VP, _VP, _I, C.c_int64, C.c_float, C.c_float, _VP], _I),
     "mtfjsp_adv_normalize": ([_VP, _VP, C.c_double, _I, C.c_int64, _VP], _I),
+    "mtfjsp_pareto_filter": ([_VP, _VP, _I, C.c_int64, _VP, _VP], _I),
+    "mtfjsp_hypervolume3": ([_VP, _VP, _I, _VP, _VP, _VP], _I),
     "mtfjsp_launch_overlap_error": ([_VP], _I),
     "mtfjsp_launch_count": ([_VP], C.c_int64),
     "mtfjsp_bytes_per_step": ([_VP, _I], C.c_int64),

@@ -16,12 +16,17 @@ neighbour of the lowest FP64 objective w_mk*mk + w_ec*(pt + idle) + w_tt*tt if t
 incumbent's.  The search stops after `rounds` rounds or at the first round in which no instance moves: one host
 synchronisation per round.  The environment decides what a sequence costs, so a neighbour's objective is exactly what
 stepping it would give, left shift included.
+
+`pareto_local_search` walks the same neighbourhood without a weighted sum: it keeps an archive of mutually
+non-dominated schedules per instance over the three targets (pareto.py) and expands it until no member is left
+unexplored.
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
+from . import pareto
 from .env import BatchedMTFJSPEnv
 from .validate import _objective
 
@@ -104,7 +109,8 @@ def local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, r
     replay call.  With max_neighbours=None the result of an instance depends neither on max_candidates nor on the other
     instances of the batch.
     -> dict of numpy arrays: actions [N,S,2] int32, final4 [S,4], objective [S], history [rounds_run+1, S] (objective
-    after each round, the start first; never increasing), accepted [rounds_run, S] bool."""
+    after each round, the start first; never increasing), accepted [rounds_run, S] bool, and replays, the number of
+    sequences replayed (the start included)."""
     t = np.asarray(instances["t"])
     S, N, M = t.shape
     J, E = N // M, np.asarray(instances["edge"]).shape[1]
@@ -124,10 +130,12 @@ def local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, r
         raise ValueError("a starting sequence has an invalid action")
     obj = _objective(final4, weights)
     history, accepted = [obj], []
+    replays = S
     inst_ids = torch.arange(S, device=dev)
     for rnd in range(int(rounds)):
         moves = neighbour_moves(cur, t_dev, max_neighbours, seed, rnd)
         R = moves.shape[0]
+        replays += R
         f4 = torch.empty((R, 4), dtype=torch.float64, device=dev)
         bad = torch.zeros((), dtype=torch.bool, device=dev)
         for c0 in range(0, R, max_candidates):
@@ -157,4 +165,147 @@ def local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, r
     env.close()
     return {"actions": cur.cpu().numpy(), "final4": final4.cpu().numpy(), "objective": obj.cpu().numpy(),
             "history": torch.stack(history).cpu().numpy(),
-            "accepted": (torch.stack(accepted) if accepted else torch.zeros((0, S), dtype=torch.bool)).cpu().numpy()}
+            "accepted": (torch.stack(accepted) if accepted else torch.zeros((0, S), dtype=torch.bool)).cpu().numpy(),
+            "replays": replays}
+
+
+def _replay_all(env, R, seqs, src, max_candidates):
+    """final4 [R,4] of R sequences, each replayed from the episode start of env src[r] ([R] int32), at most
+    max_candidates per replay call; seqs(c0, c1) builds the [N, c1 - c0, 2] sequences of candidates c0 .. c1 - 1.
+    Also a device flag: some action was invalid."""
+    f4 = torch.empty((R, 4), dtype=torch.float64, device=env.device)
+    bad = torch.zeros((), dtype=torch.bool, device=env.device)
+    for c0 in range(0, R, max_candidates):
+        c1 = min(R, c0 + max_candidates)
+        f4[c0:c1], _, fi = env.replay(seqs(c0, c1), src[c0:c1])
+        bad |= (fi != -1).any()
+    return f4, bad
+
+
+def _merge(count, arch_f4, new_inst, new_f4, cap):
+    """One archive-first merge.  The archive (arch_f4 [S,A,4], the first count[s] slots of row s valid) in archive order,
+    then the new points (new_f4 [R,4] of instances new_inst [R], grouped by instance in candidate order), per instance;
+    filtered by mtfjsp_pareto_filter, fronts of more than `cap` points cut by crowding distance.
+    -> survivors in merged order as (is_new, index: archive flat index s * A + a or new candidate index, instance, slot),
+       their count [S] and truncated [S] bool."""
+    S, A = arch_f4.shape[0], arch_f4.shape[1]
+    dev = arch_f4.device
+    oi, oa = (torch.arange(A, device=dev)[None, :] < count[:, None]).nonzero(as_tuple=True)
+    inst = torch.cat((oi, new_inst))
+    is_new = torch.cat((torch.zeros_like(oi, dtype=torch.bool), torch.ones_like(new_inst, dtype=torch.bool)))
+    idx = torch.cat((oi * A + oa, torch.arange(new_inst.shape[0], device=dev)))
+    order = torch.sort(inst * 2 + is_new.long(), stable=True)[1]            # instance; the archive first; list order
+    inst, is_new, idx = inst[order], is_new[order], idx[order]
+    obj = pareto.objectives(torch.cat((arch_f4.view(S * A, 4)[oi * A + oa], new_f4))[order])
+    cnt = torch.bincount(inst, minlength=S)
+    seg = torch.cat((torch.zeros(1, dtype=torch.int64, device=dev), torch.cumsum(cnt, 0)))
+    keep = pareto.pareto_filter(obj, seg, max_len=inst.shape[0])
+    inst, is_new, idx, obj = inst[keep], is_new[keep], idx[keep], obj[keep]
+    truncated = torch.bincount(inst, minlength=S) > cap
+    cut = pareto.crowding_truncate(obj, inst, S, cap)
+    inst, is_new, idx = inst[cut], is_new[cut], idx[cut]
+    count = torch.bincount(inst, minlength=S)
+    slot = torch.arange(inst.shape[0], device=dev) - (torch.cumsum(count, 0) - count)[inst]
+    return is_new, idx, inst, slot, count, truncated
+
+
+def pareto_local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, rounds=200, expand=8,
+                        max_archive=256, max_neighbours=None, seed=0, max_candidates=65536, device=None):
+    """Pareto local search over the three targets (mk, ec = pt + idle, tt; pareto.objectives) from the start sequences
+    `actions` ([N,S,2] or [N,K,S,2] integers, numpy or torch: complete valid schedules of the instances
+    {"t","p","transT","edge"} [S,...]).
+
+    Each instance keeps an archive of mutually non-dominated schedules, at most `max_archive` (<= 4,096) of them.  The
+    start set is filtered into it in k order.  Each round, per instance, the first `expand` unexplored members in archive
+    order are marked explored, and their neighbourhoods (neighbour_moves with each member as one column; max_neighbours
+    samples as there) are replayed from the instance's episode start, at most `max_candidates` per replay call.  The
+    archive in archive order, then the neighbours in (member, move) order, go through mtfjsp_pareto_filter, which keeps
+    the first of equal cost vectors: an archive member beats a neighbour of the same costs.  New survivors start
+    unexplored.  A front of more than max_archive points keeps the max_archive of the largest crowding distance
+    (pareto.crowding_truncate); survivors keep their merged order.  The search stops when no instance has an unexplored
+    member, or after `rounds` rounds: one host synchronisation per round.  `weights` are the env's reward weights; they
+    do not change the costs.  With max_neighbours=None the result of an instance depends neither on max_candidates nor
+    on the other instances of the batch.
+    -> dict of numpy arrays, A = max_archive: actions [N,S,A,2] int32 (-1 past count), final4 [S,A,4] and objectives
+       [S,A,3] (NaN past count), count [S], explored [S,A] bool, ref [S,3] (1.1 x the componentwise max of the start
+       set's objectives, 1.0 where that max is 0), hypervolume [rounds_run+1, S] (the archive's in ref, the start first),
+       truncated [rounds_run, S] bool, and replays, the number of candidates replayed (the start set included)."""
+    t = np.asarray(instances["t"])
+    S, N, M = t.shape
+    J, E = N // M, np.asarray(instances["edge"]).shape[1]
+    A = int(max_archive)
+    if max_candidates < 1 or expand < 1 or not 1 <= A <= pareto.HV_MAX_POINTS:
+        raise ValueError("max_candidates and expand must be >= 1, and 1 <= max_archive <= %d" % pareto.HV_MAX_POINTS)
+    env = BatchedMTFJSPEnv(S, J, M, E, left_shift=left_shift, weights=weights, device=device, obs_dtype=torch.float32)
+    dev = env.device
+    env.load(*(np.asarray(instances[k]) for k in ("t", "p", "transT", "edge")))
+    env.scaler_init()
+    env.reset(np.tile(np.asarray(weights, dtype=np.float64), (S, 1)))
+    start = torch.as_tensor(np.asarray(actions) if not torch.is_tensor(actions) else actions).to(dev, torch.int32)
+    if start.dim() == 3:
+        start = start[:, None]
+    if start.dim() != 4 or (start.shape[0], start.shape[2], start.shape[3]) != (N, S, 2):
+        raise ValueError("actions must have shape [%d, %d, 2] or [%d, K, %d, 2]" % (N, S, N, S))
+    K = start.shape[1]
+    start = start.transpose(1, 2).reshape(N, S * K, 2)                       # column s * K + k
+    s_inst = torch.arange(S, device=dev).repeat_interleave(K)
+    f4, bad = _replay_all(env, S * K, lambda a, b: start[:, a:b], s_inst.to(torch.int32), max_candidates)
+    if bool(bad):
+        raise ValueError("a starting sequence has an invalid action")
+    replays = S * K
+    ref = torch.as_tensor(pareto.reference_point(pareto.objectives(f4).view(S, K, 3).transpose(0, 1).cpu().numpy()),
+                          device=dev)
+    t_dev = torch.as_tensor(t, device=dev)
+    arch_act = torch.full((N, S, A, 2), -1, dtype=torch.int32, device=dev)
+    arch_f4 = torch.full((S, A, 4), float("nan"), dtype=torch.float64, device=dev)
+    explored = torch.zeros((S, A), dtype=torch.bool, device=dev)
+    count = torch.zeros((S,), dtype=torch.int64, device=dev)
+    seg_a = torch.arange(S + 1, dtype=torch.int64, device=dev) * A
+
+    def merge(new_inst, new_f4, new_seqs):
+        nonlocal arch_act, arch_f4, explored, count
+        is_new, idx, inst, slot, count, trunc = _merge(count, arch_f4, new_inst, new_f4, A)
+        act2 = torch.full_like(arch_act, -1)
+        f42 = torch.full_like(arch_f4, float("nan"))
+        exp2 = torch.zeros_like(explored)
+        o, n = ~is_new, is_new
+        act2[:, inst[o], slot[o]] = arch_act.view(N, S * A, 2)[:, idx[o]]
+        f42[inst[o], slot[o]] = arch_f4.view(S * A, 4)[idx[o]]
+        exp2[inst[o], slot[o]] = explored.view(S * A)[idx[o]]
+        act2[:, inst[n], slot[n]] = new_seqs(idx[n])
+        f42[inst[n], slot[n]] = new_f4[idx[n]]
+        arch_act, arch_f4, explored = act2, f42, exp2
+        return trunc
+
+    def archive_hv():
+        return pareto.hypervolume(pareto.objectives(arch_f4).view(S * A, 3), seg_a, ref)
+
+    merge(s_inst, f4, lambda i: start[:, i])
+    history, truncated = [archive_hv()], []
+    for rnd in range(int(rounds)):
+        valid = torch.arange(A, device=dev)[None, :] < count[:, None]
+        open_ = valid & ~explored
+        pick = open_ & (torch.cumsum(open_.long(), 1) <= expand)             # the first `expand` unexplored members
+        ms, ma = pick.nonzero(as_tuple=True)                                 # members in (instance, archive) order
+        explored = explored | pick
+        members = arch_act[:, ms, ma]                                        # [N,Msel,2], one member per column
+        moves = neighbour_moves(members, t_dev[ms], max_neighbours, seed, rnd)
+        nb_inst = ms[moves[:, 0]]
+        f4n, badn = _replay_all(env, moves.shape[0], lambda a, b: apply_moves(members, moves[a:b]),
+                                nb_inst.to(torch.int32), max_candidates)
+        replays += int(moves.shape[0])
+        truncated.append(merge(nb_inst, f4n, lambda i: apply_moves(members, moves[i])))
+        history.append(archive_hv())
+        valid = torch.arange(A, device=dev)[None, :] < count[:, None]
+        flags = torch.stack(((valid & ~explored).any(), badn)).cpu()
+        if bool(flags[1]):
+            raise RuntimeError("a neighbour replayed with an invalid action")
+        if not bool(flags[0]):
+            break
+    env.close()
+    return {"actions": arch_act.cpu().numpy(), "final4": arch_f4.cpu().numpy(),
+            "objectives": pareto.objectives(arch_f4).cpu().numpy(), "count": count.cpu().numpy(),
+            "explored": explored.cpu().numpy(), "ref": ref.cpu().numpy(),
+            "hypervolume": torch.stack(history).cpu().numpy(),
+            "truncated": (torch.stack(truncated) if truncated else torch.zeros((0, S), dtype=torch.bool)).cpu().numpy(),
+            "replays": replays}

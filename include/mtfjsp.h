@@ -416,6 +416,27 @@ int mtfjsp_gae4(const float* r, const float* v, const float* v_next, const float
 /* adv <- (adv - mean) / (std + 1e-5) per stream over `count` values (unbiased std), ppo_algorithm.py:485, 532. */
 int mtfjsp_adv_normalize(float* adv, const double* stats, double count, int T, int64_t B, void* stream);
 
+/* Pareto fronts over the three targets (pareto.py).  Handle-free, asynchronous on `stream`, no env state.
+ * obj3 [P,3] f64 row-major points; seg [S+1] int64 CSR offsets (seg[0] = 0, non-decreasing): segment s is the point
+ * range [seg[s], seg[s+1]), one instance's set.  All on the device.
+ *
+ * mtfjsp_pareto_filter: keep[p] = 1 iff point p of segment s is finite, no finite q of segment s dominates it (q <= p in
+ * every component and q < p in one), and no finite q < p of segment s equals it in all three components (of duplicates
+ * the first is kept); else 0.  Non-finite points get 0 and dominate nothing.  Pure comparisons: exact bits.  max_len
+ * only sizes the grid (the kernel strides over longer segments); empty segments are allowed.  keep is written for the
+ * points of every segment and nowhere else.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer, S < 0 or max_len < 0. */
+int mtfjsp_pareto_filter(const double* obj3, const int64_t* seg, int S, int64_t max_len, uint8_t* keep, void* stream);
+/* mtfjsp_hypervolume3: hv[s] = the exact hypervolume of segment s's points normalised by ref3[s] ([S,3] f64):
+ * u_d = v_d / ref_d; only finite points with every u_d < 1 take part (they need not be non-dominated).  Participants
+ * are ordered by u_z ascending (ties: index); slice i's area A_i is the 2-D area of the participants of z-rank <= i,
+ * visited by u_x ascending (ties: u_y, then index), carrying m = min(m, u_y) from m = 1.0 and adding
+ * (x_next - x_k) * (1.0 - m_k) to a sum from 0.0, x_next = 1.0 after the last.  hv = sum over i in slice order, from 0.0,
+ * of A_i * (z_{i+1} - z_i), z_n = 1.0; an empty set gives 0.0.  One block per segment.  NaN for a segment of more than
+ * 4096 points or a ref3 row not finite and > 0 in every component.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer or S < 0. */
+int mtfjsp_hypervolume3(const double* obj3, const int64_t* seg, int S, const double* ref3, double* hv, void* stream);
+
 /* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
  * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
  * word: it reflects the launches the device has finished so far (read it after synchronising). */
