@@ -252,6 +252,41 @@ struct EnvSmem {
     }
 };
 
+// The transition's pieces on raw views of the records, shared by the generic step (env_transition, env_estimates,
+// env_reward: env_kernel, replay_kernel) and the one-step lookahead (peek_kernel), whose shared-memory layout differs.
+
+// term g of the flat-order idle-time sum (DGenv_func.py:144-170): the gap in front of op ord[g] on its machine
+__device__ __forceinline__ double idle_term(const double* st, const double* ft, const int16_t* ord, const int16_t* rpred,
+                                            int g) {
+    const int v = ord[g], rp = rpred[v];
+    return (rp < 0) ? (st[v] - 0.0) : (st[v] - ft[rp]);
+}
+
+// op v's term of the energy estimate (SS:896): scheduled ? duration * energy rate : minimum energy
+__device__ __forceinline__ double energy_est(const int16_t* mach, const double* dur, const double* psel,
+                                             const double* minpt, int v) {
+    return (mach[v] >= 0) ? dur[v] * psel[v] : minpt[v];
+}
+
+// step reward of a valid transition (wrk_reward_function, SS:1066-1132) from the previous-step scalars scal = (mk_prev,
+// e_prev, trans_prev, idle_prev) and the step's makespan estimate mkv, energy estimate env, transport and idle sums:
+// (total before the divisor, r_mk, r_idle, r_pt, r_tt)
+struct StepReward {
+    double total, r_t, r_idle, r_pt, r_tt;
+};
+__device__ __forceinline__ StepReward reward_terms(const double* scal, const double* cfgw, int N, double mkv, double env,
+                                                   double trans, double idle) {
+    const double mk_prev = scal[0], e_prev = scal[1], trans_prev = scal[2], idle_prev = scal[3];
+    StepReward w;
+    w.r_t = 1.0 * mk_prev - mkv;
+    double r_pt = 1.0 * e_prev - env;
+    w.r_pt = r_pt / (double)N;
+    w.r_tt = 1.0 * trans_prev - trans;
+    w.r_idle = 1.0 * idle_prev - idle;
+    w.total = cfgw[0] * w.r_t + cfgw[1] * (w.r_pt + 1.0 * w.r_idle) + cfgw[2] * w.r_tt * 1.0;
+    return w;
+}
+
 // what one transition leaves for the step's reward epilogue and incremental observation
 struct StepOut {
     bool valid, done;
@@ -380,11 +415,7 @@ __device__ __forceinline__ StepOut env_transition(const Layout& L, const EnvSmem
         const int nsched = nsched0 + 1;
         o.done = (nsched == N);
         // ---- idle time: sequential sum in (machine, route) order = flat order, DGenv_func.py:144-170 ----
-        for (int g = lane; g < nsched; g += 32) {
-            const int v = S.ord[g], rp = S.rpred[v];
-            const double term = (rp < 0) ? (S.st[v] - 0.0) : (S.st[v] - S.ft[rp]);
-            S.pt[g] = term * 1.0;
-        }
+        for (int g = lane; g < nsched; g += 32) S.pt[g] = idle_term(S.st, S.ft, S.ord, S.rpred, g) * 1.0;
         __syncwarp();
         double idle = 0.0;
         if (L.nich) {  // large instances: running sum in front of every 32nd term (the specialised kernel restarts there)
@@ -432,7 +463,7 @@ __device__ __forceinline__ void env_estimates(const Layout& L, const PwPlan& pw,
     __syncwarp();
     double mx = -INFINITY;
     for (int v = lane; v < N; v += 32) {
-        S.pt[v] = (S.mach[v] >= 0) ? S.dur[v] * S.psel[v] : S.minpt[v];
+        S.pt[v] = energy_est(S.mach, S.dur, S.psel, S.minpt, v);
         mx = fmax(mx, S.ft[v]);
     }
     __syncwarp();
@@ -442,22 +473,13 @@ __device__ __forceinline__ void env_estimates(const Layout& L, const PwPlan& pw,
     }
 }
 
-// step reward of a valid transition (wrk_reward_function, SS:1066-1132): (total before the divisor, r_mk, r_idle, r_pt,
-// r_tt); lane 0 then advances the machine accumulators (SS:2323-2338) and the previous-step scalars (SS:932-936)
-struct StepReward {
-    double total, r_t, r_idle, r_pt, r_tt;
-};
+// step reward of a valid transition (reward_terms); lane 0 then advances the machine accumulators (SS:2323-2338) and the
+// previous-step scalars (SS:932-936)
 __device__ __forceinline__ StepReward env_reward(const Layout& L, const EnvSmem& S, const double* cfgw, int m, double mkv,
                                                  double env, const StepOut& o, int lane) {
     const int N = L.N;
-    const double mk_prev = S.scal[0], e_prev = S.scal[1], trans_prev = S.scal[2], idle_prev = S.scal[3];
-    StepReward w;
-    w.r_t = 1.0 * mk_prev - mkv;
-    double r_pt = 1.0 * e_prev - env;
-    w.r_pt = r_pt / (double)N;
-    w.r_tt = 1.0 * trans_prev - o.trans;
-    w.r_idle = 1.0 * idle_prev - o.idle;
-    w.total = cfgw[0] * w.r_t + cfgw[1] * (w.r_pt + 1.0 * w.r_idle) + cfgw[2] * w.r_tt * 1.0;
+    const StepReward w = reward_terms(S.scal, cfgw, N, mkv, env, o.trans, o.idle);
+    const double idle_prev = S.scal[3];  // read after reward_terms: the scalar loads keep their order in the SASS
     __syncwarp();
     if (lane == 0) {
         S.macc[m * 3 + 0] += o.ec / (double)N;
@@ -2327,6 +2349,10 @@ size_t gather_env_bytes(const Layout& L) {
 //              combined by the plan's postfix program;
 //   idle time  the flat-order sequential sum: the unchanged prefix in front of a's slot (prefix sums computed once per
 //              block), a's term, its route follower's term against a's new finish, then the unchanged rest.
+// The idle term (idle_term), the per-op energy estimate (energy_est) and the reward (reward_terms) are the step's own
+// device code.  The validity test, the placement scan, the leaf pass and the postfix fold stay restated here: shared
+// with env_transition / pairwise_sum, each of them changed the SASS of the generic step and replay kernels and made the
+// replay slower at J6M6 and J10M10.
 struct PeekArgs {
     Layout L;
     PwPlan pw;
@@ -2425,7 +2451,7 @@ __global__ void __launch_bounds__(128) peek_kernel(const __grid_constant__ PeekA
     const double* s_minpt = s_xs + L.o_minpt;
     const double* s_tt = s_xs + L.o_tt;
     // the env's per-op energy estimate (env_kernel's s_pt)
-    const auto est = [&](int v) { return (s_mach[v] >= 0) ? s_dur[v] * s_psel[v] : s_minpt[v]; };
+    const auto est = [&](int v) { return energy_est(s_mach, s_dur, s_psel, s_minpt, v); };
     if (warp == 0) {  // base leaf results, four leaves at a time as pairwise_sum
         for (int L0 = 0; L0 < pw.nleaves; L0 += 4) {
             const int Lx = L0 + (lane >> 3);
@@ -2443,9 +2469,7 @@ __global__ void __launch_bounds__(128) peek_kernel(const __grid_constant__ PeekA
         double idle = 0.0;
         for (int g = 0; g < nsched0; g++) {
             s_pre[g] = idle;
-            const int v = s_ord[g], rp = s_rpred[v];
-            const double term = (rp < 0) ? (s_st[v] - 0.0) : (s_st[v] - s_ft[rp]);
-            idle = idle + term * 1.0;
+            idle = idle + idle_term(s_st, s_ft, s_ord, s_rpred, g) * 1.0;
         }
         s_pre[nsched0] = idle;
     }
@@ -2577,21 +2601,11 @@ __global__ void __launch_bounds__(128) peek_kernel(const __grid_constant__ PeekA
                 idle = idle + (s_st[next] - ft) * 1.0;
                 g++;
             }
-            for (; g < nsched0; g++) {
-                const int v = s_ord[g], rp = s_rpred[v];
-                const double term = (rp < 0) ? (s_st[v] - 0.0) : (s_st[v] - s_ft[rp]);
-                idle = idle + term * 1.0;
-            }
-            const double mk_prev = s_scal[0], e_prev = s_scal[1], trans_prev = s_scal[2], idle_prev = s_scal[3];
-            const double r_t = 1.0 * mk_prev - r[2];
-            double r_pt = 1.0 * e_prev - r[3];
-            r_pt = r_pt / (double)N;
-            const double r_tt = 1.0 * trans_prev - r[4];
-            const double r_idle = 1.0 * idle_prev - idle;
-            const double total = A.cfgw[0] * r_t + A.cfgw[1] * (r_pt + 1.0 * r_idle) + A.cfgw[2] * r_tt * 1.0;
+            for (; g < nsched0; g++) idle = idle + idle_term(s_st, s_ft, s_ord, s_rpred, g) * 1.0;
+            const StepReward w = reward_terms(s_scal, A.cfgw, N, r[2], r[3], r[4], idle);
             if (A.reward5) {
                 double* r5 = A.reward5 + o * 5;
-                r5[0] = total / A.divisor; r5[1] = r_t; r5[2] = r_idle; r5[3] = r_pt; r5[4] = r_tt;
+                r5[0] = w.total / A.divisor; r5[1] = w.r_t; r5[2] = w.r_idle; r5[3] = w.r_pt; r5[4] = w.r_tt;
             }
             if (A.invalid) A.invalid[o] = 0;
         }
@@ -2610,7 +2624,8 @@ size_t peek_env_bytes(const Layout& L, int K) {
 // (the reset snapshot sd0 / si0) and leaves the costs, the summed rewards and the index of its first invalid action.
 // One warp per candidate, in env_kernel's lane layout and shared-memory slice (Layout::sm_*), so every size the handle
 // accepts fits: the warp stages the snapshot records and the static doubles once, then runs every transition on that
-// copy with env_kernel's own device code (env_transition, env_estimates, env_reward) and writes 4 + 5 doubles and an int.
+// copy with env_kernel's own device code (env_transition, env_estimates, env_reward; peek_kernel shares their idle_term,
+// energy_est and reward_terms) and writes 4 + 5 doubles and an int.
 // The actions are read 32 at a time, one (op, machine) pair per lane in one coalesced 256-byte read, and broadcast by
 // shuffle.  Nothing of the handle is written.
 struct ReplayArgs {
