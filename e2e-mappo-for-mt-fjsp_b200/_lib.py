@@ -9,6 +9,8 @@ import ctypes as C
 import os
 import subprocess
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 SRC_DIR = os.path.join(_HERE, "csrc")
 # MTFJSP_LIB: load another build of the same library (A/B runs of kernel variants on the GPU box); default in-tree .so
@@ -139,6 +141,16 @@ def lib():
             fn.argtypes = argtypes
             fn.restype = restype
     return _lib
+
+
+def _ptr(t):
+    """A tensor's address for the C ABI; None passes NULL (optional operands; the library rejects a missing one)."""
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def _stream():
+    """The current torch stream of the current device, as the library's `void* stream`."""
+    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
 class MTFJSPError(RuntimeError):

@@ -8,21 +8,12 @@ algorithm/ppo_algorithm.py:438-536; advantage normalisation uses sums that are a
 runs normalise over the same [steps, B_total] block a single GPU would (SURVEY.md 8e)."""
 from __future__ import annotations
 
-import ctypes as C
 
 import torch
 import torch.distributed as dist
 
 from . import _lib
-from ._lib import check
-
-
-def _ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+from ._lib import _ptr, _stream, check
 
 
 def gae4(r, v, v_next, done, gamma=0.99, lam=0.98, normalize=True):

@@ -15,7 +15,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include "../../include/mtfjsp.h"
+#include "mtfjsp_launch.cuh"
 
 namespace {
 
@@ -468,11 +468,23 @@ __global__ void __launch_bounds__(256) select_kernel(const float* __restrict__ s
     }
 }
 
-// Operand alignment, checked on the host before any launch: the kernels read and write 16 bytes (float4) or 8 bytes
-// (float2: adj_w) at a time.  NULL passes (optional pointers are checked for presence separately).
-template <class... P>
-bool al16(P... p) { return ((((uintptr_t)p & 15) == 0) && ...); }
-bool al8(const void* p) { return ((uintptr_t)p & 7) == 0; }
+// Calls launch(b0, total, c4_shift) for consecutive runs of whole envs: b0 is a run's first env, total = its envs * N * C4
+// threads < 2^31, so that a launch indexes in 32 bits and the machine-predecessor gather stays inside an env.
+// c4_shift = log2(C4), or -1 when C4 is not a power of two.
+template <class F>
+int for_env_chunks(const char* what, int64_t B, int N, int C4, F launch) {
+    int c4_shift = -1;
+    for (int k = 0; k < 16; k++)
+        if ((1 << k) == C4) c4_shift = k;
+    const long long per_env = (long long)N * C4;
+    const long long chunk = (long long)0x7fffff00 / per_env;
+    if (chunk < 1) return fail(MTFJSP_E_ARG, what);
+    for (long long b0 = 0; b0 < B; b0 += chunk) {
+        const long long nb = B - b0 < chunk ? B - b0 : chunk;
+        launch(b0, (unsigned)(nb * per_env), c4_shift);
+    }
+    return launched(what);
+}
 
 }  // namespace
 
@@ -481,172 +493,156 @@ extern "C" {
 int mtfjsp_enc_select(const float* scores, const uint8_t* mask, const int32_t* cand, float scale, int R, int64_t B, int greedy,
                       uint64_t seed, const int64_t* counter, int stream_id, float* prob, int64_t* action, float* log_a,
                       int64_t* task, void* stream) {
-    if (!scores || !mask || !prob || !action || !log_a || R < 1 || R > 32 || B < 1 || (!greedy && !counter)) return MTFJSP_E_ARG;
+    if (!scores || !mask || !prob || !action || !log_a || R < 1 || R > 32 || B < 1 || (!greedy && !counter))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_select: bad argument");
     select_kernel<<<(unsigned)((B + 7) / 8), 256, 0, (cudaStream_t)stream>>>(scores, mask, cand, scale, R, B, greedy, seed, counter,
                                                                            stream_id, prob, action, log_a, task);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_gae4(const float* r, const float* v, const float* v_next, const float* done, float* adv, double* stats, int T,
                 int64_t B, float gamma, float lam, void* stream) {
-    if (!r || !v || !v_next || !done || !adv || T < 1 || B < 1) return MTFJSP_E_ARG;
+    if (!r || !v || !v_next || !done || !adv || T < 1 || B < 1) return fail(MTFJSP_E_ARG, "mtfjsp_gae4: bad argument");
     const long long n = (long long)B * 4;
     gae4_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(r, v, v_next, done, adv, stats, T, B, gamma, lam);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_adv_normalize(float* adv, const double* stats, double count, int T, int64_t B, void* stream) {
-    if (!adv || !stats || count < 2 || T < 1 || B < 1) return MTFJSP_E_ARG;
+    if (!adv || !stats || count < 2 || T < 1 || B < 1) return fail(MTFJSP_E_ARG, "mtfjsp_adv_normalize: bad argument");
     const long long total = (long long)T * B * 4;
     adv_normalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(adv, stats, count, total);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 
 int mtfjsp_enc_aggregate(const float* h, const float* adj_w, const int16_t* adj_src, float* out, int64_t B, int N,
                          int C, const float* in_scale, const float* in_shift, int in_relu, void* stream) {
-    if (!h || !adj_w || !adj_src || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return MTFJSP_E_ARG;
+    if (!h || !adj_w || !adj_src || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate: in_scale and in_shift go together");
+    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate: misaligned operand");
     const int C4 = C / 4;
-    int c4_shift = -1;
-    for (int k = 0; k < 16; k++)
-        if ((1 << k) == C4) c4_shift = k;
-    // 32-bit indexing inside a launch; whole envs per launch (the machine-predecessor gather stays inside an env)
-    const long long per_env = (long long)N * C4;
-    const long long chunk = (long long)0x7fffff00 / per_env;
-    if (chunk < 1) return MTFJSP_E_ARG;
-    for (long long b0 = 0; b0 < B; b0 += chunk) {
-        const long long nb = B - b0 < chunk ? B - b0 : chunk;
-        const unsigned total = (unsigned)(nb * per_env);
+    return for_env_chunks(__func__, B, N, C4, [&](long long b0, unsigned total, int c4_shift) {
         const long long r0 = b0 * N;
         aggregate_kernel<false><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
             reinterpret_cast<const float4*>(h) + r0 * C4, reinterpret_cast<const float2*>(adj_w) + r0, adj_src + r0,
             reinterpret_cast<float4*>(out) + r0 * C4, total, N, C4, c4_shift, reinterpret_cast<const float4*>(in_scale),
             reinterpret_cast<const float4*>(in_shift), in_relu);
-    }
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    });
 }
 
 int mtfjsp_enc_ell_invert(const int16_t* adj_src, int16_t* adj_dst, int64_t B, int N, void* stream) {
-    if (!adj_src || !adj_dst || B < 1 || N < 1 || (long long)B * N > 0x7fffff00LL) return MTFJSP_E_ARG;
+    if (!adj_src || !adj_dst || B < 1 || N < 1 || (long long)B * N > 0x7fffff00LL)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_ell_invert: bad argument");
     const unsigned rows = (unsigned)(B * N);
-    if (cudaMemsetAsync(adj_dst, 0xff, (size_t)rows * 2, (cudaStream_t)stream) != cudaSuccess) return MTFJSP_E_CUDA;
+    CK(cudaMemsetAsync(adj_dst, 0xff, (size_t)rows * 2, (cudaStream_t)stream), __func__);
     ell_invert_kernel<<<(rows + 255) / 256, 256, 0, (cudaStream_t)stream>>>(adj_src, adj_dst, rows, N);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_aggregate_bwd(const float* g, const float* adj_w, const int16_t* adj_src, const int16_t* adj_dst, float* out,
                              int64_t B, int N, int C, void* stream) {
-    if (!g || !adj_w || !adj_src || !adj_dst || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
-    if (!al16(g, out) || !al8(adj_w)) return MTFJSP_E_ARG;
+    if (!g || !adj_w || !adj_src || !adj_dst || !out || B < 1 || N < 1 || C < 4 || (C % 4) != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_bwd: bad argument");
+    if (!al16(g, out) || !al8(adj_w)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_bwd: misaligned operand");
     const int C4 = C / 4;
-    int c4_shift = -1;
-    for (int k = 0; k < 16; k++)
-        if ((1 << k) == C4) c4_shift = k;
-    const long long per_env = (long long)N * C4;
-    const long long chunk = (long long)0x7fffff00 / per_env;
-    if (chunk < 1) return MTFJSP_E_ARG;
-    for (long long b0 = 0; b0 < B; b0 += chunk) {
-        const long long nb = B - b0 < chunk ? B - b0 : chunk;
-        const unsigned total = (unsigned)(nb * per_env);
+    return for_env_chunks(__func__, B, N, C4, [&](long long b0, unsigned total, int c4_shift) {
         const long long r0 = b0 * N;
         aggregate_bwd_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
             reinterpret_cast<const float4*>(g) + r0 * C4, reinterpret_cast<const float2*>(adj_w) + r0, adj_src + r0,
             adj_dst + r0, reinterpret_cast<float4*>(out) + r0 * C4, total, N, C4, c4_shift);
-    }
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    });
 }
 
 static bool bn_args_ok(int64_t G, int64_t R, int C) { return G >= 1 && G <= 65535 && R >= 1 && C >= 4 && C <= 1024 && (C % 4) == 0; }
 
 int mtfjsp_enc_bn_fwd(const float* x, const float* w, const float* b, float eps, int64_t G, int64_t R, int C, int relu, float* y,
                       float* mean, float* rstd, double* workspace, void* stream) {
-    if (!x || !w || !b || !y || !mean || !rstd || !workspace || !bn_args_ok(G, R, C)) return MTFJSP_E_ARG;
-    if (!al16(x, w, b, y, mean, rstd) || !al8(workspace)) return MTFJSP_E_ARG;
+    if (!x || !w || !b || !y || !mean || !rstd || !workspace || !bn_args_ok(G, R, C))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_fwd: bad argument");
+    if (!al16(x, w, b, y, mean, rstd) || !al8(workspace)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_fwd: misaligned operand");
     cudaStream_t s = (cudaStream_t)stream;
     const int C4 = C / 4, ny = 256 / C4 > 0 ? 256 / C4 : 1;
     const int threads = C4 * ny > 256 ? C4 : 256;
     const dim3 grid((unsigned)((R + BN_ROWS - 1) / BN_ROWS), (unsigned)G);
     const size_t smem = (size_t)2 * (threads / C4) * C * sizeof(double);
-    if (cudaMemsetAsync(workspace, 0, (size_t)G * 2 * C * sizeof(double), s) != cudaSuccess) return MTFJSP_E_CUDA;
+    CK(cudaMemsetAsync(workspace, 0, (size_t)G * 2 * C * sizeof(double), s), __func__);
     bn_reduce_kernel<0><<<grid, threads, smem, s>>>(reinterpret_cast<const float4*>(x), nullptr, w, b, nullptr, nullptr, workspace,
                                                     R, C4, 0);
     bn_stats_finalize_kernel<<<(unsigned)((G * C + 255) / 256), 256, 0, s>>>(workspace, x, R, 1.0 / (double)R, eps, mean, rstd,
                                                                           (int)G, C);
     bn_apply_kernel<0><<<grid, threads, 0, s>>>(reinterpret_cast<const float4*>(x), nullptr, w, b, mean, rstd, nullptr,
                                                 reinterpret_cast<float4*>(y), R, C4, relu, 0.f);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_bn_bwd(const float* x, const float* gy, const float* w, const float* b, const float* mean, const float* rstd,
                       int64_t G, int64_t R, int C, int relu, float* dx, double* sums, void* stream) {
-    if (!x || !gy || !w || !b || !mean || !rstd || !dx || !sums || !bn_args_ok(G, R, C)) return MTFJSP_E_ARG;
-    if (!al16(x, gy, w, b, mean, rstd, dx) || !al8(sums)) return MTFJSP_E_ARG;
+    if (!x || !gy || !w || !b || !mean || !rstd || !dx || !sums || !bn_args_ok(G, R, C))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_bwd: bad argument");
+    if (!al16(x, gy, w, b, mean, rstd, dx) || !al8(sums)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_bwd: misaligned operand");
     cudaStream_t s = (cudaStream_t)stream;
     const int C4 = C / 4, ny = 256 / C4 > 0 ? 256 / C4 : 1;
     const int threads = C4 * ny > 256 ? C4 : 256;
     const dim3 grid((unsigned)((R + BN_ROWS - 1) / BN_ROWS), (unsigned)G);
     const size_t smem = (size_t)2 * (threads / C4) * C * sizeof(double);
-    if (cudaMemsetAsync(sums, 0, (size_t)G * 2 * C * sizeof(double), s) != cudaSuccess) return MTFJSP_E_CUDA;
+    CK(cudaMemsetAsync(sums, 0, (size_t)G * 2 * C * sizeof(double), s), __func__);
     bn_reduce_kernel<1><<<grid, threads, smem, s>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<const float4*>(gy), w, b, mean,
                                                     rstd, sums, R, C4, relu);
     bn_apply_kernel<1><<<grid, threads, 0, s>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<const float4*>(gy), w, b, mean,
                                                 rstd, sums, reinterpret_cast<float4*>(dx), R, C4, relu, 1.0f / (float)R);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_graph_mean(const float* h, float* out, int64_t B, int N, int C, const float* in_scale,
                           const float* in_shift, int in_relu, void* stream) {
-    if (!h || !out || B < 1 || N < 1 || C < 1) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
+    if (!h || !out || B < 1 || N < 1 || C < 1) return fail(MTFJSP_E_ARG, "mtfjsp_enc_graph_mean: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_graph_mean: in_scale and in_shift go together");
     graph_mean_kernel<false><<<(unsigned)B, C < 128 ? 32 * ((C + 31) / 32) : 128, 0, (cudaStream_t)stream>>>(h, out, N, C, in_scale,
                                                                                                    in_shift, in_relu);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_aggregate_grouped(const float* h, const float* adj_w, const int16_t* adj_src, float* out, int64_t B, int N, int C,
                                  const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, void* stream) {
-    if (!h || !adj_w || !adj_src || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 4 || (C % 4) != 0) return MTFJSP_E_ARG;
-    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
-    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return MTFJSP_E_ARG;
+    if (!h || !adj_w || !adj_src || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 4 || (C % 4) != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_grouped: bad argument");
+    if (envs_per_group < 1 || B % envs_per_group != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_grouped: envs_per_group must divide B");
+    if (!al16(h, out, in_scale, in_shift) || !al8(adj_w)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_grouped: misaligned operand");
     const int C4 = C / 4;
-    int c4_shift = -1;
-    for (int k = 0; k < 16; k++)
-        if ((1 << k) == C4) c4_shift = k;
-    const long long per_env = (long long)N * C4;
-    const long long chunk = (long long)0x7fffff00 / per_env;
-    if (chunk < 1) return MTFJSP_E_ARG;
-    for (long long b0 = 0; b0 < B; b0 += chunk) {
-        const long long nb = B - b0 < chunk ? B - b0 : chunk;
-        const unsigned total = (unsigned)(nb * per_env);
+    return for_env_chunks(__func__, B, N, C4, [&](long long b0, unsigned total, int c4_shift) {
         const long long r0 = b0 * N;
         aggregate_kernel<true><<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
             reinterpret_cast<const float4*>(h) + r0 * C4, reinterpret_cast<const float2*>(adj_w) + r0, adj_src + r0,
             reinterpret_cast<float4*>(out) + r0 * C4, total, N, C4, c4_shift, reinterpret_cast<const float4*>(in_scale),
             reinterpret_cast<const float4*>(in_shift), in_relu, b0, envs_per_group);
-    }
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    });
 }
 
 int mtfjsp_enc_graph_mean_grouped(const float* h, float* out, int64_t B, int N, int C, const float* in_scale, const float* in_shift,
                                   int in_relu, int envs_per_group, void* stream) {
-    if (!h || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 1) return MTFJSP_E_ARG;
-    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
+    if (!h || !out || !in_scale || !in_shift || B < 1 || N < 1 || C < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_graph_mean_grouped: bad argument");
+    if (envs_per_group < 1 || B % envs_per_group != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_graph_mean_grouped: envs_per_group must divide B");
     graph_mean_kernel<true><<<(unsigned)B, C < 128 ? 32 * ((C + 31) / 32) : 128, 0, (cudaStream_t)stream>>>(h, out, N, C, in_scale,
                                                                                                          in_shift, in_relu,
                                                                                                          envs_per_group);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_gat_attend(const float* t, const float* a_src, const float* a_dst, float* out, int64_t R, int mode,
                           void* stream) {
-    if (!t || !a_src || !a_dst || !out || R < 1 || mode < 0 || mode > 2) return MTFJSP_E_ARG;
-    if (!al16(t, a_src, a_dst, out)) return MTFJSP_E_ARG;
+    if (!t || !a_src || !a_dst || !out || R < 1 || mode < 0 || mode > 2) return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_attend: bad argument");
+    if (!al16(t, a_src, a_dst, out)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_attend: misaligned operand");
     gat_attend_kernel<<<(unsigned)((R + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4*>(t), reinterpret_cast<const float4*>(a_src), reinterpret_cast<const float4*>(a_dst),
         reinterpret_cast<float4*>(out), R, mode);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_gat_attend_bwd_blocks(int64_t R) {
@@ -656,12 +652,13 @@ int mtfjsp_enc_gat_attend_bwd_blocks(int64_t R) {
 
 int mtfjsp_enc_gat_attend_bwd(const float* t, const float* a_src, const float* a_dst, const float* g, float* dt, float* dparts,
                               int64_t R, int mode, void* stream) {
-    if (!t || !a_src || !a_dst || !g || !dt || !dparts || R < 1 || mode < 0 || mode > 2) return MTFJSP_E_ARG;
-    if (!al16(t, a_src, a_dst, g, dt, dparts)) return MTFJSP_E_ARG;
+    if (!t || !a_src || !a_dst || !g || !dt || !dparts || R < 1 || mode < 0 || mode > 2)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_attend_bwd: bad argument");
+    if (!al16(t, a_src, a_dst, g, dt, dparts)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_attend_bwd: misaligned operand");
     gat_attend_bwd_kernel<<<mtfjsp_enc_gat_attend_bwd_blocks(R), 256, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4*>(t), reinterpret_cast<const float4*>(a_src), reinterpret_cast<const float4*>(a_dst),
         reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(dt), dparts, R, mode);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 

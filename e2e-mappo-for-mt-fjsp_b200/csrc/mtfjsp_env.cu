@@ -41,7 +41,7 @@
 
 #include <new>
 
-#include "../../include/mtfjsp.h"
+#include "mtfjsp_launch.cuh"
 
 #define MAX_LEAVES 64
 #define MAX_PROG 128
@@ -2700,14 +2700,6 @@ __global__ void __launch_bounds__(256) replay_kernel(const __grid_constant__ Rep
     }
 }
 
-thread_local char g_err[512] = "";
-
-int fail(int code, const char* msg, cudaError_t e = cudaSuccess) {
-    if (e != cudaSuccess) snprintf(g_err, sizeof g_err, "%s: %s", msg, cudaGetErrorString(e));
-    else snprintf(g_err, sizeof g_err, "%s", msg);
-    return code;
-}
-
 int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
 void build_plan_rec(int off, int n, PwPlan& pw) {
@@ -2782,11 +2774,11 @@ struct mtfjsp_env {
     unsigned *ovl_err, *ovl_err_d;
 };
 
-#define CK(call, msg)                                            \
-    do {                                                         \
-        cudaError_t e_ = (call);                                 \
-        if (e_ != cudaSuccess) return fail(MTFJSP_E_CUDA, msg, e_); \
-    } while (0)
+// the tail of every launch on a handle: counts it (mtfjsp_launch_count), then reports a launch error
+static int counted(mtfjsp_env* h, const char* what) {
+    h->launches++;
+    return launched(what);
+}
 
 static Params make_params(mtfjsp_env* h) {
     Params P;
@@ -2806,16 +2798,14 @@ static int flush_reset(mtfjsp_env* h, cudaStream_t s) {
     if (h->pend_reset || h->pend_scaler) h->ovl_chain = false;
     if (h->pend_reset) {
         reset_copy_kernel<<<L.B, 128, 0, s>>>(L, h->sd0, h->si0, h->pend_w, h->sd, h->si, h->jm_fin, h->jm_esa, h->cand);
-        h->launches++;
         h->pend_reset = false;
-        CK(cudaGetLastError(), "reset_copy_kernel");
+        if (const int rc = counted(h, "reset_copy_kernel")) return rc;
     }
     if (h->pend_scaler) {
         const size_t n = (size_t)L.B * 4;
         scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(L, h->sd, 0);
-        h->launches++;
         h->pend_scaler = false;
-        CK(cudaGetLastError(), "scaler_kernel");
+        if (const int rc = counted(h, "scaler_kernel")) return rc;
     }
     return MTFJSP_OK;
 }
@@ -2836,20 +2826,11 @@ static int launch_env(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     int rc = flush_reset(h, s);
     if (rc != MTFJSP_OK) return rc;
     size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
-    static thread_local int configured_dev = -1;
-    static thread_local size_t configured_smem = 0;
-    if (configured_dev != h->device || configured_smem < smem) {
-        CK(cudaFuncSetAttribute(env_kernel<MODE, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-           "cudaFuncSetAttribute");
-        configured_dev = h->device;
-        configured_smem = smem;
-    }
+    CK(opt_in_smem(env_kernel<MODE, OutT>, smem), "cudaFuncSetAttribute");
     int blocks = (L.B + L.warps_per_block - 1) / L.warps_per_block;
     env_kernel<MODE, OutT><<<blocks, L.warps_per_block * 32, smem, s>>>(P);
-    h->launches++;
     h->ovl_chain = false;
-    CK(cudaGetLastError(), "env_kernel launch");
-    return MTFJSP_OK;
+    return counted(h, "env_kernel launch");
 }
 
 template <class S, int MODE, typename OutT>
@@ -2871,12 +2852,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
         if (rc != MTFJSP_OK) return rc;
     }
     const size_t smem = (size_t)S::WARPS * S::EPW * S::ENV_BYTES + (S::BAR_IN_PAD ? 0 : 16 * ((S::WARPS * 8 + 15) / 16));
-    static thread_local int configured_dev = -1;
-    if (configured_dev != h->device) {
-        CK(cudaFuncSetAttribute(env_kernel_s<S, MODE, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
-           "cudaFuncSetAttribute");
-        configured_dev = h->device;
-    }
+    CK(opt_in_smem(env_kernel_s<S, MODE, OutT>, smem), "cudaFuncSetAttribute");
     const int per_block = S::WARPS * S::EPW;
     const int blocks = (L.B + per_block - 1) / per_block;
     Params Q = P;
@@ -2930,8 +2906,7 @@ static int launch_spec(mtfjsp_env* h, const Params& P, cudaStream_t s) {
     }
     h->ovl_chain = false;
     CK(cudaLaunchKernelEx(&cfg, env_kernel_s<S, MODE, OutT>, Q), "env_kernel_s launch");
-    h->launches++;
-    CK(cudaGetLastError(), "env_kernel_s launch");
+    if (const int rc = counted(h, "env_kernel_s launch")) return rc;
     if (Q.ep) {  // only a launch that was issued releases its epoch
         h->ep = Q.ep;
         h->ovl_chain = true;
@@ -2999,9 +2974,8 @@ static int launch_prestep(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, con
             prestep_kernel<MM, float, POLICY><<<blocks, 128, 0, s>>>(L, h->t, h->p, h->xs, h->si, h->edge_id, jm,     \
                                                                     h->cand, seed, env_offset, op, mach, (float*)out, \
                                                                     mmask);                                          \
-        h->launches++;                                                                                               \
-        CK(cudaGetLastError(), "prestep_kernel");                                                                    \
-        return 1;                                                                                                    \
+        const int rc = counted(h, "prestep_kernel");                                                                 \
+        return rc == MTFJSP_OK ? 1 : rc;                                                                             \
     }
     PRESTEP(6)
     PRESTEP(10)
@@ -3213,8 +3187,7 @@ int mtfjsp_load(mtfjsp_env* h, const double* t, const double* p, const double* t
     CK(cudaMemcpyAsync(h->p, p, n, cudaMemcpyDeviceToDevice, s), "copy p");
     size_t total = (size_t)L.B * (size_t)(L.N > L.M * L.M ? L.N : L.M * L.M);
     load_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(L, h->t, h->p, tt, edge, W, h->xs, h->edge_id);
-    h->launches++;
-    CK(cudaGetLastError(), "load_kernel");
+    if (const int rc = counted(h, "load_kernel")) return rc;
     h->loaded = true;
     h->reset_done = false;
     h->obs_synced = false;
@@ -3228,9 +3201,7 @@ int mtfjsp_scaler_init(mtfjsp_env* h, void* stream) {
     if (rc) return rc;
     size_t n = (size_t)h->L.B * 13;
     scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, 1);
-    h->launches++;
-    CK(cudaGetLastError(), "scaler_kernel");
-    return MTFJSP_OK;
+    return counted(h, "scaler_kernel");
 }
 
 int mtfjsp_scaler_reset(mtfjsp_env* h, void* stream) {
@@ -3243,9 +3214,7 @@ int mtfjsp_scaler_reset(mtfjsp_env* h, void* stream) {
     if (rc) return rc;
     size_t n = (size_t)h->L.B * 4;
     scaler_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, 0);
-    h->launches++;
-    CK(cudaGetLastError(), "scaler_kernel");
-    return MTFJSP_OK;
+    return counted(h, "scaler_kernel");
 }
 
 int mtfjsp_reset(mtfjsp_env* h, const double* weights, void* stream) {
@@ -3336,9 +3305,7 @@ int mtfjsp_mfea1(mtfjsp_env* h, const int32_t* op, void* mfea1, uint8_t* mach_ma
         mfea1_kernel<float><<<blocks, 128, 0, s>>>(L, h->t, h->p, h->xs, h->si, h->edge_id, op, (float*)mfea1, mach_mask);
     else
         return fail(MTFJSP_E_ARG, "dtype must be MTFJSP_F32 or MTFJSP_F64");
-    h->launches++;
-    CK(cudaGetLastError(), "mfea1_kernel");
-    return MTFJSP_OK;
+    return counted(h, "mfea1_kernel");
 }
 
 int mtfjsp_dense_adj(mtfjsp_env* h, void* adj, int dtype, void* stream) {
@@ -3352,9 +3319,7 @@ int mtfjsp_dense_adj(mtfjsp_env* h, void* adj, int dtype, void* stream) {
     if (dtype == MTFJSP_F64) dense_adj_kernel<double><<<h->L.B, 256, 0, s>>>(h->L, h->tmp_adj_w, h->tmp_adj_src, (double*)adj);
     else if (dtype == MTFJSP_F32) dense_adj_kernel<float><<<h->L.B, 256, 0, s>>>(h->L, h->tmp_adj_w, h->tmp_adj_src, (float*)adj);
     else return fail(MTFJSP_E_ARG, "dtype must be MTFJSP_F32 or MTFJSP_F64");
-    h->launches++;
-    CK(cudaGetLastError(), "dense_adj_kernel");
-    return MTFJSP_OK;
+    return counted(h, "dense_adj_kernel");
 }
 
 int mtfjsp_raw_adj(mtfjsp_env* h, int32_t* adj, void* stream) {
@@ -3367,9 +3332,7 @@ int mtfjsp_raw_adj(mtfjsp_env* h, int32_t* adj, void* stream) {
     CK(cudaMemsetAsync(adj, 0, (size_t)L.B * L.N * L.N * sizeof(int32_t), s), "cudaMemsetAsync");
     const size_t n = (size_t)L.B * L.N;
     raw_adj_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(L, h->sd, h->si, h->xs, adj);
-    h->launches++;
-    CK(cudaGetLastError(), "raw_adj_kernel");
-    return MTFJSP_OK;
+    return counted(h, "raw_adj_kernel");
 }
 
 int mtfjsp_generate_instances(int B, int J, int M, int E, uint64_t seed, uint64_t env_offset, double* t, double* p, double* tt,
@@ -3382,8 +3345,7 @@ int mtfjsp_generate_instances(int B, int J, int M, int E, uint64_t seed, uint64_
     if ((long long)M * M > (long long)J * M) return fail(MTFJSP_E_ARG, "mtfjsp_generate_instances: needs J >= M");
     const size_t n = (size_t)B * J * M;
     instance_gen_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(B, J, M, E, W, seed, env_offset, t, p, tt, edge);
-    CK(cudaGetLastError(), "instance_gen_kernel");
-    return MTFJSP_OK;
+    return launched("instance_gen_kernel");
 }
 
 int mtfjsp_costs(mtfjsp_env* h, double* cost4, double* total_e1, void* stream) {
@@ -3391,9 +3353,7 @@ int mtfjsp_costs(mtfjsp_env* h, double* cost4, double* total_e1, void* stream) {
     int rc = enter(h, (cudaStream_t)stream);
     if (rc) return rc;
     costs_kernel<<<(h->L.B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, cost4, total_e1);
-    h->launches++;
-    CK(cudaGetLastError(), "costs_kernel");
-    return MTFJSP_OK;
+    return counted(h, "costs_kernel");
 }
 
 int mtfjsp_export_state(mtfjsp_env* h, int32_t* mach, double* st, double* ft, int32_t* routes, void* stream) {
@@ -3409,9 +3369,7 @@ int mtfjsp_export_state(mtfjsp_env* h, int32_t* mach, double* st, double* ft, in
     }
     size_t n = (size_t)L.B * L.N;
     export_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(L, h->sd, h->si, mach, st, ft, routes);
-    h->launches++;
-    CK(cudaGetLastError(), "export_kernel");
-    return MTFJSP_OK;
+    return counted(h, "export_kernel");
 }
 
 int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int64_t* n, void* stream) {
@@ -3419,9 +3377,7 @@ int mtfjsp_export_scaler(mtfjsp_env* h, double* R, double* mean, double* S, int6
     int rc = enter(h, (cudaStream_t)stream);
     if (rc) return rc;
     export_scaler_kernel<<<(h->L.B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->L, h->sd, R, mean, S, n);
-    h->launches++;
-    CK(cudaGetLastError(), "export_scaler_kernel");
-    return MTFJSP_OK;
+    return counted(h, "export_scaler_kernel");
 }
 
 int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, void* stream) {
@@ -3452,8 +3408,7 @@ int mtfjsp_gather(mtfjsp_env* dst, const mtfjsp_env* src, const int32_t* idx, vo
     A.d_edge_id = dst->edge_id; A.d_jm_fin = dst->jm_fin; A.d_jm_esa = dst->jm_esa; A.d_dn = dst->dn; A.d_inv = dst->inv;
     A.d_cand = dst->cand;
     gather_kernel<<<Ld.B, 128, 0, s>>>(A);
-    dst->launches++;
-    CK(cudaGetLastError(), "gather_kernel");
+    if (const int rc = counted(dst, "gather_kernel")) return rc;
     dst->loaded = true;
     dst->reset_done = hs->reset_done;
     dst->reset_snap = hs->reset_snap;
@@ -3473,13 +3428,7 @@ int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, do
     // a non-step call: a recorded reset runs now, and the next step waits for the peek in full
     int rc = enter(h, s);
     if (rc) return rc;
-    static thread_local int configured_dev = -1;
-    static thread_local size_t configured_smem = 0;
-    if (smem > 48 * 1024 && (configured_dev != h->device || configured_smem < smem)) {
-        CK(cudaFuncSetAttribute(peek_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute");
-        configured_dev = h->device;
-        configured_smem = smem;
-    }
+    CK(opt_in_smem(peek_kernel, smem), "cudaFuncSetAttribute");
     PeekArgs A;
     memset(&A, 0, sizeof A);
     A.L = L; A.pw = h->pw;
@@ -3488,9 +3437,7 @@ int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, do
     A.cfgw[0] = h->cfgw[0]; A.cfgw[1] = h->cfgw[1]; A.cfgw[2] = h->cfgw[2]; A.divisor = h->divisor;
     A.reward5 = reward5; A.invalid = invalid;
     peek_kernel<<<L.B, warps * 32, smem, s>>>(A);
-    h->launches++;
-    CK(cudaGetLastError(), "peek_kernel");
-    return MTFJSP_OK;
+    return counted(h, "peek_kernel");
 }
 
 int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, double* cost4, double* return5,
@@ -3503,13 +3450,7 @@ int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actio
     int rc = enter(h, s);
     if (rc) return rc;
     const size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
-    static thread_local int configured_dev = -1;
-    static thread_local size_t configured_smem = 0;
-    if (configured_dev != h->device || configured_smem < smem) {
-        CK(cudaFuncSetAttribute(replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute");
-        configured_dev = h->device;
-        configured_smem = smem;
-    }
+    CK(opt_in_smem(replay_kernel, smem), "cudaFuncSetAttribute");
     ReplayArgs A;
     memset(&A, 0, sizeof A);
     A.L = L; A.pw = h->pw;
@@ -3519,9 +3460,7 @@ int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actio
     A.cost4 = cost4; A.return5 = return5; A.first_invalid = first_invalid;
     const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
     replay_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
-    h->launches++;
-    CK(cudaGetLastError(), "replay_kernel");
-    return MTFJSP_OK;
+    return counted(h, "replay_kernel");
 }
 
 int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int mask_mode, int32_t* op,
@@ -3532,9 +3471,7 @@ int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int 
     if (rc) return rc;
     const uint8_t* jm = mask_mode == MTFJSP_MASK_ESA ? h->jm_esa : h->jm_fin;
     policy_kernel<<<(h->L.B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->L, h->t, h->si, jm, h->cand, seed, env_offset, op, mach);
-    h->launches++;
-    CK(cudaGetLastError(), "policy_kernel");
-    return MTFJSP_OK;
+    return counted(h, "policy_kernel");
 }
 
 int mtfjsp_random_step(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int32_t* op, int32_t* mach, void* mfea1,

@@ -21,7 +21,7 @@
 
 #include <type_traits>
 
-#include "../../include/mtfjsp.h"
+#include "mtfjsp_launch.cuh"
 
 namespace {
 
@@ -1638,43 +1638,28 @@ __global__ void __launch_bounds__(ESA_HEAD_WARPS * 32, 1) esa_head_tf32_kernel(
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256));
 }
 
-// Operand alignment, checked on the host before any launch: cp.async, TMA and the float4 loads / stores move 16 bytes at a
-// time, adj_w and fea1 are read as float2.  NULL passes (optional pointers are checked for presence separately).
-template <class... P>
-bool al16(P... p) { return ((((uintptr_t)p & 15) == 0) && ...); }
-bool al8(const void* p) { return ((uintptr_t)p & 7) == 0; }
-
 }  // namespace
 
 // nodes > 0: the grouped form (env-aligned tiles of `nodes`-row envs, per-env statistics; see linear_tf32_kernel)
 template <int KP, bool GROUPED = false>
-static int launch_linear(const float* X, int64_t rows, int K, const float* W, const float* bias, const float* in_scale,
-                         const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream, int nodes = 0) {
+static int launch_linear(const char* what, const float* X, int64_t rows, int K, const float* W, const float* bias,
+                         const float* in_scale, const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream,
+                         int nodes = 0) {
     const size_t smem = (size_t)TILE_N * KP * 4 + (size_t)NSTAGE * TILE_M * (KP > 64 ? 64 : KP) * 4 +
                         (size_t)NEPI * 32 * STG_W * 4 + (TILE_N + 256) * 4 + (4 + NSTAGE) * 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_kernel<KP, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(linear_tf32_kernel<KP, GROUPED>, smem), what);
     const int P = GROUPED ? (nodes + TILE_M - 1) / TILE_M : 1, rpt = GROUPED && P == 1 ? (TILE_M / nodes) * nodes : TILE_M;
     const long long tiles = GROUPED ? (P == 1 ? (rows + rpt - 1) / rpt : rows / nodes * P) : (rows + TILE_M - 1) / TILE_M;
-    const int grid = (int)(tiles < sms ? tiles : sms);
+    const int grid = persistent_grid(tiles);
     if constexpr (GROUPED)
         linear_tf32_kernel<KP, true><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, nullptr, nullptr, 0, Z, stats,
                                                                              tiles, rpt, nodes, P);
     else
         linear_tf32_kernel<KP, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z,
                                                                               stats, tiles);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(what);
 }
 
-// K = 128 through the TMA kernel (X 16-byte aligned, checked by the caller); returns 1 if launched, 0 if the driver entry
-// point is not available (caller falls back)
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1691,103 +1676,71 @@ static EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
-static int launch_linear_tma(const float* X, int64_t rows, const float* W, const float* bias, const float* in_scale,
-                             const float* in_shift, int in_relu, float* Z, double* stats, cudaStream_t stream) {
-    EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return 0;
-    CUtensorMap map;
+// The A operand of the K = 128 TMA kernel: X [rows, 128] f32 (16-byte aligned, checked by the caller) in boxes of 32 columns
+// x box_rows rows, 128-byte swizzled.  False when the driver lacks the entry point or rejects the map (the caller falls back).
+static bool a_operand_map(CUtensorMap* map, const float* X, long long rows, int box_rows) {
+    const EncodeTiledFn enc = encode_tiled_fn();
+    if (!enc) return false;
     const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
     const cuuint64_t strides[1] = {512};
-    const cuuint32_t box[2] = {32, 128};
+    const cuuint32_t box[2] = {32, (cuuint32_t)box_rows};
     const cuuint32_t estr[2] = {1, 1};
-    if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)X, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return 0;
+    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)X, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// K = 128 through the TMA kernel; 1 launched, 0 not available (the caller falls back), < 0 error
+static int launch_linear_tma(const char* what, const float* X, int64_t rows, const float* W, const float* bias,
+                             const float* in_scale, const float* in_shift, int in_relu, float* Z, double* stats,
+                             cudaStream_t stream) {
+    CUtensorMap map;
+    if (!a_operand_map(&map, X, rows, TILE_M)) return 0;
     const size_t smem = (size_t)TILE_N * 128 * 4 + (size_t)NSTAGE * TILE_M * 64 * 4 + (size_t)NEPI * 32 * STG_W * 4 +
                         (TILE_N + 256) * 4 + (4 + 2 * NSTAGE) * 8 + 16 + 128 * 10;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(linear_tf32_tma_kernel<false, false>, smem), what);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    linear_tf32_tma_kernel<false, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles,
-                                                                         TILE_M, 0, nullptr, nullptr);
-    return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
+    linear_tf32_tma_kernel<false, false><<<persistent_grid(tiles), GEMM_WARPS * 32, smem, stream>>>(
+        map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles, TILE_M, 0, nullptr, nullptr);
+    const int rc = launched(what);
+    return rc == MTFJSP_OK ? 1 : rc;
 }
 
 // aggregation + layer in one launch (K = 128, N <= 128 nodes per env); 1 launched, 0 not available, < 0 error
-static int launch_linear_tma_agg(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src, const float* W,
-                                 const float* bias, const float* in_scale, const float* in_shift, int in_relu, float* Z,
-                                 double* stats, cudaStream_t stream) {
-    EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc || N > TILE_M) return 0;
+static int launch_linear_tma_agg(const char* what, const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
+                                 const float* W, const float* bias, const float* in_scale, const float* in_shift, int in_relu,
+                                 float* Z, double* stats, cudaStream_t stream) {
+    if (N > TILE_M) return 0;
     const int rpt = (TILE_M / N) * N;
     const long long rows = (long long)B * N;
     CUtensorMap map;
-    const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {512};
-    const cuuint32_t box[2] = {32, (cuuint32_t)rpt};
-    const cuuint32_t estr[2] = {1, 1};
-    if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)X, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return 0;
+    if (!a_operand_map(&map, X, rows, rpt)) return 0;
     const size_t smem = (size_t)TILE_N * 128 * 4 + (size_t)3 * TILE_M * 64 * 4 + (size_t)TILE_M * TILE_N * 4 + (TILE_N + 256) * 4 +
                         (4 + 2 * 3) * 8 + 16 + 128 * 10;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(linear_tf32_tma_kernel<true, false>, smem), what);
     const long long tiles = (rows + rpt - 1) / rpt;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    linear_tf32_tma_kernel<true, false><<<grid, GEMM_WARPS * 32, smem, stream>>>(map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles, rpt,
-                                                                        N, reinterpret_cast<const float2*>(adj_w), adj_src);
-    return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
+    linear_tf32_tma_kernel<true, false><<<persistent_grid(tiles), GEMM_WARPS * 32, smem, stream>>>(
+        map, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, tiles, rpt, N, reinterpret_cast<const float2*>(adj_w), adj_src);
+    const int rc = launched(what);
+    return rc == MTFJSP_OK ? 1 : rc;
 }
 
 // the grouped K = 128 layers (both forms: agg = the aggregation + layer of launch_linear_tma_agg, nodes <= 128); in_scale /
 // in_shift [G,128]; 1 launched, 0 TMA not available, < 0 error
-static int launch_linear_tma_grouped(bool agg, const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
-                                     const float* W, const float* bias, const float* in_scale, const float* in_shift, int in_relu,
-                                     int epg, float* Z, double* env_stats, cudaStream_t stream) {
-    EncodeTiledFn enc = encode_tiled_fn();
-    if (!enc) return 0;
+static int launch_linear_tma_grouped(const char* what, bool agg, const float* X, int64_t B, int N, const float* adj_w,
+                                     const int16_t* adj_src, const float* W, const float* bias, const float* in_scale,
+                                     const float* in_shift, int in_relu, int epg, float* Z, double* env_stats, cudaStream_t stream) {
     const int P = (N + TILE_M - 1) / TILE_M, rpt = P == 1 ? (TILE_M / N) * N : TILE_M;
     const long long rows = (long long)B * N;
     CUtensorMap map;
-    const cuuint64_t dims[2] = {128, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {512};
-    const cuuint32_t box[2] = {32, (cuuint32_t)rpt};
-    const cuuint32_t estr[2] = {1, 1};
-    if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)X, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return 0;
+    if (!a_operand_map(&map, X, rows, rpt)) return 0;
     const size_t smem_agg = (size_t)TILE_N * 128 * 4 + (size_t)3 * TILE_M * 64 * 4 + (size_t)TILE_M * TILE_N * 4 + (TILE_N + 256) * 4 +
                             (4 + 2 * 3) * 8 + 16 + 128 * 10;
     const size_t smem_lin = (size_t)TILE_N * 128 * 4 + (size_t)NSTAGE * TILE_M * 64 * 4 + (size_t)NEPI * 32 * STG_W * 4 +
                             (TILE_N + 256) * 4 + (4 + 2 * NSTAGE) * 8 + 16 + 128 * 10;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(linear_tf32_tma_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_agg) != cudaSuccess ||
-            cudaFuncSetAttribute(linear_tf32_tma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_lin) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(linear_tf32_tma_kernel<true, true>, smem_agg), what);
+    CK(opt_in_smem(linear_tf32_tma_kernel<false, true>, smem_lin), what);
     const long long tiles = P == 1 ? (rows + rpt - 1) / rpt : B * P;
-    const int grid = (int)(tiles < sms ? tiles : sms);
+    const int grid = persistent_grid(tiles);
     if (agg)
         linear_tf32_tma_kernel<true, true><<<grid, GEMM_WARPS * 32, smem_agg, stream>>>(
             map, rows, W, bias, in_scale, in_shift, in_relu, Z, env_stats, tiles, rpt, N, reinterpret_cast<const float2*>(adj_w), adj_src,
@@ -1795,75 +1748,62 @@ static int launch_linear_tma_grouped(bool agg, const float* X, int64_t B, int N,
     else
         linear_tf32_tma_kernel<false, true><<<grid, GEMM_WARPS * 32, smem_lin, stream>>>(
             map, rows, W, bias, in_scale, in_shift, in_relu, Z, env_stats, tiles, rpt, N, nullptr, nullptr, P, epg);
-    return cudaGetLastError() == cudaSuccess ? 1 : MTFJSP_E_CUDA;
+    const int rc = launched(what);
+    return rc == MTFJSP_OK ? 1 : rc;
 }
 
 extern "C" {
 
 int mtfjsp_enc_linear_tf32(const float* X, int64_t rows, int K, const float* W, const float* bias, const float* in_scale,
                            const float* in_shift, int in_relu, float* Z, double* stats, void* stream) {
-    if (!X || !W || !Z || rows < 1 || K < 4 || K > 128 || (K % 4) != 0) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(X, W, Z) || !al8(stats)) return MTFJSP_E_ARG;
+    if (!X || !W || !Z || rows < 1 || K < 4 || K > 128 || (K % 4) != 0) return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32: in_scale and in_shift go together");
+    if (!al16(X, W, Z) || !al8(stats)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32: misaligned operand");
     cudaStream_t s = (cudaStream_t)stream;
     if (K == 128 && rows >= 4096) {  // the big layers: A operand by TMA (falls through when the driver lacks the entry point)
-        const int rc = launch_linear_tma(X, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
+        const int rc = launch_linear_tma(__func__, X, rows, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
         if (rc != 0) return rc < 0 ? rc : MTFJSP_OK;
     }
-    if (K <= 16) return launch_linear<16>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
-    if (K <= 32) return launch_linear<32>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
-    if (K <= 64) return launch_linear<64>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
-    return launch_linear<128>(X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
+    if (K <= 16) return launch_linear<16>(__func__, X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
+    if (K <= 32) return launch_linear<32>(__func__, X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
+    if (K <= 64) return launch_linear<64>(__func__, X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
+    return launch_linear<128>(__func__, X, rows, K, W, bias, in_scale, in_shift, in_relu, Z, stats, s);
 }
 
 int mtfjsp_enc_head_tf32(const float* X, const int32_t* cand, int64_t B, int rows_per_env, int nodes_per_env,
                          const float* in_scale, const float* in_shift, int in_relu, const float* Wa, const float* bias_env,
                          int64_t bias_rows, const float* W1, const float* b1, const float* w2, const float* b2, float* out,
                          void* stream) {
-    if (!X || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(X, Wa, bias_env, W1)) return MTFJSP_E_ARG;
-    if (bias_rows != 1 && bias_rows != B) return MTFJSP_E_ARG;
-    if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL)) return MTFJSP_E_ARG;
+    if (!X || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: in_scale and in_shift go together");
+    if (!al16(X, Wa, bias_env, W1)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: misaligned operand");
+    if (bias_rows != 1 && bias_rows != B) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: bias_rows must be 1 or B");
+    if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: candidate nodes out of range");
     const long long rows = (long long)B * rows_per_env;
-    if (rows > 0x7fffffffLL) return MTFJSP_E_ARG;
+    if (rows > 0x7fffffffLL) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32: more than 2^31 - 1 rows");
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (4 * 128 + 4 * 128) * 4 + 256 * 4 + 2 * 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(head_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(head_tf32_kernel<false>, smem), __func__);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    head_tf32_kernel<false><<<grid, HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(X, cand, rows, rows_per_env, nodes_per_env, in_scale,
-                                                                          in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2, b2,
-                                                                          out, tiles);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    head_tf32_kernel<false><<<persistent_grid(tiles), HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(
+        X, cand, rows, rows_per_env, nodes_per_env, in_scale, in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2, b2, out, tiles);
+    return launched(__func__);
 }
 
 int mtfjsp_enc_gat_trunk_tf32(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
                               const float* a_src, const float* a_dst, float* out, double* stats, int64_t R, void* stream) {
-    if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || R < 1) return MTFJSP_E_ARG;
-    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(stats)) return MTFJSP_E_ARG;
+    if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || R < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_trunk_tf32: bad argument");
+    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(stats)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_trunk_tf32: misaligned operand");
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(gat_trunk2_tf32_kernel<false>, smem), __func__);
     const long long tiles = (R + 127) / 128;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    gat_trunk2_tf32_kernel<false><<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
-                                                                                          stats, R, tiles, 128, 1);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    gat_trunk2_tf32_kernel<false><<<persistent_grid(tiles), TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(
+        fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out, stats, R, tiles, 128, 1);
+    return launched(__func__);
 }
 
 int mtfjsp_enc_gat_trunk_tf32_grouped(const float* fea1, const float* fea2, const float* W1p, const float* W2p, const float* Wt,
@@ -1871,34 +1811,29 @@ int mtfjsp_enc_gat_trunk_tf32_grouped(const float* fea1, const float* fea2, cons
                                       void* stream) {
     if (!fea1 || !fea2 || !W1p || !W2p || !Wt || !a_src || !a_dst || !out || !env_stats || B < 1 || M < 1 || M > 128 ||
         B * M > 0x7fffff00LL)
-        return MTFJSP_E_ARG;
-    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(env_stats)) return MTFJSP_E_ARG;
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_trunk_tf32_grouped: bad argument");
+    if (!al16(fea2, Wt, out) || !al8(fea1) || !al8(env_stats))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_gat_trunk_tf32_grouped: misaligned operand");
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (3 * 4 * 128 + 256 + 128 * 14) * 4 + 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(gat_trunk2_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(gat_trunk2_tf32_kernel<true>, smem), __func__);
     const int epT = 128 / M;  // whole envs per tile
     const long long tiles = (B + epT - 1) / epT;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    gat_trunk2_tf32_kernel<true><<<grid, TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out,
-                                                                                         env_stats, B * M, tiles, epT * M, M);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    gat_trunk2_tf32_kernel<true><<<persistent_grid(tiles), TRUNK_WARPS * 32, smem, (cudaStream_t)stream>>>(
+        fea1, fea2, W1p, W2p, Wt, a_src, a_dst, out, env_stats, B * M, tiles, epT * M, M);
+    return launched(__func__);
 }
 
 int mtfjsp_enc_aggregate_linear_tf32(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src, const float* W,
                                      const float* bias, const float* in_scale, const float* in_shift, int in_relu, float* Z,
                                      double* stats, void* stream) {
-    if (!X || !adj_w || !adj_src || !W || !Z || B < 1 || N < 1) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(X, W, Z) || !al8(adj_w) || !al8(stats)) return MTFJSP_E_ARG;
-    const int rc = launch_linear_tma_agg(X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, Z, stats, (cudaStream_t)stream);
-    if (rc == 0) return MTFJSP_E_STATE;  // not available for this size / driver: the caller runs the two kernels
+    if (!X || !adj_w || !adj_src || !W || !Z || B < 1 || N < 1) return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32: in_scale and in_shift go together");
+    if (!al16(X, W, Z) || !al8(adj_w) || !al8(stats)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32: misaligned operand");
+    const int rc = launch_linear_tma_agg(__func__, X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, Z, stats,
+                                         (cudaStream_t)stream);
+    if (rc == 0)  // the caller runs the two kernels
+        return fail(MTFJSP_E_STATE, "mtfjsp_enc_aggregate_linear_tf32: not available for this size or driver");
     return rc < 0 ? rc : MTFJSP_OK;
 }
 
@@ -1907,170 +1842,160 @@ static bool grouped_args_ok(int64_t B, int N, int epg) { return B >= 1 && N >= 1
 int mtfjsp_enc_linear_tf32_grouped(const float* X, int64_t B, int rows_per_env, int K, const float* W, const float* bias,
                                    const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, float* Z,
                                    double* env_stats, void* stream) {
-    if (!X || !W || !Z || !env_stats || !grouped_args_ok(B, rows_per_env, envs_per_group)) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(X, W, Z, in_scale, in_shift) || !al8(env_stats)) return MTFJSP_E_ARG;
+    if (!X || !W || !Z || !env_stats || !grouped_args_ok(B, rows_per_env, envs_per_group))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32_grouped: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32_grouped: in_scale and in_shift go together");
+    if (!al16(X, W, Z, in_scale, in_shift) || !al8(env_stats))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32_grouped: misaligned operand");
     if (K == 128) {
-        const int rc = launch_linear_tma_grouped(false, X, B, rows_per_env, nullptr, nullptr, W, bias, in_scale, in_shift, in_relu,
-                                                 envs_per_group, Z, env_stats, (cudaStream_t)stream);
-        return rc == 0 ? MTFJSP_E_STATE : rc < 0 ? rc : MTFJSP_OK;
+        const int rc = launch_linear_tma_grouped(__func__, false, X, B, rows_per_env, nullptr, nullptr, W, bias, in_scale, in_shift,
+                                                 in_relu, envs_per_group, Z, env_stats, (cudaStream_t)stream);
+        if (rc == 0) return fail(MTFJSP_E_STATE, "mtfjsp_enc_linear_tf32_grouped: TMA not available");
+        return rc < 0 ? rc : MTFJSP_OK;
     }
-    if (K < 4 || K > 16 || (K % 4) != 0 || in_scale) return MTFJSP_E_ARG;
-    return launch_linear<16, true>(X, B * rows_per_env, K, W, bias, nullptr, nullptr, 0, Z, env_stats, (cudaStream_t)stream, rows_per_env);
+    if (K < 4 || K > 16 || (K % 4) != 0 || in_scale)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_linear_tf32_grouped: K must be 128, or 4..16 without an input affine");
+    return launch_linear<16, true>(__func__, X, B * rows_per_env, K, W, bias, nullptr, nullptr, 0, Z, env_stats, (cudaStream_t)stream,
+                                   rows_per_env);
 }
 
 int mtfjsp_enc_aggregate_linear_tf32_grouped(const float* X, int64_t B, int N, const float* adj_w, const int16_t* adj_src,
                                              const float* W, const float* bias, const float* in_scale, const float* in_shift,
                                              int in_relu, int envs_per_group, float* Z, double* env_stats, void* stream) {
-    if (!X || !adj_w || !adj_src || !W || !Z || !env_stats || !grouped_args_ok(B, N, envs_per_group)) return MTFJSP_E_ARG;
-    if ((in_scale == nullptr) != (in_shift == nullptr)) return MTFJSP_E_ARG;
-    if (!al16(X, W, Z, in_scale, in_shift) || !al8(adj_w) || !al8(env_stats)) return MTFJSP_E_ARG;
-    if (N > TILE_M) return MTFJSP_E_STATE;  // the caller runs mtfjsp_enc_aggregate_grouped + mtfjsp_enc_linear_tf32_grouped
-    const int rc = launch_linear_tma_grouped(true, X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu, envs_per_group, Z,
-                                             env_stats, (cudaStream_t)stream);
-    return rc == 0 ? MTFJSP_E_STATE : rc < 0 ? rc : MTFJSP_OK;
+    if (!X || !adj_w || !adj_src || !W || !Z || !env_stats || !grouped_args_ok(B, N, envs_per_group))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32_grouped: bad argument");
+    if ((in_scale == nullptr) != (in_shift == nullptr))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32_grouped: in_scale and in_shift go together");
+    if (!al16(X, W, Z, in_scale, in_shift) || !al8(adj_w) || !al8(env_stats))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_aggregate_linear_tf32_grouped: misaligned operand");
+    // the caller runs mtfjsp_enc_aggregate_grouped + mtfjsp_enc_linear_tf32_grouped
+    if (N > TILE_M) return fail(MTFJSP_E_STATE, "mtfjsp_enc_aggregate_linear_tf32_grouped: more than 128 nodes per env");
+    const int rc = launch_linear_tma_grouped(__func__, true, X, B, N, adj_w, adj_src, W, bias, in_scale, in_shift, in_relu,
+                                             envs_per_group, Z, env_stats, (cudaStream_t)stream);
+    if (rc == 0) return fail(MTFJSP_E_STATE, "mtfjsp_enc_aggregate_linear_tf32_grouped: TMA not available");
+    return rc < 0 ? rc : MTFJSP_OK;
 }
 
 int mtfjsp_enc_head_tf32_grouped(const float* X, const int32_t* cand, int64_t B, int rows_per_env, int nodes_per_env,
                                  const float* in_scale, const float* in_shift, int in_relu, int envs_per_group, const float* Wa,
                                  const float* bias_env, int64_t bias_rows, const float* W1, const float* b1, const float* w2,
                                  const float* b2, float* out, void* stream) {
-    if (!X || !in_scale || !in_shift || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1) return MTFJSP_E_ARG;
-    if (envs_per_group < 1 || B % envs_per_group != 0) return MTFJSP_E_ARG;
-    if (bias_rows != 1 && bias_rows != B) return MTFJSP_E_ARG;
-    if (!al16(X, Wa, bias_env, W1, in_scale, in_shift)) return MTFJSP_E_ARG;
-    if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL)) return MTFJSP_E_ARG;
+    if (!X || !in_scale || !in_shift || !Wa || !bias_env || !W1 || !w2 || !out || B < 1 || rows_per_env < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: bad argument");
+    if (envs_per_group < 1 || B % envs_per_group != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: envs_per_group must divide B");
+    if (bias_rows != 1 && bias_rows != B) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: bias_rows must be 1 or B");
+    if (!al16(X, Wa, bias_env, W1, in_scale, in_shift)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: misaligned operand");
+    if (cand && (nodes_per_env < 1 || (long long)B * nodes_per_env > 0x7fffffffLL))
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: candidate nodes out of range");
     const long long rows = (long long)B * rows_per_env;
-    if (rows > 0x7fffffffLL) return MTFJSP_E_ARG;
+    if (rows > 0x7fffffffLL) return fail(MTFJSP_E_ARG, "mtfjsp_enc_head_tf32_grouped: more than 2^31 - 1 rows");
     const size_t smem = 3 * (size_t)TILE_N * 128 * 4 + (4 * 128 + 4 * 128) * 4 + 256 * 4 + 2 * 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(head_tf32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(head_tf32_kernel<true>, smem), __func__);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    head_tf32_kernel<true><<<grid, HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(X, cand, rows, rows_per_env, nodes_per_env, in_scale,
-                                                                                in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2,
-                                                                                b2, out, tiles, envs_per_group);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    head_tf32_kernel<true><<<persistent_grid(tiles), HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(
+        X, cand, rows, rows_per_env, nodes_per_env, in_scale, in_shift, in_relu, Wa, bias_env, bias_rows, W1, b1, w2, b2, out, tiles,
+        envs_per_group);
+    return launched(__func__);
 }
 
 int mtfjsp_enc_bn_finalize_grouped(const double* env_stats, int64_t B, int rows_per_env, int envs_per_group, const float* gamma,
                                    const float* beta, float eps, float* scale, float* shift, int C, void* stream) {
     if (!env_stats || !gamma || !beta || !scale || !shift || C < 1 || !grouped_args_ok(B, rows_per_env, envs_per_group))
-        return MTFJSP_E_ARG;
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_finalize_grouped: bad argument");
     const long long G = B / envs_per_group;
     const int P = (rows_per_env + TILE_M - 1) / TILE_M;
     bn_finalize_grouped_kernel<<<(unsigned)((G * C + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         env_stats, G, P, envs_per_group, 1.0 / ((double)envs_per_group * rows_per_env), gamma, beta, eps, scale, shift, C);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_bn_finalize(const double* stats, int64_t rows, const float* gamma, const float* beta, float eps,
                            float* scale, float* shift, int C, void* stream) {
-    if (!stats || !gamma || !beta || !scale || !shift || rows < 1 || C < 1) return MTFJSP_E_ARG;
+    if (!stats || !gamma || !beta || !scale || !shift || rows < 1 || C < 1) return fail(MTFJSP_E_ARG, "mtfjsp_enc_bn_finalize: bad argument");
     bn_finalize_kernel<<<(C + 127) / 128, 128, 0, (cudaStream_t)stream>>>(stats, 1.0 / (double)rows, gamma, beta, eps, scale,
                                                                         shift, C);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int64_t mtfjsp_enc_esa_mach_stats_workspace_doubles(void) { return (int64_t)ESA_STATS_BLOCKS * 128; }
 
 int mtfjsp_enc_esa_mach_stats(const float* fea1, const float* fea2, int64_t B, int M, double* moments, float* env_mean,
                               double* workspace, void* stream) {
-    if (!fea1 || !fea2 || !moments || !env_mean || !workspace || B < 1 || M < 1 || M > ESA_STATS_ROWS) return MTFJSP_E_ARG;
+    if (!fea1 || !fea2 || !moments || !env_mean || !workspace || B < 1 || M < 1 || M > ESA_STATS_ROWS)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_esa_mach_stats: bad argument");
     const int epc = ESA_STATS_ROWS / M;
     const long long chunks = (B + epc - 1) / epc;
     const int grid = (int)(chunks < ESA_STATS_BLOCKS ? chunks : ESA_STATS_BLOCKS);
     esa_stats_kernel<<<grid, ESA_STATS_THREADS, 0, (cudaStream_t)stream>>>(fea1, fea2, B, M, epc, workspace, env_mean);
-    if (cudaGetLastError() != cudaSuccess) return MTFJSP_E_CUDA;
+    const int rc = launched(__func__);
+    if (rc != MTFJSP_OK) return rc;
     esa_stats_reduce_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(workspace, grid, moments);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_esa_mach_fold(const double* moments, int64_t rows, const float* W1, const float* W2, const float* gamma,
                              const float* beta, float eps, const float* W0, const float* b0, float* Wf, float* Wp, float* bp,
                              float* b0f, void* stream) {
-    if (!moments || !W1 || !W2 || !gamma || !beta || !W0 || !b0 || !Wf || !Wp || !bp || !b0f || rows < 1) return MTFJSP_E_ARG;
+    if (!moments || !W1 || !W2 || !gamma || !beta || !W0 || !b0 || !Wf || !Wp || !bp || !b0f || rows < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_esa_mach_fold: bad argument");
     esa_fold_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(moments, 1.0 / (double)rows, W1, W2, gamma, beta, eps, W0, b0, Wf, Wp, bp, b0f);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_enc_esa_mach_head_tf32(const float* fea1, const float* fea2, int64_t B, int M, const float* W0f, const float* bias_env,
                                   const float* W1, const float* b1, const float* w2, const float* b2, float* out, void* stream) {
-    if (!fea1 || !fea2 || !W0f || !bias_env || !W1 || !w2 || !out || B < 1 || M < 1) return MTFJSP_E_ARG;
-    if (!al16(W0f, bias_env, W1)) return MTFJSP_E_ARG;
+    if (!fea1 || !fea2 || !W0f || !bias_env || !W1 || !w2 || !out || B < 1 || M < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_esa_mach_head_tf32: bad argument");
+    if (!al16(W0f, bias_env, W1)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_esa_mach_head_tf32: misaligned operand");
     const long long rows = (long long)B * M;
     const size_t smem = 2 * (size_t)TILE_N * 128 * 4 + 2 * (size_t)TILE_M * 16 * 4 + (4 * 128 + 2 * 128) * 4 + 2 * 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(esa_head_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CK(opt_in_smem(esa_head_tf32_kernel, smem), __func__);
     const long long tiles = (rows + TILE_M - 1) / TILE_M;
-    const int grid = (int)(tiles < sms ? tiles : sms);
-    esa_head_tf32_kernel<<<grid, ESA_HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(fea1, fea2, rows, M, W0f, bias_env, W1, b1, w2, b2,
-                                                                                  out, tiles);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    esa_head_tf32_kernel<<<persistent_grid(tiles), ESA_HEAD_WARPS * 32, smem, (cudaStream_t)stream>>>(
+        fea1, fea2, rows, M, W0f, bias_env, W1, b1, w2, b2, out, tiles);
+    return launched(__func__);
 }
 
 }  // extern "C"
 
 template <int NP>
-static int launch_wgrad(const float* dY, const float* X, int64_t rows, int K, float* dW, float* db, float* ws, int sms,
-                        cudaStream_t stream) {
+static int launch_wgrad(const float* dY, const float* X, int64_t rows, int K, float* dW, float* db, float* ws, cudaStream_t stream) {
     const size_t smem = (size_t)WG_NSTAGE * (16 + NP / 8) * WG_SBO + (size_t)WG_WARPS * 128 * 8 + (WG_NSTAGE + 1) * 8 + 16;
-    static thread_local bool configured = false;
-    if (!configured) {
-        if (cudaFuncSetAttribute(wgrad_tf32_kernel<NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-            return MTFJSP_E_CUDA;
-        configured = true;
-    }
+    CK(opt_in_smem(wgrad_tf32_kernel<NP>, smem), "mtfjsp_enc_wgrad_tf32");
+    const int sms = sm_count();  // the workspace holds one partial per SM (mtfjsp_enc_wgrad_workspace_floats)
     const long long stages = (rows + WG_KS - 1) / WG_KS;
     const int grid = (int)(stages < sms ? stages : sms);
     float* parts = ws;
     float* dbparts = ws + (size_t)sms * TILE_M * NP;
     wgrad_tf32_kernel<NP><<<grid, WG_WARPS * 32, smem, stream>>>(dY, X, rows, K, parts, dbparts, stages);
-    if (cudaGetLastError() != cudaSuccess) return MTFJSP_E_CUDA;
+    const int rc = launched("mtfjsp_enc_wgrad_tf32");
+    if (rc != MTFJSP_OK) return rc;
     wgrad_reduce_kernel<<<(TILE_M * K + 255) / 256, 256, 0, stream>>>(parts, dbparts, grid, NP, K, dW, db);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched("mtfjsp_enc_wgrad_tf32");
 }
 
-static int wgrad_sms() {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return sms;
-}
 static int wgrad_np(int K) { return K <= 16 ? 16 : K <= 32 ? 32 : K <= 64 ? 64 : 128; }
 
 extern "C" {
 
 int64_t mtfjsp_enc_wgrad_workspace_floats(int K) {
     if (K < 4 || K > 128) return 0;
-    return (int64_t)wgrad_sms() * (TILE_M * wgrad_np(K) + 128);
+    return (int64_t)sm_count() * (TILE_M * wgrad_np(K) + 128);
 }
 
 int mtfjsp_enc_wgrad_tf32(const float* dY, const float* X, int64_t rows, int K, float* dW, float* db, float* workspace,
                           void* stream) {
-    if (!dY || !X || !dW || !workspace || rows < 1 || K < 4 || K > 128 || (K % 4) != 0) return MTFJSP_E_ARG;
-    if (!al16(dY, X, workspace)) return MTFJSP_E_ARG;
+    if (!dY || !X || !dW || !workspace || rows < 1 || K < 4 || K > 128 || (K % 4) != 0)
+        return fail(MTFJSP_E_ARG, "mtfjsp_enc_wgrad_tf32: bad argument");
+    if (!al16(dY, X, workspace)) return fail(MTFJSP_E_ARG, "mtfjsp_enc_wgrad_tf32: misaligned operand");
     cudaStream_t s = (cudaStream_t)stream;
-    const int sms = wgrad_sms();
     switch (wgrad_np(K)) {
-        case 16: return launch_wgrad<16>(dY, X, rows, K, dW, db, workspace, sms, s);
-        case 32: return launch_wgrad<32>(dY, X, rows, K, dW, db, workspace, sms, s);
-        case 64: return launch_wgrad<64>(dY, X, rows, K, dW, db, workspace, sms, s);
-        default: return launch_wgrad<128>(dY, X, rows, K, dW, db, workspace, sms, s);
+        case 16: return launch_wgrad<16>(dY, X, rows, K, dW, db, workspace, s);
+        case 32: return launch_wgrad<32>(dY, X, rows, K, dW, db, workspace, s);
+        case 64: return launch_wgrad<64>(dY, X, rows, K, dW, db, workspace, s);
+        default: return launch_wgrad<128>(dY, X, rows, K, dW, db, workspace, s);
     }
 }
 

@@ -8,7 +8,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include "../../include/mtfjsp.h"
+#include "mtfjsp_launch.cuh"
 
 namespace {
 
@@ -155,21 +155,20 @@ __global__ void __launch_bounds__(HV_THREADS) hypervolume3_kernel(const double* 
 extern "C" {
 
 int mtfjsp_pareto_filter(const double* obj3, const int64_t* seg, int S, int64_t max_len, uint8_t* keep, void* stream) {
-    if (!obj3 || !seg || !keep || S < 0 || max_len < 0) return MTFJSP_E_ARG;
+    if (!obj3 || !seg || !keep || S < 0 || max_len < 0) return fail(MTFJSP_E_ARG, "mtfjsp_pareto_filter: bad argument");
     if (S == 0) return MTFJSP_OK;
     const int64_t tiles = (max_len + FILTER_THREADS - 1) / FILTER_THREADS;
     const dim3 grid((unsigned)S, (unsigned)(tiles < 1 ? 1 : (tiles > 65535 ? 65535 : tiles)));
     pareto_filter_kernel<<<grid, FILTER_THREADS, 0, (cudaStream_t)stream>>>(obj3, seg, keep);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 int mtfjsp_hypervolume3(const double* obj3, const int64_t* seg, int S, const double* ref3, double* hv, void* stream) {
-    if (!obj3 || !seg || !ref3 || !hv || S < 0) return MTFJSP_E_ARG;
+    if (!obj3 || !seg || !ref3 || !hv || S < 0) return fail(MTFJSP_E_ARG, "mtfjsp_hypervolume3: bad argument");
     if (S == 0) return MTFJSP_OK;
-    if (cudaFuncSetAttribute(hypervolume3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HV_SMEM) != cudaSuccess)
-        return MTFJSP_E_CUDA;
+    CK(opt_in_smem(hypervolume3_kernel, HV_SMEM), __func__);
     hypervolume3_kernel<<<(unsigned)S, HV_THREADS, HV_SMEM, (cudaStream_t)stream>>>(obj3, seg, ref3, hv);
-    return cudaGetLastError() == cudaSuccess ? MTFJSP_OK : MTFJSP_E_CUDA;
+    return launched(__func__);
 }
 
 }  // extern "C"

@@ -20,7 +20,6 @@ BatchNorm uses batch statistics exactly as the reference does (its modules are n
 """
 from __future__ import annotations
 
-import ctypes as C
 import weakref
 
 import numpy as np
@@ -28,19 +27,7 @@ import torch
 import torch.nn.functional as F
 
 from . import _lib
-from ._lib import check
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr())
-
-
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
-def _optr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
+from ._lib import _ptr, _stream, check
 
 
 def _aggregate_raw(h, adj_w, adj_src, in_scale=None, in_shift=None, relu=False):
@@ -52,8 +39,8 @@ def _aggregate_raw(h, adj_w, adj_src, in_scale=None, in_shift=None, relu=False):
                                                       _ptr(in_shift), int(relu), B // in_scale.shape[0], _stream()),
               "mtfjsp_enc_aggregate_grouped")
         return out
-    check(_lib.lib().mtfjsp_enc_aggregate(_ptr(h), _ptr(adj_w), _ptr(adj_src), _ptr(out), B, N, Cc, _optr(in_scale),
-                                          _optr(in_shift), int(relu), _stream()), "mtfjsp_enc_aggregate")
+    check(_lib.lib().mtfjsp_enc_aggregate(_ptr(h), _ptr(adj_w), _ptr(adj_src), _ptr(out), B, N, Cc, _ptr(in_scale),
+                                          _ptr(in_shift), int(relu), _stream()), "mtfjsp_enc_aggregate")
     return out
 
 
@@ -114,8 +101,8 @@ def aggregate_linear_tf32(h, adj_w, adj_src, weight, bias, in_scale=None, in_shi
     if N > 128 or h.shape[2] != 128:
         return None
     z = torch.empty((B * N, 128), dtype=torch.float32, device=h.device)
-    rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _optr(bias),
-                                                     _optr(in_scale), _optr(in_shift), 1 if relu else 0, _ptr(z), _optr(stats),
+    rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _ptr(bias),
+                                                     _ptr(in_scale), _ptr(in_shift), 1 if relu else 0, _ptr(z), _ptr(stats),
                                                      _stream())
     if rc == -3:  # MTFJSP_E_STATE: this form is not available here (driver without the TMA entry point)
         return None
@@ -136,8 +123,8 @@ def select(scores, mask, cand, scale, greedy, rng, stream_id):
     m8 = mask.reshape(B, R)
     m8 = (m8 if m8.dtype == torch.uint8 else m8.to(torch.uint8)).contiguous()
     seed, counter = rng if rng is not None else (0, None)
-    check(_lib.lib().mtfjsp_enc_select(_ptr(scores.contiguous()), _ptr(m8), _optr(cand), float(scale), R, B, 1 if greedy else 0,
-                                       int(seed) & 0xFFFFFFFFFFFFFFFF, _optr(counter), stream_id, _ptr(prob), _ptr(action),
+    check(_lib.lib().mtfjsp_enc_select(_ptr(scores.contiguous()), _ptr(m8), _ptr(cand), float(scale), R, B, 1 if greedy else 0,
+                                       int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(counter), stream_id, _ptr(prob), _ptr(action),
                                        _ptr(log_a), _ptr(task), _stream()), "mtfjsp_enc_select")
     return prob, action, log_a, task
 
@@ -148,13 +135,13 @@ def head_tf32(x, cand, B, rows_per_env, nodes_per_env, in_scale, in_shift, Wa, b
     BatchNorm group of B / G envs (mtfjsp_enc_head_tf32_grouped)."""
     out = torch.empty((B, rows_per_env), dtype=torch.float32, device=x.device)
     if in_scale is not None and in_scale.dim() == 2:
-        check(_lib.lib().mtfjsp_enc_head_tf32_grouped(_ptr(x), _optr(cand), B, rows_per_env, nodes_per_env, _ptr(in_scale),
+        check(_lib.lib().mtfjsp_enc_head_tf32_grouped(_ptr(x), _ptr(cand), B, rows_per_env, nodes_per_env, _ptr(in_scale),
                                                       _ptr(in_shift), 1 if relu else 0, B // in_scale.shape[0], _ptr(Wa),
-                                                      _ptr(bias_env), bias_env.shape[0], _ptr(W1), _optr(b1), _ptr(w2), _optr(b2),
+                                                      _ptr(bias_env), bias_env.shape[0], _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2),
                                                       _ptr(out), _stream()), "mtfjsp_enc_head_tf32_grouped")
         return out
-    check(_lib.lib().mtfjsp_enc_head_tf32(_ptr(x), _optr(cand), B, rows_per_env, nodes_per_env, _optr(in_scale), _optr(in_shift),
-                                          1 if relu else 0, _ptr(Wa), _ptr(bias_env), bias_env.shape[0], _ptr(W1), _optr(b1), _ptr(w2), _optr(b2),
+    check(_lib.lib().mtfjsp_enc_head_tf32(_ptr(x), _ptr(cand), B, rows_per_env, nodes_per_env, _ptr(in_scale), _ptr(in_shift),
+                                          1 if relu else 0, _ptr(Wa), _ptr(bias_env), bias_env.shape[0], _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2),
                                           _ptr(out), _stream()), "mtfjsp_enc_head_tf32")
     return out
 
@@ -165,7 +152,7 @@ def gat_trunk_tf32(fea1, fea2, W1p, W2p, Wt, a_src, a_dst, stats=None):
     R = fea1.shape[0]
     out = torch.empty((R, 128), dtype=torch.float32, device=fea1.device)
     check(_lib.lib().mtfjsp_enc_gat_trunk_tf32(_ptr(fea1), _ptr(fea2), _ptr(W1p), _ptr(W2p), _ptr(Wt), _ptr(a_src), _ptr(a_dst),
-                                               _ptr(out), _optr(stats), R, _stream()), "mtfjsp_enc_gat_trunk_tf32")
+                                               _ptr(out), _ptr(stats), R, _stream()), "mtfjsp_enc_gat_trunk_tf32")
     return out
 
 
@@ -188,7 +175,7 @@ def _graph_mean_raw(h, in_scale=None, in_shift=None, relu=False):
         check(_lib.lib().mtfjsp_enc_graph_mean_grouped(_ptr(h), _ptr(out), B, N, Cc, _ptr(in_scale), _ptr(in_shift), int(relu),
                                                        B // in_scale.shape[0], _stream()), "mtfjsp_enc_graph_mean_grouped")
         return out
-    check(_lib.lib().mtfjsp_enc_graph_mean(_ptr(h), _ptr(out), B, N, Cc, _optr(in_scale), _optr(in_shift), int(relu),
+    check(_lib.lib().mtfjsp_enc_graph_mean(_ptr(h), _ptr(out), B, N, Cc, _ptr(in_scale), _ptr(in_shift), int(relu),
                                            _stream()), "mtfjsp_enc_graph_mean")
     return out
 
@@ -207,8 +194,8 @@ def linear_tf32(x, weight, bias, in_scale=None, in_shift=None, relu=False, stats
     rows, K = x.shape
     assert weight.shape == (128, K) and x.dtype == torch.float32
     z = torch.empty((rows, 128), dtype=torch.float32, device=x.device)
-    check(_lib.lib().mtfjsp_enc_linear_tf32(_ptr(x.contiguous()), rows, K, _ptr(weight), _optr(bias), _optr(in_scale),
-                                            _optr(in_shift), int(relu), _ptr(z), _optr(stats), _stream()),
+    check(_lib.lib().mtfjsp_enc_linear_tf32(_ptr(x.contiguous()), rows, K, _ptr(weight), _ptr(bias), _ptr(in_scale),
+                                            _ptr(in_shift), int(relu), _ptr(z), _ptr(stats), _stream()),
           "mtfjsp_enc_linear_tf32")
     return z
 
@@ -225,8 +212,8 @@ def linear_tf32_grouped(x, rows_per_env, weight, bias, in_scale, in_shift, relu,
     B = rows // rows_per_env
     z = torch.empty((rows, 128), dtype=torch.float32, device=x.device)
     epg = 1 if in_scale is None else B // in_scale.shape[0]
-    check(_lib.lib().mtfjsp_enc_linear_tf32_grouped(_ptr(x.contiguous()), B, rows_per_env, K, _ptr(weight), _optr(bias),
-                                                    _optr(in_scale), _optr(in_shift), int(relu), epg, _ptr(z), _ptr(env_stats),
+    check(_lib.lib().mtfjsp_enc_linear_tf32_grouped(_ptr(x.contiguous()), B, rows_per_env, K, _ptr(weight), _ptr(bias),
+                                                    _ptr(in_scale), _ptr(in_shift), int(relu), epg, _ptr(z), _ptr(env_stats),
                                                     _stream()), "mtfjsp_enc_linear_tf32_grouped")
     return z
 
@@ -238,8 +225,8 @@ def aggregate_linear_tf32_grouped(h, adj_w, adj_src, weight, bias, in_scale, in_
         return None
     z = torch.empty((B * N, 128), dtype=torch.float32, device=h.device)
     epg = 1 if in_scale is None else B // in_scale.shape[0]
-    rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32_grouped(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _optr(bias),
-                                                             _optr(in_scale), _optr(in_shift), int(relu), epg, _ptr(z),
+    rc = _lib.lib().mtfjsp_enc_aggregate_linear_tf32_grouped(_ptr(h), B, N, _ptr(adj_w), _ptr(adj_src), _ptr(weight), _ptr(bias),
+                                                             _ptr(in_scale), _ptr(in_shift), int(relu), epg, _ptr(z),
                                                              _ptr(env_stats), _stream())
     if rc == -3:  # MTFJSP_E_STATE
         return None
@@ -272,7 +259,7 @@ def wgrad_tf32(gz, x, want_bias=True):
         _WGRAD_WS[key] = torch.empty(int(lib.mtfjsp_enc_wgrad_workspace_floats(K)), dtype=torch.float32, device=x.device)
     dW = torch.empty((128, K), dtype=torch.float32, device=x.device)
     db = torch.empty(128, dtype=torch.float32, device=x.device) if want_bias else None
-    check(lib.mtfjsp_enc_wgrad_tf32(_ptr(gz.contiguous()), _ptr(x.contiguous()), rows, K, _ptr(dW), _optr(db),
+    check(lib.mtfjsp_enc_wgrad_tf32(_ptr(gz.contiguous()), _ptr(x.contiguous()), rows, K, _ptr(dW), _ptr(db),
                                     _ptr(_WGRAD_WS[key]), _stream()), "mtfjsp_enc_wgrad_tf32")
     return dW, db
 

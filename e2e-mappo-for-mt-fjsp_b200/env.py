@@ -12,18 +12,10 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import check
+from ._lib import _ptr, _stream, check
 
 F32, F64 = 0, 1
 MASK_FINISHED, MASK_ESA = 0, 1
-
-
-def _ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
 def _to_dev(x, device, dtype):

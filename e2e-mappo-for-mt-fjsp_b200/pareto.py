@@ -17,23 +17,14 @@ search (search.pareto_local_search) uses to bound its archive.
 """
 from __future__ import annotations
 
-import ctypes as C
 
 import numpy as np
 import torch
 
 from . import _lib
-from ._lib import check
+from ._lib import _ptr, _stream, check
 
 HV_MAX_POINTS = 4096
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr())
-
-
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
 def objectives(final4):

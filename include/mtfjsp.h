@@ -13,7 +13,8 @@
  *     caller-owned; the library allocates only in mtfjsp_create;
  *   - every call is asynchronous on `stream` (a cudaStream_t passed as void*) and never synchronises
  *     the host, except the *_host entry points, which return after their device->host copy is done;
- *   - return value: 0 ok, negative = error (MTFJSP_E_*); nothing throws;
+ *   - return value: 0 ok, negative = error (MTFJSP_E_*); nothing throws; every call that returns an
+ *     error leaves its reason in mtfjsp_last_error (one message per thread);
  *   - an invalid (operation, machine) pair does not fail the batch: the env's `invalid` flag is set
  *     and its state is left untouched (the reference silently corrupts its state, SS:1495-1528);
  *   - not thread-safe per handle; handles are independent.
