@@ -1,10 +1,11 @@
 // mtfjsp_pareto.cu -- multi-objective kernels for sm_100a over the three targets (mk, ec, tt) of finished schedules:
-// a per-segment non-dominated filter and the exact per-segment hypervolume (pareto.py wraps both).
+// a per-segment non-dominated filter, the exact per-segment hypervolume and the per-segment non-dominated sorting rank
+// (pareto.py wraps all three).
 //
-// Both are handle-free and run on the caller's stream.  Points are FP64 [P,3] row-major; segment s is the CSR range
-// [seg[s], seg[s+1]).  The filter is pure comparisons, so its bits are exact.  The hypervolume restates, operation for
-// operation, the slice sweep documented in include/mtfjsp.h (pareto.hypervolume3_reference is the numpy form); this file
-// is built with -fmad=false so that no product is contracted into the sum that follows it.
+// All three are handle-free and run on the caller's stream.  Points are FP64 [P,3] row-major; segment s is the CSR range
+// [seg[s], seg[s+1]).  The filter and the rank are pure comparisons, so their results are exact.  The hypervolume
+// restates, operation for operation, the slice sweep documented in include/mtfjsp.h (pareto.hypervolume3_reference is
+// the numpy form); this file is built with -fmad=false so that no product is contracted into the sum that follows it.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -150,6 +151,121 @@ __global__ void __launch_bounds__(HV_THREADS) hypervolume3_kernel(const double* 
     }
 }
 
+// Non-dominated sorting, one block per segment (Deb's domination counts): cnt[p] = how many points beat p, one O(n^2)
+// pass; then front f + 1 is every point whose count reaches 0 once the beats of front f's members are subtracted, so the
+// peeling does O(n^2) work in all.  Shared: the point coordinates when the segment fits `cap` (non-finite rows as NaN,
+// which beat nothing), cnt[RANK_MAX] int32 (-1 once ranked), two front lists of RANK_MAX int16 and two list lengths.
+constexpr int RANK_THREADS = 1024;
+constexpr int RANK_MAX = 4096;              // = HV_MAX: pareto.HV_MAX_POINTS
+constexpr size_t RANK_FIXED_SMEM = (size_t)RANK_MAX * (sizeof(int32_t) + 2 * sizeof(int16_t)) + 4 * sizeof(int32_t);
+
+// q beats p: both finite (a NaN coordinate fails every test), q <= p in every coordinate, and q != p or q has the lower
+// index -- the filter's relation
+__device__ __forceinline__ bool beats(double qx, double qy, double qz, int q, double px, double py, double pz, int p) {
+    const bool le = qx <= px && qy <= py && qz <= pz;
+    const bool eq = qx == px && qy == py && qz == pz;
+    return le && (!eq || q < p);
+}
+
+template <bool STAGED>
+__device__ void rank_segment(const double* __restrict__ pts, int n, int cap, double* smem, int32_t* __restrict__ rank) {
+    double* sx = smem;
+    double* sy = sx + cap;
+    double* sz = sy + cap;
+    int32_t* cnt = reinterpret_cast<int32_t*>(sz + cap);
+    int16_t* lists = reinterpret_cast<int16_t*>(cnt + RANK_MAX);  // front list i at lists + i * RANK_MAX
+    int32_t* len = reinterpret_cast<int32_t*>(lists + 2 * RANK_MAX);
+    auto get = [&](int i, double& x, double& y, double& z) {
+        if (STAGED) {
+            x = sx[i]; y = sy[i]; z = sz[i];
+        } else {
+            x = pts[3 * i]; y = pts[3 * i + 1]; z = pts[3 * i + 2];
+            if (!finite3(x, y, z)) x = y = z = __longlong_as_double(0x7ff8000000000000LL);
+        }
+    };
+    if (STAGED) {
+        for (int i = threadIdx.x; i < n; i += RANK_THREADS) {
+            double x = pts[3 * i], y = pts[3 * i + 1], z = pts[3 * i + 2];
+            if (!finite3(x, y, z)) x = y = z = __longlong_as_double(0x7ff8000000000000LL);
+            sx[i] = x; sy[i] = y; sz[i] = z;
+        }
+    }
+    if (threadIdx.x == 0) len[0] = len[1] = 0;
+    __syncthreads();
+    // domination counts; front 0 straight away
+    for (int p = threadIdx.x; p < n; p += RANK_THREADS) {
+        double px, py, pz;
+        get(p, px, py, pz);
+        if (isnan(px)) {
+            rank[p] = INT32_MAX;
+            cnt[p] = -1;
+            continue;
+        }
+        int c = 0;
+        for (int q = 0; q < n; ++q) {
+            double qx, qy, qz;
+            get(q, qx, qy, qz);
+            c += beats(qx, qy, qz, q, px, py, pz, p);
+        }
+        cnt[p] = c;
+        if (c == 0) {
+            lists[atomicAdd(&len[0], 1)] = (int16_t)p;
+            rank[p] = 0;
+            cnt[p] = -1;
+        }
+    }
+    __syncthreads();
+    int L = len[0];
+    for (int f = 0; L > 0; ++f) {
+        const int cur = f & 1;
+        const int16_t* fr = lists + cur * RANK_MAX;
+        // thread p owns cnt[p] for the whole peel
+        for (int p = threadIdx.x; p < n; p += RANK_THREADS) {
+            if (cnt[p] <= 0) continue;
+            double px, py, pz;
+            get(p, px, py, pz);
+            int d = 0;
+            for (int k = 0; k < L; ++k) {
+                const int q = fr[k];
+                double qx, qy, qz;
+                get(q, qx, qy, qz);
+                d += beats(qx, qy, qz, q, px, py, pz, p);
+            }
+            if (d == 0) continue;
+            if (cnt[p] == d) {
+                lists[(cur ^ 1) * RANK_MAX + atomicAdd(&len[cur ^ 1], 1)] = (int16_t)p;
+                rank[p] = f + 1;
+                cnt[p] = -1;
+            } else {
+                cnt[p] -= d;
+            }
+        }
+        // Every thread read this round's L = len[cur] before starting the round, so before this barrier; the barrier
+        // also ends the appends to len[cur ^ 1].  After it, len[cur] may be cleared for the next round's appends, and
+        // the second barrier orders the clear before them and every read of len[cur ^ 1] before the next round's clear.
+        __syncthreads();
+        if (threadIdx.x == 0) len[cur] = 0;
+        L = len[cur ^ 1];
+        __syncthreads();
+    }
+}
+
+// grid S; segment s ranked in shared memory when it has at most `cap` points, else read from global memory
+__global__ void __launch_bounds__(RANK_THREADS) pareto_rank_kernel(const double* __restrict__ obj3,
+                                                                  const int64_t* __restrict__ seg, int cap,
+                                                                  int32_t* __restrict__ rank) {
+    extern __shared__ double rsmem[];
+    const int s = blockIdx.x;
+    const int64_t b0 = seg[s], len = seg[s + 1] - b0;
+    if (len <= 0) return;
+    if (len > RANK_MAX) {
+        for (int64_t i = threadIdx.x; i < len; i += RANK_THREADS) rank[b0 + i] = -2;
+        return;
+    }
+    if (len <= cap) rank_segment<true>(obj3 + 3 * b0, (int)len, cap, rsmem, rank + b0);
+    else rank_segment<false>(obj3 + 3 * b0, (int)len, cap, rsmem, rank + b0);
+}
+
 }  // namespace
 
 extern "C" {
@@ -168,6 +284,17 @@ int mtfjsp_hypervolume3(const double* obj3, const int64_t* seg, int S, const dou
     if (S == 0) return MTFJSP_OK;
     CK(opt_in_smem(hypervolume3_kernel, HV_SMEM), __func__);
     hypervolume3_kernel<<<(unsigned)S, HV_THREADS, HV_SMEM, (cudaStream_t)stream>>>(obj3, seg, ref3, hv);
+    return launched(__func__);
+}
+
+int mtfjsp_pareto_rank(const double* obj3, const int64_t* seg, int S, int64_t max_len, int32_t* rank, void* stream) {
+    if (!obj3 || !seg || !rank || S < 0 || max_len < 0) return fail(MTFJSP_E_ARG, "mtfjsp_pareto_rank: bad argument");
+    if (S == 0) return MTFJSP_OK;
+    // coordinates staged for segments up to max_len points (at least one, at most RANK_MAX); longer ones read global
+    const int cap = (int)(max_len < 1 ? 1 : (max_len > RANK_MAX ? RANK_MAX : max_len));
+    const size_t smem = (size_t)cap * 3 * sizeof(double) + RANK_FIXED_SMEM;
+    CK(opt_in_smem(pareto_rank_kernel, smem), __func__);
+    pareto_rank_kernel<<<(unsigned)S, RANK_THREADS, smem, (cudaStream_t)stream>>>(obj3, seg, cap, rank);
     return launched(__func__);
 }
 

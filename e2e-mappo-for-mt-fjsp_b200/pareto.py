@@ -3,17 +3,20 @@ time tt (the three the reward weights (w_mk, w_ec, w_tt) name).
 
 Every method of the package scores a schedule by one weighted sum; this module keeps the cost vectors apart.  A set of
 points is given in CSR form: obj [P,3] f64 and seg [S+1] int64 offsets, segment s = one instance's points
-obj[seg[s]:seg[s+1]].  The two hot operations are kernels of csrc/mtfjsp_pareto.cu:
+obj[seg[s]:seg[s+1]].  The hot operations are kernels of csrc/mtfjsp_pareto.cu:
 
   pareto_filter   the non-dominated points of every segment (mtfjsp_pareto_filter): O(P^2) comparisons per segment, the
                   comparison points streamed through shared memory; of equal points the first is kept;
   hypervolume     the exact hypervolume of every segment inside a per-segment reference point (mtfjsp_hypervolume3), a
-                  z-slice sweep of one block per segment, up to 4,096 points.
+                  z-slice sweep of one block per segment, up to 4,096 points;
+  pareto_rank     the non-dominated-sorting front of every point (mtfjsp_pareto_rank), Deb's domination counts peeled
+                  front by front in one block per segment, up to 4,096 points; rank 0 is pareto_filter's keep.
 
-`pareto_filter_reference` and `hypervolume3_reference` restate both in numpy, expression for expression and in the same
-order; they are the specification the kernels are tested against.  `front` and `hypervolume_table` apply the kernels to
-the [K,S,4] cost layouts the validators return; `crowding_truncate` is the NSGA-II crowding-distance cut the Pareto local
-search (search.pareto_local_search) uses to bound its archive.
+`pareto_filter_reference`, `hypervolume3_reference` and `pareto_rank_reference` restate them in numpy, expression for
+expression and in the same order; they are the specification the kernels are tested against.  `front` and
+`hypervolume_table` apply the kernels to the [K,S,4] cost layouts the validators return; `crowding_truncate` is the
+NSGA-II crowding-distance cut the Pareto local search (search.pareto_local_search) uses to bound its archive, and
+`crowding_distance` the distance evolve.nsga2 selects by.
 """
 from __future__ import annotations
 
@@ -78,6 +81,23 @@ def hypervolume(obj, seg, ref):
         o = torch.zeros((1, 3), dtype=torch.float64, device=o.device)
     check(_lib.lib().mtfjsp_hypervolume3(_ptr(o), _ptr(sg), S, _ptr(r), _ptr(hv), _stream()), "mtfjsp_hypervolume3")
     return hv
+
+
+def pareto_rank(obj, seg, max_len=None):
+    """Non-dominated sorting rank of every point within its segment (mtfjsp_pareto_rank): int32 [P] on the device, 0 for
+    the first front.  q beats p when both are finite, q <= p in every component and q != p or q has the lower index (the
+    filter's relation); a point's rank is 0 when nothing beats it, else 1 + the largest rank of the points that beat it.
+    INT32_MAX for a non-finite point, -2 for every point of a segment of more than 4,096.  obj [P,3], seg [S+1] as
+    pareto_filter; max_len, the longest segment if known (else one synchronisation reads it), only sizes the launch."""
+    o, sg = _segments(obj, seg)
+    S = sg.shape[0] - 1
+    if max_len is None:
+        max_len = int((sg[1:] - sg[:-1]).max()) if S else 0
+    rank = torch.empty((o.shape[0],), dtype=torch.int32, device=o.device)
+    if o.shape[0] == 0:
+        return rank
+    check(_lib.lib().mtfjsp_pareto_rank(_ptr(o), _ptr(sg), S, int(max_len), _ptr(rank), _stream()), "mtfjsp_pareto_rank")
+    return rank
 
 
 def _layout(final4):
@@ -201,6 +221,39 @@ def pareto_filter_reference(obj, seg):
             dom[c0:c0 + 512] |= (le & (~eq | (idx[None, :] < idx[c0:c0 + 512, None]))).any(1)
         keep[a:b] = ~dom
     return keep
+
+
+def pareto_rank_reference(obj, seg):
+    """numpy restatement of mtfjsp_pareto_rank: rank [P] int32, by domination counts peeled front by front."""
+    obj = np.asarray(obj, dtype=np.float64)
+    seg = np.asarray(seg, dtype=np.int64)
+    rank = np.zeros(obj.shape[0], dtype=np.int32)
+    for s in range(len(seg) - 1):
+        a, b = int(seg[s]), int(seg[s + 1])
+        if b <= a:
+            continue
+        if b - a > HV_MAX_POINTS:
+            rank[a:b] = -2
+            continue
+        p = obj[a:b]
+        fin = np.isfinite(p).all(axis=1)
+        q = np.where(fin[:, None], p, np.nan)                               # non-finite: beats nothing
+        idx = np.arange(b - a)
+        le = (q[:, None, :] <= q[None, :, :]).all(-1)                       # [q, p]
+        eq = (q[:, None, :] == q[None, :, :]).all(-1)
+        beats = le & (~eq | (idx[:, None] < idx[None, :]))
+        cnt = beats.sum(0)
+        r = np.full(b - a, np.iinfo(np.int32).max, dtype=np.int32)
+        front = fin & (cnt == 0)
+        f = 0
+        while front.any():
+            r[front] = f
+            cnt = cnt - beats[front].sum(0)
+            cnt[front] = -1
+            front = fin & (cnt == 0)
+            f += 1
+        rank[a:b] = r
+    return rank
 
 
 def hypervolume3_reference(obj, seg, ref):

@@ -437,6 +437,37 @@ int mtfjsp_pareto_filter(const double* obj3, const int64_t* seg, int S, int64_t 
  * 4096 points or a ref3 row not finite and > 0 in every component.
  * MTFJSP_E_ARG, nothing written: a NULL pointer or S < 0. */
 int mtfjsp_hypervolume3(const double* obj3, const int64_t* seg, int S, const double* ref3, double* hv, void* stream);
+/* mtfjsp_pareto_rank: rank[p] = the non-dominated-sorting front of point p within its segment, 0 for the first.  q
+ * beats p when both are finite, q <= p in every component, and q != p or q < p (the filter's relation, a strict partial
+ * order: of equal points the later falls to a later front).  rank is 0 when nothing beats p, else 1 + the largest rank
+ * of the points that beat it, so rank == 0 is the filter's keep bit for bit.  INT32_MAX for a non-finite point; -2 for
+ * every point of a segment of more than 4096 points.  Pure comparisons: exact.  max_len only sizes the launch (segments
+ * up to max_len points are ranked in shared memory, longer ones from global memory).  One block per segment.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer, S < 0 or max_len < 0. */
+int mtfjsp_pareto_rank(const double* obj3, const int64_t* seg, int S, int64_t max_len, int32_t* rank, void* stream);
+
+/* Variation of (op, machine) sequences for evolutionary search (evolve.py).  Handle-free, asynchronous on `stream`.
+ * t [S,N,M] f64 processing times of the S instances (t < 0: machine infeasible for the op), N = J*M; parents [P,N,2] and
+ * children [C,N,2] int32 (op, machine) sequences, one contiguous run per sequence; pair [C,2] int32 the parent indices
+ * of each child, inst [C] int32 its instance.  A child works on the job-sequence view (position s holds job op_s / M,
+ * each op's machine apart) and is decoded with op = j*M + the number of earlier occurrences of j: every child of valid
+ * parents is a complete valid sequence.  Draw k of child c is u = splitmix64(seed ^ splitmix64(c * 0x100000001B3 +
+ * k * 0x9E3779B97F4A7C15)) >> 11, times 2^-53; an integer draw below n is min(floor(u * n), n - 1).
+ *   pair[c,0] >= 0: POX -- job j is kept when draw j < 0.5 (j < J); positions of kept jobs take parent 1's entries, the
+ *     others parent 2's non-kept jobs in parent 2's order; op o's machine is parent 1's when draw J + o < 0.5, else
+ *     parent 2's.  Then with draw J+N < p_swap, positions draws J+N+1 and J+N+2 (below N) of the job sequence swap;
+ *     op o with draw J+N+3+2o < p_mach takes the (draw J+N+4+2o below F)-th of its F feasible machines in machine order.
+ *   pair[c,0] == -1: a random child -- draws [1, N) shuffle the job sequence 0..0 1..1 ... (each job M times) by
+ *     Fisher-Yates (for i = N-1 down to 1, swap i with draw i below i+1), op o takes the (draw N+o below F)-th feasible
+ *     machine; no mutation.
+ * A child whose pair[c,0] is outside [-1, P), whose pair[c,1] is outside [0, P) when pair[c,0] >= 0, whose inst[c] is
+ * outside [0, S), or one of whose parents holds an op outside [0, N) or a machine outside [0, M), is all -1; the other
+ * children are unaffected.  Parents that are in range but not valid sequences give unspecified children.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer, S, P or C < 0, or (J, M) outside mtfjsp_create's range (J >= 1,
+ * 2 <= M <= 64, N <= 4096). */
+int mtfjsp_offspring(const double* t, int S, int J, int M, const int32_t* parents, int P, const int32_t* pair,
+                     const int32_t* inst, int C, uint64_t seed, double p_swap, double p_mach, int32_t* children,
+                     void* stream);
 
 /* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
  * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
