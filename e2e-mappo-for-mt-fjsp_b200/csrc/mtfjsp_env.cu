@@ -2700,6 +2700,188 @@ __global__ void __launch_bounds__(256) replay_kernel(const __grid_constant__ Rep
     }
 }
 
+// Episode completion (mtfjsp_complete): candidate r starts from the CURRENT state of env src[r], runs T forced (op,
+// machine) actions, then lets a base policy pick every further action until the schedule is complete, and leaves the
+// costs, the summed rewards, the index of its first invalid action and the base policy's actions.  replay_kernel's shape:
+// one warp per candidate in env_kernel's shared-memory slice, the forced actions read 32 at a time, every transition by
+// env_transition / env_estimates / env_reward on the staged copy.  The base decision is made in the warp, one job per
+// lane: the job mask is env_kernel's rule (restated, not shared: env_kernel's SASS stays as it is), the random base makes
+// policy_kernel's draws keyed by (seed, r, ops scheduled), the priority base takes the open job whose candidate op has the
+// smallest key (ties to the lowest job).  An invalid base action ends the run.  Nothing of the handle is written.
+struct CompleteArgs {
+    Layout L;
+    PwPlan pw;
+    const double *sd, *xs, *t, *p;
+    const int16_t* si;
+    const int32_t *src, *actions;
+    int R, T, base, mask_mode;
+    const double* key;
+    const int32_t* key_mach;
+    uint64_t seed;
+    double cfgw[3], divisor;
+    double *cost4, *return5;
+    int32_t *first_invalid, *base_actions;
+};
+
+// a priority key as an unsigned integer of the same order (-0.0 counts as +0.0, NaN above +inf)
+__device__ __forceinline__ unsigned long long key_order(double x) {
+    if (x != x) return ~0ull;
+    const unsigned long long u = (unsigned long long)__double_as_longlong(x + 0.0);
+    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+
+__global__ void __launch_bounds__(256) complete_kernel(const __grid_constant__ CompleteArgs A) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const Layout& L = A.L;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int r = blockIdx.x * L.warps_per_block + warp;
+    if (r >= A.R) return;
+    const int N = L.N, M = L.M, J = L.J;
+    const int src = A.src[r];
+    int32_t* bact = A.base_actions ? A.base_actions + (size_t)r * N * 2 : nullptr;
+    if (src < 0 || src >= L.B) {  // a source index is data: -2, zero rows and no base actions
+        if (A.cost4 && lane < 4) A.cost4[(size_t)r * 4 + lane] = 0.0;
+        if (A.return5 && lane < 5) A.return5[(size_t)r * 5 + lane] = 0.0;
+        if (A.first_invalid && lane == 0) A.first_invalid[r] = -2;
+        if (bact) for (int i = lane; i < 2 * N; i += 32) bact[i] = -1;
+        return;
+    }
+    const EnvSmem S(L, smem_raw + (size_t)warp * L.smem_per_warp);
+    {
+        const uint4* g = reinterpret_cast<const uint4*>(A.sd + (size_t)src * L.sd_stride);
+        uint4* d = reinterpret_cast<uint4*>(S.sd);
+        for (int i = lane; i < L.sd_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.xs + (size_t)src * L.xs_stride);
+        d = reinterpret_cast<uint4*>(S.xs);
+        for (int i = lane; i < L.xs_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.si + (size_t)src * L.si_stride);
+        d = reinterpret_cast<uint4*>(S.si);
+        for (int i = lane; i < L.si_stride / 8; i += 32) d[i] = __ldg(g + i);
+    }
+    __syncwarp();
+    {  // nxt and the ESA key of the live state (what the step kernels derived the handle's masks from)
+        double mkv, env;
+        env_estimates<false>(L, A.pw, S, lane, &mkv, &env);
+    }
+    double ret[5] = {0.0, 0.0, 0.0, 0.0, 0.0};  // lane 0: the step-order sums of the step's reward5
+    int bad = -1;
+    // one transition with its reward summed into ret; false for an invalid action (a no-op)
+    auto run = [&](const int a, const int m) {
+        const StepOut so = env_transition<false>(L, S, A.t, A.p, (size_t)src, a, m, nullptr, nullptr, lane);
+        double r5[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+        if (so.valid) {
+            double mkv, env;
+            env_estimates<true>(L, A.pw, S, lane, &mkv, &env);
+            const StepReward rw = env_reward(L, S, A.cfgw, m, mkv, env, so, lane);
+            r5[0] = rw.total / A.divisor; r5[1] = rw.r_t; r5[2] = rw.r_idle; r5[3] = rw.r_pt; r5[4] = rw.r_tt;
+            __syncwarp();
+        }
+#pragma unroll
+        for (int k = 0; k < 5; k++) ret[k] += r5[k];
+        return so.valid;
+    };
+    const int32_t* act = A.actions + (size_t)r * A.T * 2;
+    int op_l = 0, mach_l = 0;
+    for (int s = 0; s < A.T; s++) {
+        if ((s & 31) == 0) {
+            op_l = s + lane < A.T ? __ldg(act + 2 * (s + lane)) : 0;
+            mach_l = s + lane < A.T ? __ldg(act + 2 * (s + lane) + 1) : 0;
+        }
+        const int a = __shfl_sync(FULL, op_l, s & 31), m = __shfl_sync(FULL, mach_l, s & 31);
+        if (!run(a, m) && bad < 0) bad = s;
+    }
+    const size_t trow = (size_t)src * N;
+    int nb = 0;
+    while (S.misc[2] < N) {
+        // the job mask of the state (env_kernel's rule): fin = finished; ESA as the reference's
+        bool first_missing = false, unfinished = false;
+        double mn = INFINITY;
+        if (A.mask_mode == MTFJSP_MASK_ESA) {
+            for (int j0 = 0; j0 < J; j0 += 32) {
+                const int j = j0 + lane;
+                const int nx = (j < J) ? (int)S.nxt[j] : M;
+                first_missing |= __any_sync(FULL, j < J && nx == 0);
+                unfinished |= __any_sync(FULL, j < J && nx < M);
+            }
+            for (int j = lane; j < J; j += 32) mn = fmin(mn, S.v[j]);
+            mn = warp_min(mn);
+        }
+        auto open = [&](const int j) {
+            if (j >= J) return false;
+            const int nx = S.nxt[j];
+            bool closed = nx == M;
+            if (A.mask_mode == MTFJSP_MASK_ESA) {
+                if (first_missing) closed = nx >= 1;
+                else if (unfinished) closed = S.v[j] != mn;
+            }
+            return !closed;
+        };
+        const uint64_t step = (uint64_t)S.misc[2];
+        int job = -1, a = -1, m = -1;
+        if (A.base == MTFJSP_BASE_RANDOM) {  // policy_kernel's draws: the k-th open job, the km-th feasible machine
+            int n = 0;
+            for (int j0 = 0; j0 < J; j0 += 32) n += __popc(__ballot_sync(FULL, open(j0 + lane)));
+            int k = (int)(((uint64_t)rand_u32(A.seed, (uint64_t)r, step, 0) * (uint64_t)n) >> 32);
+            for (int j0 = 0; j0 < J; j0 += 32) {
+                const unsigned bits = __ballot_sync(FULL, open(j0 + lane));
+                const int c = __popc(bits);
+                if (k < c) { job = j0 + kth_set_bit(bits, k, 32); break; }
+                k -= c;
+            }
+            if (job >= 0) {
+                a = job * M + min((int)S.nxt[job], M - 1);
+                const double* tr = A.t + (trow + a) * M;
+                int nf = 0;
+                for (int m0 = 0; m0 < M; m0 += 32)
+                    nf += __popc(__ballot_sync(FULL, m0 + lane < M && __ldg(tr + m0 + lane) >= 0));
+                int km = (int)(((uint64_t)rand_u32(A.seed, (uint64_t)r, step, 1) * (uint64_t)nf) >> 32);
+                for (int m0 = 0; m0 < M; m0 += 32) {
+                    const unsigned bits = __ballot_sync(FULL, m0 + lane < M && __ldg(tr + m0 + lane) >= 0);
+                    const int c = __popc(bits);
+                    if (km < c) { m = m0 + kth_set_bit(bits, km, 32); break; }
+                    km -= c;
+                }
+            }
+        } else {  // MTFJSP_BASE_PRIORITY: the open job of the smallest (key of its candidate op, job index)
+            unsigned long long bk = ~0ull;
+            int bj = J;
+            for (int j = lane; j < J; j += 32)
+                if (open(j)) {
+                    const unsigned long long kk = key_order(__ldg(A.key + trow + j * M + min((int)S.nxt[j], M - 1)));
+                    if (bj == J || kk < bk) { bk = kk; bj = j; }
+                }
+            unsigned long long wk = bk;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const unsigned long long x = __shfl_xor_sync(FULL, wk, o);
+                wk = x < wk ? x : wk;
+            }
+            job = (int)__reduce_min_sync(FULL, (unsigned)((bj < J && bk == wk) ? bj : J));
+            if (job < J) {
+                a = job * M + min((int)S.nxt[job], M - 1);
+                m = __ldg(A.key_mach + trow + a);
+            }
+        }
+        if (bact && lane == 0) { bact[2 * nb] = a; bact[2 * nb + 1] = m; }
+        const bool ok = run(a, m);
+        nb++;
+        if (!ok) {  // an invalid base action is data: the run ends there
+            if (bad < 0) bad = A.T + nb - 1;
+            break;
+        }
+    }
+    if (bact) for (int i = 2 * nb + lane; i < 2 * N; i += 32) bact[i] = -1;
+    if (lane == 0) {
+        if (A.cost4) {  // costs_kernel's expressions
+            double* c = A.cost4 + (size_t)r * 4;
+            c[0] = S.scal[0]; c[1] = S.scal[1] / (double)L.N; c[2] = S.scal[2]; c[3] = S.scal[3];
+        }
+        if (A.return5)
+            for (int k = 0; k < 5; k++) A.return5[(size_t)r * 5 + k] = ret[k];
+        if (A.first_invalid) A.first_invalid[r] = bad;
+    }
+}
+
 int align_up(int x, int a) { return (x + a - 1) / a * a; }
 
 void build_plan_rec(int off, int n, PwPlan& pw) {
@@ -3461,6 +3643,35 @@ int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actio
     const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
     replay_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
     return counted(h, "replay_kernel");
+}
+
+int mtfjsp_complete(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, int base, const double* key,
+                    const int32_t* key_mach, uint64_t seed, int mask_mode, double* cost4, double* return5,
+                    int32_t* first_invalid, int32_t* base_actions, void* stream) {
+    if (!h || !src || R < 1 || T < 0 || T > h->L.N || (T > 0 && !actions) ||
+        (base != MTFJSP_BASE_RANDOM && base != MTFJSP_BASE_PRIORITY) ||
+        (mask_mode != MTFJSP_MASK_FINISHED && mask_mode != MTFJSP_MASK_ESA) ||
+        (base == MTFJSP_BASE_PRIORITY && (!key || !key_mach)))
+        return fail(MTFJSP_E_ARG, "mtfjsp_complete: bad argument");
+    if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_complete before mtfjsp_reset");
+    const Layout& L = h->L;
+    cudaStream_t s = (cudaStream_t)stream;
+    // a non-step call: a recorded reset runs now, and the next step waits for the completion in full
+    int rc = enter(h, s);
+    if (rc) return rc;
+    const size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
+    CK(opt_in_smem(complete_kernel, smem), "cudaFuncSetAttribute");
+    CompleteArgs A;
+    memset(&A, 0, sizeof A);
+    A.L = L; A.pw = h->pw;
+    A.sd = h->sd; A.xs = h->xs; A.t = h->t; A.p = h->p; A.si = h->si;
+    A.src = src; A.actions = actions; A.R = R; A.T = T; A.base = base; A.mask_mode = mask_mode;
+    A.key = key; A.key_mach = key_mach; A.seed = seed;
+    A.cfgw[0] = h->cfgw[0]; A.cfgw[1] = h->cfgw[1]; A.cfgw[2] = h->cfgw[2]; A.divisor = h->divisor;
+    A.cost4 = cost4; A.return5 = return5; A.first_invalid = first_invalid; A.base_actions = base_actions;
+    const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
+    complete_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
+    return counted(h, "complete_kernel");
 }
 
 int mtfjsp_policy_random(mtfjsp_env* h, uint64_t seed, uint64_t env_offset, int mask_mode, int32_t* op,

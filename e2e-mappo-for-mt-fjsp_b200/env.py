@@ -16,6 +16,7 @@ from ._lib import _ptr, _stream, check
 
 F32, F64 = 0, 1
 MASK_FINISHED, MASK_ESA = 0, 1
+BASE_RANDOM, BASE_PRIORITY = 0, 1
 
 
 def _to_dev(x, device, dtype):
@@ -317,6 +318,52 @@ class BatchedMTFJSPEnv:
         check(self._lib.mtfjsp_replay(self._h, _ptr(src), R, _ptr(act), T, _ptr(final4), _ptr(ret5), _ptr(finv),
                                       _stream()), "mtfjsp_replay")
         return final4, ret5, finv
+
+    # ---- episode completion ------------------------------------------------------------------------------------------
+    def complete(self, src, actions=None, base="random", key=None, mach=None, seed=0, mask_mode=None):
+        """What the rest of the episode costs for R candidates, each from the CURRENT state of env src[r]: T forced actions,
+        then a base policy to the end of the schedule, without changing the env (mtfjsp_complete).  src: [R] integers
+        (duplicates and permutations allowed); actions: None (T = 0) or a [T,R,2] integer (op, machine) tensor on this
+        env's device, T <= N.  base "random": policy_random's draws, keyed by (seed, r, ops scheduled); base "priority":
+        the selectable job whose candidate op c has the smallest key[src[r], c] (ties to the lowest job), on machine
+        mach[src[r], c]; key [B,N] float64 and mach [B,N] integers (rules.priority_table).  Selectable: the mask_mode job
+        mask (default: this env's).  Returns new tensors final4 [R,4] f64 (what `costs` would return), return5 [R,5] f64
+        (the step-order sum of every step's reward5), first_invalid [R] int32 (-1, the index of the first invalid action,
+        T + i for the i-th base action, which ends the run, or -2 where src is outside [0, B), with zero rows) and
+        base_actions [N,R,2] int32 (the base policy's actions in order, -1 after its last)."""
+        _on(self.device, src, actions, key, mach)
+        mm = self.mask_mode if mask_mode is None else mask_mode
+        if src.dim() != 1:
+            raise ValueError("src must have shape [R]")
+        R = int(src.shape[0])
+        if actions is None:
+            T, act = 0, None
+        else:
+            if actions.dim() != 3 or actions.shape[1] != R or actions.shape[2] != 2:
+                raise ValueError("actions must have shape [T, %d, 2]" % R)
+            T = int(actions.shape[0])
+            act = actions.to(torch.int32).transpose(0, 1).contiguous()           # [R,T,2]: one contiguous run per candidate
+            if T == 0:
+                act = None
+        if base == "random":
+            b = BASE_RANDOM
+            key = mach = None
+        elif base == "priority":
+            b = BASE_PRIORITY
+            if key is None or mach is None or tuple(key.shape) != (self.B, self.N) or tuple(mach.shape) != (self.B, self.N):
+                raise ValueError("the priority base needs key and mach of shape [%d, %d]" % (self.B, self.N))
+            key = key.to(torch.float64).contiguous()
+            mach = mach.to(torch.int32).contiguous()
+        else:
+            raise ValueError("base must be 'random' or 'priority'")
+        src = src.to(torch.int32).contiguous()
+        final4 = torch.empty((R, 4), dtype=torch.float64, device=self.device)
+        ret5 = torch.empty((R, 5), dtype=torch.float64, device=self.device)
+        finv = torch.empty((R,), dtype=torch.int32, device=self.device)
+        bact = torch.empty((R, self.N, 2), dtype=torch.int32, device=self.device)
+        check(self._lib.mtfjsp_complete(self._h, _ptr(src), R, _ptr(act), T, b, _ptr(key), _ptr(mach), seed, mm,
+                                        _ptr(final4), _ptr(ret5), _ptr(finv), _ptr(bact), _stream()), "mtfjsp_complete")
+        return final4, ret5, finv, bact.transpose(0, 1)
 
     # ---- views ---------------------------------------------------------------------------------------------------
     def dense_adj(self, dtype=torch.float64):

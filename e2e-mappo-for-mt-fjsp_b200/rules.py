@@ -55,12 +55,16 @@ def _row_mean_positive(x):
     return np.where(cnt > 0, acc / np.maximum(cnt, 1), 0.0)
 
 
-def op_rule(name, t, p, n_job, n_machine):
-    """-> [S,N] op order (0-based op ids, position s = the op scheduled at step s)."""
+def _op_rule_walk(name, t, p, n_job, n_machine):
+    """The op rule's loop (pdrs.py:186-197) -> ([S,N] op order, [S,N] f64 priority key of every op).
+    The key of op j*M + k is the rule's value of job j when that op is next: refer[j] after k subtractions (LWKR), its
+    negation (MWKR), the op index (FIFO); +inf for an op the loop never reaches because its job was finished by
+    refer == 0.  Taking, at every step, the job whose next op has the smallest key, ties to the lowest job, gives the
+    order back."""
     S, N, M = t.shape
     J = n_job
     if name == "FIFO":
-        return np.tile(np.arange(N), (S, 1))
+        return np.tile(np.arange(N), (S, 1)), np.tile(np.arange(N, dtype=np.float64), (S, 1))
     least = name.startswith("LWKR")
     if name.endswith("_PT"):
         sel = _row_mean_positive(t * np.abs(p))
@@ -70,15 +74,32 @@ def op_rule(name, t, p, n_job, n_machine):
     refer = np.sum(tn, axis=2)                      # np.sum over the job's ops (pairwise order = numpy's)
     nxt = np.zeros((S, J), dtype=np.int64)
     order = np.zeros((S, N), dtype=np.int64)
+    key = np.full((S, N), np.inf)
     ar = np.arange(S)
     for s in range(N):                              # pdrs.py:186-197
         j = np.argmin(refer, axis=1) if least else np.argmax(refer, axis=1)
         order[:, s] = j * M + nxt[ar, j]
+        key[ar, order[:, s]] = refer[ar, j] if least else -refer[ar, j]
         refer[ar, j] = refer[ar, j] - tn[ar, j, nxt[ar, j]]
         nxt[ar, j] += 1
         fin = (refer[ar, j] == 0) | (nxt[ar, j] > M - 1)
         refer[ar, j] = np.where(fin, np.inf if least else -np.inf, refer[ar, j])
-    return order
+    return order, key
+
+
+def op_rule(name, t, p, n_job, n_machine):
+    """-> [S,N] op order (0-based op ids, position s = the op scheduled at step s)."""
+    return _op_rule_walk(name, t, p, n_job, n_machine)[0]
+
+
+def priority_table(op_rule_name, machine_rule_name, t, p, n_job, n_machine):
+    """A static rule pair as priority tables for the device completion (BatchedMTFJSPEnv.complete, base "priority"):
+    key [S,N] f64 and mach [S,N] int32.  From the reset state, with the FINISHED job mask, the priority completion
+    schedules exactly op_rule's order on machine_rule's machines, as evaluate_rules steps them."""
+    t = np.asarray(t, dtype=np.float64)
+    p = np.asarray(p, dtype=np.float64)
+    key = _op_rule_walk(op_rule_name, t, p, n_job, n_machine)[1]
+    return key, machine_rule(machine_rule_name, t, p).astype(np.int32)
 
 
 def lookahead_choice(name, r_idle, invalid):

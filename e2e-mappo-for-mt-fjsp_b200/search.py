@@ -20,6 +20,10 @@ stepping it would give, left shift included.
 `pareto_local_search` walks the same neighbourhood without a weighted sum: it keeps an archive of mutually
 non-dominated schedules per instance over the three targets (pareto.py) and expands it until no member is left
 unexplored.
+
+`pilot_search` is constructive instead: the rollout algorithm (pilot method) on the environment's episode completion
+(BatchedMTFJSPEnv.complete, mtfjsp_complete).  At every decision it lets a base heuristic finish the schedule after each
+candidate action and takes the candidate whose completion is best.
 """
 from __future__ import annotations
 
@@ -27,7 +31,8 @@ import numpy as np
 import torch
 
 from . import pareto
-from .env import BatchedMTFJSPEnv
+from .env import MASK_FINISHED, BatchedMTFJSPEnv
+from .rules import priority_table
 from .validate import _objective
 
 REASSIGN, INSERT = 0, 1
@@ -309,3 +314,134 @@ def pareto_local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=
             "hypervolume": torch.stack(history).cpu().numpy(),
             "truncated": (torch.stack(truncated) if truncated else torch.zeros((0, S), dtype=torch.bool)).cpu().numpy(),
             "replays": replays}
+
+
+def pilot_search(instances, base=("MWKR_T", "SPT"), candidates="all", weights=(0.4, 0.4, 0.2), left_shift=False,
+                 mask_mode=MASK_FINISHED, samples=1, seed=0, max_candidates=65536, device=None):
+    """The pilot method (rollout algorithm) on the instances {"t","p","transT","edge"} [S,...] under the reward weights
+    `weights`, with a base heuristic finishing every candidate's schedule on the device (BatchedMTFJSPEnv.complete).
+
+    base: an (operation rule, machine rule) pair of rules.OP_RULES x rules.MACHINE_RULES, run as its priority table
+    (rules.priority_table), or "random" (policy_random's draws).  One live env of the S instances makes N decisions.  At
+    each, the candidates of an instance are every (candidate op of a selectable job, machine) pair (candidates="all",
+    flat index j*M + m) or the candidate op of every selectable job on the base rule's machine ("rule", flat index j;
+    not for the random base); selectable means open under the `mask_mode` job mask.  One completion per candidate (T = 1,
+    src = its instance; `samples` completions under the random base, the candidate scoring their minimum), at most
+    `max_candidates` per call, scores it by the FP64 objective w_mk*mk + w_ec*(pt + idle) + w_tt*tt of its final costs;
+    a candidate that is not selectable, or whose completion met an invalid action, scores +inf.  The lowest score wins,
+    ties to the lowest flat index, and the live env steps it.  Each instance keeps an incumbent: the best complete
+    sequence seen (ties keep the earlier), built from the pilot's prefix, the candidate and the base's actions.
+    Shapes are static: no decision reads the device; there is one synchronisation at the end.
+
+    With a deterministic base whose own choice is always a candidate (the priority base, under either candidate set),
+    history never increases: the best completion's next action is a candidate at the next decision and completes to the
+    same final state.  With the priority base an instance's result depends neither on the batch nor on max_candidates.
+    With the random base the draws are keyed by (seed, decision, row of the completion call), so an instance's result
+    depends on its row in the batch, as evolve.nsga2's does, and on max_candidates where that splits the candidates
+    over several calls.  left_shift=False (the default) runs the rules as evaluate_rules does, so history[0] equals
+    the rule's row there.
+    -> dict: actions [N,S,2] int32 (the incumbents), final4 [S,4], objective [S] (= history.min(0)), history [N+1,S]
+       (history[0] the base's own completion from the start, history[k+1] the best candidate score at decision k),
+       base_objective [S] (= history[0]), completions (completion runs) and env_steps (steps they took)."""
+    t = np.asarray(instances["t"], dtype=np.float64)
+    p = np.asarray(instances["p"], dtype=np.float64)
+    S, N, M = t.shape
+    J, E = N // M, np.asarray(instances["edge"]).shape[1]
+    Q = int(samples)
+    if candidates not in ("all", "rule"):
+        raise ValueError("candidates must be 'all' or 'rule'")
+    if isinstance(base, str):
+        if base != "random":
+            raise ValueError("base must be 'random' or an (operation rule, machine rule) pair")
+        if candidates == "rule":
+            raise ValueError("candidates='rule' needs a rule pair as the base")
+        kind = "random"
+    else:
+        kind = "priority"
+        if Q != 1:
+            raise ValueError("samples applies to the random base only")
+    if Q < 1 or max_candidates < 1:
+        raise ValueError("samples and max_candidates must be >= 1")
+    env = BatchedMTFJSPEnv(S, J, M, E, left_shift=left_shift, weights=weights, device=device, obs_dtype=torch.float32,
+                           mask_mode=mask_mode)
+    dev = env.device
+    env.load(t, p, np.asarray(instances["transT"]), np.asarray(instances["edge"]))
+    env.scaler_init()
+    env.reset(np.tile(np.asarray(weights, dtype=np.float64), (S, 1)))
+    key = mach_tab = None
+    if kind == "priority":
+        k_np, m_np = priority_table(base[0], base[1], t, p, J, M)
+        key, mach_tab = torch.as_tensor(k_np, device=dev), torch.as_tensor(m_np, device=dev)
+    C = J * M if candidates == "all" else J
+    inst = torch.arange(S, device=dev)
+    env_steps = torch.zeros((), dtype=torch.int64, device=dev)
+    completions = 0
+
+    def best_completion(per, act, closed, k):
+        """Completions of S * per rows, row r from instance r // per, forced actions act [T, S*per, 2] or None; closed
+        [S*per] bool rows scoring +inf, or None.  -> per instance the lowest score, its row (the lowest of equal
+        scores), final4 [S,4] and base actions [N,S,2]."""
+        nonlocal env_steps, completions
+        R = S * per
+        ds = int(np.random.SeedSequence([int(seed), k]).generate_state(1, dtype=np.uint64)[0])
+        src = torch.arange(R, device=dev, dtype=torch.int32) // per
+        b_obj = torch.full((S,), float("inf"), dtype=torch.float64, device=dev)
+        b_row = torch.zeros((S,), dtype=torch.int64, device=dev)
+        b_f4 = torch.zeros((S, 4), dtype=torch.float64, device=dev)
+        b_act = torch.full((N, S, 2), -1, dtype=torch.int32, device=dev)
+        for c0 in range(0, R, max_candidates):
+            c1 = min(R, c0 + max_candidates)
+            f4, _, fi, ba = env.complete(src[c0:c1], None if act is None else act[:, c0:c1], base=kind, key=key,
+                                         mach=mach_tab, seed=ds, mask_mode=mask_mode)
+            T = 0 if act is None else act.shape[0]
+            env_steps += (ba[..., 0] >= 0).sum() + T * (c1 - c0)
+            ok = fi == -1
+            if closed is not None:
+                ok &= ~closed[c0:c1]
+            o = torch.where(ok, _objective(f4, weights), float("inf"))
+            si = src[c0:c1].long()
+            cmin = torch.full((S,), float("inf"), dtype=torch.float64, device=dev).scatter_reduce(0, si, o, "amin")
+            rows = torch.arange(c0, c1, device=dev)
+            crow = torch.full((S,), R, dtype=torch.int64, device=dev).scatter_reduce(
+                0, si, torch.where(o == cmin[si], rows, R), "amin")
+            better = cmin < b_obj                                             # a later chunk's equal score has a later row
+            loc = torch.clamp(crow - c0, 0, c1 - c0 - 1)
+            b_obj = torch.where(better, cmin, b_obj)
+            b_row = torch.where(better, crow, b_row)
+            b_f4 = torch.where(better[:, None], f4[loc], b_f4)
+            b_act = torch.where(better[None, :, None], ba[:, loc], b_act)
+            completions += c1 - c0
+        return b_obj, b_row, b_f4, b_act
+
+    obj0, _, inc_f4, inc_act = best_completion(Q, None, None, 0)
+    inc_obj = obj0
+    history = [obj0]
+    env.obs(mask_mode)
+    acts = torch.full((N, S, 2), -1, dtype=torch.int32, device=dev)
+    jj = torch.arange(C, device=dev) // M if candidates == "all" else torch.arange(C, device=dev)
+    for k in range(N):
+        cand = env.candidate                                                   # [S,J], current after obs / step_obs
+        closed = env.job_mask.bool()
+        op = cand[:, jj]                                                       # [S,C]
+        if candidates == "all":
+            mc = (torch.arange(C, device=dev) % M).to(torch.int32).expand(S, C)
+        else:
+            mc = torch.gather(mach_tab, 1, op.long())
+        pair = torch.stack((op, mc), 2).repeat_interleave(Q, dim=1).reshape(1, S * C * Q, 2)
+        cl = closed[:, jj].repeat_interleave(Q, dim=1).reshape(S * C * Q)
+        b_obj, b_row, b_f4, b_act = best_completion(C * Q, pair, cl, k + 1)
+        c = (b_row % (C * Q)) // Q
+        a = torch.stack((op[inst, c], mc[inst, c]), 1)                         # [S,2]
+        new = torch.cat((acts[:k], a[None], b_act[:N - k - 1]))
+        better = b_obj < inc_obj
+        inc_act = torch.where(better[None, :, None], new, inc_act)
+        inc_f4 = torch.where(better[:, None], b_f4, inc_f4)
+        inc_obj = torch.where(better, b_obj, inc_obj)
+        history.append(b_obj)
+        acts[k] = a
+        env.step_obs(a[:, 0].contiguous(), a[:, 1].contiguous(), mask_mode)
+    out = {"actions": inc_act.cpu().numpy(), "final4": inc_f4.cpu().numpy(), "objective": inc_obj.cpu().numpy(),
+           "history": torch.stack(history).cpu().numpy(), "base_objective": obj0.cpu().numpy(),
+           "completions": completions, "env_steps": int(env_steps.item())}
+    env.close()
+    return out

@@ -188,6 +188,34 @@ int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, do
 int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, double* cost4, double* return5,
                   int32_t* first_invalid, void* stream);
 
+/* Episode completion: for R candidates, what the rest of the episode costs when T forced actions and then a base policy
+ * finish the schedule, without changing the handle.  Candidate r starts from the CURRENT state of env src[r] (src [R]
+ * int32; duplicates and permutations allowed), runs actions [R,T,2] int32 (op, machine), 0 <= T <= N (NULL when T = 0;
+ * an invalid forced action is a no-op, as in mtfjsp_step, and the run goes on), then one base action at a time until
+ * every op is scheduled.  The selectable jobs are those the mask_mode job mask leaves open after the same steps (the
+ * mask mtfjsp_policy_random reads).
+ *   MTFJSP_BASE_RANDOM: mtfjsp_policy_random's draws with env_offset 0 and env index r: the k-th selectable job by
+ *     draw (seed, r, ops scheduled, stream 0), the k-th feasible machine by stream 1.  key / key_mach are not read.
+ *   MTFJSP_BASE_PRIORITY: the selectable job whose candidate op c has the smallest key[src[r], c] ([B,N] f64; -0.0 equals
+ *     +0.0, NaN ranks above +inf), ties to the lowest job index, on machine key_mach[src[r], c] ([B,N] int32).
+ * A base action that is invalid (e.g. an infeasible key_mach entry) is data: the completion stops there.
+ * Outputs, any of which may be NULL: cost4 [R,4] f64 what mtfjsp_costs would return after the run; return5 [R,5] f64 the
+ * step-order FP64 sum, from 0.0, of the reward5 of every step, forced and base; first_invalid [R] int32 -1 if every action
+ * was valid, else the index of the first invalid one (T + i for the i-th base action); base_actions [R,N,2] int32 the
+ * base policy's actions in order, padded with -1.  The bits equal those of: mtfjsp_gather into an R-env handle with
+ * idx = src, T mtfjsp_step calls with the forced actions, then mtfjsp_policy_random(seed, 0, mask_mode) (or the priority
+ * choice) and mtfjsp_step until done, then mtfjsp_costs.  A src[r] outside [0, B) is data: -2 in first_invalid, zero
+ * rows in cost4 / return5 and -1 in base_actions.
+ * Read-only: nothing of the handle is written.  A non-step call: a recorded reset (mtfjsp_reset) is performed first, and
+ * the next step waits for the completion in full.
+ * MTFJSP_E_ARG, nothing written: a NULL handle or src, R < 1, T outside [0, N], T > 0 with NULL actions, a bad base or
+ * mask_mode, or MTFJSP_BASE_PRIORITY with a NULL key or key_mach.  MTFJSP_E_STATE, nothing written: before the first
+ * mtfjsp_reset since mtfjsp_load. */
+enum { MTFJSP_BASE_RANDOM = 0, MTFJSP_BASE_PRIORITY = 1 };
+int mtfjsp_complete(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, int base, const double* key,
+                    const int32_t* key_mach, uint64_t seed, int mask_mode, double* cost4, double* return5,
+                    int32_t* first_invalid, int32_t* base_actions, void* stream);
+
 /* Uniform random valid action from the env's current masks: a selectable job (under mask_mode), its candidate
  * op, and a feasible machine for it; counter-based, keyed by (seed, env_offset + env, ops scheduled so far).
  * Mirrors tester/pdrs.py Random_task / Random_m (:75-86, :139-156).  op, mach [B] int32 (-1 when done). */
