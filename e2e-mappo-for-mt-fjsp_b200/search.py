@@ -31,7 +31,8 @@ import numpy as np
 import torch
 
 from . import pareto
-from .env import MASK_FINISHED, BatchedMTFJSPEnv
+from ._lib import _ptr, _stream, check, lib
+from .env import MASK_ESA, MASK_FINISHED, BatchedMTFJSPEnv
 from .rules import priority_table
 from .validate import _objective
 
@@ -443,5 +444,349 @@ def pilot_search(instances, base=("MWKR_T", "SPT"), candidates="all", weights=(0
     out = {"actions": inc_act.cpu().numpy(), "final4": inc_f4.cpu().numpy(), "objective": inc_obj.cpu().numpy(),
            "history": torch.stack(history).cpu().numpy(), "base_objective": obj0.cpu().numpy(),
            "completions": completions, "env_steps": int(env_steps.item())}
+    env.close()
+    return out
+
+
+# ---- Monte Carlo tree search on the episode completion ------------------------------------------------------------------
+# node fields of a tree pool (include/mtfjsp.h, mtfjsp_mcts_select)
+PARENT, FIRST, NCHILD, OP, MACH, VISITS, VIRTUAL = range(7)
+
+
+def mcts_trees(S, max_nodes, device=None):
+    """S fresh trees of max_nodes nodes each, as mtfjsp_mcts_select / mtfjsp_mcts_backup read them: node [S,P,7] int32,
+    vmin [S,P] f64, root [S] and count [S] int32, lohi [S,2] f64.  Node 0 is every tree's root; nothing is scored.
+    device None: torch tensors on the current CUDA device; "numpy": numpy arrays (mcts_reference's form)."""
+    P = int(max_nodes)
+    if device == "numpy":
+        xp, kw = np, {}
+    else:
+        xp, kw = torch, {"device": torch.device("cuda", torch.cuda.current_device()) if device is None else device}
+    node = xp.zeros((S, P, 7), dtype=xp.int32, **kw)
+    node[..., PARENT] = -1
+    node[..., FIRST] = -1
+    node[..., OP] = -1
+    node[..., MACH] = -1
+    lohi = xp.zeros((S, 2), dtype=xp.float64, **kw)
+    lohi[:, 0], lohi[:, 1] = float("inf"), float("-inf")
+    return {"node": node, "vmin": xp.full((S, P), float("inf"), dtype=xp.float64, **kw),
+            "root": xp.zeros(S, dtype=xp.int32, **kw), "count": xp.ones(S, dtype=xp.int32, **kw), "lohi": lohi}
+
+
+def mcts_select(t, next_op, tree, leaves, c, mach=None, max_depth=None):
+    """One round of `leaves` selections per tree on the device (mtfjsp_mcts_select).  t [S,N,M] f64 and next_op [S,J]
+    int32 (the root's next op index of every job, M when finished) on the trees' device; mach [S,N] int32 for the "rule"
+    candidates, None for "all".  Updates `tree` in place.  -> paths [S*L, D, 2] int32 (D = max_depth, default N),
+    depth [S*L] and leaf [S*L] int32."""
+    node = tree["node"]
+    S, P = node.shape[0], node.shape[1]
+    N, M = t.shape[1], t.shape[2]
+    J = N // M
+    L, D = int(leaves), N if max_depth is None else int(max_depth)
+    dev = node.device
+    paths = torch.empty((S * L, D, 2), dtype=torch.int32, device=dev)
+    depth = torch.empty((S * L,), dtype=torch.int32, device=dev)
+    leaf = torch.empty((S * L,), dtype=torch.int32, device=dev)
+    t = t.to(torch.float64).contiguous()
+    nx = next_op.to(torch.int32).contiguous()
+    m = None if mach is None else mach.to(torch.int32).contiguous()
+    check(lib().mtfjsp_mcts_select(_ptr(t), _ptr(m), S, J, M, _ptr(nx), L, P, D, float(c), _ptr(node), _ptr(tree["vmin"]),
+                                   _ptr(tree["root"]), _ptr(tree["count"]), _ptr(tree["lohi"]), _ptr(paths), _ptr(depth),
+                                   _ptr(leaf), _stream()), "mtfjsp_mcts_select")
+    return paths, depth, leaf
+
+
+def mcts_backup(tree, leaf, objective):
+    """Backs the round's S*L objectives (f64, +inf for a failed completion) up the paths ending at `leaf`
+    (mtfjsp_mcts_backup).  Updates `tree` in place."""
+    node = tree["node"]
+    S, P = node.shape[0], node.shape[1]
+    L = leaf.shape[0] // S
+    obj = objective.to(torch.float64).contiguous()
+    check(lib().mtfjsp_mcts_backup(S, L, P, _ptr(leaf), _ptr(obj), _ptr(node), _ptr(tree["vmin"]), _ptr(tree["root"]),
+                                   _ptr(tree["count"]), _ptr(tree["lohi"]), _stream()), "mtfjsp_mcts_backup")
+
+
+def _ref_children(ts, rule, nx, M):
+    """(op, machine) children of a node, in flat-index order, from its per-job next op index nx."""
+    out = []
+    for j, k in enumerate(nx):
+        if not 0 <= k < M:
+            continue
+        op = j * M + int(k)
+        if rule is None:
+            out += [(op, m) for m in range(M) if ts[op, m] >= 0.0]
+        elif 0 <= rule[op] < M and ts[op, rule[op]] >= 0.0:
+            out.append((op, int(rule[op])))
+    return out
+
+
+def _ref_select(t, next_op, tree, L, c, mach, D):
+    node, vm, lohi = tree["node"], tree["vmin"], tree["lohi"]
+    S, P = node.shape[0], node.shape[1]
+    M = t.shape[2]
+    N = t.shape[1]
+    paths = np.full((S * L, D, 2), -1, dtype=np.int32)
+    depth = np.zeros(S * L, dtype=np.int32)
+    leaf = np.zeros(S * L, dtype=np.int32)
+    for s in range(S):
+        nd = node[s]
+        lo, hi = lohi[s, 0], lohi[s, 1]
+        cnt, r0 = int(tree["count"][s]), int(tree["root"][s])
+        ok = 1 <= cnt <= P and 0 <= r0 < cnt
+        for l in range(L):
+            row = s * L + l
+            nx = next_op[s].astype(np.int64).copy()
+            x, d = (r0 if ok else -1), 0
+            while x >= 0:
+                seen = int(nd[x, VISITS]) + int(nd[x, VIRTUAL])
+                fc, nc = int(nd[x, FIRST]), int(nd[x, NCHILD])
+                nd[x, VIRTUAL] += 1
+                if fc == -1 and nc == 0:
+                    if seen == 0 or d >= D:
+                        break
+                    ch = _ref_children(t[s], None if mach is None else mach[s], nx, M)
+                    if not ch or len(ch) > P - cnt:
+                        break
+                    for i, (op, m) in enumerate(ch):
+                        nd[cnt + i] = (x, -1, 0, op, m, 0, 0)
+                        vm[s, cnt + i] = np.inf
+                    nd[x, FIRST], nd[x, NCHILD] = cnt, len(ch)
+                    child = cnt
+                    cnt += len(ch)
+                else:
+                    if fc < 0 or nc < 1 or fc > cnt - nc or d >= D:
+                        break
+                    n, v = nd[fc:fc + nc, VISITS].astype(np.int64), nd[fc:fc + nc, VIRTUAL].astype(np.int64)
+                    fresh = np.nonzero(n + v == 0)[0]
+                    if fresh.size:
+                        child = fc + int(fresh[0])
+                    else:
+                        u = np.float64(c) * np.sqrt(np.float64(seen + 1))
+                        best, bi = None, -1
+                        for i in range(nc):
+                            vc = vm[s, fc + i]
+                            q = np.float64(0.0) if vc == np.inf else (np.float64(1.0) if hi == lo else (hi - vc) / (hi - lo))
+                            sc = q * np.float64(n[i]) / np.float64(n[i] + v[i]) + u / np.float64(1 + n[i] + v[i])
+                            if best is None or sc > best:
+                                best, bi = sc, i
+                        child = fc + bi
+                op, m = int(nd[child, OP]), int(nd[child, MACH])
+                paths[row, d] = (op, m)
+                if 0 <= op < N:
+                    nx[op // M] += 1
+                d += 1
+                x = child
+            depth[row], leaf[row] = d, x
+        tree["count"][s] = cnt
+    return paths, depth, leaf
+
+
+def _ref_backup(tree, leaf, obj):
+    node, vm, lohi = tree["node"], tree["vmin"], tree["lohi"]
+    S = node.shape[0]
+    L = leaf.shape[0] // S
+    for s in range(S):
+        cnt, r0 = min(int(tree["count"][s]), node.shape[1]), int(tree["root"][s])
+        for l in range(L):
+            v, x = np.float64(obj[s * L + l]), int(leaf[s * L + l])
+            if not 0 <= x < cnt:
+                continue
+            for _ in range(cnt):
+                node[s, x, VISITS] += 1
+                node[s, x, VIRTUAL] -= 1
+                if v < vm[s, x]:
+                    vm[s, x] = v
+                if x == r0:
+                    break
+                x = int(node[s, x, PARENT])
+                if not 0 <= x < cnt:
+                    break
+            if np.isfinite(v):
+                lohi[s, 0] = min(lohi[s, 0], v)
+                lohi[s, 1] = max(lohi[s, 1], v)
+
+
+def mcts_reference(t, next_op, tree, leaves, c, objectives, mach=None, max_depth=None):
+    """numpy restatement of mtfjsp_mcts_select and mtfjsp_mcts_backup (include/mtfjsp.h), bit for bit.  For every row of
+    objectives ([R, S*L] f64) one round: `leaves` selections per tree, then the backup of that row.  t [S,N,M], next_op
+    [S,J], mach [S,N] or None ("all"), tree as mcts_trees(..., device="numpy") returns it (copied, not changed).
+    -> paths [R, S*L, D, 2], depth [R, S*L], leaf [R, S*L] (each round's selection) and the tree after the last backup."""
+    t = np.asarray(t, dtype=np.float64)
+    tree = {k: np.array(v, copy=True) for k, v in tree.items()}
+    next_op = np.asarray(next_op)
+    mach = None if mach is None else np.asarray(mach)
+    D = t.shape[1] if max_depth is None else int(max_depth)
+    out = []
+    for obj in np.asarray(objectives, dtype=np.float64).reshape(-1, next_op.shape[0] * int(leaves)):
+        out.append(_ref_select(t, next_op, tree, int(leaves), c, mach, D))
+        _ref_backup(tree, out[-1][2], obj)
+    paths, depth, leaf = (np.stack([o[i] for o in out]) for i in range(3))
+    return paths, depth, leaf, tree
+
+
+def mcts_search(instances, base=("MWKR_T", "SPT"), candidates="all", simulations=256, leaves=64, c=1.0,
+                max_nodes=65536, weights=(0.4, 0.4, 0.2), left_shift=False, mask_mode=MASK_FINISHED, seed=0,
+                max_candidates=65536, device=None):
+    """Monte Carlo tree search over joint (op, machine) actions on the instances {"t","p","transT","edge"} [S,...] under
+    the reward weights `weights`, with leaves scored by the device episode completion (BatchedMTFJSPEnv.complete).
+
+    base and candidates are pilot_search's: an (operation rule, machine rule) pair run as its priority table, or
+    "random"; children are every (candidate op of an open job, feasible machine) pair (candidates="all", flat index
+    j*M + m) or the candidate op of every open job on the base rule's machine ("rule", flat index j; not for the random
+    base).  Open means unfinished: only the FINISHED job mask is supported.  One tree per instance, a pool of max_nodes
+    nodes (mcts_trees; 36 bytes a node).  One live env of the S instances makes N decisions.  Each decision runs
+    ceil(simulations / leaves) rounds of `leaves` selections per tree (mtfjsp_mcts_select: unvisited children first in
+    flat-index order, then the largest q*n/(n+v) + c*sqrt(Np+Vp)/(1+n+v) with q the child's best objective rescaled to
+    [0, 1] by the least and largest the tree has seen, 1 the best), one completion per selected path (its actions forced,
+    padded with (-1, -1) to the round's deepest path; src = its instance; at most max_candidates per call), and the
+    backup of the FP64 objectives w_mk*mk + w_ec*(pt + idle) + w_tt*tt (mtfjsp_mcts_backup).  A node whose child block
+    does not fit in the pool stays a leaf.  The decision commits to the root child of the least vmin (the best objective
+    through it), ties to the most visits, then the lowest index; the live env steps its action and the root moves there,
+    keeping its subtree (no compaction).  A root without children at decision time (its block never fit, or the budget
+    never reached it twice) commits to the first action of the decision's best completion -- the base's own action, as
+    every path of that decision was the root itself -- and the tree restarts from a fresh root.  Each instance keeps an
+    incumbent: the best complete sequence seen (ties keep the earlier), built from the committed prefix, the path and
+    the base's actions.  The host reads the round's deepest path once per round.
+
+    With the priority base and simulations >= C + 1 (C the number of candidates, J*M for "all", J for "rule") every root
+    child is scored before each decision, so history never increases: the root's own completion begins with the base's
+    action, which is a candidate, and that child completes to the same final state, so the least child vmin is at most
+    the root's, and the kept subtree carries the value forward.  Below that budget a child nothing reached has vmin =
+    +inf and history may increase; the incumbent still never gets worse, so objective <= base_objective always.  With
+    the priority base an instance's result depends neither on the batch nor on max_candidates.  With the random base the
+    draws are keyed by (seed, decision, round, row of the completion call), so a result depends on the instance's row
+    and on how max_candidates splits the rows.
+    -> dict: actions [N,S,2] int32 (the incumbents), final4 [S,4], objective [S], history [N+1,S] (history[0] the base's
+       completion from the start, history[k+1] the vmin of the child committed at decision k, or the root's for a root
+       without children), base_objective [S], completions (completion runs), env_steps (steps they took) and nodes [S]
+       (the most pool nodes a tree used at once)."""
+    t = np.asarray(instances["t"], dtype=np.float64)
+    p = np.asarray(instances["p"], dtype=np.float64)
+    S, N, M = t.shape
+    J, E = N // M, np.asarray(instances["edge"]).shape[1]
+    if candidates not in ("all", "rule"):
+        raise ValueError("candidates must be 'all' or 'rule'")
+    if isinstance(base, str):
+        if base != "random":
+            raise ValueError("base must be 'random' or an (operation rule, machine rule) pair")
+        if candidates == "rule":
+            raise ValueError("candidates='rule' needs a rule pair as the base")
+        kind = "random"
+    else:
+        kind = "priority"
+    if mask_mode == MASK_ESA:
+        raise ValueError("mcts_search supports the FINISHED job mask only: the ESA mask needs state estimates per node")
+    if mask_mode != MASK_FINISHED:
+        raise ValueError("mask_mode must be MASK_FINISHED")
+    if int(simulations) < 1 or int(leaves) < 1 or int(max_nodes) < 1 or max_candidates < 1:
+        raise ValueError("simulations, leaves, max_nodes and max_candidates must be >= 1")
+    if not (np.isfinite(c) and c >= 0):
+        raise ValueError("c must be finite and >= 0")
+    L = int(leaves)
+    rounds = -(-int(simulations) // L)
+    env = BatchedMTFJSPEnv(S, J, M, E, left_shift=left_shift, weights=weights, device=device, obs_dtype=torch.float32,
+                           mask_mode=mask_mode)
+    dev = env.device
+    env.load(t, p, np.asarray(instances["transT"]), np.asarray(instances["edge"]))
+    env.scaler_init()
+    env.reset(np.tile(np.asarray(weights, dtype=np.float64), (S, 1)))
+    key = mach_tab = None
+    if kind == "priority":
+        k_np, m_np = priority_table(base[0], base[1], t, p, J, M)
+        key, mach_tab = torch.as_tensor(k_np, device=dev), torch.as_tensor(m_np, device=dev)
+    rule = mach_tab if candidates == "rule" else None
+    C = J * M if candidates == "all" else J
+    t_dev = torch.as_tensor(t, device=dev)
+    tree = mcts_trees(S, max_nodes, dev)
+    inst = torch.arange(S, device=dev)
+    R = S * L
+    src = (torch.arange(R, device=dev) // L).to(torch.int32)
+    steps_n = torch.arange(N, device=dev)[:, None]
+    env_steps = torch.zeros((), dtype=torch.int64, device=dev)
+    bad = torch.zeros((), dtype=torch.bool, device=dev)
+    completions = S
+
+    f4, _, fi, ba = env.complete(inst.to(torch.int32), None, base=kind, key=key, mach=mach_tab,
+                                 seed=int(np.random.SeedSequence([int(seed), 0]).generate_state(1, dtype=np.uint64)[0]),
+                                 mask_mode=mask_mode)
+    env_steps += (ba[..., 0] >= 0).sum()
+    obj0 = torch.where(fi == -1, _objective(f4, weights), float("inf"))
+    inc_obj, inc_f4, inc_act = obj0, f4, ba.clone()
+    history = [obj0]
+    nodes = tree["count"].clone()
+    env.obs(mask_mode)
+    acts = torch.full((N, S, 2), -1, dtype=torch.int32, device=dev)
+    fresh_tree = mcts_trees(1, 1, dev)
+    for k in range(N):
+        next_op = torch.where(env.job_mask.bool(), M,
+                              env.candidate - torch.arange(J, dtype=torch.int32, device=dev) * M).to(torch.int32)
+        dec_obj = torch.full((S,), float("inf"), dtype=torch.float64, device=dev)
+        dec_first = torch.full((S, 2), -1, dtype=torch.int32, device=dev)
+        for rnd in range(rounds):
+            paths, depth, leaf = mcts_select(t_dev, next_op, tree, L, c, rule, N)
+            T = int(depth.max())                                              # the one read of the round
+            act = paths[:, :T].transpose(0, 1) if T else None
+            ds = int(np.random.SeedSequence([int(seed), k + 1, rnd]).generate_state(1, dtype=np.uint64)[0])
+            f4 = torch.empty((R, 4), dtype=torch.float64, device=dev)
+            fi = torch.empty((R,), dtype=torch.int32, device=dev)
+            ba = torch.empty((N, R, 2), dtype=torch.int32, device=dev)
+            for c0 in range(0, R, max_candidates):
+                c1 = min(R, c0 + max_candidates)
+                f4[c0:c1], _, fi[c0:c1], ba[:, c0:c1] = env.complete(
+                    src[c0:c1], None if act is None else act[:, c0:c1], base=kind, key=key, mach=mach_tab, seed=ds,
+                    mask_mode=mask_mode)
+            completions += R
+            env_steps += (ba[..., 0] >= 0).sum() + depth.sum()
+            ok = (fi == -1) | (fi == depth)
+            bad |= ~ok.all()
+            obj = torch.where(ok, _objective(f4, weights), float("inf"))
+            mcts_backup(tree, leaf, obj)
+            nodes = torch.maximum(nodes, tree["count"])
+            # the round's best completion per instance: committed prefix, path, base actions
+            b_obj, b_l = obj.view(S, L).min(1)
+            row = inst * L + b_l
+            d = depth[row].long()[None, :]
+            pth = paths[row].transpose(0, 1)                                  # [N,S,2]
+            via_path = torch.gather(pth, 0, torch.clamp(steps_n - k, 0, N - 1)[..., None].expand(N, S, 2))
+            via_base = torch.gather(ba[:, row], 0, torch.clamp(steps_n - k - d, 0, N - 1)[..., None].expand(N, S, 2))
+            seq = torch.where((steps_n < k)[..., None], acts,
+                              torch.where((steps_n < k + d)[..., None], via_path, via_base))
+            better = b_obj < inc_obj
+            inc_act = torch.where(better[None, :, None], seq, inc_act)
+            inc_f4 = torch.where(better[:, None], f4[row], inc_f4)
+            inc_obj = torch.where(better, b_obj, inc_obj)
+            dbetter = b_obj < dec_obj
+            dec_first = torch.where(dbetter[:, None], seq[k], dec_first)
+            dec_obj = torch.where(dbetter, b_obj, dec_obj)
+        # commit: the root child of the least vmin, ties to the most visits, then the lowest index
+        node, vmin = tree["node"], tree["vmin"]
+        root = tree["root"].long()
+        fc, nc = node[inst, root, FIRST].long(), node[inst, root, NCHILD].long()
+        has = nc > 0
+        ci = torch.arange(C, device=dev)[None, :]
+        valid = ci < nc[:, None]
+        idx = torch.where(valid, fc[:, None] + ci, 0)
+        cv = torch.where(valid, vmin[inst[:, None], idx], float("inf"))
+        cn = torch.where(valid, node[inst[:, None], idx, VISITS], -1)
+        tie = valid & (cv == cv.min(1, keepdim=True)[0])
+        cn = torch.where(tie, cn, -1)
+        pick = (tie & (cn == cn.max(1, keepdim=True)[0])).long().argmax(1)
+        chosen = idx[inst, pick]
+        a = torch.where(has[:, None], node[inst, chosen][:, OP:MACH + 1], dec_first)
+        history.append(torch.where(has, vmin[inst, chosen], vmin[inst, root]))
+        acts[k] = a
+        env.step_obs(a[:, 0].contiguous(), a[:, 1].contiguous(), mask_mode)
+        # move the root, or restart a tree whose root had no child
+        tree["root"] = torch.where(has, chosen, 0).to(torch.int32)
+        tree["count"] = torch.where(has, tree["count"], 1).to(torch.int32)
+        tree["lohi"] = torch.where(has[:, None], tree["lohi"], fresh_tree["lohi"])
+        tree["node"][:, 0] = torch.where(has[:, None], node[:, 0], fresh_tree["node"][:, 0])
+        tree["vmin"][:, 0] = torch.where(has, vmin[:, 0], fresh_tree["vmin"][:, 0])
+    if bool(bad):
+        raise RuntimeError("a completion met an invalid action other than its path's padding")
+    out = {"actions": inc_act.cpu().numpy(), "final4": inc_f4.cpu().numpy(), "objective": inc_obj.cpu().numpy(),
+           "history": torch.stack(history).cpu().numpy(), "base_objective": obj0.cpu().numpy(),
+           "completions": completions, "env_steps": int(env_steps.item()), "nodes": nodes.cpu().numpy()}
     env.close()
     return out

@@ -497,6 +497,42 @@ int mtfjsp_offspring(const double* t, int S, int J, int M, const int32_t* parent
                      const int32_t* inst, int C, uint64_t seed, double p_swap, double p_mach, int32_t* children,
                      void* stream);
 
+/* Monte Carlo tree search over joint (op, machine) actions (search.mcts_search).  Handle-free, asynchronous on `stream`.
+ * S trees, one per instance, each a pool of P = max_nodes nodes in caller-owned device arrays: node [S,P,7] int32 holds
+ * per node (parent, first_child, n_children, op, mach, visits, virtual) -- parent -1 at a tree's first root, first_child
+ * -1 and n_children 0 until the node is expanded, (op, mach) the action of the edge from its parent; vmin [S,P] f64 the
+ * least objective backed up through the node (+inf until then); root [S] and count [S] int32 (nodes in use, node 0 ..
+ * count - 1); lohi [S,2] f64 the least and largest finite objective the tree has seen (+inf, -inf before any).  A node
+ * stands for the state its path of edge actions from the root reaches; no env state is stored.
+ * Children: with rule_mach == NULL, flat index j*M + m for every job j with next op k = next_op[s,j] < M (k = M: finished)
+ * and every machine m with t[s, j*M+k, m] >= 0; with rule_mach [S,N] int32, flat index j on machine rule_mach[s, j*M+k]
+ * when t >= 0 there.  An expanded node's valid children are one contiguous block, in flat-index order, allocated at count.
+ * The job mask is MTFJSP_MASK_FINISHED's.  t [S,N,M] f64, next_op [S,J] int32 the root's state; N = J*M.
+ *
+ * mtfjsp_mcts_select: one warp per tree makes L selections in order l = 0 .. L-1.  A selection starts at the root; at each
+ * node x, with seen = visits + virtual of x read first, virtual[x] += 1, then:
+ *   unexpanded: the path ends at x when seen == 0, at depth max_depth, when x has no valid child (terminal: scored
+ *     again), or when its block does not fit (count + n > P: x stays a leaf); else x is expanded and the walk steps into
+ *     its first child;
+ *   expanded: the lowest child with visits + virtual == 0; if none, the child of the largest score
+ *     q*n/(n+v) + c*sqrt(Nx + Vx)/(1+n+v) (n, v the child's counts; Nx + Vx = seen + 1, x's counts with this path;
+ *     q = 0 for vmin = +inf, else 1 when hi == lo, else (hi - vmin)/(hi - lo); FP64, evaluated in that order, no FMA),
+ *     ties to the lowest child.  At depth max_depth the path ends at x.
+ * paths [S*L, max_depth, 2] int32 receives row s*L + l's edge actions root-first, padded with -1; depth [S*L] its length;
+ * leaf [S*L] its last node (-1 when the tree's root or count is out of range: that tree's rows are all padding and the
+ * tree is not written).  A malformed block (first_child out of [0, count - n_children]) ends the path at its node.
+ * mtfjsp_mcts_backup: one thread per tree takes objective [S*L] f64 (+inf for a failed completion) and, for l = 0 .. L-1
+ * in order, walks from leaf[s*L+l] up the parents to the root: visits += 1, virtual -= 1, vmin = v if v < vmin; then,
+ * if v is finite, lo = min(lo, v) and hi = max(hi, v).  A leaf outside [0, count) is skipped; a parent outside [0,
+ * count) ends the walk.  The serial order makes the trees bit-reproducible.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer (rule_mach may be NULL), S < 1, L < 1, max_nodes < 1, max_depth < 0, or
+ * (J, M) outside mtfjsp_create's range (J >= 1, 2 <= M <= 64, N <= 4096). */
+int mtfjsp_mcts_select(const double* t, const int32_t* rule_mach, int S, int J, int M, const int32_t* next_op, int L,
+                       int max_nodes, int max_depth, double c, int32_t* node, double* vmin, const int32_t* root,
+                       int32_t* count, const double* lohi, int32_t* paths, int32_t* depth, int32_t* leaf, void* stream);
+int mtfjsp_mcts_backup(int S, int L, int max_nodes, const int32_t* leaf, const double* objective, int32_t* node,
+                       double* vmin, const int32_t* root, const int32_t* count, double* lohi, void* stream);
+
 /* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
  * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
  * word: it reflects the launches the device has finished so far (read it after synchronising). */
