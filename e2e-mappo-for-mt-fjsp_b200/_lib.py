@@ -17,7 +17,7 @@ SRC_DIR = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("MTFJSP_LIB") or os.path.join(_HERE, "libmtfjsp_b200.so")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "mtfjsp.h")
 SOURCES = ["mtfjsp_env.cu", "mtfjsp_encoder.cu", "mtfjsp_gemm.cu", "mtfjsp_pareto.cu", "mtfjsp_evolve.cu",
-           "mtfjsp_mcts.cu"]
+           "mtfjsp_mcts.cu", "mtfjsp_tabu.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 # the env kernels restate the reference's FP64 arithmetic operation by operation, and the hypervolume and the MCTS score
 # their numpy specifications: no FMA contraction there
@@ -79,6 +79,7 @@ SIGNATURES = {
     "mtfjsp_gather": ([_VP, _VP, _VP, _VP], _I),
     "mtfjsp_peek": ([_VP, _VP, _VP, _I, _VP, _VP, _VP], _I),
     "mtfjsp_replay": ([_VP, _VP, _I, _VP, _I, _VP, _VP, _VP, _VP], _I),
+    "mtfjsp_replay_moves": ([_VP, _VP, _I, _VP, _VP, _I, _VP, _VP, _VP, _VP], _I),
     "mtfjsp_complete": ([_VP, _VP, _I, _VP, _I, _I, _VP, _VP, _U64, _I, _VP, _VP, _VP, _VP, _VP], _I),
     "mtfjsp_policy_random": ([_VP, _U64, _U64, _I, _VP, _VP, _VP], _I),
     "mtfjsp_random_step": ([_VP, _U64, _U64] + [_VP] * 14 + [_I, _I, _VP], _I),
@@ -121,6 +122,7 @@ SIGNATURES = {
     "mtfjsp_offspring": ([_VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _U64, _D, _D, _VP, _VP], _I),
     "mtfjsp_mcts_select": ([_VP, _VP, _I, _I, _I, _VP, _I, _I, _I, _D] + [_VP] * 9, _I),
     "mtfjsp_mcts_backup": ([_I, _I, _I] + [_VP] * 8, _I),
+    "mtfjsp_tabu_move": ([_I, _I, _I, _VP, C.c_int64, _VP, _VP, _VP, _I, _I, _I] + [_VP] * 10, _I),
     "mtfjsp_launch_overlap_error": ([_VP], _I),
     "mtfjsp_launch_count": ([_VP], C.c_int64),
     "mtfjsp_bytes_per_step": ([_VP, _I], C.c_int64),

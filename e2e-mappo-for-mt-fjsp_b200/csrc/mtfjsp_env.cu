@@ -2700,6 +2700,95 @@ __global__ void __launch_bounds__(256) replay_kernel(const __grid_constant__ Rep
     }
 }
 
+// Neighbour replay (mtfjsp_replay_moves): candidate r is base row moves[r,0] with the single move r applied, replayed
+// over all N steps from the episode start of env base_src[row].  replay_kernel's shape and step loop, kept a kernel of
+// its own so that replay_kernel's SASS stays as it is; only the action read differs: lane k of a 32-step window computes
+// the source index of entry s0 + k from the move (search.apply_moves' index arithmetic) and reads that entry of the base
+// row, which every candidate of the row shares through L2.  The neighbour sequence is never written.
+struct ReplayMovesArgs {
+    Layout L;
+    PwPlan pw;
+    const double *sd0, *xs, *t, *p;
+    const int16_t* si0;
+    const int32_t *base_src, *base, *moves;
+    int Q, R;
+    double cfgw[3], divisor;
+    double *cost4, *return5;
+    int32_t* first_invalid;
+};
+
+__global__ void __launch_bounds__(256) replay_moves_kernel(const __grid_constant__ ReplayMovesArgs A) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const Layout& L = A.L;
+    const int N = L.N;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int r = blockIdx.x * L.warps_per_block + warp;
+    if (r >= A.R) return;
+    const int32_t* mv = A.moves + (size_t)r * 4;
+    const int row = __ldg(mv), kind = __ldg(mv + 1), ms = __ldg(mv + 2), arg = __ldg(mv + 3);
+    const bool ins = kind == 1;
+    int src = -1;
+    if (row >= 0 && row < A.Q && (kind == 0 || ins) && ms >= 0 && ms < N && (!ins || (arg >= 0 && arg < N)))
+        src = __ldg(A.base_src + row);
+    if (src < 0 || src >= L.B) {  // a malformed move is data: this candidate gets -2 and zero rows, the others run
+        if (A.cost4 && lane < 4) A.cost4[(size_t)r * 4 + lane] = 0.0;
+        if (A.return5 && lane < 5) A.return5[(size_t)r * 5 + lane] = 0.0;
+        if (A.first_invalid && lane == 0) A.first_invalid[r] = -2;
+        return;
+    }
+    const EnvSmem S(L, smem_raw + (size_t)warp * L.smem_per_warp);
+    {
+        const uint4* g = reinterpret_cast<const uint4*>(A.sd0 + (size_t)src * L.sd_stride);
+        uint4* d = reinterpret_cast<uint4*>(S.sd);
+        for (int i = lane; i < L.sd_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.xs + (size_t)src * L.xs_stride);
+        d = reinterpret_cast<uint4*>(S.xs);
+        for (int i = lane; i < L.xs_stride / 2; i += 32) d[i] = __ldg(g + i);
+        g = reinterpret_cast<const uint4*>(A.si0 + (size_t)src * L.si_stride);
+        d = reinterpret_cast<uint4*>(S.si);
+        for (int i = lane; i < L.si_stride / 8; i += 32) d[i] = __ldg(g + i);
+    }
+    __syncwarp();
+    const int32_t* act = A.base + (size_t)row * N * 2;
+    double ret[5] = {0.0, 0.0, 0.0, 0.0, 0.0};  // lane 0: the step-order sums of the step's reward5
+    int bad = -1, op_l = 0, mach_l = 0;
+    for (int s = 0; s < N; s++) {
+        if ((s & 31) == 0) {
+            const int n = s + lane;
+            int from = n;  // a reassignment keeps every entry in place
+            if (ins) {     // entry ms removed, then inserted at index arg of the remaining N - 1
+                const int rest = n < arg ? n : n - 1;
+                from = n == arg ? ms : (rest < ms ? rest : rest + 1);
+            }
+            op_l = n < N ? __ldg(act + 2 * from) : 0;
+            mach_l = n < N ? (!ins && n == ms ? arg : __ldg(act + 2 * from + 1)) : 0;
+        }
+        const int a = __shfl_sync(FULL, op_l, s & 31), m = __shfl_sync(FULL, mach_l, s & 31);
+        const StepOut so = env_transition<false>(L, S, A.t, A.p, (size_t)src, a, m, nullptr, nullptr, lane);
+        double r5[5] = {0.0, 0.0, 0.0, 0.0, 0.0};  // what the step writes for an invalid action
+        if (so.valid) {
+            double mkv, env;
+            env_estimates<true>(L, A.pw, S, lane, &mkv, &env);
+            const StepReward rw = env_reward(L, S, A.cfgw, m, mkv, env, so, lane);
+            r5[0] = rw.total / A.divisor; r5[1] = rw.r_t; r5[2] = rw.r_idle; r5[3] = rw.r_pt; r5[4] = rw.r_tt;
+            __syncwarp();
+        } else if (bad < 0) {
+            bad = s;
+        }
+#pragma unroll
+        for (int k = 0; k < 5; k++) ret[k] += r5[k];
+    }
+    if (lane == 0) {
+        if (A.cost4) {  // costs_kernel's expressions
+            double* c = A.cost4 + (size_t)r * 4;
+            c[0] = S.scal[0]; c[1] = S.scal[1] / (double)L.N; c[2] = S.scal[2]; c[3] = S.scal[3];
+        }
+        if (A.return5)
+            for (int k = 0; k < 5; k++) A.return5[(size_t)r * 5 + k] = ret[k];
+        if (A.first_invalid) A.first_invalid[r] = bad;
+    }
+}
+
 // Episode completion (mtfjsp_complete): candidate r starts from the CURRENT state of env src[r], runs T forced (op,
 // machine) actions, then lets a base policy pick every further action until the schedule is complete, and leaves the
 // costs, the summed rewards, the index of its first invalid action and the base policy's actions.  replay_kernel's shape:
@@ -3643,6 +3732,30 @@ int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actio
     const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
     replay_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
     return counted(h, "replay_kernel");
+}
+
+int mtfjsp_replay_moves(mtfjsp_env* h, const int32_t* base_src, int Q, const int32_t* base, const int32_t* moves, int R,
+                        double* cost4, double* return5, int32_t* first_invalid, void* stream) {
+    if (!h || !base_src || !base || !moves || Q < 1 || R < 1)
+        return fail(MTFJSP_E_ARG, "mtfjsp_replay_moves: bad argument");
+    if (!h->reset_done) return fail(MTFJSP_E_STATE, "mtfjsp_replay_moves before mtfjsp_reset");
+    const Layout& L = h->L;
+    cudaStream_t s = (cudaStream_t)stream;
+    // a non-step call: a recorded reset runs now, and the next step waits for the replay in full
+    int rc = enter(h, s);
+    if (rc) return rc;
+    const size_t smem = (size_t)L.smem_per_warp * L.warps_per_block;
+    CK(opt_in_smem(replay_moves_kernel, smem), "cudaFuncSetAttribute");
+    ReplayMovesArgs A;
+    memset(&A, 0, sizeof A);
+    A.L = L; A.pw = h->pw;
+    A.sd0 = h->sd0; A.xs = h->xs; A.t = h->t; A.p = h->p; A.si0 = h->si0;
+    A.base_src = base_src; A.base = base; A.moves = moves; A.Q = Q; A.R = R;
+    A.cfgw[0] = h->cfgw[0]; A.cfgw[1] = h->cfgw[1]; A.cfgw[2] = h->cfgw[2]; A.divisor = h->divisor;
+    A.cost4 = cost4; A.return5 = return5; A.first_invalid = first_invalid;
+    const unsigned blocks = (unsigned)((R + L.warps_per_block - 1) / L.warps_per_block);
+    replay_moves_kernel<<<blocks, L.warps_per_block * 32, smem, s>>>(A);
+    return counted(h, "replay_moves_kernel");
 }
 
 int mtfjsp_complete(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, int base, const double* key,

@@ -319,6 +319,36 @@ class BatchedMTFJSPEnv:
                                       _stream()), "mtfjsp_replay")
         return final4, ret5, finv
 
+    def replay_moves(self, base, moves, base_src=None):
+        """replay of single-move neighbours without building them (mtfjsp_replay_moves): candidate r is base column
+        moves[r, 0] with move r applied (search.apply_moves), replayed over all N steps from the episode start of env
+        base_src[moves[r, 0]].  base: [N,Q,2] integer (op, machine) sequences on this env's device, the layout
+        greedy_validate and search.local_search use (transposed once here); moves: [R,4] integers (row, kind, s, arg) in
+        search.neighbour_moves' form; base_src: [Q] integers, None means arange(Q) and needs Q == B.  Returns what
+        replay(apply_moves(base, moves), base_src[moves[:, 0]]) returns, bit for bit; a malformed move (include/mtfjsp.h)
+        gets -2 in first_invalid and zero rows."""
+        _on(self.device, base, moves, base_src)
+        if base.dim() != 3 or base.shape[0] != self.N or base.shape[2] != 2:
+            raise ValueError("base must have shape [%d, Q, 2]" % self.N)
+        if moves.dim() != 2 or moves.shape[1] != 4:
+            raise ValueError("moves must have shape [R, 4]")
+        Q, R = int(base.shape[1]), int(moves.shape[0])
+        if base_src is None:
+            if Q != self.B:
+                raise ValueError("base_src=None replays row q from env q: needs Q == B = %d" % self.B)
+            base_src = torch.arange(Q, dtype=torch.int32, device=self.device)
+        elif tuple(base_src.shape) != (Q,):
+            raise ValueError("base_src must have shape [%d]" % Q)
+        base_src = base_src.to(torch.int32).contiguous()
+        b = base.to(torch.int32).transpose(0, 1).contiguous()                  # [Q,N,2]: one contiguous run per row
+        mv = moves.to(torch.int32).contiguous()
+        final4 = torch.empty((R, 4), dtype=torch.float64, device=self.device)
+        ret5 = torch.empty((R, 5), dtype=torch.float64, device=self.device)
+        finv = torch.empty((R,), dtype=torch.int32, device=self.device)
+        check(self._lib.mtfjsp_replay_moves(self._h, _ptr(base_src), Q, _ptr(b), _ptr(mv), R, _ptr(final4), _ptr(ret5),
+                                            _ptr(finv), _stream()), "mtfjsp_replay_moves")
+        return final4, ret5, finv
+
     # ---- episode completion ------------------------------------------------------------------------------------------
     def complete(self, src, actions=None, base="random", key=None, mach=None, seed=0, mask_mode=None):
         """What the rest of the episode costs for R candidates, each from the CURRENT state of env src[r]: T forced actions,

@@ -17,6 +17,11 @@ incumbent's.  The search stops after `rounds` rounds or at the first round in wh
 synchronisation per round.  The environment decides what a sequence costs, so a neighbour's objective is exactly what
 stepping it would give, left shift included.
 
+`tabu_search` walks the same neighbourhood past local optima: every iteration it moves to the best neighbour that is not
+tabu, improving or not, and a short memory of recent moves keeps it from walking straight back.  Neighbours are
+replayed from the incumbent and the move list (BatchedMTFJSPEnv.replay_moves, mtfjsp_replay_moves) without being built,
+and the move decision is one launch for every instance (mtfjsp_tabu_move).
+
 `pareto_local_search` walks the same neighbourhood without a weighted sum: it keeps an archive of mutually
 non-dominated schedules per instance over the three targets (pareto.py) and expands it until no member is left
 unexplored.
@@ -172,6 +177,173 @@ def local_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, r
     return {"actions": cur.cpu().numpy(), "final4": final4.cpu().numpy(), "objective": obj.cpu().numpy(),
             "history": torch.stack(history).cpu().numpy(),
             "accepted": (torch.stack(accepted) if accepted else torch.zeros((0, S), dtype=torch.bool)).cpu().numpy(),
+            "replays": replays}
+
+
+# ---- tabu search on the neighbour replay -------------------------------------------------------------------------------
+# the defaults come from a sweep on device-generated J6M6E2 instances (profiles/README.md, "Tabu search" (d))
+TENURE_MACH, TENURE_INS = 20, 80
+_TABU_STATE = ("cur", "cur_obj", "cur_f4", "best", "best_obj", "best_f4", "mach_until", "op_until")
+
+
+def tabu_state(cur, f4, weights, M):
+    """A fresh tabu state of S instances at the sequences cur ([S,N,2] int32) of final costs f4 ([S,4] f64), in the form
+    mtfjsp_tabu_move updates: cur, cur_obj, cur_f4, best (= cur), best_obj, best_f4, mach_until [S,N,M] and op_until
+    [S,N] int32 (all 0: nothing tabu).  Torch tensors on cur's device, or numpy arrays for numpy input."""
+    if isinstance(cur, np.ndarray):
+        xp, kw, cp = np, {}, np.copy
+    else:
+        xp, kw, cp = torch, {"device": cur.device}, torch.clone
+    S, N = cur.shape[0], cur.shape[1]
+    obj = _objective(f4, weights)
+    return {"cur": cp(cur), "cur_obj": cp(obj), "cur_f4": cp(f4), "best": cp(cur), "best_obj": cp(obj), "best_f4": cp(f4),
+            "mach_until": xp.zeros((S, N, M), dtype=xp.int32, **kw), "op_until": xp.zeros((S, N), dtype=xp.int32, **kw)}
+
+
+def tabu_move(state, moves, seg, obj, f4, it, tenure_mach=TENURE_MACH, tenure_ins=TENURE_INS):
+    """One tabu iteration's move for every instance on the device (mtfjsp_tabu_move; rules in include/mtfjsp.h): state
+    as tabu_state returns it, updated in place; moves [R,4] integers grouped by instance in neighbour_moves' order, seg
+    [S+1] integers (instance s's moves are moves[seg[s]:seg[s+1]]), obj [R] and f4 [R,4] f64 their objectives and costs.
+    -> chosen [S] int32: the move taken, -1 for none admissible, -2 for a malformed segment."""
+    cur, mu = state["cur"], state["mach_until"]
+    S, N, M = cur.shape[0], cur.shape[1], mu.shape[2]
+    R = int(moves.shape[0])
+    mv = moves.to(torch.int32).contiguous()
+    sg = seg.to(torch.int64).contiguous()
+    o = obj.to(torch.float64).contiguous()
+    f = f4.to(torch.float64).contiguous()
+    chosen = torch.empty((S,), dtype=torch.int32, device=cur.device)
+    check(lib().mtfjsp_tabu_move(S, N // M, M, _ptr(mv if R else None), R, _ptr(sg), _ptr(o if R else None),
+                                 _ptr(f if R else None), int(it), int(tenure_mach), int(tenure_ins),
+                                 *(_ptr(state[k]) for k in _TABU_STATE), _ptr(chosen), _stream()), "mtfjsp_tabu_move")
+    return chosen
+
+
+def tabu_reference(state, moves, seg, obj, f4, it, tenure_mach=TENURE_MACH, tenure_ins=TENURE_INS):
+    """numpy restatement of mtfjsp_tabu_move, move for move: state as tabu_state(..., numpy) (copied, not changed),
+    moves [R,4], seg [S+1], obj [R], f4 [R,4].  -> (the state after the move, chosen [S] int32)."""
+    st = {k: np.array(v, copy=True) for k, v in state.items()}
+    moves, seg = np.asarray(moves, dtype=np.int64), np.asarray(seg, dtype=np.int64)
+    obj, f4 = np.asarray(obj, dtype=np.float64), np.asarray(f4, dtype=np.float64)
+    S, N, M = st["cur"].shape[0], st["cur"].shape[1], st["mach_until"].shape[2]
+    R = moves.shape[0]
+    chosen = np.empty(S, dtype=np.int32)
+    for s in range(S):
+        lo, hi = int(seg[s]), int(seg[s + 1])
+        if lo < 0 or hi < lo or hi > R:
+            chosen[s] = -2
+            continue
+        row = st["cur"][s].copy()
+        bo = st["best_obj"][s]
+        bi, v = -1, None
+        for r in range(lo, hi):
+            i, kind, ms, arg = (int(x) for x in moves[r])
+            if i != s or not 0 <= ms < N or not 0 <= row[ms, 0] < N:
+                continue
+            o = int(row[ms, 0])
+            if kind == REASSIGN:
+                if not (0 <= arg < M and 0 <= row[ms, 1] < M):
+                    continue
+                tabu = st["mach_until"][s, o, arg] > it
+            elif kind == INSERT:
+                if not 0 <= arg < N:
+                    continue
+                tabu = st["op_until"][s, o] > it
+            else:
+                continue
+            x = obj[r]
+            if np.isnan(x) or (tabu and not x < bo):
+                continue
+            if bi < 0 or x < v:
+                bi, v = r, x
+        if bi < 0:
+            chosen[s] = -1
+            continue
+        _, kind, ms, arg = (int(x) for x in moves[bi])
+        o = int(row[ms, 0])
+        if kind == INSERT:
+            rest = np.delete(row, ms, axis=0)
+            st["cur"][s] = np.insert(rest, arg, row[ms], axis=0)
+            st["op_until"][s, o] = it + 1 + tenure_ins
+        else:
+            st["cur"][s, ms, 1] = arg
+            st["mach_until"][s, o, row[ms, 1]] = it + 1 + tenure_mach
+        st["cur_obj"][s] = v
+        st["cur_f4"][s] = f4[bi]
+        if v < bo:
+            st["best"][s] = st["cur"][s]
+            st["best_obj"][s] = v
+            st["best_f4"][s] = f4[bi]
+        chosen[s] = bi
+    return st, chosen
+
+
+def tabu_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, iterations=500, tenure_mach=TENURE_MACH,
+                tenure_ins=TENURE_INS, max_neighbours=None, seed=0, max_candidates=65536, device=None):
+    """Tabu search from the S sequences `actions` ([N,S,2] integers, numpy or torch: complete valid schedules of the
+    instances {"t","p","transT","edge"} [S,...]) under the reward weights `weights`, on local_search's neighbourhood and
+    FP64 objective.  Every iteration `it` runs neighbour_moves of the current sequences (max_neighbours samples as
+    there, keyed by (seed, it)), replays them from the incumbent and the move list with BatchedMTFJSPEnv.replay_moves
+    (src = their instance, at most max_candidates per call), and makes one mtfjsp_tabu_move: each instance moves to its
+    admissible neighbour of the least objective, improving or not.  A reassignment of op o away from machine m makes
+    (o, m) tabu for tenure_mach iterations; an insertion of o makes o's insertions tabu for tenure_ins iterations; a tabu
+    move is admissible when it beats the instance's best (aspiration).  An instance with no admissible move stays put.
+    Exactly `iterations` iterations run.  The histories stay on the device and the invalid-replay flag is read once, at
+    the end; neighbour_moves' nonzero still synchronises once per iteration.
+
+    While an instance descends, its current and best objectives are equal, so the steepest improving neighbour is
+    admissible and wins with local_search's tie-break: with max_neighbours=None history follows local_search's history
+    for as long as local_search accepts moves, and the result is never worse than local_search's.  With
+    max_neighbours=None an instance's result depends neither on max_candidates nor on the other instances of the batch.
+    -> dict of numpy arrays: actions [N,S,2] int32, final4 [S,4] and objective [S] of the best schedule, history
+       [iterations+1, S] (the current objective, the start first), best_history [iterations+1, S] (never increasing),
+       chosen [iterations, S] (mtfjsp_tabu_move's output) and replays, the number of sequences replayed (the start
+       included)."""
+    t = np.asarray(instances["t"])
+    S, N, M = t.shape
+    J, E = N // M, np.asarray(instances["edge"]).shape[1]
+    if max_candidates < 1:
+        raise ValueError("max_candidates must be >= 1")
+    if int(iterations) < 0 or int(tenure_mach) < 0 or int(tenure_ins) < 0:
+        raise ValueError("iterations and the tenures must be >= 0")
+    env = BatchedMTFJSPEnv(S, J, M, E, left_shift=left_shift, weights=weights, device=device, obs_dtype=torch.float32)
+    dev = env.device
+    env.load(*(np.asarray(instances[k]) for k in ("t", "p", "transT", "edge")))
+    env.scaler_init()
+    env.reset(np.tile(np.asarray(weights, dtype=np.float64), (S, 1)))
+    start = torch.as_tensor(np.asarray(actions) if not torch.is_tensor(actions) else actions).to(dev, torch.int32)
+    if tuple(start.shape) != (N, S, 2):
+        raise ValueError("actions must have shape [%d, %d, 2]" % (N, S))
+    t_dev = torch.as_tensor(t, device=dev)
+    final4, _, finv = env.replay(start)
+    if bool((finv != -1).any()):
+        raise ValueError("a starting sequence has an invalid action")
+    st = tabu_state(start.transpose(0, 1).contiguous(), final4, weights, M)
+    history, best_history, chosen = [st["cur_obj"].clone()], [st["best_obj"].clone()], []
+    replays = S
+    bad = torch.zeros((), dtype=torch.bool, device=dev)
+    zero = torch.zeros(1, dtype=torch.int64, device=dev)
+    for it in range(int(iterations)):
+        base = st["cur"].transpose(0, 1)                                      # [N,S,2] view of the current sequences
+        moves = neighbour_moves(base, t_dev, max_neighbours, seed, it)
+        R = moves.shape[0]
+        replays += R
+        f4 = torch.empty((R, 4), dtype=torch.float64, device=dev)
+        for c0 in range(0, R, max_candidates):
+            mv = moves[c0:c0 + max_candidates]
+            f4[c0:c0 + mv.shape[0]], _, fi = env.replay_moves(base, mv)
+            bad |= (fi != -1).any()
+        seg = torch.cat((zero, torch.cumsum(torch.bincount(moves[:, 0], minlength=S), 0)))
+        chosen.append(tabu_move(st, moves, seg, _objective(f4, weights), f4, it, tenure_mach, tenure_ins))
+        history.append(st["cur_obj"].clone())
+        best_history.append(st["best_obj"].clone())
+    if bool(bad):
+        raise RuntimeError("a neighbour replayed with an invalid action")
+    env.close()
+    return {"actions": st["best"].transpose(0, 1).cpu().numpy(), "final4": st["best_f4"].cpu().numpy(),
+            "objective": st["best_obj"].cpu().numpy(), "history": torch.stack(history).cpu().numpy(),
+            "best_history": torch.stack(best_history).cpu().numpy(),
+            "chosen": (torch.stack(chosen) if chosen else torch.zeros((0, S), dtype=torch.int32)).cpu().numpy(),
             "replays": replays}
 
 

@@ -188,6 +188,23 @@ int mtfjsp_peek(mtfjsp_env* h, const int32_t* op, const int32_t* mach, int K, do
 int mtfjsp_replay(mtfjsp_env* h, const int32_t* src, int R, const int32_t* actions, int T, double* cost4, double* return5,
                   int32_t* first_invalid, void* stream);
 
+/* Neighbour replay: mtfjsp_replay of R single-move neighbours of Q base sequences, without writing the neighbours.
+ * base [Q,N,2] int32 holds Q complete (op, machine) sequences, contiguous per row; base_src [Q] int32 the env whose
+ * episode start row q is replayed from; moves [R,4] int32 (row, kind, s, arg): kind 0 (reassignment) runs entry s of
+ * base row `row` on machine arg, kind 1 (insertion) removes entry s and inserts it at index arg of the remaining N - 1
+ * (search.neighbour_moves / search.apply_moves).  All on the device.  Candidate r is replayed over all N steps; the
+ * outputs are mtfjsp_replay's (any may be NULL) and their bits equal mtfjsp_replay with src = base_src[moves[:,0]] and
+ * the neighbour sequences apply_moves would build, T = N.  A malformed move is data: a row outside [0, Q), a kind other
+ * than 0 or 1, s outside [0, N), an insertion with arg outside [0, N), or base_src[row] outside [0, B) gives -2 in
+ * first_invalid and zero rows in cost4 / return5, and the other moves are unaffected.  A reassignment to an infeasible
+ * or out-of-range machine, and an insertion that breaks job order, are well-formed: they replay, and their first
+ * invalid action is reported as mtfjsp_replay reports it.
+ * Read-only and a non-step call, as mtfjsp_replay.
+ * MTFJSP_E_ARG, nothing written: a NULL handle, base_src, base or moves, Q < 1 or R < 1.  MTFJSP_E_STATE, nothing
+ * written: before the first mtfjsp_reset since mtfjsp_load. */
+int mtfjsp_replay_moves(mtfjsp_env* h, const int32_t* base_src, int Q, const int32_t* base, const int32_t* moves, int R,
+                        double* cost4, double* return5, int32_t* first_invalid, void* stream);
+
 /* Episode completion: for R candidates, what the rest of the episode costs when T forced actions and then a base policy
  * finish the schedule, without changing the handle.  Candidate r starts from the CURRENT state of env src[r] (src [R]
  * int32; duplicates and permutations allowed), runs actions [R,T,2] int32 (op, machine), 0 <= T <= N (NULL when T = 0;
@@ -532,6 +549,31 @@ int mtfjsp_mcts_select(const double* t, const int32_t* rule_mach, int S, int J, 
                        int32_t* count, const double* lohi, int32_t* paths, int32_t* depth, int32_t* leaf, void* stream);
 int mtfjsp_mcts_backup(int S, int L, int max_nodes, const int32_t* leaf, const double* objective, int32_t* node,
                        double* vmin, const int32_t* root, const int32_t* count, double* lohi, void* stream);
+
+/* One tabu-search iteration's move for S instances, applied in place (search.tabu_search).  Handle-free, asynchronous on
+ * `stream`, one warp per instance.  N = J*M.  moves [R,4] int32 (instance, kind, s, arg) are the iteration's moves in
+ * search.neighbour_moves' form and order, instance s's in moves[seg[s] .. seg[s+1]) (seg [S+1] int64); obj [R] f64 their
+ * objectives and f4 [R,4] f64 their final costs (moves, obj and f4 may be NULL when R = 0).  State, updated in place:
+ * cur [S,N,2] int32, cur_obj [S], cur_f4 [S,4], best [S,N,2] int32, best_obj [S], best_f4 [S,4] f64; mach_until [S,N,M]
+ * int32, the first iteration at which op o may again be reassigned to machine m; op_until [S,N] int32, the first
+ * iteration at which op o may again be moved by insertion.  With o the op at index s of cur: a reassignment (s, m') is
+ * tabu iff mach_until[o,m'] > it, an insertion iff op_until[o] > it.  A move is admissible iff it is not tabu or its
+ * objective is strictly below best_obj (aspiration).  The admissible move of the least objective is taken, ties to the
+ * lowest move index; a NaN objective never wins.  Taking it: cur becomes search.apply_moves(cur, move); a reassignment
+ * sets mach_until[o, m_old] = it + 1 + tenure_mach, an insertion op_until[o] = it + 1 + tenure_ins; cur_obj and cur_f4
+ * take the move's obj and f4; if that objective is below the previous best_obj, cur is copied to best and best_obj /
+ * best_f4 take it too.  chosen [S] int32 receives the move's index in moves, -1 when the instance has no admissible move
+ * (an empty segment included) and stays put, or -2 when its segment is malformed (seg[s] < 0, seg[s+1] < seg[s] or
+ * seg[s+1] > R) and it stays put.  A move is never taken when its instance field is not s, its kind is not 0 or 1, s is
+ * outside [0, N), its arg is outside [0, M) (reassignment) or [0, N) (insertion), or the entry of cur it names holds an
+ * op outside [0, N) or, for a reassignment, a machine outside [0, M).
+ * MTFJSP_E_ARG, nothing written: a NULL pointer (see above), S < 1, (J, M) outside mtfjsp_create's range (J >= 1,
+ * 2 <= M <= 64, N <= 4096), R < 0 or R > INT32_MAX, it, tenure_mach or tenure_ins < 0, or it + 1 + a tenure above
+ * INT32_MAX. */
+int mtfjsp_tabu_move(int S, int J, int M, const int32_t* moves, int64_t R, const int64_t* seg, const double* obj,
+                     const double* f4, int it, int tenure_mach, int tenure_ins, int32_t* cur, double* cur_obj,
+                     double* cur_f4, int32_t* best, double* best_obj, double* best_f4, int32_t* mach_until,
+                     int32_t* op_until, int32_t* chosen, void* stream);
 
 /* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
  * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
