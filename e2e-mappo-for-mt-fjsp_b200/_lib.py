@@ -17,11 +17,12 @@ SRC_DIR = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("MTFJSP_LIB") or os.path.join(_HERE, "libmtfjsp_b200.so")
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "mtfjsp.h")
 SOURCES = ["mtfjsp_env.cu", "mtfjsp_encoder.cu", "mtfjsp_gemm.cu", "mtfjsp_pareto.cu", "mtfjsp_evolve.cu",
-           "mtfjsp_mcts.cu", "mtfjsp_tabu.cu"]
+           "mtfjsp_mcts.cu", "mtfjsp_tabu.cu", "mtfjsp_anneal.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
-# the env kernels restate the reference's FP64 arithmetic operation by operation, and the hypervolume and the MCTS score
-# their numpy specifications: no FMA contraction there
-EXTRA_FLAGS = {"mtfjsp_env.cu": ["-fmad=false"], "mtfjsp_pareto.cu": ["-fmad=false"], "mtfjsp_mcts.cu": ["-fmad=false"]}
+# the env kernels restate the reference's FP64 arithmetic operation by operation, and the hypervolume, the MCTS score and
+# the annealer's acceptance test their numpy specifications: no FMA contraction there
+EXTRA_FLAGS = {"mtfjsp_env.cu": ["-fmad=false"], "mtfjsp_pareto.cu": ["-fmad=false"], "mtfjsp_mcts.cu": ["-fmad=false"],
+               "mtfjsp_anneal.cu": ["-fmad=false"]}
 
 
 def _stale() -> bool:
@@ -123,6 +124,8 @@ SIGNATURES = {
     "mtfjsp_mcts_select": ([_VP, _VP, _I, _I, _I, _VP, _I, _I, _I, _D] + [_VP] * 9, _I),
     "mtfjsp_mcts_backup": ([_I, _I, _I] + [_VP] * 8, _I),
     "mtfjsp_tabu_move": ([_I, _I, _I, _VP, C.c_int64, _VP, _VP, _VP, _I, _I, _I] + [_VP] * 10, _I),
+    "mtfjsp_anneal_propose": ([_VP, _I, _I, _I, _I, _VP, _U64, _I, _VP, _VP], _I),
+    "mtfjsp_anneal_step": ([_I, _I, _I, _I] + [_VP] * 5 + [_U64, _I, _I] + [_VP] * 9, _I),
     "mtfjsp_launch_overlap_error": ([_VP], _I),
     "mtfjsp_launch_count": ([_VP], C.c_int64),
     "mtfjsp_bytes_per_step": ([_VP, _I], C.c_int64),

@@ -22,6 +22,11 @@ tabu, improving or not, and a short memory of recent moves keeps it from walking
 replayed from the incumbent and the move list (BatchedMTFJSPEnv.replay_moves, mtfjsp_replay_moves) without being built,
 and the move decision is one launch for every instance (mtfjsp_tabu_move).
 
+`anneal_search` is parallel tempering on the same neighbourhood: K Markov chains per instance, each at its own
+temperature, propose one uniformly drawn neighbour each per iteration (mtfjsp_anneal_propose), replay only that, take it
+by the Metropolis rule and exchange states between adjacent temperatures (mtfjsp_anneal_step).  It spends one replay per
+proposal where tabu search spends a whole neighbourhood per move.
+
 `pareto_local_search` walks the same neighbourhood without a weighted sum: it keeps an archive of mutually
 non-dominated schedules per instance over the three targets (pareto.py) and expands it until no member is left
 unexplored.
@@ -345,6 +350,258 @@ def tabu_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, it
             "best_history": torch.stack(best_history).cpu().numpy(),
             "chosen": (torch.stack(chosen) if chosen else torch.zeros((0, S), dtype=torch.int32)).cpu().numpy(),
             "replays": replays}
+
+
+# ---- parallel tempering on the neighbour replay ------------------------------------------------------------------------
+# the defaults come from a sweep on device-generated J6M6E2 instances (profiles/README.md, "Parallel tempering" (a))
+ANNEAL_CHAINS, ANNEAL_T_MAX, ANNEAL_T_MIN, ANNEAL_SWAP_EVERY = 32, 0.03, 1e-3, 1
+_ANNEAL_STATE = ("cur", "cur_obj", "cur_f4", "best", "best_obj", "best_f4", "accepted", "swapped")
+# exp_neg's constants (include/mtfjsp.h): Cody-Waite ln 2, 1/i! for the degree-13 Horner polynomial, the zero point
+_INV_LN2, _LN2_HI, _LN2_LO, _EXP_NEG_ZERO = 1.4426950408889634, 0.6931471803691238, 1.9082149292705877e-10, 746.0
+_INV_FACT = (1.0, 1.0, 0.5, 0.16666666666666666, 0.041666666666666664, 0.008333333333333333, 0.001388888888888889,
+             0.0001984126984126984, 2.48015873015873e-05, 2.7557319223985893e-06, 2.755731922398589e-07,
+             2.505210838544172e-08, 2.08767569878681e-09, 1.6059043836821613e-10)
+
+
+def exp_neg_reference(x):
+    """mtfjsp_anneal.cu's exp_neg in numpy, bit for bit: e^-x for x > 0, 1 for x <= 0, NaN for NaN, 0 past 746.  Cody-Waite
+    reduction x = n ln2 + r, the degree-13 Taylor polynomial of e^z at z = -r in Horner form, and ldexp(p, -n)."""
+    x = np.asarray(x, dtype=np.float64)
+    with np.errstate(invalid="ignore", over="ignore"):
+        xc = np.where((x > 0.0) & (x <= _EXP_NEG_ZERO), x, 1.0)
+        n = np.rint(xc * _INV_LN2)
+        z = -((xc - n * _LN2_HI) - n * _LN2_LO)
+        p = np.full_like(z, _INV_FACT[13])
+        for c in _INV_FACT[12::-1]:
+            p = p * z + c
+        out = np.ldexp(p, -n.astype(np.int64))
+    out = np.where(x <= 0.0, 1.0, np.where(x > _EXP_NEG_ZERO, 0.0, out))
+    out = np.where(np.isnan(x), x, out)
+    return out[()] if out.ndim == 0 else out
+
+
+def anneal_ladder(K=ANNEAL_CHAINS, t_max=ANNEAL_T_MAX, t_min=ANNEAL_T_MIN):
+    """The default ladder of K relative temperatures, ascending and geometric from t_min to t_max; K = 1 gives [t_max]."""
+    K = int(K)
+    if K < 1 or not 0 < t_min <= t_max or not np.isfinite(t_max):
+        raise ValueError("anneal_ladder needs K >= 1 and 0 < t_min <= t_max < inf")
+    if K == 1:
+        return np.array([float(t_max)])
+    lad = float(t_min) * (float(t_max) / float(t_min)) ** (np.arange(K) / (K - 1))
+    lad[0], lad[-1] = t_min, t_max
+    return np.maximum.accumulate(lad)
+
+
+def anneal_state(cur, f4, weights, K):
+    """A fresh annealing state of S instances with K chains each, every chain at its instance's sequence of cur ([S,N,2]
+    int32) of final costs f4 ([S,4] f64), in the form mtfjsp_anneal_step updates: cur [S*K,N,2], cur_obj [S*K], cur_f4
+    [S*K,4], best (= cur [S,N,2]), best_obj [S], best_f4 [S,4], and the per-call flags accepted [S*K] and swapped [S*K]
+    int32.  Torch tensors on cur's device, or numpy arrays for numpy input."""
+    if isinstance(cur, np.ndarray):
+        xp, kw, cp, rep = np, {}, np.copy, lambda a: np.repeat(a, K, axis=0)
+    else:
+        xp, kw, cp, rep = torch, {"device": cur.device}, torch.clone, lambda a: torch.repeat_interleave(a, K, 0)
+    S = cur.shape[0]
+    obj = _objective(f4, weights)
+    return {"cur": rep(cur), "cur_obj": rep(obj), "cur_f4": rep(f4), "best": cp(cur), "best_obj": cp(obj),
+            "best_f4": cp(f4), "accepted": xp.zeros(S * K, dtype=xp.int32, **kw),
+            "swapped": xp.zeros(S * K, dtype=xp.int32, **kw)}
+
+
+def anneal_propose(t, cur, seed, it):
+    """One uniformly drawn neighbour per chain on the device (mtfjsp_anneal_propose; rules in include/mtfjsp.h): t [S,N,M]
+    f64 processing times, cur [S*K,N,2] int32 chain rows (row q = s*K + k), on one device.  -> moves [S*K,4] int32
+    (row, kind, s, arg) in neighbour_moves' form, (q, -1, 0, 0) for a row without moves."""
+    S, N, M = t.shape
+    Q = int(cur.shape[0])
+    if Q % S or tuple(cur.shape[1:]) != (N, 2):
+        raise ValueError("cur must have shape [S*K, %d, 2]" % N)
+    tt = t.to(torch.float64).contiguous()
+    c = cur.to(torch.int32).contiguous()
+    moves = torch.empty((Q, 4), dtype=torch.int32, device=cur.device)
+    check(lib().mtfjsp_anneal_propose(_ptr(tt), S, N // M, M, Q // S, _ptr(c), int(seed) & 0xFFFFFFFFFFFFFFFF, int(it),
+                                      _ptr(moves), _stream()), "mtfjsp_anneal_propose")
+    return moves
+
+
+def anneal_step(state, moves, first_invalid, obj, f4, temp, seed, it, swap_parity, M):
+    """One iteration's Metropolis decisions, exchanges and best update on the device (mtfjsp_anneal_step; rules in
+    include/mtfjsp.h): state as anneal_state returns it, updated in place (accepted and swapped rewritten); moves [S*K,4],
+    first_invalid [S*K], obj [S*K] and f4 [S*K,4] the proposals' replay, temp [S,K] absolute temperatures; swap_parity 0
+    or 1 exchanges the pairs (k, k+1) with k of that parity, anything else none; M the machine count (N = J*M)."""
+    S, K = temp.shape
+    N = state["cur"].shape[1]
+    args = [x.to(dt).contiguous() for x, dt in ((moves, torch.int32), (first_invalid, torch.int32),
+                                                 (obj, torch.float64), (f4, torch.float64), (temp, torch.float64))]
+    check(lib().mtfjsp_anneal_step(S, N // M, M, K, *(_ptr(a) for a in args), int(seed) & 0xFFFFFFFFFFFFFFFF, int(it),
+                                   int(swap_parity), *(_ptr(state[k]) for k in _ANNEAL_STATE), _stream()),
+          "mtfjsp_anneal_step")
+
+
+def anneal_propose_reference(t, cur, seed, it):
+    """numpy restatement of mtfjsp_anneal_propose, draw for draw: row q's move is neighbour_moves(row q, t[s])
+    [_below(u0, R_q)] with its row field set to q, (q, -1, 0, 0) when R_q = 0.  t [S,N,M], cur [S*K,N,2]; valid
+    sequences only (the kernel's output for others is not restated)."""
+    from .evolve import _below, _draws
+    t = np.asarray(t, dtype=np.float64)
+    cur = np.asarray(cur, dtype=np.int64)
+    S, N, M = t.shape
+    Q = cur.shape[0]
+    K = Q // S
+    inst = np.arange(Q) // K
+    allm = neighbour_moves(torch.as_tensor(cur.transpose(1, 0, 2)), torch.as_tensor(t[inst])).numpy()
+    count = np.bincount(allm[:, 0], minlength=Q)
+    start = np.cumsum(count) - count
+    out = np.zeros((Q, 4), dtype=np.int32)
+    for q in range(Q):
+        R = int(count[q])
+        if R == 0:
+            out[q] = (q, -1, 0, 0)
+            continue
+        u0 = _draws(seed, (int(it) << 32) | (q % K), 3)[0]
+        out[q] = allm[start[q] + _below(u0, R)]
+    return out
+
+
+def anneal_step_reference(state, moves, first_invalid, obj, f4, temp, seed, it, swap_parity, M):
+    """numpy restatement of mtfjsp_anneal_step, decision for decision: arguments as anneal_step, numpy; state copied, not
+    changed.  -> the state after the step (accepted and swapped included)."""
+    from .evolve import _draws
+    st = {k: np.array(v, copy=True) for k, v in state.items()}
+    moves, finv = np.asarray(moves, dtype=np.int64), np.asarray(first_invalid, dtype=np.int64)
+    obj, f4, temp = (np.asarray(a, dtype=np.float64) for a in (obj, f4, temp))
+    S, K = temp.shape
+    N = st["cur"].shape[1]
+    st["accepted"][:] = 0
+    st["swapped"][:] = 0
+    for s in range(S):
+        u = [_draws(seed, (int(it) << 32) | k, 3) for k in range(K)]
+        for k in range(K):
+            q = s * K + k
+            row, kind, ms, arg = (int(x) for x in moves[q])
+            ok = row == q and kind in (REASSIGN, INSERT) and 0 <= ms < N and finv[q] == -1
+            if ok:
+                o, mo = (int(x) for x in st["cur"][q, ms])
+                ok = 0 <= o < N and ((0 <= arg < M and 0 <= mo < M) if kind == REASSIGN else 0 <= arg < N)
+            if not ok or np.isnan(obj[q]):
+                continue
+            delta, T = obj[q] - st["cur_obj"][q], temp[s, k]
+            if not (delta <= 0.0 or (T > 0.0 and u[k][1] < exp_neg_reference(delta / T))):
+                continue
+            if kind == INSERT:
+                r = st["cur"][q]
+                st["cur"][q] = np.insert(np.delete(r, ms, axis=0), arg, r[ms], axis=0)
+            else:
+                st["cur"][q, ms, 1] = arg
+            st["cur_obj"][q], st["cur_f4"][q] = obj[q], f4[q]
+            st["accepted"][q] = 1
+        if swap_parity in (0, 1):
+            for k in range(int(swap_parity), K - 1, 2):
+                a, b = s * K + k, s * K + k + 1
+                d, Ta, Tb = st["cur_obj"][b] - st["cur_obj"][a], temp[s, k], temp[s, k + 1]
+                with np.errstate(divide="ignore", invalid="ignore"):
+                    swap = d <= 0.0 or (Ta > 0.0 and u[k][2] < exp_neg_reference(d * (1.0 / Ta - 1.0 / Tb)))
+                if swap:
+                    for key in ("cur", "cur_obj", "cur_f4"):
+                        st[key][[a, b]] = st[key][[b, a]]
+                    st["swapped"][a] = 1
+        v, bk = st["best_obj"][s], -1
+        for k in range(K):
+            if st["cur_obj"][s * K + k] < v:
+                v, bk = st["cur_obj"][s * K + k], k
+        if bk >= 0:
+            st["best"][s], st["best_obj"][s], st["best_f4"][s] = st["cur"][s * K + bk], v, st["cur_f4"][s * K + bk]
+    return st
+
+
+def _swap_parity(it, swap_every):
+    return (it // swap_every) % 2 if swap_every > 0 and (it + 1) % swap_every == 0 else -1
+
+
+def _check_ladder(ladder):
+    lad = np.asarray(ladder, dtype=np.float64)
+    if lad.ndim != 1 or lad.shape[0] < 1 or not np.isfinite(lad).all() or (lad < 0).any() or (np.diff(lad) < 0).any():
+        raise ValueError("ladder must be a non-empty 1-D array of finite, nonnegative, nondecreasing temperatures")
+    return lad
+
+
+def anneal_search(instances, actions, weights=(0.4, 0.4, 0.2), left_shift=True, iterations=2000, ladder=None,
+                  swap_every=ANNEAL_SWAP_EVERY, seed=0, max_candidates=65536, device=None):
+    """Parallel tempering (replica-exchange simulated annealing) from the S sequences `actions` ([N,S,2] integers, numpy
+    or torch: complete valid schedules of the instances {"t","p","transT","edge"} [S,...]) under the reward weights
+    `weights`, on local_search's neighbourhood and FP64 objective.  Each instance runs K = len(ladder) chains, all starting
+    from its sequence, chain k at the absolute temperature ladder[k] * the start objective (ladder: relative temperatures,
+    finite, >= 0 and nondecreasing; None is anneal_ladder()'s defaults).  Every iteration `it` runs one anneal_propose (one
+    uniform neighbour per chain), BatchedMTFJSPEnv.replay_moves of the S*K proposals (src = their instance, at most
+    max_candidates per call), and one anneal_step: the Metropolis test per chain, then, on iterations with
+    (it + 1) % swap_every == 0, exchanges of the adjacent pairs (k, k+1) with k = (it // swap_every) % 2 (mod 2);
+    swap_every = 0 never exchanges.  Exactly `iterations` iterations run with no host synchronisation; the invalid-replay
+    flag is read once, at the end.  Draws are keyed by (seed, it, k) only, so an instance's result depends neither on
+    max_candidates nor on the other instances of the batch or its row in it.
+    -> dict of numpy arrays: actions [N,S,2] int32, final4 [S,4] and objective [S] of the best schedule visited,
+       best_history [iterations+1, S] (never increasing, the start first), current [S,K] (the chains' final objectives),
+       accept_rate [K] (per rung, over instances and iterations), swap_rate [K-1] (per adjacent pair, over instances and
+       the iterations that tried it; NaN if none did) and replays, the number of sequences replayed (the start
+       included)."""
+    t = np.asarray(instances["t"])
+    S, N, M = t.shape
+    J, E = N // M, np.asarray(instances["edge"]).shape[1]
+    lad = anneal_ladder() if ladder is None else _check_ladder(ladder)
+    K = lad.shape[0]
+    if max_candidates < 1:
+        raise ValueError("max_candidates must be >= 1")
+    if int(iterations) < 0 or int(swap_every) < 0:
+        raise ValueError("iterations and swap_every must be >= 0")
+    if tuple(actions.shape if torch.is_tensor(actions) else np.shape(actions)) != (N, S, 2):
+        raise ValueError("actions must have shape [%d, %d, 2]" % (N, S))
+    env = BatchedMTFJSPEnv(S, J, M, E, left_shift=left_shift, weights=weights, device=device, obs_dtype=torch.float32)
+    dev = env.device
+    start = torch.as_tensor(np.asarray(actions) if not torch.is_tensor(actions) else actions).to(dev, torch.int32)
+    env.load(*(np.asarray(instances[k]) for k in ("t", "p", "transT", "edge")))
+    env.scaler_init()
+    env.reset(np.tile(np.asarray(weights, dtype=np.float64), (S, 1)))
+    t_dev = torch.as_tensor(t, device=dev, dtype=torch.float64)
+    final4, _, finv = env.replay(start)
+    if bool((finv != -1).any()):
+        raise ValueError("a starting sequence has an invalid action")
+    st = anneal_state(start.transpose(0, 1).contiguous(), final4, weights, K)
+    temp = torch.as_tensor(lad, device=dev)[None, :] * st["best_obj"][:, None]                 # [S,K]
+    Q = S * K
+    row_src = torch.arange(Q, dtype=torch.int32, device=dev) // K                 # chain row -> its instance's env
+    best_history = [st["best_obj"].clone()]
+    acc_sum = torch.zeros(Q, dtype=torch.int64, device=dev)
+    swap_sum = torch.zeros(Q, dtype=torch.int64, device=dev)
+    tries = np.zeros(2, dtype=np.int64)                                            # exchanges tried per parity
+    bad = torch.zeros((), dtype=torch.bool, device=dev)
+    f4 = torch.empty((Q, 4), dtype=torch.float64, device=dev)
+    fi = torch.empty((Q,), dtype=torch.int32, device=dev)
+    for it in range(int(iterations)):
+        moves = anneal_propose(t_dev, st["cur"], seed, it)
+        base = st["cur"].transpose(0, 1)                                           # [N,S*K,2] view of the chain rows
+        for c0 in range(0, Q, max_candidates):
+            c1 = min(c0 + max_candidates, Q)
+            f4[c0:c1], _, fi[c0:c1] = env.replay_moves(base, moves[c0:c1], row_src)
+        bad |= (fi >= 0).any()
+        par = _swap_parity(it, int(swap_every))
+        if par >= 0:
+            tries[par] += 1
+        anneal_step(st, moves, fi, _objective(f4, weights), f4, temp, seed, it, par, M)
+        acc_sum += st["accepted"]
+        swap_sum += st["swapped"]
+        best_history.append(st["best_obj"].clone())
+    if bool(bad):
+        raise RuntimeError("a neighbour replayed with an invalid action")
+    env.close()
+    pair_tries = tries[np.arange(K - 1) % 2] * S
+    sw = swap_sum.view(S, K)[:, :K - 1].sum(0).cpu().numpy().astype(np.float64)
+    acc = acc_sum.view(S, K).sum(0).cpu().numpy().astype(np.float64)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        swap_rate = np.where(pair_tries > 0, sw / pair_tries, np.nan)
+        accept_rate = acc / float(S * int(iterations))
+    return {"actions": st["best"].transpose(0, 1).cpu().numpy(), "final4": st["best_f4"].cpu().numpy(),
+            "objective": st["best_obj"].cpu().numpy(), "best_history": torch.stack(best_history).cpu().numpy(),
+            "current": st["cur_obj"].view(S, K).cpu().numpy(),
+            "accept_rate": accept_rate, "swap_rate": swap_rate, "replays": S + int(iterations) * Q}
 
 
 def _replay_all(env, R, seqs, src, max_candidates):

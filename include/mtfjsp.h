@@ -575,6 +575,51 @@ int mtfjsp_tabu_move(int S, int J, int M, const int32_t* moves, int64_t R, const
                      double* cur_f4, int32_t* best, double* best_obj, double* best_f4, int32_t* mach_until,
                      int32_t* op_until, int32_t* chosen, void* stream);
 
+/* Parallel tempering over finished schedules (search.anneal_search): S instances with K Markov chains each.  Handle-free,
+ * asynchronous on `stream`.  N = J*M.  Chain row q = s*K + k (instance s, chain k); cur [S*K,N,2] int32 holds the rows'
+ * complete (op, machine) sequences, contiguous per row.
+ * Draws: chain k's draws at iteration it are u_j = evolve._draws(seed, (it << 32) | k, 3)[j], i.e.
+ * x = splitmix64(seed ^ splitmix64(c * 0x100000001B3 + j * 0x9E3779B97F4A7C15)), u_j = (x >> 11) * 2^-53 with
+ * c = (it << 32) | k (all mod 2^64); u0 is the proposal, u1 the Metropolis test, u2 the exchange of the pair whose lower
+ * chain is k.  The instance row is not in the key, so an instance's run depends neither on the batch nor on its row.
+ * below(u, n) = min(floor(u * n), n - 1) with u * n an FP64 product.
+ * exp_neg(x): NaN for NaN, 1 for x <= 0, 0 for x > 746; otherwise, in FP64 with every operation correctly rounded and
+ * none contracted: n = rint(x * 1.4426950408889634) (ties to even), z = -((x - n * LN2_HI) - n * LN2_LO) with
+ * LN2_HI = 0x3fe62e42fee00000 (0.6931471803691238) and LN2_LO = 1.9082149292705877e-10, p = c13 and then p = p * z + c_i
+ * for i = 12 .. 0 with c_i = 1/i! rounded to double, and the result scalbn(p, -n), correctly rounded (subnormals too).
+ * mtfjsp_anneal_propose writes moves [S*K,4] int32 (row, kind, s, arg) in search.neighbour_moves' form with row = q.
+ * Row q's neighbourhood is neighbour_moves' for its sequence and t [S,N,M] f64 (t < 0: infeasible) of instance s, in its
+ * order: reassignments (s, m') for every entry s and every machine m' != m_s with t[s][o_s][m'] >= 0, in (s, m') order,
+ * then insertions (s, s') for every s' in (pos(pred), pos(succ)) other than s and s - 1, in (s, s') order, where pos(pred)
+ * is the index of o_s - 1 if o_s % M > 0, else -1, and pos(succ) the index of o_s + 1 if o_s % M < M - 1, else N.  With
+ * R_q moves, chain q takes move number below(u0, R_q).  A row with R_q = 0, and a row whose ops are not a permutation of
+ * [0, N), get (q, -1, 0, 0): a malformed move.
+ * mtfjsp_anneal_step makes iteration it's decisions for every chain and applies them in place.  moves [S*K,4] int32 are
+ * the proposals (row q's is moves[q]), first_invalid [S*K] int32, obj [S*K] f64 and f4 [S*K,4] f64 their replay's first
+ * invalid index, objective and final costs; temp [S,K] f64 absolute temperatures (T of chain q is temp[q]).  State,
+ * updated in place: cur, cur_obj [S*K], cur_f4 [S*K,4] f64; best [S,N,2] int32, best_obj [S], best_f4 [S,4] f64.
+ * accepted [S*K] and swapped [S*K] int32 are written every call.  Per instance, in this order:
+ *  1. Metropolis: chain q takes its proposal iff the move is well formed for row q (row == q, kind 0 or 1, s in [0, N),
+ *     the op at index s of cur[q] in [0, N), and for a reassignment arg and that entry's machine in [0, M), for an
+ *     insertion arg in [0, N)), first_invalid[q] == -1, obj[q] is not NaN, and delta = obj[q] - cur_obj[q] <= 0 or
+ *     T > 0 and u1 < exp_neg(delta / T).  Taking it sets cur[q] = search.apply_moves(cur[q], move), cur_obj[q] = obj[q]
+ *     and cur_f4[q] = f4[q].  accepted[q] = 1 if it was taken, else 0.
+ *  2. Exchange, only when swap_parity is 0 or 1: for every pair a = s*K + k, b = a + 1 with k = swap_parity (mod 2) and
+ *     k + 1 < K, with d = cur_obj[b] - cur_obj[a] after step 1, the pair swaps iff d <= 0, or temp[a] > 0 and
+ *     u2 (of chain k) < exp_neg(d * (1 / temp[a] - 1 / temp[b])).  A swap exchanges the two rows of cur, cur_obj and
+ *     cur_f4 (not the temperatures).  swapped[a] = 1 if the pair (k, k + 1) swapped; every other entry is 0.
+ *  3. Best: the least cur_obj over the instance's chains that is strictly below best_obj[s], ties to the lowest k (NaN
+ *     never wins), is copied with its row and cur_f4 to best[s], best_obj[s] and best_f4[s].
+ * Every index and value in device memory is data and never a fault.
+ * MTFJSP_E_ARG, nothing written: a NULL pointer, S < 1, K < 1, S*K > INT32_MAX, it < 0, or (J, M) outside mtfjsp_create's
+ * range (J >= 1, 2 <= M <= 64, N <= 4096). */
+int mtfjsp_anneal_propose(const double* t, int S, int J, int M, int K, const int32_t* cur, uint64_t seed, int it,
+                          int32_t* moves, void* stream);
+int mtfjsp_anneal_step(int S, int J, int M, int K, const int32_t* moves, const int32_t* first_invalid,
+                       const double* obj, const double* f4, const double* temp, uint64_t seed, int it, int swap_parity,
+                       int32_t* cur, double* cur_obj, double* cur_f4, int32_t* best, double* best_obj, double* best_f4,
+                       int32_t* accepted, int32_t* swapped, void* stream);
+
 /* Nonzero if a step launch of this handle waited more than 1 s for the previous one to finish the same envs
  * (MTFJSP_LAUNCH_OVERLAP) and went on; every later call on the handle then returns MTFJSP_E_CUDA.  Reads a mapped host
  * word: it reflects the launches the device has finished so far (read it after synchronising). */
